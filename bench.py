@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the AC-move hot path (BASELINE.json config 2).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the batched ``ACEnv.step`` kernel over one batch of 1 Mi synthetic
@@ -34,6 +34,7 @@ HORIZON = 200
 # relator lengths travel with the state (ACS_FLAG_LENS_VALID).  BENCH_FLAGS=0 times the general variant.
 FLAGS = int(os.environ.get("BENCH_FLAGS", "6"))
 L2_BYTES = 126 * 1024 * 1024
+DUMP_BYTES = 48 << 20  # --dump-outputs: 161 319 of the 1 Mi rows at mrl 36
 
 
 def parse_args():
@@ -54,7 +55,13 @@ def parse_args():
     ap.add_argument("--skip-barcode", action="store_true")
     ap.add_argument("--skip-ppo", action="store_true")
     ap.add_argument("--greedy-budget", type=int, default=1_000_000)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0's rows; a fixed sample of them "
+                         "when they exceed DUMP_BYTES) to DIR/<name>.npy as float32")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl b200 and --steps >= 1")
+    return args
 
 
 def dist_env():
@@ -385,6 +392,10 @@ def run_b200(args):
     ev1.record(stream)
     torch.cuda.synchronize()
     sampler.phase = "post"
+    if args.dump_outputs and rank == 0:
+        b = (args.warmup + args.steps - 1) % nbuf  # the buffers the last timed step updated in place
+        dump_outputs(args.dump_outputs, state=states[b], reward=reward, done=done, truncated=trunc, step_count=stepc[b],
+                     lengths=lens[b])
     ms = ev0.elapsed_time(ev1)
     if dist is not None:
         t = torch.tensor([ms], device="cuda", dtype=torch.float64)
@@ -640,6 +651,20 @@ def run_b200(args):
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, **outputs):
+    """Each [rows, ...] device output to out_dir/<name>.npy as float32: every row, or the same seeded sample of rows
+    for all outputs when every row would take more than DUMP_BYTES."""
+    import torch
+
+    rows = len(next(iter(outputs.values())))
+    n = min(rows, DUMP_BYTES // (4 * sum(t[0].numel() for t in outputs.values())))
+    idx = np.arange(rows) if n == rows else np.sort(np.random.default_rng(0).choice(rows, n, replace=False))
+    idx = torch.from_numpy(idx)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(0, idx.to(t.device)).cpu().numpy().astype(np.float32))
 
 
 def ncu_traffic():

