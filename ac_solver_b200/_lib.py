@@ -102,6 +102,12 @@ _SIGS = {
     "acs_bfs_run": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(SearchResult)]),
     "acs_bfs_visited": (C.c_int, [_P, _P, C.c_int64, C.POINTER(C.c_int64)]),
     "acs_bfs_destroy": (None, [_P]),
+    "acs_bfs_batch_bytes": (C.c_int, [C.c_int, C.c_int, _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "acs_bfs_batch_create": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, C.c_int, C.c_int64, C.POINTER(_P)]),
+    "acs_bfs_batch_run": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(SearchResult)]),
+    "acs_bfs_batch_paths": (C.c_int, [_P, _P, C.c_int]),
+    "acs_bfs_batch_visited": (C.c_int, [_P, C.c_int, _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "acs_bfs_batch_destroy": (None, [_P]),
     "acs_greedy_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, C.POINTER(_P)]),
     "acs_greedy_run": (C.c_int, [_P, _P, _P, _P]),
     "acs_greedy_visited": (C.c_int, [_P, C.c_int, _P, C.c_int64, C.POINTER(C.c_int64)]),

@@ -1,0 +1,1008 @@
+// mbfs.cu -- batched breadth-first search: many independent searches of one max_relator_length
+// and one `cyclical` flag advance together through the same kernel launches on one GPU.
+//
+// Contract: for every search, the result equals acs_bfs_run on that presentation (pbfs.cu, and so
+// the reference's ac_solver/search/breadth_first.py:15-97): solved flag and path, counters,
+// budget cut, raising row, "New minimal length" sequence and the visited array in FIFO order.
+//
+// Design.  Search s owns a slab of budget_s + 16 nodes (the reference overshoots its budget by at
+// most 11: the test runs after a parent's 12 children), so a node's slab index is its FIFO id and
+// parent links stay inside the slab.  A combined chunk concatenates one segment per active search:
+// segment k covers parents [head_k, head_k + F_k) of search seg_search[k] (within its current
+// level) at chunk offset off_k, and a child gets the candidate id c = 12*(off_k + gid - head_k) + a.
+// Within a search that is the reference's order; across searches the (search, state) keys differ,
+// so "smallest candidate id wins per (search, state)" is exact.  One chunk is
+//
+//   prep     reset the bitmap, the record cursor and the per-segment control minima
+//   expand   one thread per parent, children appended to the chunk's record log (key, c, search)
+//   insert   one shared exact open-addressing table keyed by (search, state): 32-byte buckets,
+//            tentative slots point at log records, smallest c wins by CAS, XOR winner bitmap
+//   scan     popcount prefix of the winner bitmap -> rank table
+//   decide   one thread per segment: budget cut by binary search, solving / raising child,
+//            minimal-length log, counters; a search that ends drops out
+//   commit   winners below their segment's limit become nodes of their slab and their table slot
+//            is re-pointed at the node; winners past the limit leave a tombstone
+//   plan     next chunk: the active searches' level remainders, in search order, up to the
+//            parents cap and the table's free room
+//
+// Table slots are fingerprint << 40 | tag | (index + 1): the tag bit 39 set means a committed node
+// (global node index), clear a record of the current chunk's log.  The log is rewritten every
+// chunk, so its size is bounded by 12 records per parent of one chunk.  The host enqueues chunks
+// ahead of the device and reads only a lagging pinned copy of the run state.
+#include <algorithm>
+#include <cstdint>
+#include <cstdio>
+#include <cstring>
+#include <string>
+#include <vector>
+
+#include <cuda_runtime.h>
+
+#include "../../include/acsolver_b200.h"
+#include "ac_core.cuh"
+#include "ac_keys.cuh"
+#include "acs_internal.h"
+#include "bfs_common.cuh"
+
+namespace acs {
+
+constexpr int kMbCtrl = 130;  // per segment: solving child, raising child, first child of each total length < 128
+constexpr int kMbSol = 0, kMbErr = 1, kMbLen0 = 2;
+constexpr uint64_t kMbNode = 1ull << 39, kMbIdx = kMbNode - 1;
+constexpr uint64_t kMbTomb = 1ull << 63;  // fingerprints are 23 bits: never equal to a tombstone's
+constexpr int kMbStage = 128;             // records staged per warp before a flush to the log
+
+enum : int { MB_IERR_TABLE_FULL = 1, MB_IERR_SLAB_FULL = 2 };
+
+// per-search state
+struct MbSearch {
+    int64_t budget, slab, cap, n_nodes, head, level_end, n_expanded, sol_gid, err_code;
+    int32_t min_len, levels, done, solved, budget_hit, status, n_minlen, pad;
+    int32_t minlen_log[128];
+};
+
+// run state (the host polls a lagging copy of it)
+struct MbState {
+    int64_t Ftot, n_seg, used, chunks, chunk_cap;
+    uint64_t tmask;
+    int32_t mrl, cyclical, n_search, done, ierr, pad;
+};
+
+struct MbEngine {
+    MbState* st;
+    MbSearch* srch;       // [n_search]
+    uint64_t* nodes;      // [sum cap][2W+2]: key words, parent link, search id
+    uint64_t* table;      // [tmask+1]
+    uint64_t* log_keys;   // [rec_cap][2W]
+    uint32_t* log_c;      // [rec_cap]
+    uint32_t* log_s;      // [rec_cap]
+    uint64_t* rec_slot;   // [rec_cap] table slot a record claimed
+    unsigned long long* cursor;
+    uint32_t* bitmap;     // [bitmap_words]
+    uint2* rt;            // [bitmap_words + 1] {winners before the word, its bits}
+    uint32_t* bsums;      // [nblk]
+    unsigned long long* ctrl;  // [n_search][kMbCtrl], indexed by segment
+    int32_t* seg_search;  // [n_search]
+    int64_t* seg_head;    // [n_search]
+    int64_t* seg_off;     // [n_search + 1]
+    int64_t* seg_limit;   // [n_search] chunk candidate id limit of the commit
+    int64_t* seg_base;    // [n_search] global node index of the segment's first winner, minus its rank
+    int32_t* seg_of;      // [n_search] segment of a search in the current chunk
+    int64_t rec_cap;
+};
+
+template <int W>
+__device__ __forceinline__ uint64_t mb_hash(const Key<W>& q, uint32_t s) {
+    return mix64(pb_hash<W>(q) ^ ((uint64_t)(s + 1) * 0x9E3779B97F4A7C15ull));
+}
+
+__device__ __forceinline__ int mb_segment(const int64_t* seg_off, int n_seg, int64_t p) {
+    int lo = 0, hi = n_seg - 1;  // last k with seg_off[k] <= p
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(seg_off + mid) <= p) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+
+__device__ __forceinline__ uint64_t mb_rank(const uint2* rt, uint64_t c) {
+    const uint2 e = rt[c >> 5];
+    return e.x + __popc(e.y & ((1u << (c & 31)) - 1u));
+}
+
+// ---- init: roots into their slabs and the table ----------------------------------------------
+template <int W>
+__global__ void mb_init_kernel(const MbEngine E, const uint64_t* roots) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= E.st->n_search || E.srch[s].done) return;
+    Key<W> q;
+#pragma unroll
+    for (int i = 0; i < 2 * W; ++i) q.k[i] = roots[(size_t)s * 2 * W + i];
+    const uint64_t idx = (uint64_t)E.srch[s].slab;
+    node_store<W>(E.nodes, idx, q, -1, s);
+    const uint64_t h = mb_hash<W>(q, (uint32_t)s), tmask = E.st->tmask;
+    const uint64_t v = ((h >> 41) << 40) | kMbNode | (idx + 1);
+    // slot by slot from the start of the 4-slot bucket: the order in which mb_insert_kernel probes
+    for (uint64_t t = (h & tmask) & ~3ull, n = 0; n <= tmask; t = (t + 1) & tmask, ++n)
+        if (atomicCAS((unsigned long long*)&E.table[t], 0ull, (unsigned long long)v) == 0ull) return;
+    atomicOr(&E.st->ierr, MB_IERR_TABLE_FULL);
+}
+
+// ---- plan: the next chunk's segments (one warp) --------------------------------------------------
+__global__ void __launch_bounds__(32) mb_plan_kernel(const MbEngine E, int first) {
+    MbState* st = E.st;
+    if (st->done) return;
+    const int lane = threadIdx.x;
+    const int n = st->n_search;
+    int64_t P = st->chunk_cap;
+    if (first) {
+        P = (int64_t)n;  // the roots, expanded without the normal-form shortcuts
+    } else {
+        // no room: more than 3/4 of the table holds nodes and tombstones -- stop with an error rather
+        // than crawl on in tiny chunks
+        const int64_t room = ((int64_t)(3 * ((st->tmask + 1) / 4)) - st->used) / 12;
+        if (room < 1) {
+            if (lane == 0) {
+                atomicOr(&st->ierr, MB_IERR_TABLE_FULL);
+                st->done = 1;
+            }
+            return;
+        }
+        P = room < P ? room : P;
+    }
+    const uint32_t lt = (1u << lane) - 1u;
+    int64_t carryD = 0;
+    int carryK = 0;
+    for (int base = 0; base < n; base += 32) {
+        const int s = base + lane;
+        int64_t d = 0, head = 0;
+        if (s < n && !E.srch[s].done) {
+            const MbSearch& M = E.srch[s];
+            head = M.head;
+            // a third of the remaining budget at most: a search ends inside its last segment, and the winners
+            // past its end stay in the table as tombstones; ~2.8 new states per parent keep them few
+            const int64_t r = (M.budget - M.n_nodes) / 3 + 1;
+            d = M.level_end - head;
+            d = d < r ? d : r;
+            d = d < P ? d : P;
+        }
+        int64_t x = d;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int64_t t = __shfl_up_sync(0xFFFFFFFFu, x, o);
+            if (lane >= o) x += t;
+        }
+        const int64_t D = carryD + x - d;
+        const bool on = d > 0 && D < P;
+        const uint32_t b = __ballot_sync(0xFFFFFFFFu, on);
+        if (on) {
+            const int k = carryK + __popc(b & lt);
+            E.seg_search[k] = s;
+            E.seg_head[k] = head;
+            E.seg_off[k] = D;
+            E.seg_of[s] = k;
+        }
+        carryD += __shfl_sync(0xFFFFFFFFu, x, 31);
+        carryK += __popc(b);
+        if (carryD >= P) break;
+    }
+    if (lane == 0) {
+        const int64_t F = carryD < P ? carryD : P;
+        E.seg_off[carryK] = F;
+        st->n_seg = carryK;
+        st->Ftot = F;
+        if (carryK == 0) st->done = 1;
+    }
+}
+
+// ---- prep ------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) mb_prep_kernel(const MbEngine E) {
+    const MbState* st = E.st;
+    if (st->done) return;
+    const int64_t nwords = (12 * st->Ftot + 31) / 32;
+    const int64_t nctrl = st->n_seg * kMbCtrl;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nwords; i += stride) E.bitmap[i] = 0;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nctrl; i += stride) E.ctrl[i] = ~0ull;
+    if (blockIdx.x == 0 && threadIdx.x == 0) *E.cursor = 0;
+}
+
+// ---- expand ----------------------------------------------------------------------------------------
+template <int W>
+__host__ __device__ constexpr int mb_stage_bytes_per_warp() {
+    return kMbStage * (16 * W + 4 + 4);
+}
+extern __shared__ __align__(16) unsigned char mb_smem[];
+
+template <int W>
+__device__ __forceinline__ void mb_flush(const MbEngine& E, const ulonglong2* sk, const uint32_t* sc, const uint32_t* ss,
+                                         uint32_t n, int lane) {
+    unsigned long long pos = 0;
+    if (lane == 0) pos = atomicAdd(E.cursor, (unsigned long long)n);
+    pos = __shfl_sync(0xFFFFFFFFu, pos, 0);
+    ulonglong2* dk = reinterpret_cast<ulonglong2*>(E.log_keys) + pos * W;
+    for (uint32_t idx = lane; idx < n; idx += 32) {  // the log holds 12 records per parent: never full
+#pragma unroll
+        for (int i = 0; i < W; ++i) dk[(size_t)idx * W + i] = sk[idx * W + i];
+        E.log_c[pos + idx] = sc[idx];
+        E.log_s[pos + idx] = ss[idx];
+    }
+    __syncwarp();
+}
+
+template <int W, bool TRUSTED>
+__global__ void __launch_bounds__(256) mb_expand_kernel(const MbEngine E) {
+    const MbState* st = E.st;
+    if (st->done) return;
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, wpb = blockDim.x >> 5;
+    unsigned char* p = mb_smem + wib * mb_stage_bytes_per_warp<W>();
+    ulonglong2* sk = reinterpret_cast<ulonglong2*>(p);
+    uint32_t* sc = reinterpret_cast<uint32_t*>(p + kMbStage * 16 * W);
+    uint32_t* ss = sc + kMbStage;
+    const int64_t F = st->Ftot;
+    const int n_seg = (int)st->n_seg;
+    const int mrl = st->mrl;
+    const bool cyc = st->cyclical != 0;
+    const int64_t gw = (int64_t)blockIdx.x * wpb + wib, nw = (int64_t)gridDim.x * wpb;
+    const uint32_t lt = (1u << lane) - 1u;
+    uint32_t staged = 0;  // warp-uniform
+    for (int64_t base = 32 * gw; base < F; base += 32 * nw) {
+        const int64_t j = base + lane;
+        const bool valid = j < F;
+        Key<W> pk;
+#pragma unroll
+        for (int i = 0; i < 2 * W; ++i) pk.k[i] = 0;
+        uint32_t skip = 0, s = 0;
+        int k = 0, min_len = 0;
+        if (valid) {
+            k = mb_segment(E.seg_off, n_seg, j);
+            s = (uint32_t)__ldg(E.seg_search + k);
+            const MbSearch& M = E.srch[s];
+            min_len = M.min_len;
+            int64_t pl, tag;
+            node_load<W>(E.nodes, (uint64_t)(M.slab + __ldg(E.seg_head + k) + (j - __ldg(E.seg_off + k))), pk, pl, tag);
+            skip = skip_moves<TRUSTED>(pl, cyc);
+        }
+        unsigned long long* ctrl = E.ctrl + (int64_t)k * kMbCtrl;
+        Rel<2 * W> p0, p1;
+        split_key<W>(pk, p0, p1);
+        const uint32_t cbase = (uint32_t)(j * 12);
+#pragma unroll 4
+        for (int a = 0; a < 12; ++a) {
+            Rel<2 * W> r0 = p0, r1 = p1;
+            bool emit = false;
+            Key<W> child;
+#pragma unroll
+            for (int i = 0; i < 2 * W; ++i) child.k[i] = 0;
+            if (valid && !((skip >> a) & 1u)) {
+                bool co;
+                const int stt = apply_move<2 * W, TRUSTED>(r0, r1, a, mrl, cyc, co);
+                const unsigned long long c = cbase + a;
+                if (stt != ST_OK) {
+                    atomicMin(&ctrl[kMbErr], (c << 2) | (unsigned)stt);
+                } else {
+                    const int L = r0.len + r1.len;
+                    if (L < min_len) atomicMin(&ctrl[kMbLen0 + L], c);
+                    if (L == 2) atomicMin(&ctrl[kMbSol], c);  // before the visited test
+                    child = make_key<W>(r0, r1);
+                    emit = !key_eq<W>(child, pk);
+                }
+            }
+            const uint32_t act = __ballot_sync(0xFFFFFFFFu, emit);
+            if (emit) {
+                const uint32_t q = staged + __popc(act & lt);
+#pragma unroll
+                for (int i = 0; i < W; ++i) sk[q * W + i] = make_ulonglong2(child.k[2 * i], child.k[2 * i + 1]);
+                sc[q] = cbase + a;
+                ss[q] = s;
+            }
+            staged += __popc(act);
+            if (staged > kMbStage - 32) {
+                __syncwarp();
+                mb_flush<W>(E, sk, sc, ss, staged, lane);
+                staged = 0;
+            }
+        }
+    }
+    if (staged) {
+        __syncwarp();
+        mb_flush<W>(E, sk, sc, ss, staged, lane);
+    }
+}
+
+// ---- insert ----------------------------------------------------------------------------------------
+template <int W>
+__global__ void __launch_bounds__(256) mb_insert_kernel(const MbEngine E) {
+    MbState* st = E.st;
+    if (st->done) return;
+    const unsigned long long n = *E.cursor;
+    const uint64_t tmask = st->tmask;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+         i += (unsigned long long)gridDim.x * blockDim.x) {
+        const Key<W> key = load_key_cg<W>(E.log_keys, i);
+        const uint32_t c = __ldcg(E.log_c + i), s = __ldcg(E.log_s + i);
+        const uint64_t h = mb_hash<W>(key, s);
+        const uint64_t fp23 = h >> 41;
+        const uint64_t mine = (fp23 << 40) | (i + 1);
+        uint64_t slot_base = (h & tmask) & ~3ull;
+        uint64_t probes = 0;
+        bool finished = false;
+        while (!finished) {
+            uint64_t vv[4];
+            load_bucket(E.table + slot_base, vv);
+#pragma unroll
+            for (int jj = 0; jj < 4 && !finished; ++jj) {
+                uint64_t cur = vv[jj];
+                const uint64_t slot = slot_base + jj;
+                unsigned long long* sp = (unsigned long long*)&E.table[slot];
+                if (cur == 0) {
+                    cur = atomicCAS(sp, 0ull, (unsigned long long)mine);
+                    if (cur == 0) {  // first sighting of this (search, state): claim
+                        E.rec_slot[i] = slot;
+                        atomicXor(&E.bitmap[c >> 5], 1u << (c & 31));
+                        finished = true;
+                        break;
+                    }
+                }
+                if ((cur >> 40) != fp23) continue;
+                if (cur & kMbNode) {  // a committed node: visited if it is this search's state
+                    Key<W> other;
+                    int64_t pl, s2;
+                    node_load<W>(E.nodes, (cur & kMbIdx) - 1, other, pl, s2);
+                    if ((uint32_t)s2 != s || !key_eq<W>(other, key)) continue;
+                    finished = true;
+                    break;
+                }
+                uint64_t p2 = (cur & kMbIdx) - 1;
+                if (__ldcg(E.log_s + p2) != s || !key_eq<W>(load_key_cg<W>(E.log_keys, p2), key)) continue;
+                // a record of this chunk with the same (search, state): the smaller candidate id keeps the slot
+                for (;;) {
+                    const uint32_t c2 = __ldcg(E.log_c + p2);
+                    if (c2 < c) break;
+                    const uint64_t old = atomicCAS(sp, (unsigned long long)cur, (unsigned long long)mine);
+                    if (old == cur) {  // displaced the holder: its claim bit flips back, mine flips on
+                        E.rec_slot[i] = slot;
+                        atomicXor(&E.bitmap[c2 >> 5], 1u << (c2 & 31));
+                        atomicXor(&E.bitmap[c >> 5], 1u << (c & 31));
+                        break;
+                    }
+                    cur = old;  // someone else replaced it meanwhile (same state): look again
+                    p2 = (cur & kMbIdx) - 1;
+                }
+                finished = true;
+            }
+            if (!finished) {
+                slot_base = (slot_base + 4) & tmask;
+                probes += 4;
+                if (probes > tmask) {  // cannot happen with the chunk sizing (table <= 3/4 full)
+                    atomicOr(&st->ierr, MB_IERR_TABLE_FULL);
+                    finished = true;
+                }
+            }
+        }
+    }
+}
+
+// ---- scan --------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(kScanT) mb_scan_sums_kernel(const MbEngine E) {
+    const MbState* st = E.st;
+    if (st->done) return;
+    const int64_t nwords = (12 * st->Ftot + 31) / 32;
+    const int64_t nblk = (nwords + kScanBlock - 1) / kScanBlock;
+    for (int64_t b = blockIdx.x; b < nblk; b += gridDim.x) {
+        uint32_t v = 0;
+#pragma unroll
+        for (int k = 0; k < kScanPer; ++k) {
+            const int64_t i = b * kScanBlock + (int64_t)k * kScanT + threadIdx.x;
+            if (i < nwords) v += __popc(__ldcg(E.bitmap + i));
+        }
+        uint32_t tot;
+        block_excl_scan(v, tot);
+        if (threadIdx.x == 0) E.bsums[b] = tot;
+        __syncthreads();
+    }
+}
+// single block: exclusive scan of the block sums in place; total to the sentinel rank-table entry
+__global__ void __launch_bounds__(kScanT) mb_scan_top_kernel(const MbEngine E) {
+    const MbState* st = E.st;
+    if (st->done) return;
+    const int64_t nwords = (12 * st->Ftot + 31) / 32;
+    const int64_t nblk = (nwords + kScanBlock - 1) / kScanBlock;
+    uint32_t carry = 0;
+    for (int64_t base = 0; base < nblk; base += kScanT) {
+        const int64_t i = base + threadIdx.x;
+        const uint32_t v = i < nblk ? __ldcg(E.bsums + i) : 0u;
+        uint32_t total;
+        const uint32_t ex = block_excl_scan(v, total);
+        if (i < nblk) E.bsums[i] = carry + ex;
+        carry += total;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) E.rt[nwords] = make_uint2(carry, 0u);
+}
+__global__ void __launch_bounds__(kScanT) mb_scan_final_kernel(const MbEngine E) {
+    const MbState* st = E.st;
+    if (st->done) return;
+    const int64_t nwords = (12 * st->Ftot + 31) / 32;
+    const int64_t nblk = (nwords + kScanBlock - 1) / kScanBlock;
+    for (int64_t b = blockIdx.x; b < nblk; b += gridDim.x) {
+        const int64_t first = b * kScanBlock + (int64_t)threadIdx.x * kScanPer;
+        uint32_t w[kScanPer], sum = 0;
+#pragma unroll
+        for (int k = 0; k < kScanPer; ++k) {
+            w[k] = first + k < nwords ? __ldcg(E.bitmap + first + k) : 0u;
+            sum += __popc(w[k]);
+        }
+        uint32_t tot;
+        uint32_t r = __ldcg(E.bsums + b) + block_excl_scan(sum, tot);
+#pragma unroll
+        for (int k = 0; k < kScanPer; ++k) {
+            if (first + k < nwords) E.rt[first + k] = make_uint2(r, w[k]);
+            r += __popc(w[k]);
+        }
+        __syncthreads();
+    }
+}
+
+// ---- decide: one thread per segment, pbfs.cu's rules on the segment ---------------------------------
+__global__ void __launch_bounds__(128) mb_decide_kernel(const MbEngine E) {
+    MbState* st = E.st;
+    if (st->done) return;
+    const int64_t Ftot = st->Ftot;
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k == 0) {  // every winner becomes a node or a tombstone
+        const int64_t nwords = (12 * Ftot + 31) / 32;
+        st->used += E.rt[nwords].x;
+        st->chunks += 1;
+    }
+    if (k >= st->n_seg) return;
+    const int s = E.seg_search[k];
+    MbSearch& M = E.srch[s];
+    const unsigned long long* red = E.ctrl + (int64_t)k * kMbCtrl;
+    const uint64_t off = (uint64_t)E.seg_off[k], F = (uint64_t)E.seg_off[k + 1] - off;
+    const uint64_t c0 = 12 * off, head = (uint64_t)M.head, n_nodes = (uint64_t)M.n_nodes;
+    const uint64_t budget = (uint64_t)M.budget;
+    const uint64_t r0 = mb_rank(E.rt, c0);
+    const uint64_t total = mb_rank(E.rt, c0 + 12 * F) - r0;
+    uint64_t limit = 12 * F;
+    bool cut = false;
+    uint64_t cut_p = 0;
+    if (n_nodes + total >= budget) {
+        // first segment-local parent p with n_nodes + #winners(parents <= p) >= budget (monotone in p)
+        uint64_t lo = 0, hi = F - 1;
+        while (lo < hi) {
+            const uint64_t mid = (lo + hi) >> 1;
+            if (n_nodes + mb_rank(E.rt, c0 + (mid + 1) * 12) - r0 >= budget) hi = mid;
+            else lo = mid + 1;
+        }
+        cut = true;
+        cut_p = lo;
+        if (12 * (cut_p + 1) < limit) limit = 12 * (cut_p + 1);
+    }
+    const unsigned long long sol = red[kMbSol], err = red[kMbErr];
+    bool sol_here = false;
+    int status = 0;
+    uint64_t sol_l = 0, err_l = 0;
+    if (sol != ~0ull && sol - c0 < limit) {  // solved at or before the cut parent
+        sol_l = sol - c0;
+        limit = sol_l;
+        sol_here = true;
+        cut = false;
+    }
+    if (err != ~0ull && (err >> 2) - c0 < limit) {  // the reference raises here, before anything later
+        err_l = (err >> 2) - c0;
+        limit = err_l;
+        status = (int)(err & 3);
+        sol_here = false;
+        cut = false;
+    }
+    // "New minimal length found" events in reference order
+    const uint64_t c_limit = limit + (sol_here ? 1 : 0);
+    int min_len = M.min_len;
+    for (;;) {
+        unsigned long long best = ~0ull;
+        int bestL = -1;
+        for (int L = 0; L < min_len && L < 128; ++L) {
+            const unsigned long long g = red[kMbLen0 + L];
+            if (g != ~0ull && g - c0 < c_limit && g < best) {
+                best = g;
+                bestL = L;
+            }
+        }
+        if (bestL < 0) break;
+        min_len = bestL;
+        if (M.n_minlen < 128) M.minlen_log[M.n_minlen++] = bestL;
+    }
+    M.min_len = min_len;
+    const uint64_t cg = mb_rank(E.rt, c0 + limit) - r0;
+    E.seg_limit[k] = (int64_t)(c0 + limit);
+    E.seg_base[k] = M.slab + (int64_t)n_nodes - (int64_t)r0;
+    if ((int64_t)(n_nodes + cg) > M.cap) atomicOr(&st->ierr, MB_IERR_SLAB_FULL);  // the commit drops the excess
+    M.n_nodes = (int64_t)(n_nodes + cg);
+    if (sol_here) {
+        M.solved = 1;
+        M.sol_gid = (int64_t)(12 * head + sol_l);
+        M.n_expanded = M.sol_gid / 12 + 1;
+    } else if (status) {
+        M.status = status;
+        M.err_code = (int64_t)(((12 * head + err_l) << 2) | (uint64_t)status);
+        M.n_expanded = (int64_t)((12 * head + err_l) / 12 + 1);
+    } else if (cut) {
+        M.budget_hit = 1;
+        M.n_expanded = (int64_t)(head + cut_p + 1);
+    } else {
+        M.n_expanded = (int64_t)(head + F);
+    }
+    M.head = (int64_t)(head + F);
+    if (M.solved || M.budget_hit || M.status || M.head >= M.n_nodes) {
+        M.done = 1;
+    } else if (M.head == M.level_end) {
+        M.level_end = M.n_nodes;
+        M.levels += 1;
+    }
+}
+
+// ---- commit ------------------------------------------------------------------------------------------
+template <int W>
+__global__ void __launch_bounds__(256) mb_commit_kernel(const MbEngine E) {
+    const MbState* st = E.st;
+    if (st->done) return;
+    const unsigned long long n = *E.cursor;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+         i += (unsigned long long)gridDim.x * blockDim.x) {
+        const uint32_t c = __ldcg(E.log_c + i);
+        const uint2 e = E.rt[c >> 5];
+        if (!((e.y >> (c & 31)) & 1u)) continue;  // an already visited state, or lost to an earlier candidate
+        const uint32_t s = __ldcg(E.log_s + i);
+        const int k = E.seg_of[s];
+        const uint64_t slot = E.rec_slot[i];
+        if ((int64_t)c >= E.seg_limit[k]) {  // past the end of its search
+            E.table[slot] = kMbTomb;
+            continue;
+        }
+        const int64_t idx = E.seg_base[k] + (int64_t)(e.x + __popc(e.y & ((1u << (c & 31)) - 1u)));
+        const MbSearch& M = E.srch[s];
+        if (idx >= M.slab + M.cap) {  // MB_IERR_SLAB_FULL was raised by decide
+            E.table[slot] = kMbTomb;
+            continue;
+        }
+        const Key<W> key = load_key_cg<W>(E.log_keys, i);
+        const int64_t pgid = E.seg_head[k] + (int64_t)(c / 12) - E.seg_off[k];
+        node_store<W>(E.nodes, (uint64_t)idx, key, (pgid << 4) | (int64_t)(c % 12), (int64_t)s);
+        E.table[slot] = ((mb_hash<W>(key, s) >> 41) << 40) | kMbNode | (uint64_t)(idx + 1);
+    }
+}
+
+// ---- results -----------------------------------------------------------------------------------------
+// path of every solved search: (action, total length) pairs from the root, then (solving action, 2)
+template <int W>
+__global__ void mb_path_kernel(const MbEngine E, int32_t* paths, int path_cap, int32_t* path_len) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= E.st->n_search) return;
+    const MbSearch& M = E.srch[s];
+    path_len[s] = 0;
+    if (!M.solved) return;
+    int32_t* path = paths + (size_t)s * path_cap * 2;
+    const int64_t node = M.sol_gid / 12;
+    int depth = 0;
+    for (int64_t g = node; g >= 0; ++depth) {
+        Key<W> k;
+        int64_t pl, tag;
+        node_load<W>(E.nodes, (uint64_t)(M.slab + g), k, pl, tag);
+        g = pl < 0 ? -1 : (pl >> 4);
+    }
+    path_len[s] = depth + 1;
+    if (depth < path_cap) {
+        path[2 * depth] = (int32_t)(M.sol_gid % 12);
+        path[2 * depth + 1] = 2;
+    }
+    int pos = depth - 1;
+    for (int64_t g = node; g >= 0; --pos) {
+        Key<W> k;
+        int64_t pl, tag;
+        node_load<W>(E.nodes, (uint64_t)(M.slab + g), k, pl, tag);
+        if (pos < path_cap) {
+            path[2 * pos] = pl < 0 ? -1 : (int32_t)(pl & 15);
+            path[2 * pos + 1] = (int32_t)(k.k[W - 1] >> 58) + (int32_t)(k.k[2 * W - 1] >> 58);
+        }
+        g = pl < 0 ? -1 : (pl >> 4);
+    }
+}
+
+template <int W>
+__global__ void mb_unpack_kernel(const uint64_t* nodes, int8_t* out, uint64_t n, int mrl) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    Rel<2 * W> r0, r1;
+    split_key<W>(node_key<W>(nodes, i), r0, r1);
+    unpack_bytes<2 * W>(out + i * 2 * mrl, r0, mrl);
+    unpack_bytes<2 * W>(out + i * 2 * mrl + mrl, r1, mrl);
+}
+
+}  // namespace acs
+
+// ---------------------------------------------------------------------------------------------------------
+using namespace acs;
+
+namespace {
+inline int mb_fail(int code, const std::string& m) {
+    acs::set_last_error(m.c_str());
+    return code;
+}
+#define MB_CUDA(call)                                                                      \
+    do {                                                                                   \
+        cudaError_t e__ = (call);                                                          \
+        if (e__ != cudaSuccess) {                                                          \
+            cudaGetLastError();                                                            \
+            return mb_fail(e__ == cudaErrorMemoryAllocation ? ACS_ERR_NOMEM : ACS_ERR_CUDA, \
+                           std::string(#call) + ": " + cudaGetErrorString(e__));           \
+        }                                                                                  \
+    } while (0)
+constexpr int kMbRing = 4, kMbLag = 2;
+
+// sizes of an engine (shared by acs_bfs_batch_bytes and acs_bfs_batch_create)
+struct MbPlan {
+    int W;
+    int64_t nodes, chunk, rec_cap, bitmap_words, nblk;
+    uint64_t tcap;
+    int64_t bytes;
+};
+
+int mb_plan(int n_search, int mrl, const int64_t* max_nodes, int64_t chunk_parents, MbPlan& P) {
+    if (n_search < 1 || !max_nodes) return mb_fail(ACS_ERR_INVALID, "bfs_batch: need at least one search");
+    if (mrl < 1 || mrl > 61) return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch needs 1 <= max_relator_length <= 61");
+    P.W = mrl <= 29 ? 1 : 2;
+    P.nodes = 0;
+    for (int s = 0; s < n_search; ++s) {
+        if (max_nodes[s] < 0) return mb_fail(ACS_ERR_INVALID, "bfs_batch: negative node budget");
+        P.nodes += max_nodes[s] + 16;
+    }
+    // the table stays <= 3/4 full: committed nodes, tombstones and one chunk's tentative claims
+    uint64_t t = 1024;
+    while (t < 5 * (uint64_t)P.nodes / 2) t <<= 1;
+    P.tcap = t;
+    if (P.nodes >= (int64_t)kMbIdx) return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch: too many nodes for one engine");
+    // parents per chunk after the first: ~4 Mi (candidate ids are 32-bit)
+    int64_t chunk = chunk_parents > 0 ? chunk_parents : (int64_t)1 << 22;
+    chunk = std::min<int64_t>(chunk, std::max<int64_t>(P.nodes, 1024));
+    chunk = std::min<int64_t>(chunk, ((int64_t)1 << 32) / 12 - 1);
+    P.chunk = chunk;
+    // the log and the bitmap also hold the first chunk, which expands every root
+    const int64_t widest = std::max<int64_t>(chunk, n_search);
+    if (widest > ((int64_t)1 << 32) / 12 - 1) return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch: too many searches");
+    P.rec_cap = 12 * widest;
+    P.bitmap_words = (12 * widest + 31) / 32 + 8;
+    P.nblk = (P.bitmap_words + kScanBlock - 1) / kScanBlock + 1;
+    const int64_t node_bytes = 8 * (2 * P.W + 2);
+    // per search: control minima, six segment arrays, the state and the root key
+    const int64_t per_search = kMbCtrl * 8 + 4 + 8 + 8 + 8 + 8 + 4 + (int64_t)sizeof(MbSearch) + 16 * P.W;
+    P.bytes = P.nodes * node_bytes + (int64_t)P.tcap * 8 + P.rec_cap * (16 * P.W + 4 + 4 + 8) + P.bitmap_words * 4 +
+              (P.bitmap_words + 1) * 8 + P.nblk * 4 + (int64_t)n_search * per_search + 8 + 8 + (int64_t)sizeof(MbState);
+    return ACS_OK;
+}
+}  // namespace
+
+struct acs_bfs_batch {
+    int device = 0, n_search = 0, mrl = 0, W = 1, cyclical = 0;
+    MbPlan plan{};
+    MbEngine E{};
+    uint64_t* d_roots = nullptr;
+    int32_t* d_paths = nullptr;
+    int32_t* d_plen = nullptr;
+    int d_path_cap = 0;
+    std::vector<int64_t> budgets;
+    std::vector<MbSearch> h_final;
+    cudaStream_t stream = nullptr;
+    cudaEvent_t ev0 = nullptr, ev1 = nullptr, ring_ev[kMbRing] = {};
+    MbState* h_ring = nullptr;  // pinned [kMbRing]
+    int sms = 148;
+    int expand_blocks = 148, expand_wpb = 8, insert_blocks = 148, commit_blocks = 148;
+    size_t expand_smem = 0;
+    bool ran = false;
+};
+
+extern "C" {
+
+int acs_bfs_batch_bytes(int n_search, int mrl, const int64_t* max_nodes, int64_t chunk_parents, int64_t* bytes_out) {
+    if (!bytes_out) return ACS_ERR_INVALID;
+    MbPlan P;
+    const int rc = mb_plan(n_search, mrl, max_nodes, chunk_parents, P);
+    if (rc != ACS_OK) return rc;
+    *bytes_out = P.bytes;
+    return ACS_OK;
+}
+
+void acs_bfs_batch_destroy(acs_bfs_batch* b) {
+    if (!b) return;
+    cudaSetDevice(b->device);
+    if (b->stream) {
+        cudaStreamSynchronize(b->stream);
+        cudaStreamDestroy(b->stream);
+    }
+    if (b->ev0) cudaEventDestroy(b->ev0);
+    if (b->ev1) cudaEventDestroy(b->ev1);
+    for (auto e : b->ring_ev)
+        if (e) cudaEventDestroy(e);
+    MbEngine& E = b->E;
+    void* ptrs[] = {E.st, E.srch, E.nodes, E.table, E.log_keys, E.log_c, E.log_s, E.rec_slot, E.cursor, E.bitmap, E.rt,
+                    E.bsums, E.ctrl, E.seg_search, E.seg_head, E.seg_off, E.seg_limit, E.seg_base, E.seg_of,
+                    b->d_roots, b->d_paths, b->d_plen};
+    for (void* p : ptrs)
+        if (p) cudaFree(p);
+    if (b->h_ring) cudaFreeHost(b->h_ring);
+    cudaGetLastError();
+    delete b;
+}
+
+int acs_bfs_batch_create(int device, int n_search, int mrl, const int64_t* max_nodes, int cyclical, int64_t chunk_parents,
+                         acs_bfs_batch** out) {
+    if (!out) return ACS_ERR_INVALID;
+    *out = nullptr;
+    MbPlan P;
+    const int rc = mb_plan(n_search, mrl, max_nodes, chunk_parents, P);
+    if (rc != ACS_OK) return rc;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
+        cudaGetLastError();
+        return mb_fail(ACS_ERR_NO_DEVICE, "no CUDA device visible; there is no CPU fallback");
+    }
+    if (device < 0 || device >= ndev) return mb_fail(ACS_ERR_INVALID, "bfs_batch: device index out of range");
+    MB_CUDA(cudaSetDevice(device));
+    acs_bfs_batch* b = new acs_bfs_batch();
+    b->device = device;
+    b->n_search = n_search;
+    b->mrl = mrl;
+    b->W = P.W;
+    b->cyclical = cyclical ? 1 : 0;
+    b->plan = P;
+    b->budgets.assign(max_nodes, max_nodes + n_search);
+    auto bail = [&](int code, const std::string& m) {
+        acs_bfs_batch_destroy(b);
+        return mb_fail(code, m);
+    };
+    MbEngine& E = b->E;
+    E.rec_cap = P.rec_cap;
+#define MB_ALLOC(ptr, bytes)                                                                             \
+    do {                                                                                                 \
+        cudaError_t e__ = cudaMalloc((void**)&(ptr), (size_t)(bytes));                                   \
+        if (e__ != cudaSuccess) {                                                                        \
+            cudaGetLastError();                                                                          \
+            return bail(ACS_ERR_NOMEM, std::string("bfs_batch: cudaMalloc(" #ptr "): ") + cudaGetErrorString(e__)); \
+        }                                                                                                \
+    } while (0)
+    MB_ALLOC(E.st, sizeof(MbState));
+    MB_ALLOC(E.srch, (size_t)n_search * sizeof(MbSearch));
+    MB_ALLOC(E.nodes, (size_t)P.nodes * 8 * (2 * P.W + 2));
+    MB_ALLOC(E.table, (size_t)P.tcap * 8);
+    MB_ALLOC(E.log_keys, (size_t)P.rec_cap * 16 * P.W);
+    MB_ALLOC(E.log_c, (size_t)P.rec_cap * 4);
+    MB_ALLOC(E.log_s, (size_t)P.rec_cap * 4);
+    MB_ALLOC(E.rec_slot, (size_t)P.rec_cap * 8);
+    MB_ALLOC(E.cursor, 8);
+    MB_ALLOC(E.bitmap, (size_t)P.bitmap_words * 4);
+    MB_ALLOC(E.rt, (size_t)(P.bitmap_words + 1) * sizeof(uint2));
+    MB_ALLOC(E.bsums, (size_t)P.nblk * 4);
+    MB_ALLOC(E.ctrl, (size_t)n_search * kMbCtrl * 8);
+    MB_ALLOC(E.seg_search, (size_t)n_search * 4);
+    MB_ALLOC(E.seg_head, (size_t)n_search * 8);
+    MB_ALLOC(E.seg_off, (size_t)(n_search + 1) * 8);
+    MB_ALLOC(E.seg_limit, (size_t)n_search * 8);
+    MB_ALLOC(E.seg_base, (size_t)n_search * 8);
+    MB_ALLOC(E.seg_of, (size_t)n_search * 4);
+    MB_ALLOC(b->d_roots, (size_t)n_search * 16 * P.W);
+#undef MB_ALLOC
+    if (cudaMallocHost((void**)&b->h_ring, kMbRing * sizeof(MbState)) != cudaSuccess)
+        return bail(ACS_ERR_NOMEM, "bfs_batch: cudaMallocHost");
+    if (cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking) != cudaSuccess)
+        return bail(ACS_ERR_CUDA, "bfs_batch: cudaStreamCreate");
+    cudaEventCreate(&b->ev0);
+    cudaEventCreate(&b->ev1);
+    for (auto& e : b->ring_ev) cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
+    cudaDeviceProp prop{};
+    if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) b->sms = prop.multiProcessorCount;
+    b->expand_smem = (size_t)b->expand_wpb * (P.W == 1 ? mb_stage_bytes_per_warp<1>() : mb_stage_bytes_per_warp<2>());
+    int per_sm = 1, ib = 1, cb = 1;
+    if (P.W == 1) {
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mb_expand_kernel<1, true>, 32 * b->expand_wpb, b->expand_smem);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ib, mb_insert_kernel<1>, 256, 0);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cb, mb_commit_kernel<1>, 256, 0);
+    } else {
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mb_expand_kernel<2, true>, 32 * b->expand_wpb, b->expand_smem);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ib, mb_insert_kernel<2>, 256, 0);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cb, mb_commit_kernel<2>, 256, 0);
+    }
+    cudaGetLastError();
+    b->expand_blocks = b->sms * std::max(per_sm, 1);
+    b->insert_blocks = b->sms * std::max(ib, 1);
+    b->commit_blocks = b->sms * std::max(cb, 1);
+    *out = b;
+    return ACS_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+// Paths of the solved searches of the last run into h_paths [n_search, path_cap, 2]; plen gets every search's
+// path length (0 if not solved).  A path longer than path_cap is an error, never truncated.
+template <int W>
+int mb_paths(acs_bfs_batch* b, int32_t* h_paths, int path_cap, std::vector<int32_t>& plen) {
+    const int n = b->n_search;
+    cudaStream_t s = b->stream;
+    MB_CUDA(cudaSetDevice(b->device));
+    const int cap = std::max(path_cap, 1);  // the kernel writes the first pair of every solved path
+    if (!b->d_paths || cap > b->d_path_cap) {
+        if (b->d_paths) cudaFree(b->d_paths);
+        b->d_paths = nullptr;
+        b->d_path_cap = 0;
+        MB_CUDA(cudaMalloc((void**)&b->d_paths, (size_t)n * cap * 2 * sizeof(int32_t)));
+        b->d_path_cap = cap;
+    }
+    if (!b->d_plen) MB_CUDA(cudaMalloc((void**)&b->d_plen, (size_t)n * sizeof(int32_t)));
+    mb_path_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(b->E, b->d_paths, cap, b->d_plen);
+    MB_CUDA(cudaGetLastError());
+    plen.resize((size_t)n);
+    MB_CUDA(cudaMemcpyAsync(plen.data(), b->d_plen, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    MB_CUDA(cudaStreamSynchronize(s));
+    for (int i = 0; i < n; ++i)
+        if (plen[i] > path_cap)
+            return mb_fail(ACS_ERR_INVALID, "bfs_batch: a solution path is longer than path_cap (see path_len)");
+    if (h_paths && path_cap > 0)
+        MB_CUDA(cudaMemcpy(h_paths, b->d_paths, (size_t)n * path_cap * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost));
+    return ACS_OK;
+}
+
+template <int W>
+int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int path_cap, acs_search_result* results) {
+    const int n = b->n_search, mrl = b->mrl;
+    MbEngine& E = b->E;
+    std::vector<MbSearch> init((size_t)n);
+    std::vector<uint64_t> roots((size_t)n * 2 * W, 0);
+    int64_t slab = 0, n_valid = 0;
+    for (int s = 0; s < n; ++s) {
+        MbSearch& M = init[s];
+        std::memset(&M, 0, sizeof(M));
+        M.budget = b->budgets[s];
+        M.cap = b->budgets[s] + 16;
+        M.slab = slab;
+        slab += M.cap;
+        M.n_nodes = 1;
+        M.level_end = 1;
+        M.sol_gid = -1;
+        Key<W> root;
+        int lens[2];
+        bool valid;
+        if (!pack_root<W>(h_pres + (size_t)s * 2 * mrl, mrl, root, lens, valid))
+            return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch: letters outside {+-1,+-2} are not supported by the packed search");
+        if (!valid) {  // breadth_first.py:36-38 asserts is_array_valid_presentation
+            M.status = ACS_ROW_ASSERT;
+            M.done = 1;
+            M.n_nodes = 0;
+            continue;
+        }
+        M.min_len = lens[0] + lens[1];
+        for (int i = 0; i < 2 * W; ++i) roots[(size_t)s * 2 * W + i] = root.k[i];
+        ++n_valid;
+    }
+    MbState st{};
+    st.chunk_cap = b->plan.chunk;
+    st.tmask = b->plan.tcap - 1;
+    st.mrl = mrl;
+    st.cyclical = b->cyclical;
+    st.n_search = n;
+    st.used = n_valid;
+    cudaStream_t s = b->stream;
+    MB_CUDA(cudaSetDevice(b->device));
+    MB_CUDA(cudaMemsetAsync(E.table, 0, b->plan.tcap * sizeof(uint64_t), s));
+    b->h_ring[0] = st;  // pinned staging for the async upload
+    MB_CUDA(cudaMemcpyAsync(E.st, &b->h_ring[0], sizeof(MbState), cudaMemcpyHostToDevice, s));
+    MB_CUDA(cudaMemcpyAsync(E.srch, init.data(), init.size() * sizeof(MbSearch), cudaMemcpyHostToDevice, s));
+    MB_CUDA(cudaMemcpyAsync(b->d_roots, roots.data(), roots.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    MB_CUDA(cudaStreamSynchronize(s));  // the staging copies above read host memory that goes out of scope
+    MB_CUDA(cudaEventRecord(b->ev0, s));
+    mb_init_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(E, b->d_roots);
+    mb_plan_kernel<<<1, 32, 0, s>>>(E, 1);
+    MB_CUDA(cudaGetLastError());
+    const int decide_blocks = (n + 127) / 128;
+    for (int64_t chunk = 0;; ++chunk) {
+        if (chunk >= kMbLag) {
+            MB_CUDA(cudaEventSynchronize(b->ring_ev[(chunk - kMbLag) % kMbRing]));
+            if (b->h_ring[(chunk - kMbLag) % kMbRing].done) break;
+        }
+        mb_prep_kernel<<<b->sms * 2, 256, 0, s>>>(E);
+        if (chunk == 0) mb_expand_kernel<W, false><<<b->expand_blocks, 32 * b->expand_wpb, b->expand_smem, s>>>(E);
+        else mb_expand_kernel<W, true><<<b->expand_blocks, 32 * b->expand_wpb, b->expand_smem, s>>>(E);
+        mb_insert_kernel<W><<<b->insert_blocks, 256, 0, s>>>(E);
+        mb_scan_sums_kernel<<<b->sms * 4, kScanT, 0, s>>>(E);
+        mb_scan_top_kernel<<<1, kScanT, 0, s>>>(E);
+        mb_scan_final_kernel<<<b->sms * 4, kScanT, 0, s>>>(E);
+        mb_decide_kernel<<<decide_blocks, 128, 0, s>>>(E);
+        mb_commit_kernel<W><<<b->commit_blocks, 256, 0, s>>>(E);
+        mb_plan_kernel<<<1, 32, 0, s>>>(E, 0);
+        MB_CUDA(cudaGetLastError());
+        MB_CUDA(cudaMemcpyAsync(&b->h_ring[chunk % kMbRing], E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
+        MB_CUDA(cudaEventRecord(b->ring_ev[chunk % kMbRing], s));
+    }
+    MB_CUDA(cudaEventRecord(b->ev1, s));
+    MbState fin{};
+    b->h_final.resize((size_t)n);
+    MB_CUDA(cudaMemcpyAsync(&fin, E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
+    MB_CUDA(cudaMemcpyAsync(b->h_final.data(), E.srch, (size_t)n * sizeof(MbSearch), cudaMemcpyDeviceToHost, s));
+    MB_CUDA(cudaStreamSynchronize(s));
+    if (fin.ierr) {
+        std::string m = "bfs_batch: internal error:";
+        if (fin.ierr & MB_IERR_TABLE_FULL) m += " visited table full (more than 3/4 of its slots used)";
+        if (fin.ierr & MB_IERR_SLAB_FULL) m += " node slab of a search full";
+        return mb_fail(ACS_ERR_CUDA, m);
+    }
+    b->ran = true;
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, b->ev0, b->ev1);
+    std::vector<int32_t> plen((size_t)n);
+    const int rc = mb_paths<W>(b, h_paths, path_cap, plen);
+    for (int i = 0; i < n; ++i) {
+        const MbSearch& f = b->h_final[i];
+        acs_search_result* r = results + i;
+        std::memset(r, 0, sizeof(*r));
+        r->solved = f.solved;
+        r->status = f.status;
+        r->budget_hit = f.budget_hit;
+        r->path_len = plen[i];
+        if (f.status == ACS_ROW_ASSERT && f.n_nodes == 0) {  // invalid root: the reference asserts before searching
+            r->seconds_device = ms * 1e-3;
+            continue;
+        }
+        r->n_visited = f.n_nodes;
+        r->n_expanded = f.n_expanded;
+        r->n_moves = f.solved ? f.sol_gid + 1 : (f.status ? (int64_t)(((uint64_t)f.err_code >> 2) + 1) : f.n_expanded * 12);
+        r->frontier_left = f.n_nodes - f.n_expanded;
+        r->n_levels = f.levels;
+        r->n_minlen = f.n_minlen;
+        for (int j = 0; j < f.n_minlen && j < 128; ++j) r->minlen_log[j] = f.minlen_log[j];
+        r->seconds_device = ms * 1e-3;
+    }
+    return rc;
+}
+
+}  // namespace
+
+extern "C" {
+
+int acs_bfs_batch_run(acs_bfs_batch* b, const int8_t* h_presentations, int32_t* h_paths, int path_cap,
+                      acs_search_result* results) {
+    if (!b || !h_presentations || !results || path_cap < 0) return ACS_ERR_INVALID;
+    return b->W == 1 ? mb_run_impl<1>(b, h_presentations, h_paths, path_cap, results)
+                     : mb_run_impl<2>(b, h_presentations, h_paths, path_cap, results);
+}
+
+int acs_bfs_batch_paths(acs_bfs_batch* b, int32_t* h_paths, int path_cap) {
+    if (!b || path_cap < 0 || (!h_paths && path_cap > 0)) return ACS_ERR_INVALID;
+    if (!b->ran) return mb_fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
+    std::vector<int32_t> plen;
+    return b->W == 1 ? mb_paths<1>(b, h_paths, path_cap, plen) : mb_paths<2>(b, h_paths, path_cap, plen);
+}
+
+int acs_bfs_batch_visited(acs_bfs_batch* b, int search, int8_t* h_out, int64_t cap_rows, int64_t* n_out) {
+    if (!b || search < 0 || search >= b->n_search || (!h_out && cap_rows > 0)) return ACS_ERR_INVALID;
+    if (!b->ran) return mb_fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
+    MB_CUDA(cudaSetDevice(b->device));
+    const MbSearch& f = b->h_final[search];
+    const int64_t n = std::min<int64_t>(f.n_nodes, std::max<int64_t>(cap_rows, 0));
+    if (n_out) *n_out = n;
+    if (n == 0) return ACS_OK;
+    int8_t* d = nullptr;
+    MB_CUDA(cudaMalloc((void**)&d, (size_t)n * 2 * b->mrl));
+    const uint64_t* slab = b->E.nodes + (size_t)f.slab * (2 * b->W + 2);
+    const unsigned grid = (unsigned)((n + 255) / 256);
+    if (b->W == 1) mb_unpack_kernel<1><<<grid, 256, 0, b->stream>>>(slab, d, (uint64_t)n, b->mrl);
+    else mb_unpack_kernel<2><<<grid, 256, 0, b->stream>>>(slab, d, (uint64_t)n, b->mrl);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(h_out, d, (size_t)n * 2 * b->mrl, cudaMemcpyDeviceToHost, b->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);
+    cudaFree(d);
+    MB_CUDA(e);
+    return ACS_OK;
+}
+
+}  // extern "C"

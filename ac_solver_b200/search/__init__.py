@@ -1,2 +1,2 @@
-from .breadth_first import bfs, bfs_device  # noqa: F401
+from .breadth_first import bfs, bfs_batch, bfs_device, bfs_groups  # noqa: F401
 from .greedy import greedy_search, greedy_search_batch, greedy_search_groups  # noqa: F401

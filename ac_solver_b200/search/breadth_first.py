@@ -63,6 +63,165 @@ def bfs_device(presentation, max_nodes_to_explore=10000, cyclically_reduce_after
     return bool(res.solved), plist, info
 
 
+DEFAULT_MAX_BYTES = 32 << 30  # device bytes of one batched engine; larger batches are split into several runs
+# device bytes of the engines bfs_groups keeps alive at once (a B200 has 180 GB); more runs in several waves
+DEFAULT_MAX_TOTAL_BYTES = 128 << 30
+
+
+def _batch_inputs(presentations, max_nodes_to_explore):
+    """Validate a batch on the host, before any GPU work -> (int8 rows, int64 budgets)."""
+    P = np.asarray(presentations)
+    if P.ndim != 2 or P.shape[1] % 2 or P.shape[1] == 0:
+        raise ValueError("presentations must be [S, 2*max_relator_length]")
+    if P.size and np.abs(P.astype(np.int64)).max() > 2:  # wide: abs(int8 -128) is -128
+        raise ValueError("the GPU search supports the two-generator alphabet {+-1, +-2} only")
+    budgets = np.broadcast_to(np.asarray(max_nodes_to_explore, dtype=np.int64), (P.shape[0],))
+    if np.ndim(max_nodes_to_explore) > 1 or (budgets < 0).any():
+        raise ValueError("max_nodes_to_explore must be one non-negative int or one per row")
+    for k in range(P.shape[0]):  # breadth_first.py:36-38
+        assert is_array_valid_presentation(P[k]), f"row {k}: {P[k].tolist()} is not a valid presentation"
+    return np.ascontiguousarray(P, dtype=np.int8), np.ascontiguousarray(budgets)
+
+
+def _engine_bytes(L, mrl, budgets, chunk_parents):
+    b, arr = C.c_int64(0), np.ascontiguousarray(budgets, dtype=np.int64)
+    _lib.check(L.acs_bfs_batch_bytes(len(arr), mrl, arr.ctypes.data, int(chunk_parents), C.byref(b)))
+    return b.value
+
+
+def _split(L, mrl, budgets, chunk_parents, max_bytes):
+    """Consecutive row ranges whose engines each need at most max_bytes (a single row may need more)
+    -> list of (lo, hi, bytes).  An engine's size grows with its rows, so each range end is found by
+    bisection."""
+    parts, lo = [], 0
+    S = len(budgets)
+    while lo < S:
+        good, bad = lo + 1, S + 1  # rows [lo, good) fit (or are a single row); [lo, bad) do not
+        if _engine_bytes(L, mrl, budgets[lo:S], chunk_parents) <= max_bytes:
+            good = S
+        while bad - good > 1 and good < S:
+            mid = (good + bad) // 2
+            if _engine_bytes(L, mrl, budgets[lo:mid], chunk_parents) <= max_bytes:
+                good = mid
+            else:
+                bad = mid
+        parts.append((lo, good, _engine_bytes(L, mrl, budgets[lo:good], chunk_parents)))
+        lo = good
+    return parts
+
+
+class _BatchEngine:
+    """One acs_bfs_batch engine over rows [lo, hi) of a validated batch."""
+
+    def __init__(self, L, dev, P8, budgets, cyclical, chunk_parents):
+        self.L, self.P8 = L, np.ascontiguousarray(P8)
+        self.S, w = P8.shape
+        self.h = C.c_void_p()
+        b = np.ascontiguousarray(budgets, dtype=np.int64)  # referenced until the call returns
+        _lib.check(L.acs_bfs_batch_create(dev, self.S, w // 2, b.ctypes.data, int(bool(cyclical)), int(chunk_parents),
+                                          C.byref(self.h)))
+
+    def run(self, want_visited):
+        L, S = self.L, self.S
+        cap = 256
+        paths = np.zeros((S, cap, 2), np.int32)
+        res = (_lib.SearchResult * S)()
+        rc = L.acs_bfs_batch_run(self.h, self.P8.ctypes.data, paths.ctypes.data, cap, res)
+        need = max(int(res[s].path_len) for s in range(S))
+        if rc == _lib.ACS_ERR_INVALID and need > cap:  # a deeper solution than the buffer: fetch the paths again
+            cap = need
+            paths = np.zeros((S, cap, 2), np.int32)
+            rc = L.acs_bfs_batch_paths(self.h, paths.ctypes.data, cap)
+        _lib.check(rc)
+        out = []
+        for s in range(S):
+            r = res[s]
+            info = {
+                "n_visited": int(r.n_visited), "n_expanded": int(r.n_expanded), "n_moves": int(r.n_moves),
+                "frontier_left": int(r.frontier_left), "budget_hit": bool(r.budget_hit),
+                "n_levels": int(r.n_levels), "status": int(r.status),
+                "minlen_log": [int(r.minlen_log[i]) for i in range(r.n_minlen)],
+                "seconds_device": float(r.seconds_device),
+            }
+            if want_visited and r.status == 0:
+                vis = np.zeros((max(int(r.n_visited), 1), self.P8.shape[1]), np.int8)
+                n_out = C.c_int64(0)
+                _lib.check(L.acs_bfs_batch_visited(self.h, s, vis.ctypes.data, vis.shape[0], C.byref(n_out)))
+                info["visited"] = vis[: n_out.value]
+            plist = [(int(a), int(l)) for a, l in paths[s, : r.path_len]] if r.solved else None
+            out.append((bool(r.solved), plist, info))
+        return out
+
+    def destroy(self):
+        if self.h:
+            self.L.acs_bfs_batch_destroy(self.h)
+            self.h = None
+
+
+def bfs_batch(presentations, max_nodes_to_explore=10000, cyclically_reduce_after_moves=False, want_visited=False,
+              device=None, chunk_parents=0, max_bytes=DEFAULT_MAX_BYTES):
+    """Breadth-first search of every row of ``presentations`` [S, 2*mrl] in one device run
+    (csrc/mbfs.cu).  ``max_nodes_to_explore`` is one budget or one per row.
+
+    Returns a list of ``(solved, path|None, info)``, element s equal to ``bfs_device(row s, ...)``.
+    A row on which the reference raises carries ``info["status"] != 0`` instead of raising.  Rows
+    are split into several engine runs when one engine would need more than ``max_bytes`` of device
+    memory; ``chunk_parents`` > 0 caps the parents expanded per chunk (the results do not depend on it)."""
+    P8, budgets = _batch_inputs(presentations, max_nodes_to_explore)
+    if P8.shape[0] == 0:
+        return []
+    L = _lib.lib()
+    dev = _lib.default_device() if device is None else device
+    out = []
+    for lo, hi, _ in _split(L, P8.shape[1] // 2, budgets, chunk_parents, max_bytes):
+        e = _BatchEngine(L, dev, P8[lo:hi], budgets[lo:hi], cyclically_reduce_after_moves, chunk_parents)
+        try:
+            out += e.run(want_visited)
+        finally:
+            e.destroy()
+    return out
+
+
+def bfs_groups(groups, max_nodes_to_explore=10000, cyclically_reduce_after_moves=False, want_visited=False, device=None,
+               chunk_parents=0, max_bytes=DEFAULT_MAX_BYTES, max_total_bytes=DEFAULT_MAX_TOTAL_BYTES, threads=8):
+    """Sweep helper: ``groups`` is a list of presentation arrays [S_k, 2*mrl_k] (one per max_relator_length).
+    Rows are split into engines of at most ``max_bytes`` each, and the engines into waves of at most
+    ``max_total_bytes`` together.  Every engine of a wave is created before any of its searches runs
+    (``cudaMalloc`` stalls behind running kernels, see ``greedy_search_groups``), then they run
+    concurrently (one stream and one host thread each).  Returns one ``bfs_batch`` result list per group."""
+    from concurrent.futures import ThreadPoolExecutor
+
+    inputs = [_batch_inputs(P, max_nodes_to_explore) for P in groups]
+    L = _lib.lib()
+    dev = _lib.default_device() if device is None else device
+    plan = []  # (group, lo, hi, bytes) in group and row order
+    for g, (P8, budgets) in enumerate(inputs):
+        if P8.shape[0]:
+            plan += [(g, lo, hi, nb) for lo, hi, nb in _split(L, P8.shape[1] // 2, budgets, chunk_parents, max_bytes)]
+    waves, total = [], 0
+    for item in plan:
+        if not waves or total + item[3] > max_total_bytes:
+            waves.append([])
+            total = 0
+        waves[-1].append(item)
+        total += item[3]
+    out = [[] for _ in groups]
+    for wave in waves:
+        engines = []
+        try:
+            for g, lo, hi, _ in wave:
+                P8, budgets = inputs[g]
+                engines.append(_BatchEngine(L, dev, P8[lo:hi], budgets[lo:hi], cyclically_reduce_after_moves, chunk_parents))
+            with ThreadPoolExecutor(max_workers=max(1, min(threads, len(engines)))) as pool:
+                raw = list(pool.map(lambda e: e.run(want_visited), engines))
+        finally:
+            for e in engines:
+                e.destroy()
+        for (g, _, _, _), rows in zip(wave, raw):
+            out[g] += rows
+    return out
+
+
 def bfs(presentation, max_nodes_to_explore=10000, verbose=False, cyclically_reduce_after_moves=False):
     """search/breadth_first.py:15-97.
 

@@ -6,9 +6,10 @@ values and output-file formats).
 What differs is where the work runs: the free + cyclic reduction of all 4^len candidate words of
 one length is ONE batched call of the GPU reduction kernel (``simplify_relator`` semantics,
 envs/utils.py:175-240) instead of a Python loop, and a greedy sweep runs all presentations of a
-group concurrently (one warp per presentation, ``greedy_search_batch``) instead of one after the
-other.  The enumeration order, the cyclic-permutation de-duplication and the file layout are the
-reference's, so the generated lists are identical.
+group concurrently (one warp per presentation, ``greedy_search_batch``; a BFS sweep likewise
+through one batched engine, ``bfs_batch``) instead of one after the other.  The enumeration order,
+the cyclic-permutation de-duplication and the file layout are the reference's, so the generated
+lists are identical.
 """
 
 from __future__ import annotations
@@ -63,6 +64,7 @@ def trivialize_miller_schupp_through_search(min_n, max_n, min_w_len, max_w_len, 
     """miller_schupp.py:95-177.  ``search_fn`` is this package's ``greedy_search`` or ``bfs``.
     Returns (solved_rels, unsolved_rels, solved_paths) in the reference's order."""
     assert search_fn.__name__ in ["greedy_search", "bfs"], f"expect search_fn to be greedy or bfs; got {search_fn.__name__}"
+    from ..breadth_first import _raise_for, bfs_batch
     from ..greedy import greedy_search_batch
 
     rels = {n: generate_miller_schupp_presentations(n, max_w_len) for n in range(min_n, max_n + 1)}
@@ -73,26 +75,15 @@ def trivialize_miller_schupp_through_search(min_n, max_n, min_w_len, max_w_len, 
             group = rels[n].get(lenw, [])
             if not group:
                 continue
-            if search_fn.__name__ == "greedy_search":  # all presentations of the group in one launch
-                from ..breadth_first import _raise_for
-
-                results = []
-                for s_, p_, info in greedy_search_batch(np.array(group, dtype=np.int8), max_nodes_to_explore, False):
-                    _raise_for(info["status"])  # the reference raises where a move empties a relator
-                    if not s_ and info["budget_hit"]:  # greedy.py:116-118 prints this per presentation
-                        print(f"Exiting search as number of explored nodes = {info['n_visited']} has exceeded the limit "
-                              f"{max_nodes_to_explore}")
-                    results.append((s_, p_))
-            else:
-                import contextlib
-                import io
-
-                results = []
-                for pres in group:
-                    with contextlib.redirect_stdout(io.StringIO()) as buf:
-                        results.append(search_fn(presentation=pres, max_nodes_to_explore=max_nodes_to_explore,
-                                                 verbose=False, cyclically_reduce_after_moves=False))
-                    print(buf.getvalue(), end="")
+            # all presentations of the group in one device run; output and errors in row order, as the reference's loop
+            batch = greedy_search_batch if search_fn.__name__ == "greedy_search" else bfs_batch
+            results = []
+            for s_, p_, info in batch(np.array(group, dtype=np.int8), max_nodes_to_explore, False):
+                _raise_for(info["status"])  # the reference raises where a move empties a relator
+                if not s_ and info["budget_hit"]:  # greedy.py:116-118 / breadth_first.py print this per presentation
+                    print(f"Exiting search as number of explored nodes = {info['n_visited']} has exceeded the limit "
+                          f"{max_nodes_to_explore}")
+                results.append((s_, p_))
             for pres, (solved, path) in zip(group, results):
                 if solved:
                     solved_rels.append(pres)

@@ -198,6 +198,28 @@ int acs_bfs_run(acs_bfs *b, const int8_t *h_presentation, int32_t *h_path, int p
 int acs_bfs_visited(acs_bfs *b, int8_t *h_out, int64_t cap_rows, int64_t *n_out);
 void acs_bfs_destroy(acs_bfs *b);
 
+/* Batched breadth-first search: n_search independent searches of the same mrl and cyclical flag,
+ * one budget each, advanced together through the same kernel launches on one GPU (csrc/mbfs.cu).
+ * Every search's result, path, counters and visited array equal acs_bfs_run on its row.
+ * acs_bfs_batch_bytes: device bytes an engine for these arguments allocates (for planning batches).
+ * chunk_parents <= 0: default chunk size.  h_presentations [n_search, 2*mrl]; h_paths
+ * [n_search, path_cap, 2] int32 (action, total_length) pairs; results [n_search].  A row the
+ * reference raises on has results[s].status != 0.  A path longer than path_cap makes the run
+ * return ACS_ERR_INVALID with every other result filled (results[s].path_len holds the needed
+ * length); acs_bfs_batch_paths then fetches the paths of that run into a larger buffer without
+ * searching again.  path_cap may be 0 (with h_paths NULL) when no search can solve.
+ * chunk_parents caps the parents expanded per chunk after the first, which expands every root. */
+typedef struct acs_bfs_batch acs_bfs_batch;
+int acs_bfs_batch_bytes(int n_search, int mrl, const int64_t *max_nodes, int64_t chunk_parents, int64_t *bytes_out);
+int acs_bfs_batch_create(int device, int n_search, int mrl, const int64_t *max_nodes /* [n_search] */,
+                         int cyclical, int64_t chunk_parents, acs_bfs_batch **out);
+int acs_bfs_batch_run(acs_bfs_batch *b, const int8_t *h_presentations, int32_t *h_paths, int path_cap,
+                      acs_search_result *results /* [n_search] */);
+int acs_bfs_batch_paths(acs_bfs_batch *b, int32_t *h_paths, int path_cap);
+/* visited states of search `search` of the last run, insertion (FIFO) order, int8 rows */
+int acs_bfs_batch_visited(acs_bfs_batch *b, int search, int8_t *h_out, int64_t cap_rows, int64_t *n_out);
+void acs_bfs_batch_destroy(acs_bfs_batch *b);
+
 /* Batched greedy search (search/greedy.py:15-121): n_search independent presentations of the
  * same mrl, one warp each, one launch.  h_presentations [n_search, 2*mrl]; h_paths
  * [n_search, path_cap, 2] int32 (action, total_length) pairs; results [n_search].  On failure

@@ -15,8 +15,6 @@ File conventions reproduced from the reference's shipped data (SURVEY 8c/8f-2):
   bfs_solved_presentations.txt     rows bfs() solves, in all_presentations order
 """
 import argparse
-import contextlib
-import io
 import json
 import os
 import sys
@@ -26,7 +24,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from ac_solver_b200.search.breadth_first import bfs_device  # noqa: E402
+from ac_solver_b200.search.breadth_first import bfs_groups  # noqa: E402
 from ac_solver_b200.search.greedy import greedy_search_groups  # noqa: E402
 from ac_solver_b200.search.miller_schupp import (generate_miller_schupp_presentations,  # noqa: E402
                                                   write_list_to_text_file)
@@ -62,13 +60,14 @@ def main():
     # the reference's bfs_solved_presentations.txt (278 rows) is reproduced by bfs() at budget 1e6 WITH cyclic reduction
     # after moves (the budget / flag are not recorded in the reference; found by search, see data/README.md);
     # the plain default (cyclically_reduce_after_moves=False) solves 52 of them
-    bfs_solved, bfs_solved_plain = [], []
-    with contextlib.redirect_stdout(io.StringIO()):
-        for k in ordered:
-            if bfs_device(np.array(rows[k], dtype=np.int8), args.bfs_budget, True)[0]:
-                bfs_solved.append(k)
-            if bfs_device(np.array(rows[k], dtype=np.int8), args.bfs_budget)[0]:
-                bfs_solved_plain.append(k)
+    groups = [np.array([rows[k] for k in ks], dtype=np.int8) for ks in key_lists]
+    solved_by_flag = {}
+    for cyc in (True, False):
+        solved_by_flag[cyc] = set()
+        for ks, out in zip(key_lists, bfs_groups(groups, args.bfs_budget, cyc)):
+            solved_by_flag[cyc].update(k for k, (ok, _, _) in zip(ks, out) if ok)
+    bfs_solved = [k for k in ordered if k in solved_by_flag[True]]
+    bfs_solved_plain = [k for k in ordered if k in solved_by_flag[False]]
     t2 = time.perf_counter()
     os.makedirs(args.out, exist_ok=True)
     write_list_to_text_file([rows[k] for k in ordered], os.path.join(args.out, "all_presentations"))
