@@ -108,6 +108,13 @@ _SIGS = {
     "acs_bfs_batch_paths": (C.c_int, [_P, _P, C.c_int]),
     "acs_bfs_batch_visited": (C.c_int, [_P, C.c_int, _P, C.c_int64, C.POINTER(C.c_int64)]),
     "acs_bfs_batch_destroy": (None, [_P]),
+    "acs_bfs_batch_set_goals": (C.c_int, [_P, _P, C.c_int]),
+    "acs_bfs_batch_goal_hits": (C.c_int, [_P, _P]),
+    "acs_goalset_from_rows": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, C.c_int64, C.POINTER(_P)]),
+    "acs_goalset_from_bfs_batch": (C.c_int, [_P, C.POINTER(_P)]),
+    "acs_goalset_size": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "acs_goalset_path": (C.c_int, [_P, C.c_int64, C.POINTER(C.c_int), _P, C.c_int, C.POINTER(C.c_int)]),
+    "acs_goalset_destroy": (None, [_P]),
     "acs_greedy_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, C.POINTER(_P)]),
     "acs_greedy_run": (C.c_int, [_P, _P, _P, _P]),
     "acs_greedy_visited": (C.c_int, [_P, C.c_int, _P, C.c_int64, C.POINTER(C.c_int64)]),

@@ -43,11 +43,14 @@
 #include "ac_keys.cuh"
 #include "acs_internal.h"
 #include "bfs_common.cuh"
+#include "goalset.cuh"
 
 namespace acs {
 
-constexpr int kMbCtrl = 130;  // per segment: solving child, raising child, first child of each total length < 128
-constexpr int kMbSol = 0, kMbErr = 1, kMbLen0 = 2;
+// per segment: solving child, raising child, first child of each total length < 128, first goal child
+// (candidate id << 32 | goal entry)
+constexpr int kMbCtrl = 131;
+constexpr int kMbSol = 0, kMbErr = 1, kMbLen0 = 2, kMbGoal = 130;
 constexpr uint64_t kMbNode = 1ull << 39, kMbIdx = kMbNode - 1;
 constexpr uint64_t kMbTomb = 1ull << 63;  // fingerprints are 23 bits: never equal to a tombstone's
 constexpr int kMbStage = 128;             // records staged per warp before a flush to the log
@@ -57,7 +60,8 @@ enum : int { MB_IERR_TABLE_FULL = 1, MB_IERR_SLAB_FULL = 2 };
 // per-search state
 struct MbSearch {
     int64_t budget, slab, cap, n_nodes, head, level_end, n_expanded, sol_gid, err_code;
-    int32_t min_len, levels, done, solved, budget_hit, status, n_minlen, pad;
+    int32_t min_len, levels, done, solved, budget_hit, status, n_minlen;
+    int32_t sol_len;  // total length of the state that ended a solved search: 2, or a goal state's
     int32_t minlen_log[128];
 };
 
@@ -65,7 +69,8 @@ struct MbSearch {
 struct MbState {
     int64_t Ftot, n_seg, used, chunks, chunk_cap;
     uint64_t tmask;
-    int32_t mrl, cyclical, n_search, done, ierr, pad;
+    int32_t mrl, cyclical, n_search, done, ierr;
+    int32_t explore;  // 1: the length-2 rule is off, searches end at a goal, their budget or exhaustion
 };
 
 struct MbEngine {
@@ -89,6 +94,8 @@ struct MbEngine {
     int64_t* seg_base;    // [n_search] global node index of the segment's first winner, minus its rank
     int32_t* seg_of;      // [n_search] segment of a search in the current chunk
     int64_t rec_cap;
+    GoalView goals;       // the goal set, if one is set
+    int64_t* goal_hit;    // [n_search] goal entry a search stopped at, or -1 (allocated with the first goal set)
 };
 
 template <int W>
@@ -384,6 +391,44 @@ __global__ void __launch_bounds__(256) mb_insert_kernel(const MbEngine E) {
     }
 }
 
+// ---- goal test (only with a goal set) ----------------------------------------------------------------
+// The reference tests a child against the goal set after the length-2 test and before the visited test.
+// Only the final winners of the bitmap need a lookup: a child whose state its search has already visited
+// cannot be a goal, because that state was generated under a smaller candidate id and the search would
+// have stopped there (roots are tested at init); a child that lost its slot to a smaller candidate id of
+// the same state is preceded by that candidate.  The first goal child per segment goes to its control slot.
+template <int W>
+__global__ void __launch_bounds__(256) mb_goal_kernel(const MbEngine E) {
+    const MbState* st = E.st;
+    if (st->done) return;
+    const unsigned long long n = *E.cursor;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+         i += (unsigned long long)gridDim.x * blockDim.x) {
+        const uint32_t c = __ldcg(E.log_c + i);
+        if (!((__ldcg(E.bitmap + (c >> 5)) >> (c & 31)) & 1u)) continue;
+        const int64_t e = goal_find<W>(E.goals, load_key_cg<W>(E.log_keys, i));
+        if (e < 0) continue;
+        const int k = E.seg_of[__ldcg(E.log_s + i)];
+        atomicMin(&E.ctrl[(int64_t)k * kMbCtrl + kMbGoal], ((unsigned long long)c << 32) | (unsigned long long)e);
+    }
+}
+
+// a root in the goal set is a hit at depth 0: one visited node, nothing expanded
+template <int W>
+__global__ void mb_goal_roots_kernel(const MbEngine E) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= E.st->n_search || E.srch[s].done) return;
+    MbSearch& M = E.srch[s];
+    const int64_t e = goal_find<W>(E.goals, node_key<W>(E.nodes, (uint64_t)M.slab));
+    if (e < 0) return;
+    M.solved = 1;
+    M.done = 1;
+    M.sol_gid = -1;
+    M.n_expanded = 0;
+    M.sol_len = M.min_len;
+    E.goal_hit[s] = e;
+}
+
 // ---- scan --------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kScanT) mb_scan_sums_kernel(const MbEngine E) {
     const MbState* st = E.st;
@@ -480,8 +525,8 @@ __global__ void __launch_bounds__(128) mb_decide_kernel(const MbEngine E) {
         cut_p = lo;
         if (12 * (cut_p + 1) < limit) limit = 12 * (cut_p + 1);
     }
-    const unsigned long long sol = red[kMbSol], err = red[kMbErr];
-    bool sol_here = false;
+    const unsigned long long sol = st->explore ? ~0ull : red[kMbSol], err = red[kMbErr], goal = red[kMbGoal];
+    bool sol_here = false, goal_here = false;
     int status = 0;
     uint64_t sol_l = 0, err_l = 0;
     if (sol != ~0ull && sol - c0 < limit) {  // solved at or before the cut parent
@@ -490,11 +535,19 @@ __global__ void __launch_bounds__(128) mb_decide_kernel(const MbEngine E) {
         sol_here = true;
         cut = false;
     }
+    if (goal != ~0ull && (goal >> 32) - c0 < limit) {  // a goal child; on the solving child itself the solve wins
+        sol_l = (goal >> 32) - c0;
+        limit = sol_l;
+        sol_here = true;
+        goal_here = true;
+        cut = false;
+    }
     if (err != ~0ull && (err >> 2) - c0 < limit) {  // the reference raises here, before anything later
         err_l = (err >> 2) - c0;
         limit = err_l;
         status = (int)(err & 3);
         sol_here = false;
+        goal_here = false;
         cut = false;
     }
     // "New minimal length found" events in reference order
@@ -524,6 +577,14 @@ __global__ void __launch_bounds__(128) mb_decide_kernel(const MbEngine E) {
         M.solved = 1;
         M.sol_gid = (int64_t)(12 * head + sol_l);
         M.n_expanded = M.sol_gid / 12 + 1;
+        M.sol_len = 2;
+        if (goal_here) {
+            const uint64_t e = goal & 0xFFFFFFFFull;
+            const int W = st->mrl <= 29 ? 1 : 2;
+            const uint64_t* q = E.goals.nodes + e * (2 * W + 2);  // the goal state's key: lengths in the top bits
+            M.sol_len = (int32_t)(q[W - 1] >> 58) + (int32_t)(q[2 * W - 1] >> 58);
+            E.goal_hit[s] = (int64_t)e;
+        }
     } else if (status) {
         M.status = status;
         M.err_code = (int64_t)(((12 * head + err_l) << 2) | (uint64_t)status);
@@ -575,7 +636,8 @@ __global__ void __launch_bounds__(256) mb_commit_kernel(const MbEngine E) {
 }
 
 // ---- results -----------------------------------------------------------------------------------------
-// path of every solved search: (action, total length) pairs from the root, then (solving action, 2)
+// path of every solved search: (action, total length) pairs from the root, then (solving action, 2) -- or
+// (action, the goal state's total length) after a goal child, or nothing more when the root is a goal
 template <int W>
 __global__ void mb_path_kernel(const MbEngine E, int32_t* paths, int path_cap, int32_t* path_len) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
@@ -584,7 +646,8 @@ __global__ void mb_path_kernel(const MbEngine E, int32_t* paths, int path_cap, i
     path_len[s] = 0;
     if (!M.solved) return;
     int32_t* path = paths + (size_t)s * path_cap * 2;
-    const int64_t node = M.sol_gid / 12;
+    const bool at_root = M.sol_gid < 0;
+    const int64_t node = at_root ? 0 : M.sol_gid / 12;
     int depth = 0;
     for (int64_t g = node; g >= 0; ++depth) {
         Key<W> k;
@@ -592,10 +655,10 @@ __global__ void mb_path_kernel(const MbEngine E, int32_t* paths, int path_cap, i
         node_load<W>(E.nodes, (uint64_t)(M.slab + g), k, pl, tag);
         g = pl < 0 ? -1 : (pl >> 4);
     }
-    path_len[s] = depth + 1;
-    if (depth < path_cap) {
+    path_len[s] = depth + (at_root ? 0 : 1);
+    if (!at_root && depth < path_cap) {
         path[2 * depth] = (int32_t)(M.sol_gid % 12);
-        path[2 * depth + 1] = 2;
+        path[2 * depth + 1] = M.sol_len;
     }
     int pos = depth - 1;
     for (int64_t g = node; g >= 0; --pos) {
@@ -618,6 +681,21 @@ __global__ void mb_unpack_kernel(const uint64_t* nodes, int8_t* out, uint64_t n,
     split_key<W>(node_key<W>(nodes, i), r0, r1);
     unpack_bytes<2 * W>(out + i * 2 * mrl, r0, mrl);
     unpack_bytes<2 * W>(out + i * 2 * mrl + mrl, r1, mrl);
+}
+
+// committed nodes of every search -> goal-set entries in (search, FIFO id) order; off [n_search + 1] holds
+// each search's first entry, slab [n_search] its first node.  Parent links are rebased onto entry indices.
+template <int W>
+__global__ void mb_adopt_kernel(const uint64_t* nodes, const int64_t* off, const int64_t* slab, int n_search,
+                                uint64_t* out, uint64_t n) {
+    for (uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (uint64_t)gridDim.x * blockDim.x) {
+        const int s = mb_segment(off, n_search, (int64_t)e);
+        const int64_t first = __ldg(off + s);
+        Key<W> k;
+        int64_t pl, tag;
+        node_load<W>(nodes, (uint64_t)(__ldg(slab + s) + ((int64_t)e - first)), k, pl, tag);
+        node_store<W>(out, e, k, pl < 0 ? -1 : (((first + (pl >> 4)) << 4) | (pl & 15)), (int64_t)s);
+    }
 }
 
 }  // namespace acs
@@ -700,6 +778,9 @@ struct acs_bfs_batch {
     int expand_blocks = 148, expand_wpb = 8, insert_blocks = 148, commit_blocks = 148;
     size_t expand_smem = 0;
     bool ran = false;
+    const acs_goalset* goals = nullptr;  // acs_bfs_batch_set_goals
+    int explore = 0;                     // stop_at_trivial == 0
+    bool adopted = false;                // the nodes went to a goal set (acs_goalset_from_bfs_batch)
 };
 
 extern "C" {
@@ -727,7 +808,7 @@ void acs_bfs_batch_destroy(acs_bfs_batch* b) {
     MbEngine& E = b->E;
     void* ptrs[] = {E.st, E.srch, E.nodes, E.table, E.log_keys, E.log_c, E.log_s, E.rec_slot, E.cursor, E.bitmap, E.rt,
                     E.bsums, E.ctrl, E.seg_search, E.seg_head, E.seg_off, E.seg_limit, E.seg_base, E.seg_of,
-                    b->d_roots, b->d_paths, b->d_plen};
+                    E.goal_hit, b->d_roots, b->d_paths, b->d_plen};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (b->h_ring) cudaFreeHost(b->h_ring);
@@ -857,6 +938,7 @@ template <int W>
 int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int path_cap, acs_search_result* results) {
     const int n = b->n_search, mrl = b->mrl;
     MbEngine& E = b->E;
+    if (b->adopted) return mb_fail(ACS_ERR_INVALID, "bfs_batch: the engine's states were handed to a goal set");
     std::vector<MbSearch> init((size_t)n);
     std::vector<uint64_t> roots((size_t)n * 2 * W, 0);
     int64_t slab = 0, n_valid = 0;
@@ -892,9 +974,11 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
     st.cyclical = b->cyclical;
     st.n_search = n;
     st.used = n_valid;
+    st.explore = b->explore;
     cudaStream_t s = b->stream;
     MB_CUDA(cudaSetDevice(b->device));
     MB_CUDA(cudaMemsetAsync(E.table, 0, b->plan.tcap * sizeof(uint64_t), s));
+    if (E.goal_hit) MB_CUDA(cudaMemsetAsync(E.goal_hit, 0xFF, (size_t)n * sizeof(int64_t), s));
     b->h_ring[0] = st;  // pinned staging for the async upload
     MB_CUDA(cudaMemcpyAsync(E.st, &b->h_ring[0], sizeof(MbState), cudaMemcpyHostToDevice, s));
     MB_CUDA(cudaMemcpyAsync(E.srch, init.data(), init.size() * sizeof(MbSearch), cudaMemcpyHostToDevice, s));
@@ -902,6 +986,7 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
     MB_CUDA(cudaStreamSynchronize(s));  // the staging copies above read host memory that goes out of scope
     MB_CUDA(cudaEventRecord(b->ev0, s));
     mb_init_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(E, b->d_roots);
+    if (b->goals) mb_goal_roots_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(E);
     mb_plan_kernel<<<1, 32, 0, s>>>(E, 1);
     MB_CUDA(cudaGetLastError());
     const int decide_blocks = (n + 127) / 128;
@@ -914,6 +999,7 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
         if (chunk == 0) mb_expand_kernel<W, false><<<b->expand_blocks, 32 * b->expand_wpb, b->expand_smem, s>>>(E);
         else mb_expand_kernel<W, true><<<b->expand_blocks, 32 * b->expand_wpb, b->expand_smem, s>>>(E);
         mb_insert_kernel<W><<<b->insert_blocks, 256, 0, s>>>(E);
+        if (b->goals) mb_goal_kernel<W><<<b->insert_blocks, 256, 0, s>>>(E);
         mb_scan_sums_kernel<<<b->sms * 4, kScanT, 0, s>>>(E);
         mb_scan_top_kernel<<<1, kScanT, 0, s>>>(E);
         mb_scan_final_kernel<<<b->sms * 4, kScanT, 0, s>>>(E);
@@ -1002,6 +1088,109 @@ int acs_bfs_batch_visited(acs_bfs_batch* b, int search, int8_t* h_out, int64_t c
     if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);
     cudaFree(d);
     MB_CUDA(e);
+    return ACS_OK;
+}
+
+}  // extern "C"
+
+// ---- goal sets ---------------------------------------------------------------------------------------------
+extern "C" {
+
+int acs_bfs_batch_set_goals(acs_bfs_batch* b, const acs_goalset* g, int stop_at_trivial) {
+    if (!b) return ACS_ERR_INVALID;
+    if (g) {
+        if (g->mrl != b->mrl)
+            return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set's max_relator_length differs from the engine's");
+        if (g->cyclical != b->cyclical)
+            return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set's cyclical flag differs from the engine's");
+        if (g->device != b->device)
+            return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set lives on another device");
+        if (g->n_entries >= (int64_t)0xFFFFFFFF)  // a hit packs the entry into 32 bits beside its candidate id
+            return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch_set_goals: goal sets of 2^32 - 1 entries or more are not supported");
+        if (!b->E.goal_hit) {
+            MB_CUDA(cudaSetDevice(b->device));
+            MB_CUDA(cudaMalloc((void**)&b->E.goal_hit, (size_t)b->n_search * sizeof(int64_t)));
+            MB_CUDA(cudaMemset(b->E.goal_hit, 0xFF, (size_t)b->n_search * sizeof(int64_t)));
+        }
+        b->E.goals = g->view();
+    } else {
+        b->E.goals = GoalView{nullptr, nullptr, 0};
+    }
+    b->goals = g;
+    b->explore = stop_at_trivial ? 0 : 1;
+    return ACS_OK;
+}
+
+int acs_bfs_batch_goal_hits(acs_bfs_batch* b, int64_t* h_entry) {
+    if (!b || !h_entry) return ACS_ERR_INVALID;
+    if (!b->ran) return mb_fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
+    if (!b->E.goal_hit) {
+        std::fill(h_entry, h_entry + b->n_search, (int64_t)-1);
+        return ACS_OK;
+    }
+    MB_CUDA(cudaSetDevice(b->device));
+    MB_CUDA(cudaMemcpyAsync(h_entry, b->E.goal_hit, (size_t)b->n_search * sizeof(int64_t), cudaMemcpyDeviceToHost,
+                            b->stream));
+    MB_CUDA(cudaStreamSynchronize(b->stream));
+    return ACS_OK;
+}
+
+int acs_goalset_from_bfs_batch(acs_bfs_batch* b, acs_goalset** out) {
+    if (!b || !out) return ACS_ERR_INVALID;
+    *out = nullptr;
+    if (!b->ran) return mb_fail(ACS_ERR_INVALID, "goalset_from_bfs_batch: the engine has no completed run");
+    const int n = b->n_search;
+    std::vector<int64_t> off((size_t)n + 1, 0), slab((size_t)n, 0);
+    for (int s = 0; s < n; ++s) {
+        off[s + 1] = off[s] + b->h_final[s].n_nodes;
+        slab[s] = b->h_final[s].slab;
+    }
+    const int64_t total = off[n];
+    MB_CUDA(cudaSetDevice(b->device));
+    MB_CUDA(cudaStreamSynchronize(b->stream));
+    // the engine is spent from here on: free its table and logs before the entries are allocated
+    MbEngine& E = b->E;
+    for (void** p : {(void**)&E.table, (void**)&E.log_keys, (void**)&E.log_c, (void**)&E.log_s, (void**)&E.rec_slot,
+                     (void**)&E.bitmap, (void**)&E.rt, (void**)&E.bsums}) {
+        if (*p) cudaFree(*p);
+        *p = nullptr;
+    }
+    b->adopted = true;
+    b->ran = false;
+    acs_goalset* g = new acs_goalset();
+    g->device = b->device;
+    g->mrl = b->mrl;
+    g->W = b->W;
+    g->cyclical = b->cyclical;
+    g->n_entries = total;
+    int64_t* d_idx = nullptr;
+    cudaError_t e = cudaMalloc((void**)&g->nodes, (size_t)std::max<int64_t>(total, 1) * 8 * (2 * b->W + 2));
+    if (e == cudaSuccess) e = cudaMalloc((void**)&d_idx, (2 * (size_t)n + 1) * sizeof(int64_t));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_idx, off.data(), off.size() * 8, cudaMemcpyHostToDevice, b->stream);
+    if (e == cudaSuccess)
+        e = cudaMemcpyAsync(d_idx + n + 1, slab.data(), slab.size() * 8, cudaMemcpyHostToDevice, b->stream);
+    if (e == cudaSuccess && total > 0) {
+        const unsigned grid = (unsigned)std::min<int64_t>((total + 255) / 256, (int64_t)b->sms * 8);
+        if (b->W == 1) mb_adopt_kernel<1><<<grid, 256, 0, b->stream>>>(E.nodes, d_idx, d_idx + n + 1, n, g->nodes, (uint64_t)total);
+        else mb_adopt_kernel<2><<<grid, 256, 0, b->stream>>>(E.nodes, d_idx, d_idx + n + 1, n, g->nodes, (uint64_t)total);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);  // the host vectors above go out of scope
+    if (d_idx) cudaFree(d_idx);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        goalset_free(g);
+        return mb_fail(e == cudaErrorMemoryAllocation ? ACS_ERR_NOMEM : ACS_ERR_CUDA,
+                       std::string("goalset_from_bfs_batch: ") + cudaGetErrorString(e));
+    }
+    cudaFree(E.nodes);
+    E.nodes = nullptr;
+    const int rc = goalset_index(g, b->stream);
+    if (rc != ACS_OK) {
+        goalset_free(g);
+        return rc;
+    }
+    *out = g;
     return ACS_OK;
 }
 

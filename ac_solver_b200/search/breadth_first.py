@@ -113,13 +113,21 @@ def _split(L, mrl, budgets, chunk_parents, max_bytes):
 class _BatchEngine:
     """One acs_bfs_batch engine over rows [lo, hi) of a validated batch."""
 
-    def __init__(self, L, dev, P8, budgets, cyclical, chunk_parents):
+    def __init__(self, L, dev, P8, budgets, cyclical, chunk_parents, goals=None, stop_at_trivial=True):
         self.L, self.P8 = L, np.ascontiguousarray(P8)
         self.S, w = P8.shape
         self.h = C.c_void_p()
+        self.goals = goals
         b = np.ascontiguousarray(budgets, dtype=np.int64)  # referenced until the call returns
         _lib.check(L.acs_bfs_batch_create(dev, self.S, w // 2, b.ctypes.data, int(bool(cyclical)), int(chunk_parents),
                                           C.byref(self.h)))
+        if goals is not None or not stop_at_trivial:
+            try:
+                _lib.check(L.acs_bfs_batch_set_goals(self.h, goals.handle if goals is not None else None,
+                                                     int(bool(stop_at_trivial))))
+            except BaseException:
+                self.destroy()
+                raise
 
     def run(self, want_visited):
         L, S = self.L, self.S
@@ -133,6 +141,10 @@ class _BatchEngine:
             paths = np.zeros((S, cap, 2), np.int32)
             rc = L.acs_bfs_batch_paths(self.h, paths.ctypes.data, cap)
         _lib.check(rc)
+        hits = None
+        if self.goals is not None:
+            hits = np.full(S, -1, np.int64)
+            _lib.check(L.acs_bfs_batch_goal_hits(self.h, hits.ctypes.data))
         out = []
         for s in range(S):
             r = res[s]
@@ -143,6 +155,8 @@ class _BatchEngine:
                 "minlen_log": [int(r.minlen_log[i]) for i in range(r.n_minlen)],
                 "seconds_device": float(r.seconds_device),
             }
+            if hits is not None:
+                info["goal"] = int(hits[s]) if hits[s] >= 0 else None
             if want_visited and r.status == 0:
                 vis = np.zeros((max(int(r.n_visited), 1), self.P8.shape[1]), np.int8)
                 n_out = C.c_int64(0)
@@ -158,23 +172,46 @@ class _BatchEngine:
             self.h = None
 
 
+def _check_goals(goals, mrl, cyclical, dev):
+    if goals is None:
+        return
+    if goals.closed:
+        raise ValueError("the goal set is closed")
+    if goals.max_relator_length != mrl:
+        raise ValueError(f"the goal set has max_relator_length {goals.max_relator_length}, the presentations {mrl}")
+    if goals.cyclical != bool(cyclical):
+        raise ValueError(f"the goal set was built with cyclically_reduce_after_moves={goals.cyclical}, "
+                         f"the search uses {bool(cyclical)}")
+    if goals.device != dev:
+        raise ValueError(f"the goal set lives on device {goals.device}, the search runs on device {dev}")
+
+
 def bfs_batch(presentations, max_nodes_to_explore=10000, cyclically_reduce_after_moves=False, want_visited=False,
-              device=None, chunk_parents=0, max_bytes=DEFAULT_MAX_BYTES):
+              device=None, chunk_parents=0, max_bytes=DEFAULT_MAX_BYTES, goals=None, stop_at_trivial=True):
     """Breadth-first search of every row of ``presentations`` [S, 2*mrl] in one device run
     (csrc/mbfs.cu).  ``max_nodes_to_explore`` is one budget or one per row.
 
     Returns a list of ``(solved, path|None, info)``, element s equal to ``bfs_device(row s, ...)``.
     A row on which the reference raises carries ``info["status"] != 0`` instead of raising.  Rows
     are split into several engine runs when one engine would need more than ``max_bytes`` of device
-    memory; ``chunk_parents`` > 0 caps the parents expanded per chunk (the results do not depend on it)."""
+    memory; ``chunk_parents`` > 0 caps the parents expanded per chunk (the results do not depend on it).
+
+    ``goals`` (a ``GoalSet`` of the same max_relator_length and ``cyclically_reduce_after_moves``):
+    a search also stops at the first generated child that is in the set, tested right after the
+    length-2 test, and reports it as solved with ``info["goal"]`` = the entry index (``None`` for
+    rows that did not stop at a goal); the path then ends with (action, total length of the goal
+    state).  A root in the set stops at depth 0 with the path ``[(-1, L0)]``.  ``stop_at_trivial=False``
+    turns the length-2 rule off: searches run until a goal, their budget or exhaustion."""
     P8, budgets = _batch_inputs(presentations, max_nodes_to_explore)
+    dev = _lib.default_device() if device is None else device
+    _check_goals(goals, P8.shape[1] // 2, cyclically_reduce_after_moves, dev)
     if P8.shape[0] == 0:
         return []
     L = _lib.lib()
-    dev = _lib.default_device() if device is None else device
     out = []
     for lo, hi, _ in _split(L, P8.shape[1] // 2, budgets, chunk_parents, max_bytes):
-        e = _BatchEngine(L, dev, P8[lo:hi], budgets[lo:hi], cyclically_reduce_after_moves, chunk_parents)
+        e = _BatchEngine(L, dev, P8[lo:hi], budgets[lo:hi], cyclically_reduce_after_moves, chunk_parents, goals,
+                         stop_at_trivial)
         try:
             out += e.run(want_visited)
         finally:

@@ -1,0 +1,190 @@
+"""Goal sets for the batched breadth-first search (csrc/goalset.cu, csrc/mbfs.cu).
+
+A goal set is a device-resident set of states.  ``bfs_batch(..., goals=g)`` stops a search at the
+first generated child that is in ``g``.  Meet-in-the-middle uses it with a large ball of states
+around the trivial presentations (``trivial_ball``): a forward search that reaches the ball is
+trivialized by the forward path followed by the ball path walked backwards
+(``bfs_meet_in_the_middle``).
+"""
+
+from __future__ import annotations
+
+import ctypes as C
+
+import numpy as np
+
+from .. import _lib
+from ..envs.utils import generate_trivial_states, is_array_valid_presentation
+from .breadth_first import DEFAULT_MAX_BYTES, _BatchEngine, _batch_inputs, bfs_batch
+
+# the move that undoes each of the 12 moves when relators are only freely reduced (bfs_common.cuh, skip_moves):
+# r1 <- r1 r0^{+-1} (0, 2), r0 <- r0 r1^{-+1} (1, 3), and conjugation by g / g^-1 (4..7 <-> 8..11)
+INVERSE_MOVE = (2, 3, 0, 1, 8, 9, 10, 11, 4, 5, 6, 7)
+
+
+def _goal_rows(rows, cyclical):
+    """Validate goal rows on the host -> int8 rows.  A row must be a state a search can generate."""
+    R = np.asarray(rows)
+    if R.ndim != 2 or R.shape[1] % 2 or R.shape[1] == 0:
+        raise ValueError("goal rows must be [n, 2*max_relator_length]")
+    if R.size and np.abs(R.astype(np.int64)).max() > 2:
+        raise ValueError("the GPU search supports the two-generator alphabet {+-1, +-2} only")
+    mrl = R.shape[1] // 2
+    R8 = np.ascontiguousarray(R, dtype=np.int8)
+    for k in range(R8.shape[0]):
+        if not is_array_valid_presentation(R8[k]):
+            raise ValueError(f"goal row {k}: {R8[k].tolist()} is not a valid presentation "
+                             "(an empty relator, or zeros before letters)")
+        for h in range(2):
+            r = R8[k, h * mrl:(h + 1) * mrl]
+            r = r[: np.count_nonzero(r)].astype(np.int64)
+            if (r[:-1] == -r[1:]).any():
+                raise ValueError(f"goal row {k}: relator {h} is not freely reduced, so no search generates it")
+            if cyclical and r.size > 1 and r[0] == -r[-1]:
+                raise ValueError(f"goal row {k}: relator {h} is not cyclically reduced, so no search with "
+                                 "cyclically_reduce_after_moves=True generates it")
+    return R8
+
+
+class GoalSet:
+    """A set of states on one GPU, built with ``from_rows`` or ``explore``.  Entry ``i`` holds a state,
+    its parent entry and the move from it, and its root; a state held by several entries is represented
+    by the smallest entry index.  Free it with ``close()`` or a ``with`` block."""
+
+    def __init__(self, handle, max_relator_length, cyclical, device, results=None):
+        self.handle = handle
+        self.max_relator_length = int(max_relator_length)
+        self.cyclical = bool(cyclical)
+        self.device = int(device)
+        self.results = results  # explore: the (solved, path, info) of every root's search
+
+    @classmethod
+    def from_rows(cls, rows, cyclically_reduce_after_moves=False, device=None):
+        """Entries are the rows [n, 2*mrl], each its own root.  Rows must be freely reduced (and
+        cyclically reduced with ``cyclically_reduce_after_moves``): no search generates other rows."""
+        R8 = _goal_rows(rows, cyclically_reduce_after_moves)
+        L = _lib.lib()
+        dev = _lib.default_device() if device is None else device
+        h = C.c_void_p()
+        _lib.check(L.acs_goalset_from_rows(dev, R8.shape[1] // 2, int(bool(cyclically_reduce_after_moves)),
+                                           R8.ctypes.data, R8.shape[0], C.byref(h)))
+        return cls(h, R8.shape[1] // 2, cyclically_reduce_after_moves, dev)
+
+    @classmethod
+    def explore(cls, roots, max_nodes_to_explore, cyclically_reduce_after_moves=False, device=None, chunk_parents=0):
+        """Breadth-first search from every root with the length-2 rule off (each search runs until its
+        budget or exhaustion), in one engine; every visited state becomes an entry, in (root, visit order)
+        order.  ``results`` keeps each root's ``(solved, path, info)``."""
+        P8, budgets = _batch_inputs(roots, max_nodes_to_explore)
+        if P8.shape[0] == 0:
+            raise ValueError("explore needs at least one root")
+        L = _lib.lib()
+        dev = _lib.default_device() if device is None else device
+        e = _BatchEngine(L, dev, P8, budgets, cyclically_reduce_after_moves, chunk_parents, None, False)
+        try:
+            results = e.run(False)
+            h = C.c_void_p()
+            _lib.check(L.acs_goalset_from_bfs_batch(e.h, C.byref(h)))
+        finally:
+            e.destroy()
+        return cls(h, P8.shape[1] // 2, cyclically_reduce_after_moves, dev, results)
+
+    @property
+    def closed(self):
+        return not self.handle
+
+    def _size(self):
+        if self.closed:
+            raise ValueError("the goal set is closed")
+        n, s, b = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        _lib.check(_lib.lib().acs_goalset_size(self.handle, C.byref(n), C.byref(s), C.byref(b)))
+        return n.value, s.value, b.value
+
+    @property
+    def n_entries(self):
+        return self._size()[0]
+
+    @property
+    def n_states(self):
+        """Distinct states among the entries."""
+        return self._size()[1]
+
+    @property
+    def nbytes(self):
+        """Device bytes the set holds."""
+        return self._size()[2]
+
+    def path(self, entry):
+        """-> (root, path): the entry's root index and ``[(-1, L_root), (action, total_length), ...]`` from the
+        root's state to the entry's state."""
+        if self.closed:
+            raise ValueError("the goal set is closed")
+        L = _lib.lib()
+        root, n = C.c_int(0), C.c_int(0)
+        cap = 256
+        buf = np.zeros((cap, 2), np.int32)
+        rc = L.acs_goalset_path(self.handle, int(entry), C.byref(root), buf.ctypes.data, cap, C.byref(n))
+        if rc == _lib.ACS_ERR_INVALID and n.value > cap:
+            cap = n.value
+            buf = np.zeros((cap, 2), np.int32)
+            rc = L.acs_goalset_path(self.handle, int(entry), C.byref(root), buf.ctypes.data, cap, C.byref(n))
+        _lib.check(rc)
+        return int(root.value), [(int(a), int(l)) for a, l in buf[: n.value]]
+
+    def close(self):
+        if self.handle:
+            _lib.lib().acs_goalset_destroy(self.handle)
+            self.handle = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def trivial_ball(max_relator_length, max_nodes_to_explore, cyclically_reduce_after_moves=False, device=None,
+                 chunk_parents=0):
+    """``GoalSet.explore`` from the eight trivial presentations (<x^+-1, y^+-1> and <y^+-1, x^+-1>), each with
+    ``max_nodes_to_explore`` nodes: a ball of states from which a path to a trivial presentation is known."""
+    return GoalSet.explore(generate_trivial_states(max_relator_length), max_nodes_to_explore,
+                           cyclically_reduce_after_moves, device, chunk_parents)
+
+
+def bfs_meet_in_the_middle(presentations, max_nodes_to_explore, ball, device=None, chunk_parents=0,
+                           max_bytes=DEFAULT_MAX_BYTES):
+    """Meet-in-the-middle breadth-first search, without cyclic reduction: ``bfs_batch`` of every row with
+    ``ball`` (usually ``trivial_ball(...)``) as its goal set.
+
+    Returns a list of ``(trivialized, path|None, info)``.  ``path`` is in the reference's format and ends at
+    total length 2: a row solved directly keeps its ``bfs`` path; a row that reached the ball gets its
+    forward path followed by the ball path from the ball's root to the meeting state, walked backwards
+    with every move replaced by its inverse (``INVERSE_MOVE``).  Then ``info["goal"]`` is the entry met,
+    ``info["ball_root"]`` and ``info["ball_path"]`` its root and path in the ball.
+
+    Only for ``cyclically_reduce_after_moves=False``: with cyclic reduction a move is not undone by a
+    single move, so no such path exists.  There, ``bfs_batch(..., goals=ball)`` gives the forward path and
+    ``ball.path(info["goal"])`` the ball path, which together certify the meeting."""
+    if ball.cyclical:
+        raise ValueError("bfs_meet_in_the_middle needs a ball built with cyclically_reduce_after_moves=False: with "
+                         "cyclic reduction the ball path cannot be walked backwards; use bfs_batch(goals=...) and "
+                         "GoalSet.path")
+    res = bfs_batch(presentations, max_nodes_to_explore, False, device=device, chunk_parents=chunk_parents,
+                    max_bytes=max_bytes, goals=ball)
+    out = []
+    for solved, path, info in res:
+        if not solved or info["goal"] is None:
+            out.append((solved, path, info))
+            continue
+        root, bpath = ball.path(info["goal"])
+        back = [(INVERSE_MOVE[bpath[k][0]], bpath[k - 1][1]) for k in range(len(bpath) - 1, 0, -1)]
+        info["ball_root"], info["ball_path"] = root, bpath
+        full = path + back
+        out.append((full[-1][1] == 2, full, info))
+    return out

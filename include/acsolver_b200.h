@@ -220,6 +220,32 @@ int acs_bfs_batch_paths(acs_bfs_batch *b, int32_t *h_paths, int path_cap);
 int acs_bfs_batch_visited(acs_bfs_batch *b, int search, int8_t *h_out, int64_t cap_rows, int64_t *n_out);
 void acs_bfs_batch_destroy(acs_bfs_batch *b);
 
+/* Goal sets (csrc/goalset.cu): device-resident sets of states keyed by the state alone, for the goal
+ * test of the batched search.  An entry holds a state, a parent link and a root index; when a state
+ * occurs more than once the smallest entry index represents it.
+ * acs_goalset_from_rows: rows [n, 2*mrl] int8; each row must be a state a search can generate (both
+ * relators non-empty, right-padded, freely reduced, and cyclically reduced when cyclical), else
+ * ACS_ERR_INVALID before any device work.  Entry i is row i, its own root.
+ * acs_goalset_from_bfs_batch: every committed node of every search of b's last run, in (search, FIFO
+ * id) order; roots are search indices.  b's memory goes to the set or is freed: b can only be destroyed.
+ * acs_goalset_path: (-1, L_root), (action, total_length), ... from the entry's root to the entry; a
+ * path longer than path_cap is ACS_ERR_INVALID with *path_len the needed length. */
+typedef struct acs_goalset acs_goalset;
+int acs_goalset_from_rows(int device, int mrl, int cyclical, const int8_t *h_rows, int64_t n, acs_goalset **out);
+int acs_goalset_from_bfs_batch(acs_bfs_batch *b, acs_goalset **out);
+int acs_goalset_size(const acs_goalset *g, int64_t *n_entries, int64_t *n_states, int64_t *bytes);
+int acs_goalset_path(const acs_goalset *g, int64_t entry, int *root, int32_t *h_path, int path_cap, int *path_len);
+void acs_goalset_destroy(acs_goalset *g);
+/* Options of the next runs of b.  g (may be NULL; must outlive those runs): a search stops at the first
+ * generated child in g, tested after the length-2 test and before the visited test, exactly as a solve
+ * stops it (solved = 1; the path ends with (action, total length of the goal state)); a root in g is a
+ * hit at depth 0.  stop_at_trivial = 0 turns the length-2 rule off, so searches run until a goal,
+ * their budget or exhaustion.  g's mrl, cyclical flag and device must be b's.  With g NULL and
+ * stop_at_trivial = 1 the engine runs exactly as without this call.
+ * acs_bfs_batch_goal_hits: per search of the last run, the goal entry it stopped at, or -1. */
+int acs_bfs_batch_set_goals(acs_bfs_batch *b, const acs_goalset *g, int stop_at_trivial);
+int acs_bfs_batch_goal_hits(acs_bfs_batch *b, int64_t *h_entry /* [n_search] */);
+
 /* Batched greedy search (search/greedy.py:15-121): n_search independent presentations of the
  * same mrl, one warp each, one launch.  h_presentations [n_search, 2*mrl]; h_paths
  * [n_search, path_cap, 2] int32 (action, total_length) pairs; results [n_search].  On failure
