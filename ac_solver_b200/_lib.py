@@ -119,6 +119,8 @@ _SIGS = {
     "acs_greedy_run": (C.c_int, [_P, _P, _P, _P]),
     "acs_greedy_visited": (C.c_int, [_P, C.c_int, _P, C.c_int64, C.POINTER(C.c_int64)]),
     "acs_greedy_destroy": (None, [_P]),
+    "acs_greedy_set_goals": (C.c_int, [_P, _P]),
+    "acs_greedy_goal_hits": (C.c_int, [_P, _P]),
     "acs_sbfs_pack_root": (C.c_int, [_P, C.c_int, _P, _P, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "acs_sbfs_owner": (C.c_int, [C.c_uint64, C.c_int]),
     "acs_sbfs_expand": (C.c_int, [_P, C.c_int, _P]),

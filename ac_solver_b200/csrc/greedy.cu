@@ -34,6 +34,7 @@
 #include "ac_core.cuh"
 #include "ac_keys.cuh"
 #include "acs_internal.h"
+#include "goalset.cuh"
 
 namespace acs {
 
@@ -47,6 +48,7 @@ struct GreedyRec {  // per-search result record (device -> host)
     int32_t final_action, final_len;
     int32_t rounds, engine;  // bucket rounds executed; 1 = bucket kernel, 2 = heap kernel (fallback or forced)
     int32_t minlen_log[128];
+    int64_t goal;  // goal entry the search stopped at, or -1 (written by the goal instantiations only)
 };
 
 struct GreedyArgs {
@@ -94,18 +96,6 @@ __device__ __forceinline__ bool entry_less(uint64_t e1, const Key<W>& k1, uint64
 }
 
 template <int W>
-__device__ __forceinline__ Key<W> load_key_cg(const uint64_t* keys, uint64_t idx) {
-    Key<W> q;
-    const ulonglong2* p = reinterpret_cast<const ulonglong2*>(keys) + idx * W;
-#pragma unroll
-    for (int i = 0; i < W; ++i) {
-        const ulonglong2 v = __ldcg(p + i);
-        q.k[2 * i] = v.x;
-        q.k[2 * i + 1] = v.y;
-    }
-    return q;
-}
-template <int W>
 __device__ __forceinline__ Key<W> shfl_key(const Key<W>& k, int src) {
     Key<W> r;
 #pragma unroll
@@ -120,8 +110,11 @@ __device__ __forceinline__ Key<W> shfl_xor_key(const Key<W>& k, int off) {
     return r;
 }
 
-template <int W>
-__global__ void __launch_bounds__(32) greedy_kernel(const GreedyArgs A) {
+// GOAL: the goal test of DESIGN.md §K9 against G -- a root in the set is a hit at depth 0, and a generated
+// child in the set ends the search like a solving child, after the length-2 test (the solve wins on the same
+// child) and before the visited test
+template <int W, bool GOAL>
+__global__ void __launch_bounds__(32) greedy_kernel(const GreedyArgs A, const GoalView G) {
     const int sidx = blockIdx.x;
     if (sidx >= A.n_search) return;
     if (A.fallback_only && A.rec[sidx].status != 99) return;
@@ -153,8 +146,16 @@ __global__ void __launch_bounds__(32) greedy_kernel(const GreedyArgs A) {
     int solved = 0, status = 0, budget_hit = 0;
     uint64_t cur = 0;
     int final_action = 11, final_len = L0;
+    int64_t goal_entry = -1;
+    if constexpr (GOAL) {
+        goal_entry = goal_find<W>(G, root);
+        if (goal_entry >= 0) {  // path [(-1, L0)]: nothing expanded
+            solved = 1;
+            final_action = -1;
+        }
+    }
 
-    while (hn > 0) {
+    while (hn > 0 && !(GOAL && solved)) {
         // ================= pop the minimum =================
         const uint64_t top = __ldcg(&heap[0]);
         cur = top & 0xFFFFFFFFull;
@@ -213,9 +214,16 @@ __global__ void __launch_bounds__(32) greedy_kernel(const GreedyArgs A) {
         }
         const unsigned err_mask = __ballot_sync(kFull, lane < 12 && st != ST_OK);
         const unsigned sol_mask = __ballot_sync(kFull, lane < 12 && st == ST_OK && L == 2);
-        const int first_event = (err_mask | sol_mask) ? (__ffs(err_mask | sol_mask) - 1) : 12;
-        const bool ev_solved = first_event < 12 && ((sol_mask >> first_event) & 1u);
-        const bool ev_error = first_event < 12 && !ev_solved;
+        // every OK child is looked up: a visited or duplicate child is never the first goal, so the extra
+        // lookups cannot change the outcome
+        int64_t ge = -1;
+        if (GOAL && lane < 12 && st == ST_OK) ge = goal_find<W>(G, child);
+        const unsigned goal_mask = GOAL ? __ballot_sync(kFull, ge >= 0) : 0u;
+        const unsigned ev_mask = err_mask | sol_mask | goal_mask;
+        const int first_event = ev_mask ? (__ffs(ev_mask) - 1) : 12;
+        const bool ev_solved = first_event < 12 && ((sol_mask >> first_event) & 1u);  // the solve wins on the same child
+        const bool ev_goal = GOAL && first_event < 12 && !ev_solved && ((goal_mask >> first_event) & 1u);
+        const bool ev_error = first_event < 12 && !ev_solved && !ev_goal;
         // children the reference evaluates: actions 0..first_event (the raising one has no length)
         const int n_eval = ev_error ? first_event : min(first_event + 1, 12);
         n_moves += (uint64_t)min(first_event + 1, 12);
@@ -331,6 +339,13 @@ __global__ void __launch_bounds__(32) greedy_kernel(const GreedyArgs A) {
             final_len = 2;
             break;
         }
+        if (GOAL && ev_goal) {
+            solved = 1;
+            final_action = first_event;
+            final_len = __shfl_sync(kFull, L, first_event);
+            goal_entry = __shfl_sync(kFull, ge, first_event);
+            break;
+        }
         if (n_nodes >= A.budget) {  // greedy.py:115-119, after all 12 children
             budget_hit = 1;
             break;
@@ -350,6 +365,7 @@ __global__ void __launch_bounds__(32) greedy_kernel(const GreedyArgs A) {
         rec->final_len = final_len;
         rec->rounds = 0;
         rec->engine = 2;
+        if constexpr (GOAL) rec->goal = goal_entry;
     }
 }
 
@@ -357,7 +373,8 @@ __global__ void __launch_bounds__(32) greedy_kernel(const GreedyArgs A) {
 #include "greedy_bucket.cuh"
 namespace acs {
 
-// path of every search: chain of its final node, then (final_action, final_len)
+// path of every search: chain of its final node, then (final_action, final_len) -- nothing more when the
+// search stopped at its root (a root in the goal set, final_action -1)
 template <int W>
 __global__ void greedy_path_kernel(const GreedyArgs A, int32_t* paths, int path_cap, int32_t* path_len) {
     const int sidx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -371,7 +388,8 @@ __global__ void greedy_path_kernel(const GreedyArgs A, int32_t* paths, int path_
         ++d;
         if (parent[q] == kNone) break;
     }
-    path_len[sidx] = d + 1;
+    const bool at_root = rec.final_action < 0;
+    path_len[sidx] = d + (at_root ? 0 : 1);
     int pos = d - 1;
     for (uint64_t q = rec.final_node;; q = parent[q] >> 4, --pos) {
         const Key<W> k = load_key<W>(keys, q);
@@ -382,7 +400,7 @@ __global__ void greedy_path_kernel(const GreedyArgs A, int32_t* paths, int path_
         }
         if (root) break;
     }
-    if (d < path_cap) {
+    if (!at_root && d < path_cap) {
         path[2 * d] = rec.final_action;
         path[2 * d + 1] = rec.final_len;
     }
@@ -408,6 +426,8 @@ struct acs_greedy {
     std::vector<GreedyRec> h_rec;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    const acs_goalset* goals = nullptr;  // acs_greedy_set_goals
+    bool ran = false, ran_with_goals = false;
 };
 
 #define GR_CUDA(call)                                                                   \
@@ -526,7 +546,7 @@ extern "C" int acs_greedy_create(int device, int n_search, int mrl, int64_t max_
 
 namespace {
 
-template <int W>
+template <int W, bool GOAL>
 int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_search_result* res) {
     GR_CUDA(cudaSetDevice(g->device));
     const int S = g->n_search;
@@ -571,16 +591,20 @@ int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_s
     A.mrl = g->mrl;
     A.cyclical = g->cyclical;
     A.fallback_only = 0;
+    const GoalView G = GOAL ? g->goals->view() : GoalView{nullptr, nullptr, 0};
     GR_CUDA(cudaEventRecord(g->ev0, st));
     g->n_fallback = 0;
     if (g->use_bucket) {
         // pass 1: small bucket directory (several CTAs per SM); pass 2: the searches that outgrew it, with a
         // large directory (one CTA per SM); whatever still does not fit is re-run by the heap kernel
-        auto smem_for = [](int buckets) { return ((sizeof(GbShared) + 15) / 16) * 16 + (size_t)buckets * sizeof(GbBucket); };
-        GR_CUDA(cudaFuncSetAttribute(greedy_bucket_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        // with goals, the goal slot follows the bucket directory
+        auto smem_for = [](int buckets) {
+            return ((sizeof(GbShared) + 15) / 16) * 16 + (size_t)buckets * sizeof(GbBucket) + (GOAL ? kGbGoalSmem : 0);
+        };
+        GR_CUDA(cudaFuncSetAttribute(greedy_bucket_kernel<W, GOAL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)smem_for(kGbBuckets2)));
         // several CTAs per SM in pass 1: ask for the largest shared-memory carve-out
-        GR_CUDA(cudaFuncSetAttribute(greedy_bucket_kernel<W>, cudaFuncAttributePreferredSharedMemoryCarveout,
+        GR_CUDA(cudaFuncSetAttribute(greedy_bucket_kernel<W, GOAL>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                      (int)cudaSharedmemCarveoutMaxShared));
         const bool debug = std::getenv("ACS_GREEDY_DEBUG") != nullptr;
         for (int pass = 0; pass < 2; ++pass) {
@@ -588,7 +612,7 @@ int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_s
             g->gb.retry_only = pass;
             cudaEvent_t e0 = pass == 0 ? g->ev0 : g->ev1;
             if (pass) GR_CUDA(cudaEventRecord(e0, st));
-            greedy_bucket_kernel<W><<<S, kGbThreads, smem_for(g->gb.max_buckets), st>>>(A, g->gb);
+            greedy_bucket_kernel<W, GOAL><<<S, kGbThreads, smem_for(g->gb.max_buckets), st>>>(A, g->gb, G);
             GR_CUDA(cudaGetLastError());
             GR_CUDA(cudaMemcpyAsync(g->h_rec.data(), g->rec, (size_t)S * sizeof(GreedyRec), cudaMemcpyDeviceToHost, st));
             GR_CUDA(cudaStreamSynchronize(st));
@@ -606,11 +630,11 @@ int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_s
         }
         if (g->n_fallback) {
             A.fallback_only = 1;
-            greedy_kernel<W><<<S, 32, 0, st>>>(A);
+            greedy_kernel<W, GOAL><<<S, 32, 0, st>>>(A, G);
             GR_CUDA(cudaGetLastError());
         }
     } else {
-        greedy_kernel<W><<<S, 32, 0, st>>>(A);
+        greedy_kernel<W, GOAL><<<S, 32, 0, st>>>(A, G);
         GR_CUDA(cudaGetLastError());
     }
     greedy_path_kernel<W><<<(S + 63) / 64, 64, 0, st>>>(A, g->d_paths, g->path_cap, g->d_path_len);
@@ -625,6 +649,8 @@ int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_s
     GR_CUDA(cudaStreamSynchronize(st));
     float ms = 0.f;
     cudaEventElapsedTime(&ms, g->ev0, g->ev1);
+    g->ran = true;
+    g->ran_with_goals = GOAL;
     for (int s = 0; s < S; ++s) {
         const GreedyRec& r = g->h_rec[s];
         acs_search_result& o = res[s];
@@ -667,12 +693,44 @@ int greedy_visited_impl(acs_greedy* g, int search, int8_t* h_out, int64_t cap_ro
 extern "C" int acs_greedy_run(acs_greedy* g, const int8_t* h_presentations, int32_t* h_paths,
                               acs_search_result* results) {
     if (!g || !h_presentations || !results) return ACS_ERR_INVALID;
-    return g->W == 1 ? greedy_run_impl<1>(g, h_presentations, h_paths, results)
-                     : greedy_run_impl<2>(g, h_presentations, h_paths, results);
+    if (g->goals)
+        return g->W == 1 ? greedy_run_impl<1, true>(g, h_presentations, h_paths, results)
+                         : greedy_run_impl<2, true>(g, h_presentations, h_paths, results);
+    return g->W == 1 ? greedy_run_impl<1, false>(g, h_presentations, h_paths, results)
+                     : greedy_run_impl<2, false>(g, h_presentations, h_paths, results);
 }
 
 extern "C" int acs_greedy_visited(acs_greedy* g, int search, int8_t* h_out, int64_t cap_rows, int64_t* n_out) {
     if (!g || search < 0 || search >= g->n_search || (!h_out && cap_rows > 0)) return ACS_ERR_INVALID;
     return g->W == 1 ? greedy_visited_impl<1>(g, search, h_out, cap_rows, n_out)
                      : greedy_visited_impl<2>(g, search, h_out, cap_rows, n_out);
+}
+
+extern "C" int acs_greedy_set_goals(acs_greedy* g, const acs_goalset* gs) {
+    if (!g) return ACS_ERR_INVALID;
+    if (gs) {
+        auto fail = [](const char* m) {
+            acs::set_last_error(m);
+            return ACS_ERR_INVALID;
+        };
+        if (gs->mrl != g->mrl) return fail("greedy_set_goals: the goal set's max_relator_length differs from the engine's");
+        if (gs->cyclical != g->cyclical) return fail("greedy_set_goals: the goal set's cyclical flag differs from the engine's");
+        if (gs->device != g->device) return fail("greedy_set_goals: the goal set lives on another device");
+        if (gs->n_entries >= (int64_t)0xFFFFFFFF) {  // the bucket kernel packs a hit's entry into 32 bits beside its candidate
+            acs::set_last_error("greedy_set_goals: goal sets of 2^32 - 1 entries or more are not supported");
+            return ACS_ERR_UNSUPPORTED;
+        }
+    }
+    g->goals = gs;
+    return ACS_OK;
+}
+
+extern "C" int acs_greedy_goal_hits(acs_greedy* g, int64_t* h_entry) {
+    if (!g || !h_entry) return ACS_ERR_INVALID;
+    if (!g->ran) {
+        acs::set_last_error("greedy: no completed run");
+        return ACS_ERR_INVALID;
+    }
+    for (int s = 0; s < g->n_search; ++s) h_entry[s] = g->ran_with_goals ? g->h_rec[s].goal : -1;
+    return ACS_OK;
 }

@@ -27,6 +27,7 @@
 
 #include "ac_core.cuh"
 #include "ac_keys.cuh"
+#include "goalset.cuh"
 
 namespace acs {
 
@@ -83,7 +84,7 @@ struct GbShared {
     uint32_t cur_key, cur_n;
     int fallback;
 };
-enum : uint32_t { GB_CONT = 0, GB_INTERRUPT = 1, GB_BUDGET = 2, GB_SOLVED = 3, GB_ERROR = 4 };
+enum : uint32_t { GB_CONT = 0, GB_INTERRUPT = 1, GB_BUDGET = 2, GB_SOLVED = 3, GB_ERROR = 4, GB_GOAL = 5 };
 
 template <int W>
 __device__ __forceinline__ uint64_t* gb_rec(uint64_t* sortbuf, uint32_t i) {
@@ -143,12 +144,19 @@ __device__ __forceinline__ int gb_find(const GbBucket* B, int nb, uint32_t key) 
     return lo;
 }
 
-template <int W>
+// GOAL: the goal test of DESIGN.md §K9 against G.  A winner of the per-tile dedup that is in the set takes
+// the minimum of (candidate << 32 | entry) in one more shared-memory word, placed after the bucket
+// directory (the launch adds kGbGoalSmem bytes), and phase C resolves it like a solving child.  Only
+// winners are looked up: a visited child was tested when it was first generated (the root at start), and a
+// child that lost its slot follows a smaller candidate id of the same state.
+constexpr int kGbGoalSmem = 16;
+template <int W, bool GOAL>
 #ifndef GB_MIN_BLOCKS
 #define GB_MIN_BLOCKS 5  // resident CTAs per SM the register allocation must allow: 48 registers, 5 x 42 KB of shared memory
                          // -> 740 searches in flight on 148 SMs (the 657 unsolved rows of config 3 run as one wave)
 #endif
-__global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS) greedy_bucket_kernel(const GreedyArgs A, const GbArgs X) {
+__global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS)
+    greedy_bucket_kernel(const GreedyArgs A, const GbArgs X, const GoalView G) {
     extern __shared__ __align__(16) unsigned char gb_smem_raw[];
     GbShared& sh = *reinterpret_cast<GbShared*>(gb_smem_raw);
     GbBucket* B = reinterpret_cast<GbBucket*>(gb_smem_raw + ((sizeof(GbShared) + 15) / 16) * 16);
@@ -198,6 +206,22 @@ __global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS) greedy_bucket_kerne
     int final_action = 11, final_len = L0;
     bool finished = false;
     int rounds = 0;
+    // with goals: the goal slot holds the winning (candidate << 32 | entry) of the current tile; after a hit
+    // nothing resets it, and sh.stop says GB_GOAL (so no register carries the entry through the rounds)
+    if constexpr (GOAL) {  // a root in the set: path [(-1, L0)], nothing expanded
+        unsigned long long& goal_slot = *reinterpret_cast<unsigned long long*>(B + X.max_buckets);
+        if (tid == 0) {
+            const int64_t e = goal_find<W>(G, root);
+            goal_slot = e < 0 ? ~0ull : (unsigned long long)e;
+            sh.stop = e < 0 ? GB_CONT : GB_GOAL;
+        }
+        __syncthreads();
+        if (goal_slot != ~0ull) {
+            solved = 1;
+            final_action = -1;
+            finished = true;
+        }
+    }
 
     while (!finished) {
         if (sh.nb == 0 || sh.fallback) break;
@@ -319,6 +343,7 @@ __global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS) greedy_bucket_kerne
                 sh.sol_c = kGbNone;
                 sh.err_c = kGbNone;
                 sh.tstar_c = kGbNone;
+                if constexpr (GOAL) *reinterpret_cast<unsigned long long*>(B + X.max_buckets) = ~0ull;
             }
             __syncthreads();
             // ---- A1: expand: candidate keys, lengths, events ----
@@ -396,6 +421,12 @@ __global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS) greedy_bucket_kerne
                 if ((uint32_t)__ldcg(&round_tab[slot]) == c + 1) {
                     atomicOr(&sh.bitmap[c >> 5], 1u << (c & 31));
                     if ((int)(cand_meta[c] & 0xFF) < Lcur) atomicMin(&sh.tstar_c, c);
+                    if constexpr (GOAL) {
+                        const int64_t e = goal_find<W>(G, load_key<W>(cand_key, c));
+                        if (e >= 0)
+                            atomicMin(reinterpret_cast<unsigned long long*>(B + X.max_buckets),
+                                      ((unsigned long long)c << 32) | (unsigned long long)e);
+                    }
                 }
             }
             __syncthreads();
@@ -450,18 +481,26 @@ __global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS) greedy_bucket_kerne
                     limit = ec;
                     st2 = GB_ERROR;
                 }
+                if constexpr (GOAL) {  // before every other event; on the solving child itself the solve wins
+                    const uint32_t gc = (uint32_t)(*reinterpret_cast<unsigned long long*>(B + X.max_buckets) >> 32);
+                    if (gc < limit) {  // kGbNone when no winner is a goal
+                        limit = gc;
+                        st2 = GB_GOAL;
+                    }
+                }
                 sh.limit = limit;
                 sh.stop = st2;
                 sh.n_commit = gb_rank(sh, limit);
-                sh.processed = (st2 == GB_SOLVED || st2 == GB_ERROR) ? limit / 12 + 1 : limit / 12;
+                sh.processed = (st2 == GB_SOLVED || st2 == GB_ERROR || (GOAL && st2 == GB_GOAL)) ? limit / 12 + 1 : limit / 12;
             }
             __syncthreads();
             const uint32_t limit = sh.limit;
             stop = sh.stop;
             const uint32_t processed = sh.processed;
+            const bool goal_hit = GOAL && stop == GB_GOAL;
             // "New minimal length found" events in candidate order (greedy.py:82-85); replicated in every thread
             {
-                const uint32_t gl = limit + (stop == GB_SOLVED ? 1u : 0u);
+                const uint32_t gl = limit + (stop == GB_SOLVED || goal_hit ? 1u : 0u);
                 for (;;) {
                     uint32_t best = kGbNone;
                     int bestL = -1;
@@ -543,16 +582,21 @@ __global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS) greedy_bucket_kerne
             // ---- counters (replicated) ----
             n_nodes += sh.n_commit;
             n_expanded += processed;
-            n_moves += (stop == GB_SOLVED || stop == GB_ERROR) ? (uint64_t)limit + 1 : (uint64_t)limit;
+            n_moves += (stop == GB_SOLVED || stop == GB_ERROR || goal_hit) ? (uint64_t)limit + 1 : (uint64_t)limit;
             if (processed > 0) {
                 cur = (uint32_t)sortbuf[(size_t)(tile0 + processed - 1) * RS + 2 * W];
-                if (stop != GB_SOLVED && stop != GB_ERROR) final_len = (int)(cand_meta[(processed - 1) * 12 + 11] & 0xFF);
+                if (stop != GB_SOLVED && stop != GB_ERROR && !goal_hit)
+                    final_len = (int)(cand_meta[(processed - 1) * 12 + 11] & 0xFF);
             }
             done_nodes = tile0 + processed;
             if (stop == GB_SOLVED) {
                 solved = 1;
                 final_action = (int)(limit % 12);
                 final_len = 2;
+            } else if (goal_hit) {
+                solved = 1;
+                final_action = (int)(limit % 12);
+                final_len = (int)(cand_meta[limit] & 0xFF);
             } else if (stop == GB_ERROR) {
                 status = (int)(sh.err_c & 3);
             } else if (stop == GB_BUDGET) {
@@ -561,7 +605,7 @@ __global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS) greedy_bucket_kerne
             __syncthreads();
         }
         if (sh.fallback) break;
-        if (stop == GB_SOLVED || stop == GB_ERROR || stop == GB_BUDGET) {
+        if (stop == GB_SOLVED || stop == GB_ERROR || stop == GB_BUDGET || (GOAL && stop == GB_GOAL)) {
             cur_rest = n - done_nodes;  // still in the reference's heap
             finished = true;
             break;
@@ -608,6 +652,10 @@ __global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS) greedy_bucket_kerne
         rec->final_len = final_len;
         rec->rounds = sh.fallback ? -sh.fallback : rounds;
         rec->engine = 1;
+        if constexpr (GOAL)  // -1 for a search handed back: it had not stopped
+            rec->goal = solved && sh.stop == GB_GOAL
+                            ? (int64_t)(*reinterpret_cast<unsigned long long*>(B + X.max_buckets) & 0xFFFFFFFFull)
+                            : -1;
     }
 }
 

@@ -1,10 +1,11 @@
-"""Goal sets for the batched breadth-first search (csrc/goalset.cu, csrc/mbfs.cu).
+"""Goal sets for the batched breadth-first and greedy searches (csrc/goalset.cu, csrc/mbfs.cu, csrc/greedy.cu).
 
 A goal set is a device-resident set of states.  ``bfs_batch(..., goals=g)`` stops a search at the
 first generated child that is in ``g``.  Meet-in-the-middle uses it with a large ball of states
 around the trivial presentations (``trivial_ball``): a forward search that reaches the ball is
 trivialized by the forward path followed by the ball path walked backwards
-(``bfs_meet_in_the_middle``).
+(``bfs_meet_in_the_middle``, ``greedy_meet_in_the_middle``).  ``greedy_search_batch(..., goals=g)``
+runs the same goal test in the greedy engine (csrc/greedy.cu).
 """
 
 from __future__ import annotations
@@ -157,6 +158,30 @@ def trivial_ball(max_relator_length, max_nodes_to_explore, cyclically_reduce_aft
                            cyclically_reduce_after_moves, device, chunk_parents)
 
 
+def _stitch_through_ball(results, ball):
+    """Meet-in-the-middle paths: every row that stopped at a ball entry gets its forward path followed by
+    the entry's ball path walked backwards, each move replaced by its inverse -> ``(trivialized, path,
+    info)`` with ``info["ball_root"]`` and ``info["ball_path"]``.  Other rows are kept as they are."""
+    out = []
+    for solved, path, info in results:
+        if not solved or info["goal"] is None:
+            out.append((solved, path, info))
+            continue
+        root, bpath = ball.path(info["goal"])
+        back = [(INVERSE_MOVE[bpath[k][0]], bpath[k - 1][1]) for k in range(len(bpath) - 1, 0, -1)]
+        info["ball_root"], info["ball_path"] = root, bpath
+        full = path + back
+        out.append((full[-1][1] == 2, full, info))
+    return out
+
+
+def _check_ball(ball, name, search):
+    if ball.cyclical:
+        raise ValueError(f"{name} needs a ball built with cyclically_reduce_after_moves=False: with "
+                         f"cyclic reduction the ball path cannot be walked backwards; use {search}(goals=...) and "
+                         "GoalSet.path")
+
+
 def bfs_meet_in_the_middle(presentations, max_nodes_to_explore, ball, device=None, chunk_parents=0,
                            max_bytes=DEFAULT_MAX_BYTES):
     """Meet-in-the-middle breadth-first search, without cyclic reduction: ``bfs_batch`` of every row with
@@ -171,20 +196,23 @@ def bfs_meet_in_the_middle(presentations, max_nodes_to_explore, ball, device=Non
     Only for ``cyclically_reduce_after_moves=False``: with cyclic reduction a move is not undone by a
     single move, so no such path exists.  There, ``bfs_batch(..., goals=ball)`` gives the forward path and
     ``ball.path(info["goal"])`` the ball path, which together certify the meeting."""
-    if ball.cyclical:
-        raise ValueError("bfs_meet_in_the_middle needs a ball built with cyclically_reduce_after_moves=False: with "
-                         "cyclic reduction the ball path cannot be walked backwards; use bfs_batch(goals=...) and "
-                         "GoalSet.path")
+    _check_ball(ball, "bfs_meet_in_the_middle", "bfs_batch")
     res = bfs_batch(presentations, max_nodes_to_explore, False, device=device, chunk_parents=chunk_parents,
                     max_bytes=max_bytes, goals=ball)
-    out = []
-    for solved, path, info in res:
-        if not solved or info["goal"] is None:
-            out.append((solved, path, info))
-            continue
-        root, bpath = ball.path(info["goal"])
-        back = [(INVERSE_MOVE[bpath[k][0]], bpath[k - 1][1]) for k in range(len(bpath) - 1, 0, -1)]
-        info["ball_root"], info["ball_path"] = root, bpath
-        full = path + back
-        out.append((full[-1][1] == 2, full, info))
-    return out
+    return _stitch_through_ball(res, ball)
+
+
+def greedy_meet_in_the_middle(presentations, max_nodes_to_explore, ball, device=None):
+    """Meet-in-the-middle greedy search, without cyclic reduction: ``greedy_search_batch`` of every row
+    with ``ball`` (usually ``trivial_ball(...)``) as its goal set.
+
+    Returns a list of ``(trivialized, path, info)``, stitched as in ``bfs_meet_in_the_middle``: a row
+    solved directly keeps its greedy path, a row that reached the ball gets its forward path followed by
+    the reversed ball path, and a row that did neither keeps greedy's failure path.  Every row plain
+    greedy search solves is trivialized: a search with goals follows the plain search until its first
+    goal, and every ball state has a path to a trivial presentation."""
+    from .greedy import greedy_search_batch
+
+    _check_ball(ball, "greedy_meet_in_the_middle", "greedy_search_batch")
+    res = greedy_search_batch(presentations, max_nodes_to_explore, False, device=device, goals=ball)
+    return _stitch_through_ball(res, ball)

@@ -11,16 +11,24 @@ import ctypes as C
 import numpy as np
 
 from .. import _lib
-from .breadth_first import _raise_for
+from .breadth_first import _check_goals, _raise_for
 
 
 def greedy_search_batch(presentations, max_nodes_to_explore=10000, cyclically_reduce_after_moves=False,
-                        want_visited=False, device=None, path_cap=None):
+                        want_visited=False, device=None, path_cap=None, goals=None):
     """Run greedy search on every row of ``presentations`` [S, 2*mrl] (same mrl) concurrently.
 
     Returns a list of ``(solved, path, info)`` per row, each identical to what the reference's
     ``greedy_search`` returns for that row (``path`` is the reference's failure path when not
-    solved).  Rows whose first move raises in the reference carry ``info["status"] != 0``."""
+    solved).  Rows whose first move raises in the reference carry ``info["status"] != 0``.
+
+    ``goals`` (a ``GoalSet`` of the same max_relator_length and ``cyclically_reduce_after_moves``):
+    a search also stops at the first generated child that is in the set, tested right after the
+    length-2 test (the solve wins on the same child) and before the visited test.  It reports the
+    row as solved with ``info["goal"]`` = the entry index (``None`` for rows that did not stop at a
+    goal), and the path ends with (action, total length of the goal state).  A root in the set
+    stops at depth 0 with the path ``[(-1, L0)]``.  Up to its first goal, a search follows the
+    plain search exactly."""
     L = _lib.lib()
     dev = _lib.default_device() if device is None else device
     P = np.asarray(presentations)
@@ -31,6 +39,7 @@ def greedy_search_batch(presentations, max_nodes_to_explore=10000, cyclically_re
     P8 = np.ascontiguousarray(P, dtype=np.int8)
     S, w = P8.shape
     mrl = w // 2
+    _check_goals(goals, mrl, cyclically_reduce_after_moves, dev)
     budget = int(max_nodes_to_explore)
     if path_cap is None:
         path_cap = int(min(budget + 4, 1 << 14))
@@ -40,9 +49,15 @@ def greedy_search_batch(presentations, max_nodes_to_explore=10000, cyclically_re
                                    C.byref(h)))
     out = []
     try:
+        if goals is not None:
+            _lib.check(L.acs_greedy_set_goals(h, goals.handle))
         paths = np.zeros((S, path_cap, 2), np.int32)
         res = (_lib.SearchResult * S)()
         _lib.check(L.acs_greedy_run(h, P8.ctypes.data, paths.ctypes.data, res))
+        hits = None
+        if goals is not None:
+            hits = np.full(S, -1, np.int64)
+            _lib.check(L.acs_greedy_goal_hits(h, hits.ctypes.data))
         for s in range(S):
             r = res[s]
             info = {
@@ -53,11 +68,13 @@ def greedy_search_batch(presentations, max_nodes_to_explore=10000, cyclically_re
                 # bucket rounds of the CTA-per-search kernel; -1: served by the one-warp heap kernel
                 "rounds": int(r.n_levels),
             }
+            if hits is not None:
+                info["goal"] = int(hits[s]) if hits[s] >= 0 else None
             if r.path_len > path_cap:  # deeper than the buffer: the reference has no limit -- run again with room
                 L.acs_greedy_destroy(h)
                 h = None
                 return greedy_search_batch(presentations, max_nodes_to_explore, cyclically_reduce_after_moves, want_visited,
-                                           device, path_cap=int(max(res[i].path_len for i in range(S))) + 4)
+                                           device, path_cap=int(max(res[i].path_len for i in range(S))) + 4, goals=goals)
             if want_visited and r.status == 0:
                 vis = np.zeros((max(int(r.n_visited), 1), w), np.int8)
                 n_out = C.c_int64(0)

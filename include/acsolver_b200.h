@@ -257,6 +257,14 @@ int acs_greedy_create(int device, int n_search, int mrl, int64_t max_nodes, int 
 int acs_greedy_run(acs_greedy *g, const int8_t *h_presentations, int32_t *h_paths, acs_search_result *results);
 int acs_greedy_visited(acs_greedy *g, int search, int8_t *h_out, int64_t cap_rows, int64_t *n_out);
 void acs_greedy_destroy(acs_greedy *g);
+/* Goal set of the next runs of g (may be NULL; must outlive those runs): a search stops at the first
+ * generated child in gs, tested after the length-2 test and before the visited test, exactly as a solve
+ * stops it (solved = 1; the path ends with (action, total length of the goal state); the solve wins on
+ * the same child); a root in gs is a hit at depth 0 with the path [(-1, L0)].  gs's mrl, cyclical flag
+ * and device must be g's, else ACS_ERR_INVALID.  NULL restores the plain engine exactly.
+ * acs_greedy_goal_hits: per search of the last run, the goal entry it stopped at, or -1. */
+int acs_greedy_set_goals(acs_greedy *g, const acs_goalset *gs);
+int acs_greedy_goal_hits(acs_greedy *g, int64_t *h_entry /* [n_search] */);
 
 /* ---- hash-partitioned multi-GPU BFS: per-rank device kernels --------------------------------- */
 /* The host loop (ac_solver_b200/search/sharded.py, one process per GPU, torch.distributed/NCCL
