@@ -31,18 +31,50 @@
 
 namespace acs {
 
+// The capacities can be lowered at compile time (-DGB_TILE=64 ...), so that tests reach multi-tile
+// buckets, the bitonic sort and every hand-back at budgets a CPU reference finishes quickly.
+#ifndef GB_TILE
+#define GB_TILE 1024
+#endif
+#ifndef GB_SMALL
+#define GB_SMALL 256
+#endif
+#ifndef GB_BUCKETS1
+#define GB_BUCKETS1 2048
+#endif
+#ifndef GB_BUCKETS2
+#define GB_BUCKETS2 12288
+#endif
+#ifndef GB_MAX_SEG
+#define GB_MAX_SEG 512
+#endif
+#ifndef GB_SEG_POOL
+#define GB_SEG_POOL (1 << 16)
+#endif
+#ifndef GB_SORT_CAP
+#define GB_SORT_CAP (1 << 16)
+#endif
 constexpr int kGbThreads = 256;
-constexpr int kGbTile = 1024;             // nodes per tile
+constexpr int kGbTile = GB_TILE;          // nodes per tile
 constexpr int kGbCand = kGbTile * 12;     // candidates per tile
 constexpr int kGbRoundSlots = 32768;      // per-round dedup table (power of two, > 2 * kGbCand)
-constexpr int kGbBuckets1 = 2048;         // open (length, depth) buckets per search: first pass ...
-constexpr int kGbBuckets2 = 12288;        // ... and for the searches that outgrow it (one CTA per SM)
-constexpr int kGbMaxSeg = 512;            // segments gathered per bucket
-constexpr int kGbSegPool = 1 << 16;       // segment records per search
-constexpr int kGbSortCap = 1 << 16;       // nodes per bucket that can be sorted
-constexpr int kGbSmall = 256;             // buckets up to this size are ranked in shared memory
+constexpr int kGbBuckets1 = GB_BUCKETS1;  // open (length, depth) buckets per search: first pass ...
+constexpr int kGbBuckets2 = GB_BUCKETS2;  // ... and for the searches that outgrow it (one CTA per SM)
+constexpr int kGbMaxSeg = GB_MAX_SEG;     // segments gathered per bucket
+constexpr int kGbSegPool = GB_SEG_POOL;   // segment records per search
+constexpr int kGbSortCap = GB_SORT_CAP;   // nodes per bucket that can be sorted
+constexpr int kGbSmall = GB_SMALL;        // buckets up to this size are ranked in shared memory
 constexpr int kGbFallback = 99;           // internal status: re-run with the heap kernel
 constexpr uint32_t kGbNone = 0xFFFFFFFFu;
+// the dedup probe wraps with a mask and stays below half full
+static_assert((kGbRoundSlots & (kGbRoundSlots - 1)) == 0 && kGbRoundSlots > 2 * kGbCand, "round table");
+// the candidate bitmap has whole words, and its prefix scan takes at most 2 words per thread
+static_assert(kGbTile > 0 && kGbCand % 32 == 0 && kGbCand / 32 <= 2 * kGbThreads, "tile size");
+// the bitonic network pads a bucket to np2 <= kGbSortCap records
+static_assert(kGbSortCap > 0 && (kGbSortCap & (kGbSortCap - 1)) == 0, "sort capacity");
+// all-pairs ranking: thread t places record t
+static_assert(kGbSmall >= 1 && kGbSmall <= kGbThreads, "all-pairs ranking");
+static_assert(kGbMaxSeg >= 1 && kGbSegPool >= 1, "segments");
 
 struct GbBucket {
     uint32_t key;       // length << 24 | depth
@@ -150,6 +182,11 @@ __device__ __forceinline__ int gb_find(const GbBucket* B, int nb, uint32_t key) 
 // winners are looked up: a visited child was tested when it was first generated (the root at start), and a
 // child that lost its slot follows a smaller candidate id of the same state.
 constexpr int kGbGoalSmem = 16;
+// both passes launch with the dynamic shared memory the host sets for kGbBuckets2 (greedy_run_impl), within the
+// 227 KB a block may opt in to; the root's bucket needs one directory entry
+static_assert(kGbBuckets1 >= 1 && kGbBuckets1 <= kGbBuckets2, "bucket directories");
+static_assert(((sizeof(GbShared) + 15) / 16) * 16 + (size_t)kGbBuckets2 * sizeof(GbBucket) + kGbGoalSmem <= 227 * 1024,
+              "the large bucket directory exceeds the shared memory of a block");
 template <int W, bool GOAL>
 #ifndef GB_MIN_BLOCKS
 #define GB_MIN_BLOCKS 5  // resident CTAs per SM the register allocation must allow: 48 registers, 5 x 42 KB of shared memory
