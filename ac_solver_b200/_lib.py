@@ -110,6 +110,14 @@ _SIGS = {
     "acs_bfs_batch_destroy": (None, [_P]),
     "acs_bfs_batch_set_goals": (C.c_int, [_P, _P, C.c_int]),
     "acs_bfs_batch_goal_hits": (C.c_int, [_P, _P]),
+    "acs_canonical_form": (C.c_int, [C.c_int, C.c_int, _P, C.c_int64, _P, _P]),
+    "acs_bfs_batch_set_symmetric": (C.c_int, [_P, C.c_int]),
+    "acs_bfs_batch_goal_hit_elements": (C.c_int, [_P, _P]),
+    "acs_goalset_from_rows_symmetric": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, C.c_int64, C.POINTER(_P)]),
+    "acs_goalset_is_symmetric": (C.c_int, [_P, C.POINTER(C.c_int)]),
+    "acs_goalset_path_frame": (C.c_int, [_P, C.c_int64, C.POINTER(C.c_int), _P, C.c_int, C.POINTER(C.c_int),
+                                         C.POINTER(C.c_int)]),
+    "acs_greedy_goal_hit_elements": (C.c_int, [_P, _P]),
     "acs_goalset_from_rows": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, C.c_int64, C.POINTER(_P)]),
     "acs_goalset_from_bfs_batch": (C.c_int, [_P, C.POINTER(_P)]),
     "acs_goalset_size": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),

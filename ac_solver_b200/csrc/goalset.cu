@@ -69,26 +69,34 @@ __global__ void __launch_bounds__(256) gs_count_kernel(const uint64_t* table, ui
     if (threadIdx.x == 0 && sum) atomicAdd(count, sum);
 }
 
-// path of one entry from its root: (-1, L_root), (action, L), ...; out[0] = length, out[1] = root
+// path of one entry from its root: (-1, L_root), (action, L), ...; out[0] = length, out[1] = root, out[2] = the
+// frame H of the path's end: end state = H.(stored state).  In a symmetric set entry j stores c_j = g_j.(the state
+// its move made from c_j-1), the actual states are a_j = h_j.c_j with h_0 = g_0^-1 and h_j = h_j-1.g_j^-1, so
+// h_j = (g_j ... g_0)^-1, and the actual move into node j is pi_{h_j-1}(m_j) with h_j-1 = P^-1.(g_k ... g_j),
+// P = g_k ... g_0: one pass for P, one pass back from the entry accumulating g_k ... g_j.
 template <int W>
 __global__ void gs_path_kernel(const uint64_t* nodes, int64_t entry, int32_t* path, int path_cap, int32_t* out) {
     int depth = 0;
     int64_t root = 0;
+    int P = 0;
     for (int64_t e = entry; e >= 0; ++depth) {
         Key<W> k;
         int64_t pl;
         node_load<W>(nodes, (uint64_t)e, k, pl, root);
+        P = sym_mul(P, (int)((uint64_t)root >> 32) & 15);
         e = pl < 0 ? -1 : (pl >> 4);
     }
     out[0] = depth;
-    out[1] = (int32_t)root;
-    int pos = depth - 1;
+    out[1] = (int32_t)(root & 0xFFFFFFFFll);
+    out[2] = sym_inv(P);
+    int pos = depth - 1, Q = 0;
     for (int64_t e = entry; e >= 0; --pos) {
         Key<W> k;
         int64_t pl, r;
         node_load<W>(nodes, (uint64_t)e, k, pl, r);
+        Q = sym_mul(Q, (int)((uint64_t)r >> 32) & 15);
         if (pos < path_cap) {
-            path[2 * pos] = pl < 0 ? -1 : (int32_t)(pl & 15);
+            path[2 * pos] = pl < 0 ? -1 : sym_pi(sym_mul(sym_inv(P), Q), (int)(pl & 15));
             path[2 * pos + 1] = (int32_t)(k.k[W - 1] >> 58) + (int32_t)(k.k[2 * W - 1] >> 58);
         }
         e = pl < 0 ? -1 : (pl >> 4);
@@ -179,17 +187,19 @@ std::string gs_row_problem(const int8_t* p, int mrl, int cyclical) {
 }
 
 template <int W>
-void gs_pack(const int8_t* h_rows, int64_t n, int mrl, std::vector<uint64_t>& nodes) {
+void gs_pack(const int8_t* h_rows, int64_t n, int mrl, int symmetric, std::vector<uint64_t>& nodes) {
     nodes.assign((size_t)std::max<int64_t>(n, 1) * (2 * W + 2), 0);
     for (int64_t i = 0; i < n; ++i) {
         Key<W> key;
         int lens[2];
         bool valid;
         pack_root<W>(h_rows + (size_t)i * 2 * mrl, mrl, key, lens, valid);
+        int g = 0;
+        if (symmetric) key = canonical<W>(key, g);
         uint64_t* q = nodes.data() + (size_t)i * (2 * W + 2);
         for (int j = 0; j < 2 * W; ++j) q[j] = key.k[j];
         q[2 * W] = ~0ull;  // parent link -1
-        q[2 * W + 1] = (uint64_t)i;
+        q[2 * W + 1] = (uint64_t)i | (uint64_t)g << 32;
     }
 }
 
@@ -197,7 +207,8 @@ void gs_pack(const int8_t* h_rows, int64_t n, int mrl, std::vector<uint64_t>& no
 
 extern "C" {
 
-int acs_goalset_from_rows(int device, int mrl, int cyclical, const int8_t* h_rows, int64_t n, acs_goalset** out) {
+namespace {
+int gs_from_rows(int device, int mrl, int cyclical, int symmetric, const int8_t* h_rows, int64_t n, acs_goalset** out) {
     if (!out) return ACS_ERR_INVALID;
     *out = nullptr;
     if (mrl < 1 || mrl > 61) return gs_fail(ACS_ERR_UNSUPPORTED, "goalset needs 1 <= max_relator_length <= 61");
@@ -224,10 +235,11 @@ int acs_goalset_from_rows(int device, int mrl, int cyclical, const int8_t* h_row
     g->mrl = mrl;
     g->W = mrl <= 29 ? 1 : 2;
     g->cyclical = cyclical ? 1 : 0;
+    g->symmetric = symmetric ? 1 : 0;
     g->n_entries = n;
     std::vector<uint64_t> h;
-    if (g->W == 1) gs_pack<1>(h_rows, n, mrl, h);
-    else gs_pack<2>(h_rows, n, mrl, h);
+    if (g->W == 1) gs_pack<1>(h_rows, n, mrl, g->symmetric, h);
+    else gs_pack<2>(h_rows, n, mrl, g->symmetric, h);
     if (cudaMalloc((void**)&g->nodes, h.size() * 8) != cudaSuccess) {
         cudaGetLastError();
         goalset_free(g);
@@ -246,6 +258,22 @@ int acs_goalset_from_rows(int device, int mrl, int cyclical, const int8_t* h_row
     *out = g;
     return ACS_OK;
 }
+}  // namespace
+
+int acs_goalset_from_rows(int device, int mrl, int cyclical, const int8_t* h_rows, int64_t n, acs_goalset** out) {
+    return gs_from_rows(device, mrl, cyclical, 0, h_rows, n, out);
+}
+
+int acs_goalset_from_rows_symmetric(int device, int mrl, int cyclical, const int8_t* h_rows, int64_t n,
+                                    acs_goalset** out) {
+    return gs_from_rows(device, mrl, cyclical, 1, h_rows, n, out);
+}
+
+int acs_goalset_is_symmetric(const acs_goalset* g, int* symmetric) {
+    if (!g || !symmetric) return ACS_ERR_INVALID;
+    *symmetric = g->symmetric;
+    return ACS_OK;
+}
 
 int acs_goalset_size(const acs_goalset* g, int64_t* n_entries, int64_t* n_states, int64_t* bytes) {
     if (!g) return ACS_ERR_INVALID;
@@ -256,6 +284,11 @@ int acs_goalset_size(const acs_goalset* g, int64_t* n_entries, int64_t* n_states
 }
 
 int acs_goalset_path(const acs_goalset* g, int64_t entry, int* root, int32_t* h_path, int path_cap, int* path_len) {
+    return acs_goalset_path_frame(g, entry, root, h_path, path_cap, path_len, nullptr);
+}
+
+int acs_goalset_path_frame(const acs_goalset* g, int64_t entry, int* root, int32_t* h_path, int path_cap, int* path_len,
+                           int* frame) {
     if (!g || path_cap < 0 || (!h_path && path_cap > 0)) return ACS_ERR_INVALID;
     if (entry < 0 || entry >= g->n_entries) return gs_fail(ACS_ERR_INVALID, "goalset_path: entry out of range");
     if (cudaSetDevice(g->device) != cudaSuccess) {
@@ -264,16 +297,16 @@ int acs_goalset_path(const acs_goalset* g, int64_t entry, int* root, int32_t* h_
     }
     const int cap = std::max(path_cap, 1);
     int32_t* d = nullptr;
-    cudaError_t e = cudaMalloc((void**)&d, ((size_t)cap * 2 + 2) * sizeof(int32_t));
-    int32_t res[2] = {0, 0};
+    cudaError_t e = cudaMalloc((void**)&d, ((size_t)cap * 2 + 4) * sizeof(int32_t));
+    int32_t res[4] = {0, 0, 0, 0};
     if (e == cudaSuccess) {
-        if (g->W == 1) gs_path_kernel<1><<<1, 1>>>(g->nodes, entry, d + 2, cap, d);
-        else gs_path_kernel<2><<<1, 1>>>(g->nodes, entry, d + 2, cap, d);
+        if (g->W == 1) gs_path_kernel<1><<<1, 1>>>(g->nodes, entry, d + 4, cap, d);
+        else gs_path_kernel<2><<<1, 1>>>(g->nodes, entry, d + 4, cap, d);
         e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaMemcpy(res, d, sizeof(res), cudaMemcpyDeviceToHost);
     if (e == cudaSuccess && res[0] <= path_cap && path_cap > 0)
-        e = cudaMemcpy(h_path, d + 2, (size_t)res[0] * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost);
+        e = cudaMemcpy(h_path, d + 4, (size_t)res[0] * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost);
     if (d) cudaFree(d);
     if (e != cudaSuccess) {
         cudaGetLastError();
@@ -281,6 +314,7 @@ int acs_goalset_path(const acs_goalset* g, int64_t entry, int* root, int32_t* h_
     }
     if (path_len) *path_len = res[0];
     if (root) *root = res[1];
+    if (frame) *frame = res[2];
     if (res[0] > path_cap) return gs_fail(ACS_ERR_INVALID, "goalset_path: the path is longer than path_cap (see path_len)");
     return ACS_OK;
 }

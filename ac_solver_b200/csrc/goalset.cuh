@@ -5,12 +5,17 @@
 // the index of the entry's root (the row, or the search that committed it).  The index is an exact
 // open-addressing table of 4-slot buckets, slot = 23-bit fingerprint << 40 | (entry + 1), at most
 // half full.  When a state occurs more than once, the smallest entry index holds its slot.
+//
+// A symmetric set holds canonical forms (ac_sym.cuh) and answers "is any image of this state in the set?":
+// goal_find canonicalizes the query first.  Its entries carry the element g with stored = g.(generated state)
+// in bits 32..35 of the root word (the layout of an orbit search's nodes, mbfs.cu).
 #pragma once
 #include <cstdint>
 
 #include <cuda_runtime.h>
 
 #include "ac_keys.cuh"
+#include "ac_sym.cuh"
 #include "bfs_common.cuh"
 
 namespace acs {
@@ -21,11 +26,20 @@ struct GoalView {
     const uint64_t* nodes;  // [n_entries][2W+2]
     const uint64_t* table;  // [tmask+1]
     uint64_t tmask;
+    int symmetric;  // entries are canonical forms: queries are canonicalized before the lookup
 };
 
-// entry index of state q, or -1
+// kept out of line so that the lookups of exact sets do not carry its registers
 template <int W>
-__device__ __forceinline__ int64_t goal_find(const GoalView& G, const Key<W>& q) {
+__device__ __noinline__ Key<W> goal_canonical(const Key<W> q) {
+    int g;
+    return canonical<W>(q, g);
+}
+
+// entry index of state q (of its canonical form in a symmetric set), or -1
+template <int W>
+__device__ __forceinline__ int64_t goal_find(const GoalView& G, Key<W> q) {
+    if (G.symmetric) q = goal_canonical<W>(q);
     const uint64_t h = pb_hash<W>(q), fp = h >> 41;
     uint64_t base = (h & G.tmask) & ~3ull;
     for (uint64_t n = 0; n <= G.tmask; n += 4, base = (base + 4) & G.tmask) {
@@ -46,12 +60,12 @@ __device__ __forceinline__ int64_t goal_find(const GoalView& G, const Key<W>& q)
 
 // host side of a goal set (shared by goalset.cu and mbfs.cu)
 struct acs_goalset {
-    int device = 0, mrl = 0, W = 1, cyclical = 0;
+    int device = 0, mrl = 0, W = 1, cyclical = 0, symmetric = 0;
     int64_t n_entries = 0, n_states = 0;
     uint64_t* nodes = nullptr;  // [max(n_entries, 1)][2W+2]
     uint64_t* table = nullptr;  // [tcap]
     uint64_t tcap = 0;
-    acs::GoalView view() const { return acs::GoalView{nodes, table, tcap - 1}; }
+    acs::GoalView view() const { return acs::GoalView{nodes, table, tcap - 1, symmetric}; }
 };
 
 namespace acs {

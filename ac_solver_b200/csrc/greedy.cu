@@ -406,6 +406,30 @@ __global__ void greedy_path_kernel(const GreedyArgs A, int32_t* paths, int path_
     }
 }
 
+// the element of every goal hit: u with u.(the state the search stopped at) = the entry's state (the identity
+// for an exact set), or -1 for a search that did not stop at a goal
+template <int W>
+__global__ void greedy_goal_elem_kernel(const GreedyArgs A, int symmetric, int32_t* out) {
+    const int sidx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (sidx >= A.n_search) return;
+    const GreedyRec& rec = A.rec[sidx];
+    if (rec.goal < 0) {
+        out[sidx] = -1;
+        return;
+    }
+    Key<W> q = load_key<W>(A.keys + (uint64_t)sidx * A.cap * 2 * W, rec.final_node);
+    if (rec.final_action >= 0) {
+        Rel<2 * W> r0, r1;
+        split_key<W>(q, r0, r1);
+        bool co;
+        apply_move<2 * W, false>(r0, r1, rec.final_action, A.mrl, A.cyclical != 0, co);
+        q = make_key<W>(r0, r1);
+    }
+    int u = 0;
+    if (symmetric) canonical<W>(q, u);
+    out[sidx] = u;
+}
+
 }  // namespace acs
 
 // ---------------------------------------------------------------------------------------
@@ -421,8 +445,9 @@ struct acs_greedy {
     GbArgs gb{};  // pools of the bucket kernel
     bool use_bucket = true;
     int n_fallback = 0;
-    int32_t *d_paths = nullptr, *d_path_len = nullptr;
+    int32_t *d_paths = nullptr, *d_path_len = nullptr, *d_goal_g = nullptr;
     int path_cap = 0;
+    std::vector<int32_t> h_goal_g;  // greedy_goal_elem_kernel of the last run with goals
     std::vector<GreedyRec> h_rec;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
@@ -464,6 +489,7 @@ extern "C" void acs_greedy_destroy(acs_greedy* g) {
     cudaFree(g->gb.round_tab);
     cudaFree(g->d_paths);
     cudaFree(g->d_path_len);
+    cudaFree(g->d_goal_g);
     delete g;
 }
 
@@ -640,6 +666,13 @@ int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_s
     greedy_path_kernel<W><<<(S + 63) / 64, 64, 0, st>>>(A, g->d_paths, g->path_cap, g->d_path_len);
     GR_CUDA(cudaGetLastError());
     GR_CUDA(cudaEventRecord(g->ev1, st));
+    if (GOAL) {
+        if (!g->d_goal_g) GR_CUDA(cudaMalloc((void**)&g->d_goal_g, (size_t)S * sizeof(int32_t)));
+        greedy_goal_elem_kernel<W><<<(S + 63) / 64, 64, 0, st>>>(A, g->goals->symmetric, g->d_goal_g);
+        GR_CUDA(cudaGetLastError());
+        g->h_goal_g.resize((size_t)S);
+        GR_CUDA(cudaMemcpyAsync(g->h_goal_g.data(), g->d_goal_g, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    }
     GR_CUDA(cudaMemcpyAsync(g->h_rec.data(), g->rec, (size_t)S * sizeof(GreedyRec), cudaMemcpyDeviceToHost, st));
     std::vector<int32_t> plen(S);
     GR_CUDA(cudaMemcpyAsync(plen.data(), g->d_path_len, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -722,6 +755,16 @@ extern "C" int acs_greedy_set_goals(acs_greedy* g, const acs_goalset* gs) {
         }
     }
     g->goals = gs;
+    return ACS_OK;
+}
+
+extern "C" int acs_greedy_goal_hit_elements(acs_greedy* g, int32_t* h_elem) {
+    if (!g || !h_elem) return ACS_ERR_INVALID;
+    if (!g->ran) {
+        acs::set_last_error("greedy: no completed run");
+        return ACS_ERR_INVALID;
+    }
+    for (int s = 0; s < g->n_search; ++s) h_elem[s] = g->ran_with_goals ? g->h_goal_g[s] : -1;
     return ACS_OK;
 }
 

@@ -29,6 +29,12 @@
 // (global node index), clear a record of the current chunk's log.  The log is rewritten every
 // chunk, so its size is bounded by 12 records per parent of one chunk.  The host enqueues chunks
 // ahead of the device and reads only a lagging pinned copy of the run state.
+//
+// Orbit search (acs_bfs_batch_set_symmetric): the same engine over canonical states (ac_sym.cuh).  The
+// root is stored as its canonical form, a child is canonicalized right after it is packed, and it is new
+// when its canonical form is unseen.  Every node records the element g with stored = g.(generated state)
+// in bits 32..35 of its search word; the path kernel turns the canonical-frame moves into moves of the
+// input row.  The move-skip rule is off in this mode: its argument is about generated, not canonical, states.
 #include <algorithm>
 #include <cstdint>
 #include <cstdio>
@@ -41,6 +47,7 @@
 #include "../../include/acsolver_b200.h"
 #include "ac_core.cuh"
 #include "ac_keys.cuh"
+#include "ac_sym.cuh"
 #include "acs_internal.h"
 #include "bfs_common.cuh"
 #include "goalset.cuh"
@@ -54,6 +61,7 @@ constexpr int kMbSol = 0, kMbErr = 1, kMbLen0 = 2, kMbGoal = 130;
 constexpr uint64_t kMbNode = 1ull << 39, kMbIdx = kMbNode - 1;
 constexpr uint64_t kMbTomb = 1ull << 63;  // fingerprints are 23 bits: never equal to a tombstone's
 constexpr int kMbStage = 128;             // records staged per warp before a flush to the log
+constexpr uint32_t kMbSymShift = 28;      // orbit search: a staged record's search id carries g in its top 4 bits
 
 enum : int { MB_IERR_TABLE_FULL = 1, MB_IERR_SLAB_FULL = 2 };
 
@@ -96,6 +104,9 @@ struct MbEngine {
     int64_t rec_cap;
     GoalView goals;       // the goal set, if one is set
     int64_t* goal_hit;    // [n_search] goal entry a search stopped at, or -1 (allocated with the first goal set)
+    uint8_t* log_g;       // [rec_cap] orbit search: the element that canonicalized each record
+    const uint8_t* root_g;  // [n_search] orbit search: the element that canonicalized each root
+    int32_t* goal_hit_g;  // [n_search] u with u.(end state of the returned path) = the goal entry's state, or -1
 };
 
 template <int W>
@@ -127,7 +138,7 @@ __global__ void mb_init_kernel(const MbEngine E, const uint64_t* roots) {
 #pragma unroll
     for (int i = 0; i < 2 * W; ++i) q.k[i] = roots[(size_t)s * 2 * W + i];
     const uint64_t idx = (uint64_t)E.srch[s].slab;
-    node_store<W>(E.nodes, idx, q, -1, s);
+    node_store<W>(E.nodes, idx, q, -1, (int64_t)s | (E.root_g ? (int64_t)E.root_g[s] << 32 : 0));
     const uint64_t h = mb_hash<W>(q, (uint32_t)s), tmask = E.st->tmask;
     const uint64_t v = ((h >> 41) << 40) | kMbNode | (idx + 1);
     // slot by slot from the start of the 4-slot bucket: the order in which mb_insert_kernel probes
@@ -222,7 +233,7 @@ __host__ __device__ constexpr int mb_stage_bytes_per_warp() {
 }
 extern __shared__ __align__(16) unsigned char mb_smem[];
 
-template <int W>
+template <int W, bool SYM>
 __device__ __forceinline__ void mb_flush(const MbEngine& E, const ulonglong2* sk, const uint32_t* sc, const uint32_t* ss,
                                          uint32_t n, int lane) {
     unsigned long long pos = 0;
@@ -233,12 +244,17 @@ __device__ __forceinline__ void mb_flush(const MbEngine& E, const ulonglong2* sk
 #pragma unroll
         for (int i = 0; i < W; ++i) dk[(size_t)idx * W + i] = sk[idx * W + i];
         E.log_c[pos + idx] = sc[idx];
-        E.log_s[pos + idx] = ss[idx];
+        if constexpr (SYM) {
+            E.log_s[pos + idx] = ss[idx] & ((1u << kMbSymShift) - 1u);
+            E.log_g[pos + idx] = (uint8_t)(ss[idx] >> kMbSymShift);
+        } else {
+            E.log_s[pos + idx] = ss[idx];
+        }
     }
     __syncwarp();
 }
 
-template <int W, bool TRUSTED>
+template <int W, bool TRUSTED, bool SYM>
 __global__ void __launch_bounds__(256) mb_expand_kernel(const MbEngine E) {
     const MbState* st = E.st;
     if (st->done) return;
@@ -269,7 +285,7 @@ __global__ void __launch_bounds__(256) mb_expand_kernel(const MbEngine E) {
             min_len = M.min_len;
             int64_t pl, tag;
             node_load<W>(E.nodes, (uint64_t)(M.slab + __ldg(E.seg_head + k) + (j - __ldg(E.seg_off + k))), pk, pl, tag);
-            skip = skip_moves<TRUSTED>(pl, cyc);
+            if constexpr (!SYM) skip = skip_moves<TRUSTED>(pl, cyc);
         }
         unsigned long long* ctrl = E.ctrl + (int64_t)k * kMbCtrl;
         Rel<2 * W> p0, p1;
@@ -280,6 +296,7 @@ __global__ void __launch_bounds__(256) mb_expand_kernel(const MbEngine E) {
             Rel<2 * W> r0 = p0, r1 = p1;
             bool emit = false;
             Key<W> child;
+            int g = 0;
 #pragma unroll
             for (int i = 0; i < 2 * W; ++i) child.k[i] = 0;
             if (valid && !((skip >> a) & 1u)) {
@@ -293,6 +310,7 @@ __global__ void __launch_bounds__(256) mb_expand_kernel(const MbEngine E) {
                     if (L < min_len) atomicMin(&ctrl[kMbLen0 + L], c);
                     if (L == 2) atomicMin(&ctrl[kMbSol], c);  // before the visited test
                     child = make_key<W>(r0, r1);
+                    if constexpr (SYM) child = canonical<W>(child, g);
                     emit = !key_eq<W>(child, pk);
                 }
             }
@@ -302,19 +320,19 @@ __global__ void __launch_bounds__(256) mb_expand_kernel(const MbEngine E) {
 #pragma unroll
                 for (int i = 0; i < W; ++i) sk[q * W + i] = make_ulonglong2(child.k[2 * i], child.k[2 * i + 1]);
                 sc[q] = cbase + a;
-                ss[q] = s;
+                ss[q] = SYM ? s | ((uint32_t)g << kMbSymShift) : s;
             }
             staged += __popc(act);
             if (staged > kMbStage - 32) {
                 __syncwarp();
-                mb_flush<W>(E, sk, sc, ss, staged, lane);
+                mb_flush<W, SYM>(E, sk, sc, ss, staged, lane);
                 staged = 0;
             }
         }
     }
     if (staged) {
         __syncwarp();
-        mb_flush<W>(E, sk, sc, ss, staged, lane);
+        mb_flush<W, SYM>(E, sk, sc, ss, staged, lane);
     }
 }
 
@@ -605,7 +623,7 @@ __global__ void __launch_bounds__(128) mb_decide_kernel(const MbEngine E) {
 }
 
 // ---- commit ------------------------------------------------------------------------------------------
-template <int W>
+template <int W, bool SYM>
 __global__ void __launch_bounds__(256) mb_commit_kernel(const MbEngine E) {
     const MbState* st = E.st;
     if (st->done) return;
@@ -630,15 +648,19 @@ __global__ void __launch_bounds__(256) mb_commit_kernel(const MbEngine E) {
         }
         const Key<W> key = load_key_cg<W>(E.log_keys, i);
         const int64_t pgid = E.seg_head[k] + (int64_t)(c / 12) - E.seg_off[k];
-        node_store<W>(E.nodes, (uint64_t)idx, key, (pgid << 4) | (int64_t)(c % 12), (int64_t)s);
+        const int64_t tag = SYM ? (int64_t)s | ((int64_t)__ldcg(E.log_g + i) << 32) : (int64_t)s;
+        node_store<W>(E.nodes, (uint64_t)idx, key, (pgid << 4) | (int64_t)(c % 12), tag);
         E.table[slot] = ((mb_hash<W>(key, s) >> 41) << 40) | kMbNode | (uint64_t)(idx + 1);
     }
 }
 
 // ---- results -----------------------------------------------------------------------------------------
 // path of every solved search: (action, total length) pairs from the root, then (solving action, 2) -- or
-// (action, the goal state's total length) after a goal child, or nothing more when the root is a goal
-template <int W>
+// (action, the goal state's total length) after a goal child, or nothing more when the root is a goal.
+// Orbit search: the walk from the node back to the root stashes each node's element beside its action,
+// then a forward pass turns the moves on stored states c_k into moves on the actual states a_k = h_k.c_k:
+// h_0 = g_0^-1, the actual move of (m_k, g_k+1) is pi_{h_k}(m_k), and h_k+1 = h_k.g_k+1^-1.
+template <int W, bool SYM>
 __global__ void mb_path_kernel(const MbEngine E, int32_t* paths, int path_cap, int32_t* path_len) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= E.st->n_search) return;
@@ -667,9 +689,42 @@ __global__ void mb_path_kernel(const MbEngine E, int32_t* paths, int path_cap, i
         node_load<W>(E.nodes, (uint64_t)(M.slab + g), k, pl, tag);
         if (pos < path_cap) {
             path[2 * pos] = pl < 0 ? -1 : (int32_t)(pl & 15);
+            if constexpr (SYM) path[2 * pos] = (path[2 * pos] & 0xFF) | (int32_t)(((uint64_t)tag >> 32) & 15) << 8;
             path[2 * pos + 1] = (int32_t)(k.k[W - 1] >> 58) + (int32_t)(k.k[2 * W - 1] >> 58);
         }
         g = pl < 0 ? -1 : (pl >> 4);
+    }
+    int hk = 0;  // orbit search: the frame of the path's last stored node
+    if constexpr (SYM) {
+        int h = 0;
+        const int n = depth < path_cap ? depth : path_cap;
+        for (int i = 0; i < n; ++i) {
+            const int v = path[2 * i], el = v >> 8;
+            if (i == 0) {
+                h = sym_inv(el);
+                path[0] = -1;
+            } else {
+                path[2 * i] = sym_pi(h, v & 0xFF);
+                h = sym_mul(h, sym_inv(el));
+            }
+        }
+        if (!at_root && depth < path_cap) path[2 * depth] = sym_pi(h, path[2 * depth]);
+        hk = h;
+    }
+    // the element of a goal hit: u.(actual end state) = the entry's state -- the identity for an exact set
+    if (E.goal_hit_g && E.goal_hit[s] >= 0) {
+        Key<W> q = node_key<W>(E.nodes, (uint64_t)(M.slab + node));
+        if (!at_root) {
+            Rel<2 * W> r0, r1;
+            split_key<W>(q, r0, r1);
+            bool co;
+            apply_move<2 * W, false>(r0, r1, (int)(M.sol_gid % 12), E.st->mrl, E.st->cyclical != 0, co);
+            q = make_key<W>(r0, r1);
+        }
+        if constexpr (SYM) q = sym_apply<W>(q, hk);
+        int u = 0;
+        if (E.goals.symmetric) canonical<W>(q, u);
+        E.goal_hit_g[s] = u;
     }
 }
 
@@ -694,7 +749,7 @@ __global__ void mb_adopt_kernel(const uint64_t* nodes, const int64_t* off, const
         Key<W> k;
         int64_t pl, tag;
         node_load<W>(nodes, (uint64_t)(__ldg(slab + s) + ((int64_t)e - first)), k, pl, tag);
-        node_store<W>(out, e, k, pl < 0 ? -1 : (((first + (pl >> 4)) << 4) | (pl & 15)), (int64_t)s);
+        node_store<W>(out, e, k, pl < 0 ? -1 : (((first + (pl >> 4)) << 4) | (pl & 15)), (int64_t)s | (tag & (15ll << 32)));
     }
 }
 
@@ -775,12 +830,14 @@ struct acs_bfs_batch {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ring_ev[kMbRing] = {};
     MbState* h_ring = nullptr;  // pinned [kMbRing]
     int sms = 148;
-    int expand_blocks = 148, expand_wpb = 8, insert_blocks = 148, commit_blocks = 148;
+    int expand_blocks = 148, expand_blocks_sym = 148, expand_wpb = 8, insert_blocks = 148, commit_blocks = 148;
     size_t expand_smem = 0;
     bool ran = false;
     const acs_goalset* goals = nullptr;  // acs_bfs_batch_set_goals
     int explore = 0;                     // stop_at_trivial == 0
     bool adopted = false;                // the nodes went to a goal set (acs_goalset_from_bfs_batch)
+    int symmetric = 0;                   // orbit search (acs_bfs_batch_set_symmetric)
+    uint8_t* d_root_g = nullptr;         // [n_search] each root's element, with E.log_g allocated by set_symmetric
 };
 
 extern "C" {
@@ -808,7 +865,7 @@ void acs_bfs_batch_destroy(acs_bfs_batch* b) {
     MbEngine& E = b->E;
     void* ptrs[] = {E.st, E.srch, E.nodes, E.table, E.log_keys, E.log_c, E.log_s, E.rec_slot, E.cursor, E.bitmap, E.rt,
                     E.bsums, E.ctrl, E.seg_search, E.seg_head, E.seg_off, E.seg_limit, E.seg_base, E.seg_of,
-                    E.goal_hit, b->d_roots, b->d_paths, b->d_plen};
+                    E.goal_hit, E.goal_hit_g, E.log_g, b->d_root_g, b->d_roots, b->d_paths, b->d_plen};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (b->h_ring) cudaFreeHost(b->h_ring);
@@ -883,18 +940,21 @@ int acs_bfs_batch_create(int device, int n_search, int mrl, const int64_t* max_n
     cudaDeviceProp prop{};
     if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) b->sms = prop.multiProcessorCount;
     b->expand_smem = (size_t)b->expand_wpb * (P.W == 1 ? mb_stage_bytes_per_warp<1>() : mb_stage_bytes_per_warp<2>());
-    int per_sm = 1, ib = 1, cb = 1;
+    int per_sm = 1, per_sm_sym = 1, ib = 1, cb = 1;
     if (P.W == 1) {
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mb_expand_kernel<1, true>, 32 * b->expand_wpb, b->expand_smem);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mb_expand_kernel<1, true, false>, 32 * b->expand_wpb, b->expand_smem);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_sym, mb_expand_kernel<1, true, true>, 32 * b->expand_wpb, b->expand_smem);
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ib, mb_insert_kernel<1>, 256, 0);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cb, mb_commit_kernel<1>, 256, 0);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cb, mb_commit_kernel<1, false>, 256, 0);
     } else {
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mb_expand_kernel<2, true>, 32 * b->expand_wpb, b->expand_smem);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mb_expand_kernel<2, true, false>, 32 * b->expand_wpb, b->expand_smem);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_sym, mb_expand_kernel<2, true, true>, 32 * b->expand_wpb, b->expand_smem);
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ib, mb_insert_kernel<2>, 256, 0);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cb, mb_commit_kernel<2>, 256, 0);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cb, mb_commit_kernel<2, false>, 256, 0);
     }
     cudaGetLastError();
     b->expand_blocks = b->sms * std::max(per_sm, 1);
+    b->expand_blocks_sym = b->sms * std::max(per_sm_sym, 1);
     b->insert_blocks = b->sms * std::max(ib, 1);
     b->commit_blocks = b->sms * std::max(cb, 1);
     *out = b;
@@ -921,7 +981,8 @@ int mb_paths(acs_bfs_batch* b, int32_t* h_paths, int path_cap, std::vector<int32
         b->d_path_cap = cap;
     }
     if (!b->d_plen) MB_CUDA(cudaMalloc((void**)&b->d_plen, (size_t)n * sizeof(int32_t)));
-    mb_path_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(b->E, b->d_paths, cap, b->d_plen);
+    if (b->symmetric) mb_path_kernel<W, true><<<(n + 127) / 128, 128, 0, s>>>(b->E, b->d_paths, cap, b->d_plen);
+    else mb_path_kernel<W, false><<<(n + 127) / 128, 128, 0, s>>>(b->E, b->d_paths, cap, b->d_plen);
     MB_CUDA(cudaGetLastError());
     plen.resize((size_t)n);
     MB_CUDA(cudaMemcpyAsync(plen.data(), b->d_plen, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
@@ -941,6 +1002,7 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
     if (b->adopted) return mb_fail(ACS_ERR_INVALID, "bfs_batch: the engine's states were handed to a goal set");
     std::vector<MbSearch> init((size_t)n);
     std::vector<uint64_t> roots((size_t)n * 2 * W, 0);
+    std::vector<uint8_t> root_g((size_t)n, 0);
     int64_t slab = 0, n_valid = 0;
     for (int s = 0; s < n; ++s) {
         MbSearch& M = init[s];
@@ -964,6 +1026,11 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
             continue;
         }
         M.min_len = lens[0] + lens[1];
+        if (b->symmetric) {
+            int g0 = 0;
+            root = canonical<W>(root, g0);
+            root_g[s] = (uint8_t)g0;
+        }
         for (int i = 0; i < 2 * W; ++i) roots[(size_t)s * 2 * W + i] = root.k[i];
         ++n_valid;
     }
@@ -979,10 +1046,13 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
     MB_CUDA(cudaSetDevice(b->device));
     MB_CUDA(cudaMemsetAsync(E.table, 0, b->plan.tcap * sizeof(uint64_t), s));
     if (E.goal_hit) MB_CUDA(cudaMemsetAsync(E.goal_hit, 0xFF, (size_t)n * sizeof(int64_t), s));
+    if (E.goal_hit_g) MB_CUDA(cudaMemsetAsync(E.goal_hit_g, 0xFF, (size_t)n * sizeof(int32_t), s));
     b->h_ring[0] = st;  // pinned staging for the async upload
     MB_CUDA(cudaMemcpyAsync(E.st, &b->h_ring[0], sizeof(MbState), cudaMemcpyHostToDevice, s));
     MB_CUDA(cudaMemcpyAsync(E.srch, init.data(), init.size() * sizeof(MbSearch), cudaMemcpyHostToDevice, s));
     MB_CUDA(cudaMemcpyAsync(b->d_roots, roots.data(), roots.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    if (b->symmetric) MB_CUDA(cudaMemcpyAsync(b->d_root_g, root_g.data(), root_g.size(), cudaMemcpyHostToDevice, s));
+    E.root_g = b->symmetric ? b->d_root_g : nullptr;
     MB_CUDA(cudaStreamSynchronize(s));  // the staging copies above read host memory that goes out of scope
     MB_CUDA(cudaEventRecord(b->ev0, s));
     mb_init_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(E, b->d_roots);
@@ -996,15 +1066,22 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
             if (b->h_ring[(chunk - kMbLag) % kMbRing].done) break;
         }
         mb_prep_kernel<<<b->sms * 2, 256, 0, s>>>(E);
-        if (chunk == 0) mb_expand_kernel<W, false><<<b->expand_blocks, 32 * b->expand_wpb, b->expand_smem, s>>>(E);
-        else mb_expand_kernel<W, true><<<b->expand_blocks, 32 * b->expand_wpb, b->expand_smem, s>>>(E);
+        const dim3 eg(b->symmetric ? b->expand_blocks_sym : b->expand_blocks), et(32 * b->expand_wpb);
+        if (b->symmetric) {
+            if (chunk == 0) mb_expand_kernel<W, false, true><<<eg, et, b->expand_smem, s>>>(E);
+            else mb_expand_kernel<W, true, true><<<eg, et, b->expand_smem, s>>>(E);
+        } else {
+            if (chunk == 0) mb_expand_kernel<W, false, false><<<eg, et, b->expand_smem, s>>>(E);
+            else mb_expand_kernel<W, true, false><<<eg, et, b->expand_smem, s>>>(E);
+        }
         mb_insert_kernel<W><<<b->insert_blocks, 256, 0, s>>>(E);
         if (b->goals) mb_goal_kernel<W><<<b->insert_blocks, 256, 0, s>>>(E);
         mb_scan_sums_kernel<<<b->sms * 4, kScanT, 0, s>>>(E);
         mb_scan_top_kernel<<<1, kScanT, 0, s>>>(E);
         mb_scan_final_kernel<<<b->sms * 4, kScanT, 0, s>>>(E);
         mb_decide_kernel<<<decide_blocks, 128, 0, s>>>(E);
-        mb_commit_kernel<W><<<b->commit_blocks, 256, 0, s>>>(E);
+        if (b->symmetric) mb_commit_kernel<W, true><<<b->commit_blocks, 256, 0, s>>>(E);
+        else mb_commit_kernel<W, false><<<b->commit_blocks, 256, 0, s>>>(E);
         mb_plan_kernel<<<1, 32, 0, s>>>(E, 0);
         MB_CUDA(cudaGetLastError());
         MB_CUDA(cudaMemcpyAsync(&b->h_ring[chunk % kMbRing], E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
@@ -1105,16 +1182,20 @@ int acs_bfs_batch_set_goals(acs_bfs_batch* b, const acs_goalset* g, int stop_at_
             return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set's cyclical flag differs from the engine's");
         if (g->device != b->device)
             return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set lives on another device");
+        if (b->symmetric && !g->symmetric)  // an orbit search knows only the orbit of a child
+            return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_goals: an orbit search needs a symmetric goal set");
         if (g->n_entries >= (int64_t)0xFFFFFFFF)  // a hit packs the entry into 32 bits beside its candidate id
             return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch_set_goals: goal sets of 2^32 - 1 entries or more are not supported");
         if (!b->E.goal_hit) {
             MB_CUDA(cudaSetDevice(b->device));
             MB_CUDA(cudaMalloc((void**)&b->E.goal_hit, (size_t)b->n_search * sizeof(int64_t)));
             MB_CUDA(cudaMemset(b->E.goal_hit, 0xFF, (size_t)b->n_search * sizeof(int64_t)));
+            MB_CUDA(cudaMalloc((void**)&b->E.goal_hit_g, (size_t)b->n_search * sizeof(int32_t)));
+            MB_CUDA(cudaMemset(b->E.goal_hit_g, 0xFF, (size_t)b->n_search * sizeof(int32_t)));
         }
         b->E.goals = g->view();
     } else {
-        b->E.goals = GoalView{nullptr, nullptr, 0};
+        b->E.goals = GoalView{nullptr, nullptr, 0, 0};
     }
     b->goals = g;
     b->explore = stop_at_trivial ? 0 : 1;
@@ -1130,6 +1211,20 @@ int acs_bfs_batch_goal_hits(acs_bfs_batch* b, int64_t* h_entry) {
     }
     MB_CUDA(cudaSetDevice(b->device));
     MB_CUDA(cudaMemcpyAsync(h_entry, b->E.goal_hit, (size_t)b->n_search * sizeof(int64_t), cudaMemcpyDeviceToHost,
+                            b->stream));
+    MB_CUDA(cudaStreamSynchronize(b->stream));
+    return ACS_OK;
+}
+
+int acs_bfs_batch_goal_hit_elements(acs_bfs_batch* b, int32_t* h_elem) {
+    if (!b || !h_elem) return ACS_ERR_INVALID;
+    if (!b->ran) return mb_fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
+    if (!b->E.goal_hit_g) {
+        std::fill(h_elem, h_elem + b->n_search, -1);
+        return ACS_OK;
+    }
+    MB_CUDA(cudaSetDevice(b->device));
+    MB_CUDA(cudaMemcpyAsync(h_elem, b->E.goal_hit_g, (size_t)b->n_search * sizeof(int32_t), cudaMemcpyDeviceToHost,
                             b->stream));
     MB_CUDA(cudaStreamSynchronize(b->stream));
     return ACS_OK;
@@ -1162,6 +1257,7 @@ int acs_goalset_from_bfs_batch(acs_bfs_batch* b, acs_goalset** out) {
     g->mrl = b->mrl;
     g->W = b->W;
     g->cyclical = b->cyclical;
+    g->symmetric = b->symmetric;
     g->n_entries = total;
     int64_t* d_idx = nullptr;
     cudaError_t e = cudaMalloc((void**)&g->nodes, (size_t)std::max<int64_t>(total, 1) * 8 * (2 * b->W + 2));
@@ -1191,6 +1287,28 @@ int acs_goalset_from_bfs_batch(acs_bfs_batch* b, acs_goalset** out) {
         return rc;
     }
     *out = g;
+    return ACS_OK;
+}
+
+}  // extern "C"
+
+// ---- orbit search ------------------------------------------------------------------------------------------
+extern "C" {
+
+int acs_bfs_batch_set_symmetric(acs_bfs_batch* b, int symmetric) {
+    if (!b) return ACS_ERR_INVALID;
+    if (symmetric) {
+        if (b->goals && !b->goals->symmetric)
+            return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_symmetric: an orbit search needs a symmetric goal set");
+        if (b->n_search >= (1 << kMbSymShift))
+            return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch_set_symmetric: orbit search supports fewer than 2^28 searches");
+        if (!b->E.log_g) {
+            MB_CUDA(cudaSetDevice(b->device));
+            MB_CUDA(cudaMalloc((void**)&b->E.log_g, (size_t)b->E.rec_cap));
+            MB_CUDA(cudaMalloc((void**)&b->d_root_g, (size_t)b->n_search));
+        }
+    }
+    b->symmetric = symmetric ? 1 : 0;
     return ACS_OK;
 }
 

@@ -113,7 +113,7 @@ def _split(L, mrl, budgets, chunk_parents, max_bytes):
 class _BatchEngine:
     """One acs_bfs_batch engine over rows [lo, hi) of a validated batch."""
 
-    def __init__(self, L, dev, P8, budgets, cyclical, chunk_parents, goals=None, stop_at_trivial=True):
+    def __init__(self, L, dev, P8, budgets, cyclical, chunk_parents, goals=None, stop_at_trivial=True, symmetric=False):
         self.L, self.P8 = L, np.ascontiguousarray(P8)
         self.S, w = P8.shape
         self.h = C.c_void_p()
@@ -121,13 +121,15 @@ class _BatchEngine:
         b = np.ascontiguousarray(budgets, dtype=np.int64)  # referenced until the call returns
         _lib.check(L.acs_bfs_batch_create(dev, self.S, w // 2, b.ctypes.data, int(bool(cyclical)), int(chunk_parents),
                                           C.byref(self.h)))
-        if goals is not None or not stop_at_trivial:
-            try:
+        try:
+            if goals is not None or not stop_at_trivial:
                 _lib.check(L.acs_bfs_batch_set_goals(self.h, goals.handle if goals is not None else None,
                                                      int(bool(stop_at_trivial))))
-            except BaseException:
-                self.destroy()
-                raise
+            if symmetric:
+                _lib.check(L.acs_bfs_batch_set_symmetric(self.h, 1))
+        except BaseException:
+            self.destroy()
+            raise
 
     def run(self, want_visited):
         L, S = self.L, self.S
@@ -145,6 +147,8 @@ class _BatchEngine:
         if self.goals is not None:
             hits = np.full(S, -1, np.int64)
             _lib.check(L.acs_bfs_batch_goal_hits(self.h, hits.ctypes.data))
+            elems = np.full(S, -1, np.int32)
+            _lib.check(L.acs_bfs_batch_goal_hit_elements(self.h, elems.ctypes.data))
         out = []
         for s in range(S):
             r = res[s]
@@ -157,6 +161,7 @@ class _BatchEngine:
             }
             if hits is not None:
                 info["goal"] = int(hits[s]) if hits[s] >= 0 else None
+                info["goal_element"] = int(elems[s]) if hits[s] >= 0 else None
             if want_visited and r.status == 0:
                 vis = np.zeros((max(int(r.n_visited), 1), self.P8.shape[1]), np.int8)
                 n_out = C.c_int64(0)
@@ -187,7 +192,8 @@ def _check_goals(goals, mrl, cyclical, dev):
 
 
 def bfs_batch(presentations, max_nodes_to_explore=10000, cyclically_reduce_after_moves=False, want_visited=False,
-              device=None, chunk_parents=0, max_bytes=DEFAULT_MAX_BYTES, goals=None, stop_at_trivial=True):
+              device=None, chunk_parents=0, max_bytes=DEFAULT_MAX_BYTES, goals=None, stop_at_trivial=True,
+              symmetric=False):
     """Breadth-first search of every row of ``presentations`` [S, 2*mrl] in one device run
     (csrc/mbfs.cu).  ``max_nodes_to_explore`` is one budget or one per row.
 
@@ -200,23 +206,60 @@ def bfs_batch(presentations, max_nodes_to_explore=10000, cyclically_reduce_after
     a search also stops at the first generated child that is in the set, tested right after the
     length-2 test, and reports it as solved with ``info["goal"]`` = the entry index (``None`` for
     rows that did not stop at a goal); the path then ends with (action, total length of the goal
-    state).  A root in the set stops at depth 0 with the path ``[(-1, L0)]``.  ``stop_at_trivial=False``
-    turns the length-2 rule off: searches run until a goal, their budget or exhaustion."""
+    state).  ``info["goal_element"]`` is the element u of the presentation symmetries with u.(the state the
+    path ends at) = the entry's stored state: 0 for an exact set, any element for a symmetric set
+    (``GoalSet.from_rows(..., symmetric=True)``), which matches a state when any of its images is in the set.  A root in the set stops at depth 0 with the path ``[(-1, L0)]``.  ``stop_at_trivial=False``
+    turns the length-2 rule off: searches run until a goal, their budget or exhaustion.
+
+    ``symmetric=True`` runs orbit searches: breadth-first search over the orbits of the 16 presentation
+    symmetries (``canonical_form``).  The root and every new state are stored as canonical forms, and a
+    child is new when its canonical form is unseen, so each stored state stands for its whole orbit and the
+    path lengths stay shortest.  Paths are moves of the input row in the format above; ``info["visited"]``
+    holds the canonical states.  The node budget then counts orbits, so at a budget cut the solved rows can
+    differ from exact search in both directions.  With ``goals`` the set must be symmetric: an orbit search
+    knows the orbit of a child, not which of its states is in the set."""
     P8, budgets = _batch_inputs(presentations, max_nodes_to_explore)
     dev = _lib.default_device() if device is None else device
     _check_goals(goals, P8.shape[1] // 2, cyclically_reduce_after_moves, dev)
+    if symmetric and goals is not None and not goals.symmetric:
+        raise ValueError("an orbit search (symmetric=True) needs a symmetric goal set: it knows only the orbit "
+                         "of a child, not which of its states is in the set")
     if P8.shape[0] == 0:
         return []
     L = _lib.lib()
     out = []
     for lo, hi, _ in _split(L, P8.shape[1] // 2, budgets, chunk_parents, max_bytes):
         e = _BatchEngine(L, dev, P8[lo:hi], budgets[lo:hi], cyclically_reduce_after_moves, chunk_parents, goals,
-                         stop_at_trivial)
+                         stop_at_trivial, symmetric)
         try:
             out += e.run(want_visited)
         finally:
             e.destroy()
     return out
+
+
+def canonical_form(rows, device=None):
+    """Canonical forms under the presentation symmetries, in one device call (csrc/sym.cu).
+
+    The group has order 16: the 8 signed permutations of the generators (swap x and y, invert x, invert y)
+    and the swap of the two relators; it maps AC' moves to AC' moves.  ``rows`` [n, 2*mrl] right-padded int8
+    -> ``(canon, elements)``: ``canon[i]`` is the smallest image of row i in the order (length of relator 0,
+    relator 0 read from its last letter, length of relator 1, relator 1 likewise; letters y < x < y^-1 <
+    x^-1), ``elements[i]`` the smallest element g = 8r + 4s + 2a + b mapping the row there (s: swap x and y,
+    then a: invert x, then b: invert y, then r: swap the relators)."""
+    P = np.asarray(rows)
+    if P.ndim != 2 or P.shape[1] % 2 or P.shape[1] == 0:
+        raise ValueError("rows must be [n, 2*max_relator_length]")
+    P8 = np.ascontiguousarray(P, dtype=np.int8)
+    if not np.array_equal(P8, P):
+        raise ValueError("rows must hold letters in {+-1, +-2} and 0 padding")
+    L = _lib.lib()
+    dev = _lib.default_device() if device is None else device
+    out = np.empty_like(P8)
+    elem = np.zeros(P8.shape[0], np.uint8)
+    _lib.check(L.acs_canonical_form(dev, P8.shape[1] // 2, P8.ctypes.data, P8.shape[0], out.ctypes.data,
+                                    elem.ctypes.data))
+    return out, elem
 
 
 def bfs_groups(groups, max_nodes_to_explore=10000, cyclically_reduce_after_moves=False, want_visited=False, device=None,

@@ -58,6 +58,8 @@ def greedy_search_batch(presentations, max_nodes_to_explore=10000, cyclically_re
         if goals is not None:
             hits = np.full(S, -1, np.int64)
             _lib.check(L.acs_greedy_goal_hits(h, hits.ctypes.data))
+            elems = np.full(S, -1, np.int32)
+            _lib.check(L.acs_greedy_goal_hit_elements(h, elems.ctypes.data))
         for s in range(S):
             r = res[s]
             info = {
@@ -70,6 +72,7 @@ def greedy_search_batch(presentations, max_nodes_to_explore=10000, cyclically_re
             }
             if hits is not None:
                 info["goal"] = int(hits[s]) if hits[s] >= 0 else None
+                info["goal_element"] = int(elems[s]) if hits[s] >= 0 else None
             if r.path_len > path_cap:  # deeper than the buffer: the reference has no limit -- run again with room
                 L.acs_greedy_destroy(h)
                 h = None

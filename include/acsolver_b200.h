@@ -246,6 +246,20 @@ void acs_goalset_destroy(acs_goalset *g);
 int acs_bfs_batch_set_goals(acs_bfs_batch *b, const acs_goalset *g, int stop_at_trivial);
 int acs_bfs_batch_goal_hits(acs_bfs_batch *b, int64_t *h_entry /* [n_search] */);
 
+/* Presentation symmetries (csrc/ac_sym.cuh): the group G of order 16 generated by the signed permutations
+ * of the generators and the swap of the relators acts on the AC' graph by automorphisms.  Element
+ * g = 8r + 4s + 2a + b: swap x <-> y (s), then invert x (a), then invert y (b), then swap the relators (r).
+ * acs_canonical_form: h_out [n, 2*mrl] the canonical form of each row (the smallest of its 16 images in the
+ * order of ac_sym.cuh) and h_elem [n] the smallest g with h_out = g.row.  Rows must be right-padded with
+ * letters in {+-1, +-2}, else ACS_ERR_INVALID.
+ * acs_bfs_batch_set_symmetric: symmetric != 0 makes the next runs of b orbit searches: breadth-first
+ * search over canonical states, the root stored canonical, a child new when its canonical form is unseen.
+ * Distances to the trivial presentations are exact; paths are moves of the input row, in the format of
+ * acs_bfs_batch_run; visited arrays hold the canonical states in insertion order.  Goal sets must be
+ * symmetric (ACS_ERR_INVALID otherwise); acs_goalset_from_bfs_batch of such an engine makes a symmetric set. */
+int acs_canonical_form(int device, int mrl, const int8_t *h_rows, int64_t n, int8_t *h_out, uint8_t *h_elem);
+int acs_bfs_batch_set_symmetric(acs_bfs_batch *b, int symmetric);
+
 /* Batched greedy search (search/greedy.py:15-121): n_search independent presentations of the
  * same mrl, one warp each, one launch.  h_presentations [n_search, 2*mrl]; h_paths
  * [n_search, path_cap, 2] int32 (action, total_length) pairs; results [n_search].  On failure
@@ -265,6 +279,22 @@ void acs_greedy_destroy(acs_greedy *g);
  * acs_greedy_goal_hits: per search of the last run, the goal entry it stopped at, or -1. */
 int acs_greedy_set_goals(acs_greedy *g, const acs_goalset *gs);
 int acs_greedy_goal_hits(acs_greedy *g, int64_t *h_entry /* [n_search] */);
+/* Symmetric goal sets hold canonical forms and answer "is any image of this state in the set?"; exact
+ * and orbit searches (bfs_batch, greedy) can stop at them.  An orbit search needs a symmetric set.
+ * acs_goalset_from_rows_symmetric: acs_goalset_from_rows storing each row's canonical form.
+ * acs_goalset_from_bfs_batch of an orbit-search engine makes a symmetric set.
+ * acs_goalset_path_frame: acs_goalset_path (moves of the root's row, also for symmetric sets) and *frame =
+ * the element H with (end state of that path) = H.(the entry's stored state); 0 for exact sets.
+ * acs_bfs_batch_goal_hit_elements / acs_greedy_goal_hit_elements: per search of the last run, the element u
+ * with u.(end state of the returned path) = the state of the entry it stopped at (0 for an exact set), or
+ * -1 when it did not stop at a goal. */
+int acs_goalset_from_rows_symmetric(int device, int mrl, int cyclical, const int8_t *h_rows, int64_t n,
+                                    acs_goalset **out);
+int acs_goalset_is_symmetric(const acs_goalset *g, int *symmetric);
+int acs_goalset_path_frame(const acs_goalset *g, int64_t entry, int *root, int32_t *h_path, int path_cap,
+                           int *path_len, int *frame);
+int acs_bfs_batch_goal_hit_elements(acs_bfs_batch *b, int32_t *h_elem /* [n_search] */);
+int acs_greedy_goal_hit_elements(acs_greedy *g, int32_t *h_elem /* [n_search] */);
 
 /* ---- hash-partitioned multi-GPU BFS: per-rank device kernels --------------------------------- */
 /* The host loop (ac_solver_b200/search/sharded.py, one process per GPU, torch.distributed/NCCL
