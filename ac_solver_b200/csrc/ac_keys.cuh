@@ -17,10 +17,31 @@ constexpr uint64_t kNone = ~0ull;
 constexpr uint64_t kIdxMask = (1ull << 40) - 1;  // table slot = 24-bit fingerprint | 40-bit (index + 1)
 
 // ---- node keys: W 64-bit words per relator, length in the top 6 bits of the last word ----
+constexpr int kKeyLenShift = 58;  // 2 bits per letter below it: 29 letters per word, 61 in two
+constexpr int kMaxKeyMrl = 61;    // the longest relator a key holds (searches refuse wider rows)
+
+// words per relator for relators of up to mrl letters (1 <= mrl <= kMaxKeyMrl)
+__host__ __device__ constexpr int key_words(int mrl) { return mrl <= kKeyLenShift / 2 ? 1 : 2; }
+// words per node record: the 2W key words, the parent link and one word the engine chooses
+__host__ __device__ constexpr int node_words(int W) { return 2 * W + 2; }
+
 template <int W>
 struct Key {
     uint64_t k[2 * W];
 };
+
+// length of relator h of a key stored as 2W words (W at run time: records of either width)
+__host__ __device__ __forceinline__ int key_len(const uint64_t* k, int W, int h) {
+    return (int)(k[h * W + W - 1] >> kKeyLenShift);
+}
+template <int W>
+__host__ __device__ __forceinline__ int key_len(const Key<W>& q, int h) {
+    return key_len(q.k, W, h);
+}
+template <int W>
+__host__ __device__ __forceinline__ int key_total_len(const Key<W>& q) {
+    return key_len<W>(q, 0) + key_len<W>(q, 1);
+}
 
 template <int W>
 __host__ __device__ __forceinline__ bool key_eq(const Key<W>& a, const Key<W>& b) {
@@ -52,8 +73,8 @@ __device__ __forceinline__ Key<W> make_key(const Rel<2 * W>& r0, const Rel<2 * W
         q.k[i] = (uint64_t)r0.b.w[2 * i] | ((uint64_t)r0.b.w[2 * i + 1] << 32);
         q.k[W + i] = (uint64_t)r1.b.w[2 * i] | ((uint64_t)r1.b.w[2 * i + 1] << 32);
     }
-    q.k[W - 1] |= (uint64_t)r0.len << 58;
-    q.k[2 * W - 1] |= (uint64_t)r1.len << 58;
+    q.k[W - 1] |= (uint64_t)r0.len << kKeyLenShift;
+    q.k[2 * W - 1] |= (uint64_t)r1.len << kKeyLenShift;
     return q;
 }
 template <int W>
@@ -65,8 +86,8 @@ __device__ __forceinline__ void split_key(const Key<W>& q, Rel<2 * W>& r0, Rel<2
         r1.b.w[2 * i] = (uint32_t)q.k[W + i];
         r1.b.w[2 * i + 1] = (uint32_t)(q.k[W + i] >> 32);
     }
-    r0.len = (int)(q.k[W - 1] >> 58);
-    r1.len = (int)(q.k[2 * W - 1] >> 58);
+    r0.len = key_len<W>(q, 0);
+    r1.len = key_len<W>(q, 1);
     r0.b.w[2 * W - 1] &= (1u << 26) - 1;
     r1.b.w[2 * W - 1] &= (1u << 26) - 1;
 }
@@ -97,12 +118,13 @@ __device__ __forceinline__ void store_key(uint64_t* keys, uint64_t idx, const Ke
     }
 }
 
-// host-side packing of a root presentation; returns false if a letter is outside {+-1,+-2};
-// `valid` reports is_array_valid_presentation (utils.py:13-54)
+// host-side packing of a root presentation.  A bad letter (outside {+-1,+-2}) is reported at once;
+// otherwise a relator that is not zero right-padded outranks an empty one (utils.py:13-54 rejects both).
+enum class RootCheck { ok, bad_letter, not_padded, empty };
 template <int W>
-inline bool pack_root(const int8_t* p, int mrl, Key<W>& key, int lens[2], bool& valid) {
+inline RootCheck pack_root(const int8_t* p, int mrl, Key<W>& key, int lens[2]) {
     std::memset(&key, 0, sizeof(key));
-    valid = true;
+    bool padded = true, empty = false;
     for (int h = 0; h < 2; ++h) {
         int len = 0;
         bool seen_zero = false;
@@ -112,29 +134,57 @@ inline bool pack_root(const int8_t* p, int mrl, Key<W>& key, int lens[2], bool& 
                 seen_zero = true;
                 continue;
             }
-            if (v < -2 || v > 2) return false;
-            if (seen_zero) valid = false;  // not right-padded
+            if (v < -2 || v > 2) return RootCheck::bad_letter;
+            if (seen_zero) padded = false;
             const uint64_t code = (uint64_t)(((v < 0) ? 2 : 0) | (v & 1));
             const int bit = 2 * len;
             key.k[h * W + bit / 64] |= code << (bit % 64);
             ++len;
         }
         lens[h] = len;
-        key.k[h * W + W - 1] |= (uint64_t)len << 58;
-        if (len == 0) valid = false;
+        key.k[h * W + W - 1] |= (uint64_t)len << kKeyLenShift;
+        if (len == 0) empty = true;
     }
-    return true;
+    return !padded ? RootCheck::not_padded : empty ? RootCheck::empty : RootCheck::ok;
 }
 
-// visited nodes -> int8 rows (insertion order)
+// the same as a bool: false for a bad letter, and `valid` only for a root that packed cleanly
+// (the valid flag of acs_sbfs_pack_root)
 template <int W>
-__global__ void keys_unpack_kernel(const uint64_t* keys, int8_t* out, uint64_t n, int mrl) {
+inline bool pack_root(const int8_t* p, int mrl, Key<W>& key, int lens[2], bool& valid) {
+    const RootCheck rc = pack_root<W>(p, mrl, key, lens);
+    valid = rc == RootCheck::ok;
+    return rc != RootCheck::bad_letter;
+}
+
+// one node record (node_words(W) words) on the host
+template <int W>
+inline void node_pack(const Key<W>& key, int64_t link, int64_t tag, uint64_t* out) {
+    for (int i = 0; i < 2 * W; ++i) out[i] = key.k[i];
+    out[2 * W] = (uint64_t)link;
+    out[2 * W + 1] = (uint64_t)tag;
+}
+
+// n records of `stride` words (2W for flat key arrays, node_words(W) for node records) -> int8 rows in
+// record order; with gid_out, also word 2W + 1 of each node record (pbfs: the node's global id)
+template <int W>
+__global__ void records_unpack_kernel(const uint64_t* recs, int stride, int64_t* gid_out, int8_t* out, uint64_t n,
+                                      int mrl) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    const uint64_t* p = recs + i * stride;
+    Key<W> q;
+#pragma unroll
+    for (int j = 0; j < W; ++j) {
+        const ulonglong2 v = reinterpret_cast<const ulonglong2*>(p)[j];
+        q.k[2 * j] = v.x;
+        q.k[2 * j + 1] = v.y;
+    }
     Rel<2 * W> r0, r1;
-    split_key<W>(load_key<W>(keys, i), r0, r1);
+    split_key<W>(q, r0, r1);
     unpack_bytes<2 * W>(out + i * 2 * mrl, r0, mrl);
     unpack_bytes<2 * W>(out + i * 2 * mrl + mrl, r1, mrl);
+    if (gid_out) gid_out[i] = (int64_t)p[2 * W + 1];
 }
 
 }  // namespace acs

@@ -70,8 +70,8 @@ __host__ __device__ __forceinline__ Key<W> sym_apply(const Key<W>& q, int g) {
         o.k[i] = q.k[h * W + i];
         o.k[W + i] = q.k[(1 - h) * W + i];
     }
-    sym_letters<W>(o.k, (int)(o.k[W - 1] >> 58), g);
-    sym_letters<W>(o.k + W, (int)(o.k[2 * W - 1] >> 58), g);
+    sym_letters<W>(o.k, key_len<W>(o, 0), g);
+    sym_letters<W>(o.k + W, key_len<W>(o, 1), g);
     return o;
 }
 
@@ -89,7 +89,7 @@ __host__ __device__ __forceinline__ bool sym_less(const Key<W>& a, const Key<W>&
 // the canonical form c = g.q of q, and g (the smallest element giving c)
 template <int W>
 __host__ __device__ __forceinline__ Key<W> canonical(const Key<W>& q, int& g_out) {
-    const int l0 = (int)(q.k[W - 1] >> 58), l1 = (int)(q.k[2 * W - 1] >> 58);
+    const int l0 = key_len<W>(q, 0), l1 = key_len<W>(q, 1);
     Key<W> best = q;
     int bg = 0;
 #pragma unroll 1

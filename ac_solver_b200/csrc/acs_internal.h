@@ -1,7 +1,26 @@
 // acs_internal.h -- declarations shared by the translation units of libacsolver_b200.so.
 #pragma once
 #include <cstdint>
+#include <string>
+
 #include <cuda_runtime.h>
+
+// return the error of a failed CUDA call (acs::cuda_fail)
+#define ACS_CUDA(call)                                                \
+    do {                                                              \
+        const cudaError_t e__ = (call);                               \
+        if (e__ != cudaSuccess) return ::acs::cuda_fail(e__, #call);  \
+    } while (0)
+// cudaMalloc, or run `cleanup` and return ACS_ERR_NOMEM with the text "cudaMalloc(<ptr>): <CUDA error string>"
+#define ACS_ALLOC(ptr, bytes, cleanup)                                                                     \
+    do {                                                                                                   \
+        const cudaError_t e__ = cudaMalloc((void**)&(ptr), (size_t)(bytes));                               \
+        if (e__ != cudaSuccess) {                                                                          \
+            cudaGetLastError();                                                                            \
+            cleanup;                                                                                       \
+            return ::acs::fail(ACS_ERR_NOMEM, std::string("cudaMalloc(" #ptr "): ") + cudaGetErrorString(e__)); \
+        }                                                                                                  \
+    } while (0)
 
 namespace acs {
 
@@ -31,6 +50,21 @@ struct StepParams {
 
 // thread-local error text behind acs_last_error() (capi.cu)
 void set_last_error(const char* msg);
+// sets the error text and returns code
+int fail(int code, const std::string& msg);
+// a failed CUDA call: clears the runtime's last error and returns ACS_ERR_NOMEM for an allocation failure,
+// ACS_ERR_CUDA for any other, with the text "<what>: <CUDA error string>"
+int cuda_fail(cudaError_t e, const std::string& what);
+// selects `device` for the calling thread: ACS_ERR_NO_DEVICE without a visible device, ACS_ERR_INVALID
+// for an index out of range ("<who>: device index out of range")
+int open_device(int device, const char* who);
+// ACS_ERR_UNSUPPORTED unless a packed key holds relators of mrl letters
+// ("<who> needs 1 <= max_relator_length <= 61")
+int check_key_mrl(int mrl, const char* who);
+// n visited records of `stride` words (see records_unpack_kernel, ac_keys.cuh) -> int8 rows in host memory,
+// and with h_gid the global id word of each node record; synchronises `s`
+int records_to_host(int W, const uint64_t* d_recs, int stride, int64_t n, int mrl, int8_t* h_rows, int64_t* h_gid,
+                    cudaStream_t s);
 
 cudaError_t launch_step(const StepParams& P, cudaStream_t s);
 

@@ -417,23 +417,6 @@ __global__ void __launch_bounds__(256) ball_count_kernel(const uint32_t* root_of
 using namespace acs;
 
 namespace {
-int ball_fail(int code, const std::string& m) {
-    acs::set_last_error(m.c_str());
-    return code;
-}
-#define BALL_CUDA(call)                                                                        \
-    do {                                                                                       \
-        cudaError_t e__ = (call);                                                              \
-        if (e__ != cudaSuccess) {                                                              \
-            cudaGetLastError();                                                                \
-            free_all();                                                                        \
-            return ball_fail(e__ == cudaErrorMemoryAllocation ? ACS_ERR_NOMEM : ACS_ERR_CUDA,  \
-                             std::string(#call) + ": " + cudaGetErrorString(e__));             \
-        }                                                                                      \
-    } while (0)
-}  // namespace
-
-namespace {
 
 // Breadth-first exploration from n_roots start presentations at once (each node carries its root's index, and
 // the visited set is keyed by (root, state), so the runs are independent but share every kernel launch).
@@ -441,22 +424,17 @@ namespace {
 int ball_run(int device, const int8_t* h_letters, const int64_t* off, int n_roots, int radius, int size_cap, int classic,
              int64_t max_nodes, int64_t* n_nodes_out, int64_t* h_counts, uint16_t* h_sizes, uint8_t* h_levels,
              int64_t cap_nodes, uint32_t* h_edges, int64_t cap_edges, int64_t* n_edges_out) {
-    if (!h_letters || !off || n_roots < 1 || max_nodes < n_roots) return ball_fail(ACS_ERR_INVALID, "ball: bad argument");
-    if (max_nodes > (int64_t)3500000000ll) return ball_fail(ACS_ERR_UNSUPPORTED, "ball: node indices are 32-bit (max_nodes <= 3.5e9)");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        return ball_fail(ACS_ERR_NO_DEVICE, "no CUDA device visible; there is no CPU fallback");
-    }
-    if (cudaSetDevice(device) != cudaSuccess) return ball_fail(ACS_ERR_CUDA, "ball: cudaSetDevice");
+    if (!h_letters || !off || n_roots < 1 || max_nodes < n_roots) return fail(ACS_ERR_INVALID, "ball: bad argument");
+    if (max_nodes > (int64_t)3500000000ll) return fail(ACS_ERR_UNSUPPORTED, "ball: node indices are 32-bit (max_nodes <= 3.5e9)");
+    if (const int rc = open_device(device, "ball")) return rc;
     int max_len = 1;
     for (int r = 0; r < n_roots; ++r) {
         const int64_t a = off[2 * r], b = off[2 * r + 1], c = off[2 * r + 2];
-        if (a > b || b > c) return ball_fail(ACS_ERR_INVALID, "ball: offsets must be non-decreasing");
+        if (a > b || b > c) return fail(ACS_ERR_INVALID, "ball: offsets must be non-decreasing");
         max_len = std::max<int>(max_len, (int)std::max(b - a, c - b));
     }
     for (int64_t i = 0; i < off[2 * n_roots]; ++i)
-        if (h_letters[i] == 0 || h_letters[i] < -2 || h_letters[i] > 2) return ball_fail(ACS_ERR_INVALID, "ball: letters must be +-1, +-2");
+        if (h_letters[i] == 0 || h_letters[i] < -2 || h_letters[i] > 2) return fail(ACS_ERR_INVALID, "ball: letters must be +-1, +-2");
     bool literal = false;  // a start word with an adjacent inverse pair: the whole run follows the reference's reduce_ literally
     for (int k = 0; k < 2 * n_roots && !literal; ++k)
         for (int64_t i = off[k]; i + 1 < off[k + 1]; ++i)
@@ -498,20 +476,24 @@ int ball_run(int device, const int8_t* h_letters, const int64_t* off, int n_root
         cudaFree(d_edges);
         cudaFree(d_counts);
     };
-    BALL_CUDA(cudaMalloc((void**)&A.nodes, cap * 2 * L));
-    BALL_CUDA(cudaMalloc((void**)&A.lens, cap * 4));
-    BALL_CUDA(cudaMalloc((void**)&A.level, cap));
-    BALL_CUDA(cudaMalloc((void**)&A.root_of, cap * 4));
-    BALL_CUDA(cudaMalloc((void**)&A.table, tcap * 8));
-    BALL_CUDA(cudaMalloc((void**)&A.cand, ccap * 2 * L));
-    BALL_CUDA(cudaMalloc((void**)&A.cand_lens, ccap * 4));
-    BALL_CUDA(cudaMalloc((void**)&A.cand_slot, ccap * 4));
-    BALL_CUDA(cudaMalloc((void**)&A.cand_node, ccap * 4));
-    BALL_CUDA(cudaMalloc((void**)&A.rank, (ccap + 1) * 4));
-    BALL_CUDA(cudaMalloc((void**)&A.win, ccap));
-    BALL_CUDA(cudaMalloc((void**)&A.ctrl, 4 * 8));
+    struct FreeOnExit {  // every return from here on releases the device buffers
+        decltype(free_all)& f;
+        ~FreeOnExit() { f(); }
+    } free_on_exit{free_all};
+    ACS_CUDA(cudaMalloc((void**)&A.nodes, cap * 2 * L));
+    ACS_CUDA(cudaMalloc((void**)&A.lens, cap * 4));
+    ACS_CUDA(cudaMalloc((void**)&A.level, cap));
+    ACS_CUDA(cudaMalloc((void**)&A.root_of, cap * 4));
+    ACS_CUDA(cudaMalloc((void**)&A.table, tcap * 8));
+    ACS_CUDA(cudaMalloc((void**)&A.cand, ccap * 2 * L));
+    ACS_CUDA(cudaMalloc((void**)&A.cand_lens, ccap * 4));
+    ACS_CUDA(cudaMalloc((void**)&A.cand_slot, ccap * 4));
+    ACS_CUDA(cudaMalloc((void**)&A.cand_node, ccap * 4));
+    ACS_CUDA(cudaMalloc((void**)&A.rank, (ccap + 1) * 4));
+    ACS_CUDA(cudaMalloc((void**)&A.win, ccap));
+    ACS_CUDA(cudaMalloc((void**)&A.ctrl, 4 * 8));
     const bool want_edges = h_edges != nullptr && cap_edges > 0;
-    if (want_edges) BALL_CUDA(cudaMalloc((void**)&d_edges, ccap * 3 * 4));
+    if (want_edges) ACS_CUDA(cudaMalloc((void**)&d_edges, ccap * 3 * 4));
     A.edges = d_edges;
     A.tmask = tcap - 1;
     A.L = L;
@@ -520,8 +502,8 @@ int ball_run(int device, const int8_t* h_letters, const int64_t* off, int n_root
     A.size_cap = size_cap;
     A.want_edges = want_edges ? 1 : 0;
     A.literal = literal ? 1 : 0;
-    BALL_CUDA(cudaMemset(A.table, 0, tcap * 8));
-    BALL_CUDA(cudaMemset(A.ctrl, 0, 32));
+    ACS_CUDA(cudaMemset(A.table, 0, tcap * 8));
+    ACS_CUDA(cudaMemset(A.ctrl, 0, 32));
     // roots: the sorted pairs (sort_, AC_UTILS_no_hash.cpp:131-147) as nodes 0 .. n_roots-1, level 0
     {
         std::vector<int8_t> rows((size_t)n_roots * 2 * L, 0);
@@ -542,10 +524,8 @@ int ball_run(int device, const int8_t* h_letters, const int64_t* off, int n_root
             const int lf = keep ? len1 : len2;
             const int8_t* sd = keep ? y : x;
             const int ls = keep ? len2 : len1;
-            if (lf > L || ls > L) {
-                free_all();
-                return ball_fail(ACS_ERR_UNSUPPORTED, "ball: relators longer than 512 letters are not supported");
-            }
+            if (lf > L || ls > L)
+                return fail(ACS_ERR_UNSUPPORTED, "ball: relators longer than 512 letters are not supported");
             int8_t* row = rows.data() + (size_t)r * 2 * L;
             std::memcpy(row, f, lf);
             std::memcpy(row + L, sd, ls);
@@ -553,10 +533,10 @@ int ball_run(int device, const int8_t* h_letters, const int64_t* off, int n_root
             lens[2 * r + 1] = (uint16_t)ls;
             roots[r] = (uint32_t)r;
         }
-        BALL_CUDA(cudaMemcpy(A.nodes, rows.data(), rows.size(), cudaMemcpyHostToDevice));
-        BALL_CUDA(cudaMemcpy(A.lens, lens.data(), lens.size() * 2, cudaMemcpyHostToDevice));
-        BALL_CUDA(cudaMemset(A.level, 0, n_roots));
-        BALL_CUDA(cudaMemcpy(A.root_of, roots.data(), roots.size() * 4, cudaMemcpyHostToDevice));
+        ACS_CUDA(cudaMemcpy(A.nodes, rows.data(), rows.size(), cudaMemcpyHostToDevice));
+        ACS_CUDA(cudaMemcpy(A.lens, lens.data(), lens.size() * 2, cudaMemcpyHostToDevice));
+        ACS_CUDA(cudaMemset(A.level, 0, n_roots));
+        ACS_CUDA(cudaMemcpy(A.root_of, roots.data(), roots.size() * 4, cudaMemcpyHostToDevice));
         ball_roots_kernel<<<(n_roots + 255) / 256, 256>>>(A, n_roots);
     }
     uint64_t n_nodes = (uint64_t)n_roots, head = 0, level_end = (uint64_t)n_roots;
@@ -580,22 +560,15 @@ int ball_run(int device, const int8_t* h_letters, const int64_t* off, int n_root
         ball_fix_kernel<<<blocks, kBallThreads>>>(A);
         if (want_edges) ball_edges_kernel<<<1, 1024>>>(A, 0);
         unsigned long long ctrl[4];
-        BALL_CUDA(cudaMemcpy(ctrl, A.ctrl, 32, cudaMemcpyDeviceToHost));
-        if (ctrl[0]) {
-            free_all();
-            return ball_fail(ACS_ERR_UNSUPPORTED, "ball: a relator outgrew the 512-letter stride");
-        }
-        if (n_nodes + ctrl[1] > cap) {
-            free_all();
-            return ball_fail(ACS_ERR_NOMEM, "ball: more states than max_nodes");
-        }
+        ACS_CUDA(cudaMemcpy(ctrl, A.ctrl, 32, cudaMemcpyDeviceToHost));
+        if (ctrl[0])
+            return fail(ACS_ERR_UNSUPPORTED, "ball: a relator outgrew the 512-letter stride");
+        if (n_nodes + ctrl[1] > cap) return fail(ACS_ERR_NOMEM, "ball: more states than max_nodes");
         if (want_edges && ctrl[2]) {
             const int64_t ne = (int64_t)ctrl[2];
-            if (n_edges + ne > cap_edges) {
-                free_all();
-                return ball_fail(ACS_ERR_NOMEM, "ball: more edges than cap_edges");
-            }
-            BALL_CUDA(cudaMemcpy(h_edges + 3 * n_edges, d_edges, (size_t)ne * 12, cudaMemcpyDeviceToHost));
+            if (n_edges + ne > cap_edges)
+                return fail(ACS_ERR_NOMEM, "ball: more edges than cap_edges");
+            ACS_CUDA(cudaMemcpy(h_edges + 3 * n_edges, d_edges, (size_t)ne * 12, cudaMemcpyDeviceToHost));
             n_edges += ne;
         }
         n_nodes += ctrl[1];
@@ -604,19 +577,18 @@ int ball_run(int device, const int8_t* h_letters, const int64_t* off, int n_root
     if (n_nodes_out) *n_nodes_out = (int64_t)n_nodes;
     if (n_edges_out) *n_edges_out = n_edges;
     if (h_counts) {
-        BALL_CUDA(cudaMalloc((void**)&d_counts, (size_t)n_roots * 8));
-        BALL_CUDA(cudaMemset(d_counts, 0, (size_t)n_roots * 8));
+        ACS_CUDA(cudaMalloc((void**)&d_counts, (size_t)n_roots * 8));
+        ACS_CUDA(cudaMemset(d_counts, 0, (size_t)n_roots * 8));
         ball_count_kernel<<<(unsigned)((n_nodes + 255) / 256), 256>>>(A.root_of, n_nodes, d_counts);
-        BALL_CUDA(cudaMemcpy(h_counts, d_counts, (size_t)n_roots * 8, cudaMemcpyDeviceToHost));
+        ACS_CUDA(cudaMemcpy(h_counts, d_counts, (size_t)n_roots * 8, cudaMemcpyDeviceToHost));
     }
     const uint64_t ncopy = std::min<uint64_t>(n_nodes, (uint64_t)std::max<int64_t>(cap_nodes, 0));
     if (h_sizes && ncopy) {
         std::vector<uint16_t> lens(2 * ncopy);
-        BALL_CUDA(cudaMemcpy(lens.data(), A.lens, ncopy * 4, cudaMemcpyDeviceToHost));
+        ACS_CUDA(cudaMemcpy(lens.data(), A.lens, ncopy * 4, cudaMemcpyDeviceToHost));
         for (uint64_t i = 0; i < ncopy; ++i) h_sizes[i] = (uint16_t)(lens[2 * i] + lens[2 * i + 1]);
     }
-    if (h_levels && ncopy) BALL_CUDA(cudaMemcpy(h_levels, A.level, ncopy, cudaMemcpyDeviceToHost));
-    free_all();
+    if (h_levels && ncopy) ACS_CUDA(cudaMemcpy(h_levels, A.level, ncopy, cudaMemcpyDeviceToHost));
     return ACS_OK;
 }
 
@@ -635,7 +607,7 @@ extern "C" {
 int acs_ball_explore(int device, const int8_t* h_letters, int len1, int len2, int radius, int size_cap, int classic,
                      int64_t max_nodes, int64_t* n_nodes_out, uint16_t* h_sizes, uint8_t* h_levels, int64_t cap_nodes,
                      uint32_t* h_edges, int64_t cap_edges, int64_t* n_edges_out) {
-    if (!h_letters || len1 < 0 || len2 < 0 || max_nodes < 1) return ball_fail(ACS_ERR_INVALID, "ball: bad argument");
+    if (!h_letters || len1 < 0 || len2 < 0 || max_nodes < 1) return fail(ACS_ERR_INVALID, "ball: bad argument");
     const int64_t off[3] = {0, len1, (int64_t)len1 + len2};
     return ball_run(device, h_letters, off, 1, radius, size_cap, classic, max_nodes, n_nodes_out, nullptr, h_sizes, h_levels,
                     cap_nodes, h_edges, cap_edges, n_edges_out);
@@ -647,7 +619,7 @@ int acs_ball_explore(int device, const int8_t* h_letters, int len1, int len2, in
  * max_nodes bounds the SUM of the ball sizes (ACS_ERR_NOMEM if exceeded: split the batch). */
 int acs_ball_sizes(int device, const int8_t* h_letters, const int64_t* h_off, int n_roots, int radius, int classic,
                    int64_t max_nodes, int64_t* h_counts) {
-    if (!h_counts || radius < 0) return ball_fail(ACS_ERR_INVALID, "ball: bad argument");
+    if (!h_counts || radius < 0) return fail(ACS_ERR_INVALID, "ball: bad argument");
     return ball_run(device, h_letters, h_off, n_roots, radius, 0, classic, max_nodes, nullptr, h_counts, nullptr, nullptr, 0,
                     nullptr, 0, nullptr);
 }

@@ -15,7 +15,7 @@ constexpr int kScanT = 256, kScanPer = 8, kScanBlock = kScanT * kScanPer;  // wo
 template <int W>
 __device__ __forceinline__ Key<W> node_key(const uint64_t* nodes, uint64_t idx) {
     Key<W> q;
-    const ulonglong2* p = reinterpret_cast<const ulonglong2*>(nodes + idx * (2 * W + 2));
+    const ulonglong2* p = reinterpret_cast<const ulonglong2*>(nodes + idx * node_words(W));
 #pragma unroll
     for (int i = 0; i < W; ++i) {
         const ulonglong2 v = p[i];
@@ -26,7 +26,7 @@ __device__ __forceinline__ Key<W> node_key(const uint64_t* nodes, uint64_t idx) 
 }
 template <int W>
 __device__ __forceinline__ void node_load(const uint64_t* nodes, uint64_t idx, Key<W>& q, int64_t& parent, int64_t& gid) {
-    const ulonglong2* p = reinterpret_cast<const ulonglong2*>(nodes + idx * (2 * W + 2));
+    const ulonglong2* p = reinterpret_cast<const ulonglong2*>(nodes + idx * node_words(W));
 #pragma unroll
     for (int i = 0; i < W; ++i) {
         const ulonglong2 v = p[i];
@@ -39,7 +39,7 @@ __device__ __forceinline__ void node_load(const uint64_t* nodes, uint64_t idx, K
 }
 template <int W>
 __device__ __forceinline__ void node_store(uint64_t* nodes, uint64_t idx, const Key<W>& q, int64_t parent, int64_t gid) {
-    uint64_t* p = nodes + idx * (2 * W + 2);
+    uint64_t* p = nodes + idx * node_words(W);
     if constexpr (W == 1) {  // one 256-bit store: one memory request per node
         asm volatile("st.global.v4.u64 [%0], {%1,%2,%3,%4};" ::"l"(p), "l"(q.k[0]), "l"(q.k[1]), "l"((uint64_t)parent),
                      "l"((uint64_t)gid)

@@ -10,25 +10,15 @@
 #include <cuda_runtime.h>
 
 #include "../../include/acsolver_b200.h"
+#include "ac_keys.cuh"
 #include "acs_internal.h"
+
+using acs::cuda_fail;
+using acs::fail;
 
 namespace {
 
 thread_local std::string g_err;
-
-int fail(int code, const char* what) {
-    g_err = what ? what : "";
-    return code;
-}
-int cuda_fail(cudaError_t e, const char* where) {
-    g_err = std::string(where) + ": " + cudaGetErrorString(e);
-    return e == cudaErrorMemoryAllocation ? ACS_ERR_NOMEM : ACS_ERR_CUDA;
-}
-#define ACS_CUDA(call)                                          \
-    do {                                                        \
-        cudaError_t e__ = (call);                               \
-        if (e__ != cudaSuccess) return cuda_fail(e__, #call);   \
-    } while (0)
 
 constexpr int kStreams = 3;
 constexpr int64_t kChunkRows = 1 << 17;  // rows per pipeline chunk of the *_host calls
@@ -62,6 +52,51 @@ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 namespace acs {
 void set_last_error(const char* msg) { g_err = msg ? msg : ""; }
+
+int fail(int code, const std::string& msg) {
+    g_err = msg;
+    return code;
+}
+
+int cuda_fail(cudaError_t e, const std::string& what) {
+    cudaGetLastError();
+    return fail(e == cudaErrorMemoryAllocation ? ACS_ERR_NOMEM : ACS_ERR_CUDA, what + ": " + cudaGetErrorString(e));
+}
+
+int open_device(int device, const char* who) {
+    int n = 0;
+    if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) {
+        cudaGetLastError();
+        return fail(ACS_ERR_NO_DEVICE, "no CUDA device visible; there is no CPU fallback");
+    }
+    if (device < 0 || device >= n) return fail(ACS_ERR_INVALID, std::string(who) + ": device index out of range");
+    ACS_CUDA(cudaSetDevice(device));
+    return ACS_OK;
+}
+
+int check_key_mrl(int mrl, const char* who) {
+    if (mrl >= 1 && mrl <= kMaxKeyMrl) return ACS_OK;
+    return fail(ACS_ERR_UNSUPPORTED, std::string(who) + " needs 1 <= max_relator_length <= " + std::to_string(kMaxKeyMrl));
+}
+
+int records_to_host(int W, const uint64_t* d_recs, int stride, int64_t n, int mrl, int8_t* h_rows, int64_t* h_gid,
+                    cudaStream_t s) {
+    if (n <= 0) return ACS_OK;
+    int8_t* d = nullptr;
+    int64_t* dg = nullptr;
+    ACS_ALLOC(d, n * 2 * mrl, (void)0);
+    if (h_gid) ACS_ALLOC(dg, n * 8, cudaFree(d));
+    const unsigned grid = (unsigned)((n + 255) / 256);
+    if (W == 1) records_unpack_kernel<1><<<grid, 256, 0, s>>>(d_recs, stride, dg, d, (uint64_t)n, mrl);
+    else records_unpack_kernel<2><<<grid, 256, 0, s>>>(d_recs, stride, dg, d, (uint64_t)n, mrl);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(h_rows, d, (size_t)n * 2 * mrl, cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess && h_gid) e = cudaMemcpyAsync(h_gid, dg, (size_t)n * 8, cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    cudaFree(dg);
+    cudaFree(d);
+    return e == cudaSuccess ? ACS_OK : cuda_fail(e, "visited rows");
+}
 }  // namespace acs
 
 struct acs_ctx {
@@ -93,10 +128,7 @@ int acs_device_count(void) {
 int acs_ctx_create(int device, acs_ctx** out) {
     if (!out) return fail(ACS_ERR_INVALID, "out is null");
     *out = nullptr;
-    int n = acs_device_count();
-    if (n <= 0) return fail(ACS_ERR_NO_DEVICE, "no CUDA device visible; this library has no CPU fallback");
-    if (device < 0 || device >= n) return fail(ACS_ERR_INVALID, "device index out of range");
-    ACS_CUDA(cudaSetDevice(device));
+    if (const int rc = acs::open_device(device, "acs_ctx_create")) return rc;
     acs_ctx* c = new acs_ctx();
     c->device = device;
     cudaError_t e = cudaSuccess;

@@ -97,15 +97,10 @@ __global__ void gs_path_kernel(const uint64_t* nodes, int64_t entry, int32_t* pa
         Q = sym_mul(Q, (int)((uint64_t)r >> 32) & 15);
         if (pos < path_cap) {
             path[2 * pos] = pl < 0 ? -1 : sym_pi(sym_mul(sym_inv(P), Q), (int)(pl & 15));
-            path[2 * pos + 1] = (int32_t)(k.k[W - 1] >> 58) + (int32_t)(k.k[2 * W - 1] >> 58);
+            path[2 * pos + 1] = key_total_len<W>(k);
         }
         e = pl < 0 ? -1 : (pl >> 4);
     }
-}
-
-inline int gs_fail(int code, const std::string& m) {
-    set_last_error(m.c_str());
-    return code;
 }
 
 int goalset_index(acs_goalset* g, cudaStream_t s) {
@@ -114,7 +109,7 @@ int goalset_index(acs_goalset* g, cudaStream_t s) {
     g->tcap = t;
     if (cudaMalloc((void**)&g->table, t * 8) != cudaSuccess) {
         cudaGetLastError();
-        return gs_fail(ACS_ERR_NOMEM, "goalset: cudaMalloc of the index failed");
+        return fail(ACS_ERR_NOMEM, "goalset: cudaMalloc of the index failed");
     }
     int* d_flag = nullptr;
     unsigned long long* d_count = nullptr;
@@ -145,9 +140,9 @@ int goalset_index(acs_goalset* g, cudaStream_t s) {
     if (d_flag) cudaFree(d_flag);
     if (e != cudaSuccess) {
         cudaGetLastError();
-        return gs_fail(ACS_ERR_CUDA, std::string("goalset: building the index: ") + cudaGetErrorString(e));
+        return fail(ACS_ERR_CUDA, std::string("goalset: building the index: ") + cudaGetErrorString(e));
     }
-    if (flag) return gs_fail(ACS_ERR_CUDA, "goalset: internal error: index full");
+    if (flag) return fail(ACS_ERR_CUDA, "goalset: internal error: index full");
     g->n_states = (int64_t)count;
     return ACS_OK;
 }
@@ -188,18 +183,14 @@ std::string gs_row_problem(const int8_t* p, int mrl, int cyclical) {
 
 template <int W>
 void gs_pack(const int8_t* h_rows, int64_t n, int mrl, int symmetric, std::vector<uint64_t>& nodes) {
-    nodes.assign((size_t)std::max<int64_t>(n, 1) * (2 * W + 2), 0);
+    nodes.assign((size_t)std::max<int64_t>(n, 1) * node_words(W), 0);
     for (int64_t i = 0; i < n; ++i) {
         Key<W> key;
         int lens[2];
-        bool valid;
-        pack_root<W>(h_rows + (size_t)i * 2 * mrl, mrl, key, lens, valid);
+        pack_root<W>(h_rows + (size_t)i * 2 * mrl, mrl, key, lens);  // gs_row_problem has accepted the row
         int g = 0;
         if (symmetric) key = canonical<W>(key, g);
-        uint64_t* q = nodes.data() + (size_t)i * (2 * W + 2);
-        for (int j = 0; j < 2 * W; ++j) q[j] = key.k[j];
-        q[2 * W] = ~0ull;  // parent link -1
-        q[2 * W + 1] = (uint64_t)i | (uint64_t)g << 32;
+        node_pack<W>(key, -1, i | (int64_t)g << 32, nodes.data() + (size_t)i * node_words(W));
     }
 }
 
@@ -211,29 +202,20 @@ namespace {
 int gs_from_rows(int device, int mrl, int cyclical, int symmetric, const int8_t* h_rows, int64_t n, acs_goalset** out) {
     if (!out) return ACS_ERR_INVALID;
     *out = nullptr;
-    if (mrl < 1 || mrl > 61) return gs_fail(ACS_ERR_UNSUPPORTED, "goalset needs 1 <= max_relator_length <= 61");
-    if (n < 0 || (n > 0 && !h_rows)) return gs_fail(ACS_ERR_INVALID, "goalset: bad row count or rows");
-    if (n >= (int64_t)kGsIdx) return gs_fail(ACS_ERR_UNSUPPORTED, "goalset: too many rows");
+    if (const int rc = check_key_mrl(mrl, "goalset")) return rc;
+    if (n < 0 || (n > 0 && !h_rows)) return fail(ACS_ERR_INVALID, "goalset: bad row count or rows");
+    if (n >= (int64_t)kGsIdx) return fail(ACS_ERR_UNSUPPORTED, "goalset: too many rows");
     for (int64_t i = 0; i < n; ++i) {
         const std::string why = gs_row_problem(h_rows + (size_t)i * 2 * mrl, mrl, cyclical);
         if (!why.empty())
-            return gs_fail(ACS_ERR_INVALID, "goalset: row " + std::to_string(i) + " has " + why +
+            return fail(ACS_ERR_INVALID, "goalset: row " + std::to_string(i) + " has " + why +
                                                 ", so no search can generate it");
     }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        return gs_fail(ACS_ERR_NO_DEVICE, "no CUDA device visible; there is no CPU fallback");
-    }
-    if (device < 0 || device >= ndev) return gs_fail(ACS_ERR_INVALID, "goalset: device index out of range");
-    if (cudaSetDevice(device) != cudaSuccess) {
-        cudaGetLastError();
-        return gs_fail(ACS_ERR_CUDA, "goalset: cudaSetDevice failed");
-    }
+    if (const int rc = open_device(device, "goalset")) return rc;
     acs_goalset* g = new acs_goalset();
     g->device = device;
     g->mrl = mrl;
-    g->W = mrl <= 29 ? 1 : 2;
+    g->W = key_words(mrl);
     g->cyclical = cyclical ? 1 : 0;
     g->symmetric = symmetric ? 1 : 0;
     g->n_entries = n;
@@ -243,12 +225,12 @@ int gs_from_rows(int device, int mrl, int cyclical, int symmetric, const int8_t*
     if (cudaMalloc((void**)&g->nodes, h.size() * 8) != cudaSuccess) {
         cudaGetLastError();
         goalset_free(g);
-        return gs_fail(ACS_ERR_NOMEM, "goalset: cudaMalloc of the entries failed");
+        return fail(ACS_ERR_NOMEM, "goalset: cudaMalloc of the entries failed");
     }
     if (cudaMemcpy(g->nodes, h.data(), h.size() * 8, cudaMemcpyHostToDevice) != cudaSuccess) {
         cudaGetLastError();
         goalset_free(g);
-        return gs_fail(ACS_ERR_CUDA, "goalset: uploading the entries failed");
+        return fail(ACS_ERR_CUDA, "goalset: uploading the entries failed");
     }
     const int rc = goalset_index(g, 0);
     if (rc != ACS_OK) {
@@ -279,7 +261,7 @@ int acs_goalset_size(const acs_goalset* g, int64_t* n_entries, int64_t* n_states
     if (!g) return ACS_ERR_INVALID;
     if (n_entries) *n_entries = g->n_entries;
     if (n_states) *n_states = g->n_states;
-    if (bytes) *bytes = std::max<int64_t>(g->n_entries, 1) * 8 * (2 * g->W + 2) + (int64_t)g->tcap * 8;
+    if (bytes) *bytes = std::max<int64_t>(g->n_entries, 1) * 8 * node_words(g->W) + (int64_t)g->tcap * 8;
     return ACS_OK;
 }
 
@@ -290,10 +272,10 @@ int acs_goalset_path(const acs_goalset* g, int64_t entry, int* root, int32_t* h_
 int acs_goalset_path_frame(const acs_goalset* g, int64_t entry, int* root, int32_t* h_path, int path_cap, int* path_len,
                            int* frame) {
     if (!g || path_cap < 0 || (!h_path && path_cap > 0)) return ACS_ERR_INVALID;
-    if (entry < 0 || entry >= g->n_entries) return gs_fail(ACS_ERR_INVALID, "goalset_path: entry out of range");
+    if (entry < 0 || entry >= g->n_entries) return fail(ACS_ERR_INVALID, "goalset_path: entry out of range");
     if (cudaSetDevice(g->device) != cudaSuccess) {
         cudaGetLastError();
-        return gs_fail(ACS_ERR_CUDA, "goalset_path: cudaSetDevice failed");
+        return fail(ACS_ERR_CUDA, "goalset_path: cudaSetDevice failed");
     }
     const int cap = std::max(path_cap, 1);
     int32_t* d = nullptr;
@@ -310,12 +292,12 @@ int acs_goalset_path_frame(const acs_goalset* g, int64_t entry, int* root, int32
     if (d) cudaFree(d);
     if (e != cudaSuccess) {
         cudaGetLastError();
-        return gs_fail(ACS_ERR_CUDA, std::string("goalset_path: ") + cudaGetErrorString(e));
+        return fail(ACS_ERR_CUDA, std::string("goalset_path: ") + cudaGetErrorString(e));
     }
     if (path_len) *path_len = res[0];
     if (root) *root = res[1];
     if (frame) *frame = res[2];
-    if (res[0] > path_cap) return gs_fail(ACS_ERR_INVALID, "goalset_path: the path is longer than path_cap (see path_len)");
+    if (res[0] > path_cap) return fail(ACS_ERR_INVALID, "goalset_path: the path is longer than path_cap (see path_len)");
     return ACS_OK;
 }
 

@@ -131,7 +131,7 @@ __global__ void __launch_bounds__(32) greedy_kernel(const GreedyArgs A, const Go
     Key<W> root;
 #pragma unroll
     for (int i = 0; i < 2 * W; ++i) root.k[i] = A.roots[(uint64_t)sidx * 2 * W + i];
-    const int L0 = (int)(root.k[W - 1] >> 58) + (int)(root.k[2 * W - 1] >> 58);
+    const int L0 = key_total_len<W>(root);
     if (lane == 0) {
         store_key<W>(keys, 0, root);
         parent[0] = kNone;
@@ -396,7 +396,7 @@ __global__ void greedy_path_kernel(const GreedyArgs A, int32_t* paths, int path_
         const bool root = parent[q] == kNone;
         if (pos < path_cap) {
             path[2 * pos] = root ? -1 : (int)(parent[q] & 15);
-            path[2 * pos + 1] = (int)(k.k[W - 1] >> 58) + (int)(k.k[2 * W - 1] >> 58);
+            path[2 * pos + 1] = key_total_len<W>(k);
         }
         if (root) break;
     }
@@ -455,16 +455,6 @@ struct acs_greedy {
     bool ran = false, ran_with_goals = false;
 };
 
-#define GR_CUDA(call)                                                                   \
-    do {                                                                                \
-        cudaError_t e__ = (call);                                                       \
-        if (e__ != cudaSuccess) {                                                       \
-            acs::set_last_error((std::string(#call) + ": " + cudaGetErrorString(e__)).c_str()); \
-            cudaGetLastError();                                                         \
-            return e__ == cudaErrorMemoryAllocation ? ACS_ERR_NOMEM : ACS_ERR_CUDA;     \
-        }                                                                               \
-    } while (0)
-
 extern "C" void acs_greedy_destroy(acs_greedy* g) {
     if (!g) return;
     cudaSetDevice(g->device);
@@ -497,25 +487,14 @@ extern "C" int acs_greedy_create(int device, int n_search, int mrl, int64_t max_
                                  acs_greedy** out) {
     if (!out) return ACS_ERR_INVALID;
     *out = nullptr;
-    if (mrl < 1 || mrl > 61) {
-        acs::set_last_error("greedy needs 1 <= max_relator_length <= 61");
-        return ACS_ERR_UNSUPPORTED;
-    }
-    if (n_search < 1 || max_nodes < 0 || path_cap < 2 || max_nodes > (1ll << 24) - 32) {
-        acs::set_last_error("greedy: need n_search >= 1, 0 <= max_nodes < 2^24 - 32, path_cap >= 2");
-        return ACS_ERR_INVALID;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        acs::set_last_error("no CUDA device visible; there is no CPU fallback");
-        return ACS_ERR_NO_DEVICE;
-    }
-    GR_CUDA(cudaSetDevice(device));
+    if (const int rc = check_key_mrl(mrl, "greedy")) return rc;
+    if (n_search < 1 || max_nodes < 0 || path_cap < 2 || max_nodes > (1ll << 24) - 32)
+        return fail(ACS_ERR_INVALID, "greedy: need n_search >= 1, 0 <= max_nodes < 2^24 - 32, path_cap >= 2");
+    if (const int rc = open_device(device, "greedy")) return rc;
     acs_greedy* g = new acs_greedy();
     g->device = device;
     g->mrl = mrl;
-    g->W = mrl <= 29 ? 1 : 2;
+    g->W = key_words(mrl);
     g->cyclical = cyclical ? 1 : 0;
     g->n_search = n_search;
     g->budget = max_nodes;
@@ -525,45 +504,34 @@ extern "C" int acs_greedy_create(int device, int n_search, int mrl, int64_t max_
     g->tcap = t;
     g->path_cap = path_cap;
     const uint64_t S = (uint64_t)n_search;
-    auto fail = [&](int rc) {
-        acs_greedy_destroy(g);
-        return rc;
-    };
-#define GR_ALLOC(ptr, bytes)                                                                        \
-    do {                                                                                            \
-        cudaError_t e__ = cudaMalloc((void**)&(ptr), (bytes));                                      \
-        if (e__ != cudaSuccess) {                                                                   \
-            acs::set_last_error((std::string("cudaMalloc(" #ptr "): ") + cudaGetErrorString(e__)).c_str()); \
-            cudaGetLastError();                                                                     \
-            return fail(ACS_ERR_NOMEM);                                                             \
-        }                                                                                           \
-    } while (0)
-    GR_ALLOC(g->keys, S * g->cap * 2 * g->W * sizeof(uint64_t));
-    GR_ALLOC(g->parent, S * g->cap * sizeof(uint64_t));
-    GR_ALLOC(g->depth, S * g->cap * sizeof(uint32_t));
-    GR_ALLOC(g->heap, S * g->cap * sizeof(uint64_t));
-    GR_ALLOC(g->table, S * g->tcap * sizeof(uint64_t));
-    GR_ALLOC(g->roots, S * 2 * g->W * sizeof(uint64_t));
-    GR_ALLOC(g->rec, S * sizeof(GreedyRec));
-    GR_ALLOC(g->d_paths, S * (size_t)path_cap * 2 * sizeof(int32_t));
-    GR_ALLOC(g->d_path_len, S * sizeof(int32_t));
+    ACS_ALLOC(g->keys, S * g->cap * 2 * g->W * sizeof(uint64_t), acs_greedy_destroy(g));
+    ACS_ALLOC(g->parent, S * g->cap * sizeof(uint64_t), acs_greedy_destroy(g));
+    ACS_ALLOC(g->depth, S * g->cap * sizeof(uint32_t), acs_greedy_destroy(g));
+    ACS_ALLOC(g->heap, S * g->cap * sizeof(uint64_t), acs_greedy_destroy(g));
+    ACS_ALLOC(g->table, S * g->tcap * sizeof(uint64_t), acs_greedy_destroy(g));
+    ACS_ALLOC(g->roots, S * 2 * g->W * sizeof(uint64_t), acs_greedy_destroy(g));
+    ACS_ALLOC(g->rec, S * sizeof(GreedyRec), acs_greedy_destroy(g));
+    ACS_ALLOC(g->d_paths, S * (size_t)path_cap * 2 * sizeof(int32_t), acs_greedy_destroy(g));
+    ACS_ALLOC(g->d_path_len, S * sizeof(int32_t), acs_greedy_destroy(g));
     {
         const char* e = std::getenv("ACS_GREEDY_KERNEL");  // "heap" forces the one-warp-per-search kernel
         g->use_bucket = !(e && std::string(e) == "heap");
     }
     if (g->use_bucket) {
-        GR_ALLOC(g->gb.segs, S * (size_t)kGbSegPool * sizeof(GbSeg));
-        GR_ALLOC(g->gb.sortbuf, S * (size_t)kGbSortCap * (2 * g->W + 2) * sizeof(uint64_t));
-        GR_ALLOC(g->gb.cand_key, S * (size_t)kGbCand * 2 * g->W * sizeof(uint64_t));
-        GR_ALLOC(g->gb.cand_meta, S * (size_t)kGbCand * sizeof(uint32_t));
-        GR_ALLOC(g->gb.cand_slot, S * (size_t)kGbCand * sizeof(uint32_t));
-        GR_ALLOC(g->gb.round_tab, S * (size_t)kGbRoundSlots * sizeof(uint64_t));
+        ACS_ALLOC(g->gb.segs, S * (size_t)kGbSegPool * sizeof(GbSeg), acs_greedy_destroy(g));
+        ACS_ALLOC(g->gb.sortbuf, S * (size_t)kGbSortCap * gb_rec_words(g->W) * sizeof(uint64_t), acs_greedy_destroy(g));
+        ACS_ALLOC(g->gb.cand_key, S * (size_t)kGbCand * 2 * g->W * sizeof(uint64_t), acs_greedy_destroy(g));
+        ACS_ALLOC(g->gb.cand_meta, S * (size_t)kGbCand * sizeof(uint32_t), acs_greedy_destroy(g));
+        ACS_ALLOC(g->gb.cand_slot, S * (size_t)kGbCand * sizeof(uint32_t), acs_greedy_destroy(g));
+        ACS_ALLOC(g->gb.round_tab, S * (size_t)kGbRoundSlots * sizeof(uint64_t), acs_greedy_destroy(g));
         g->gb.frontier = reinterpret_cast<uint32_t*>(g->heap);  // the heap pool doubles as the frontier array
         g->gb.fcap = 2 * g->cap;
     }
-#undef GR_ALLOC
     g->h_rec.resize(S);
-    if (cudaStreamCreateWithFlags(&g->stream, cudaStreamNonBlocking) != cudaSuccess) return fail(ACS_ERR_CUDA);
+    if (cudaStreamCreateWithFlags(&g->stream, cudaStreamNonBlocking) != cudaSuccess) {
+        acs_greedy_destroy(g);
+        return ACS_ERR_CUDA;
+    }
     cudaEventCreate(&g->ev0);
     cudaEventCreate(&g->ev1);
     *out = g;
@@ -574,34 +542,24 @@ namespace {
 
 template <int W, bool GOAL>
 int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_search_result* res) {
-    GR_CUDA(cudaSetDevice(g->device));
+    ACS_CUDA(cudaSetDevice(g->device));
     const int S = g->n_search;
     std::vector<uint64_t> roots((size_t)S * 2 * W);
-    std::vector<int> skip(S, 0);
+    bool padded = true;
     for (int s = 0; s < S; ++s) {
         Key<W> k;
         int lens[2];
-        bool valid;
-        if (!pack_root<W>(h_pres + (size_t)s * 2 * g->mrl, g->mrl, k, lens, valid)) {
-            acs::set_last_error("greedy: letters outside {+-1,+-2} are not supported by the packed search");
-            return ACS_ERR_UNSUPPORTED;
-        }
         // a mis-padded root cannot be represented; empty relators can (the first move raises)
-        for (int h = 0; h < 2; ++h) {
-            const int8_t* p = h_pres + (size_t)s * 2 * g->mrl + h * g->mrl;
-            for (int t = lens[h]; t < g->mrl; ++t)
-                if (p[t] != 0) skip[s] = 1;
-        }
+        const RootCheck rc = pack_root<W>(h_pres + (size_t)s * 2 * g->mrl, g->mrl, k, lens);
+        if (rc == RootCheck::bad_letter)
+            return fail(ACS_ERR_UNSUPPORTED, "greedy: letters outside {+-1,+-2} are not supported by the packed search");
+        padded = padded && rc != RootCheck::not_padded;
         std::memcpy(&roots[(size_t)s * 2 * W], k.k, sizeof(k.k));
     }
-    for (int s = 0; s < S; ++s)
-        if (skip[s]) {
-            acs::set_last_error("greedy: presentation is not zero right-padded");
-            return ACS_ERR_INVALID;
-        }
+    if (!padded) return fail(ACS_ERR_INVALID, "greedy: presentation is not zero right-padded");
     cudaStream_t st = g->stream;
-    GR_CUDA(cudaMemcpyAsync(g->roots, roots.data(), roots.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    GR_CUDA(cudaMemsetAsync(g->table, 0, (size_t)S * g->tcap * sizeof(uint64_t), st));
+    ACS_CUDA(cudaMemcpyAsync(g->roots, roots.data(), roots.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    ACS_CUDA(cudaMemsetAsync(g->table, 0, (size_t)S * g->tcap * sizeof(uint64_t), st));
     GreedyArgs A{};
     A.keys = g->keys;
     A.parent = g->parent;
@@ -618,7 +576,7 @@ int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_s
     A.cyclical = g->cyclical;
     A.fallback_only = 0;
     const GoalView G = GOAL ? g->goals->view() : GoalView{nullptr, nullptr, 0};
-    GR_CUDA(cudaEventRecord(g->ev0, st));
+    ACS_CUDA(cudaEventRecord(g->ev0, st));
     g->n_fallback = 0;
     if (g->use_bucket) {
         // pass 1: small bucket directory (several CTAs per SM); pass 2: the searches that outgrew it, with a
@@ -627,21 +585,21 @@ int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_s
         auto smem_for = [](int buckets) {
             return ((sizeof(GbShared) + 15) / 16) * 16 + (size_t)buckets * sizeof(GbBucket) + (GOAL ? kGbGoalSmem : 0);
         };
-        GR_CUDA(cudaFuncSetAttribute(greedy_bucket_kernel<W, GOAL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        ACS_CUDA(cudaFuncSetAttribute(greedy_bucket_kernel<W, GOAL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)smem_for(kGbBuckets2)));
         // several CTAs per SM in pass 1: ask for the largest shared-memory carve-out
-        GR_CUDA(cudaFuncSetAttribute(greedy_bucket_kernel<W, GOAL>, cudaFuncAttributePreferredSharedMemoryCarveout,
+        ACS_CUDA(cudaFuncSetAttribute(greedy_bucket_kernel<W, GOAL>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                      (int)cudaSharedmemCarveoutMaxShared));
         const bool debug = std::getenv("ACS_GREEDY_DEBUG") != nullptr;
         for (int pass = 0; pass < 2; ++pass) {
             g->gb.max_buckets = pass == 0 ? kGbBuckets1 : kGbBuckets2;
             g->gb.retry_only = pass;
             cudaEvent_t e0 = pass == 0 ? g->ev0 : g->ev1;
-            if (pass) GR_CUDA(cudaEventRecord(e0, st));
+            if (pass) ACS_CUDA(cudaEventRecord(e0, st));
             greedy_bucket_kernel<W, GOAL><<<S, kGbThreads, smem_for(g->gb.max_buckets), st>>>(A, g->gb, G);
-            GR_CUDA(cudaGetLastError());
-            GR_CUDA(cudaMemcpyAsync(g->h_rec.data(), g->rec, (size_t)S * sizeof(GreedyRec), cudaMemcpyDeviceToHost, st));
-            GR_CUDA(cudaStreamSynchronize(st));
+            ACS_CUDA(cudaGetLastError());
+            ACS_CUDA(cudaMemcpyAsync(g->h_rec.data(), g->rec, (size_t)S * sizeof(GreedyRec), cudaMemcpyDeviceToHost, st));
+            ACS_CUDA(cudaStreamSynchronize(st));
             g->n_fallback = 0;
             for (int s = 0; s < S; ++s)
                 if (g->h_rec[s].status == kGbFallback) {
@@ -649,7 +607,7 @@ int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_s
                     if (debug)
                         std::fprintf(stderr, "greedy: pass %d, search %d handed back (reason %d, %llu nodes)\n", pass, s,
                                      -g->h_rec[s].rounds, (unsigned long long)g->h_rec[s].n_nodes);
-                    GR_CUDA(cudaMemsetAsync(g->table + (size_t)s * g->tcap, 0, g->tcap * sizeof(uint64_t), st));
+                    ACS_CUDA(cudaMemsetAsync(g->table + (size_t)s * g->tcap, 0, g->tcap * sizeof(uint64_t), st));
                 }
             if (debug) std::fprintf(stderr, "greedy: bucket pass %d, %d searches, mrl %d: %d handed back\n", pass, S, g->mrl, g->n_fallback);
             if (!g->n_fallback) break;
@@ -657,29 +615,29 @@ int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_s
         if (g->n_fallback) {
             A.fallback_only = 1;
             greedy_kernel<W, GOAL><<<S, 32, 0, st>>>(A, G);
-            GR_CUDA(cudaGetLastError());
+            ACS_CUDA(cudaGetLastError());
         }
     } else {
         greedy_kernel<W, GOAL><<<S, 32, 0, st>>>(A, G);
-        GR_CUDA(cudaGetLastError());
+        ACS_CUDA(cudaGetLastError());
     }
     greedy_path_kernel<W><<<(S + 63) / 64, 64, 0, st>>>(A, g->d_paths, g->path_cap, g->d_path_len);
-    GR_CUDA(cudaGetLastError());
-    GR_CUDA(cudaEventRecord(g->ev1, st));
+    ACS_CUDA(cudaGetLastError());
+    ACS_CUDA(cudaEventRecord(g->ev1, st));
     if (GOAL) {
-        if (!g->d_goal_g) GR_CUDA(cudaMalloc((void**)&g->d_goal_g, (size_t)S * sizeof(int32_t)));
+        if (!g->d_goal_g) ACS_CUDA(cudaMalloc((void**)&g->d_goal_g, (size_t)S * sizeof(int32_t)));
         greedy_goal_elem_kernel<W><<<(S + 63) / 64, 64, 0, st>>>(A, g->goals->symmetric, g->d_goal_g);
-        GR_CUDA(cudaGetLastError());
+        ACS_CUDA(cudaGetLastError());
         g->h_goal_g.resize((size_t)S);
-        GR_CUDA(cudaMemcpyAsync(g->h_goal_g.data(), g->d_goal_g, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        ACS_CUDA(cudaMemcpyAsync(g->h_goal_g.data(), g->d_goal_g, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     }
-    GR_CUDA(cudaMemcpyAsync(g->h_rec.data(), g->rec, (size_t)S * sizeof(GreedyRec), cudaMemcpyDeviceToHost, st));
+    ACS_CUDA(cudaMemcpyAsync(g->h_rec.data(), g->rec, (size_t)S * sizeof(GreedyRec), cudaMemcpyDeviceToHost, st));
     std::vector<int32_t> plen(S);
-    GR_CUDA(cudaMemcpyAsync(plen.data(), g->d_path_len, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    ACS_CUDA(cudaMemcpyAsync(plen.data(), g->d_path_len, (size_t)S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     if (h_paths)
-        GR_CUDA(cudaMemcpyAsync(h_paths, g->d_paths, (size_t)S * g->path_cap * 2 * sizeof(int32_t),
+        ACS_CUDA(cudaMemcpyAsync(h_paths, g->d_paths, (size_t)S * g->path_cap * 2 * sizeof(int32_t),
                                 cudaMemcpyDeviceToHost, st));
-    GR_CUDA(cudaStreamSynchronize(st));
+    ACS_CUDA(cudaStreamSynchronize(st));
     float ms = 0.f;
     cudaEventElapsedTime(&ms, g->ev0, g->ev1);
     g->ran = true;
@@ -704,23 +662,6 @@ int greedy_run_impl(acs_greedy* g, const int8_t* h_pres, int32_t* h_paths, acs_s
     return ACS_OK;
 }
 
-template <int W>
-int greedy_visited_impl(acs_greedy* g, int search, int8_t* h_out, int64_t cap_rows, int64_t* n_out) {
-    GR_CUDA(cudaSetDevice(g->device));
-    const uint64_t n = std::min<uint64_t>(g->h_rec[search].n_nodes, (uint64_t)std::max<int64_t>(cap_rows, 0));
-    if (n_out) *n_out = (int64_t)n;
-    if (n == 0) return ACS_OK;
-    int8_t* d = nullptr;
-    GR_CUDA(cudaMalloc((void**)&d, n * 2 * g->mrl));
-    keys_unpack_kernel<W><<<(unsigned)((n + 255) / 256), 256, 0, g->stream>>>(
-        g->keys + (uint64_t)search * g->cap * 2 * W, d, n, g->mrl);
-    cudaError_t e = cudaMemcpyAsync(h_out, d, n * 2 * g->mrl, cudaMemcpyDeviceToHost, g->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(g->stream);
-    cudaFree(d);
-    GR_CUDA(e);
-    return ACS_OK;
-}
-
 }  // namespace
 
 extern "C" int acs_greedy_run(acs_greedy* g, const int8_t* h_presentations, int32_t* h_paths,
@@ -735,24 +676,23 @@ extern "C" int acs_greedy_run(acs_greedy* g, const int8_t* h_presentations, int3
 
 extern "C" int acs_greedy_visited(acs_greedy* g, int search, int8_t* h_out, int64_t cap_rows, int64_t* n_out) {
     if (!g || search < 0 || search >= g->n_search || (!h_out && cap_rows > 0)) return ACS_ERR_INVALID;
-    return g->W == 1 ? greedy_visited_impl<1>(g, search, h_out, cap_rows, n_out)
-                     : greedy_visited_impl<2>(g, search, h_out, cap_rows, n_out);
+    ACS_CUDA(cudaSetDevice(g->device));
+    const int64_t n = (int64_t)std::min<uint64_t>(g->h_rec[search].n_nodes, (uint64_t)std::max<int64_t>(cap_rows, 0));
+    if (n_out) *n_out = n;
+    return records_to_host(g->W, g->keys + (uint64_t)search * g->cap * 2 * g->W, 2 * g->W, n, g->mrl, h_out, nullptr,
+                           g->stream);
 }
 
 extern "C" int acs_greedy_set_goals(acs_greedy* g, const acs_goalset* gs) {
     if (!g) return ACS_ERR_INVALID;
     if (gs) {
-        auto fail = [](const char* m) {
-            acs::set_last_error(m);
-            return ACS_ERR_INVALID;
-        };
-        if (gs->mrl != g->mrl) return fail("greedy_set_goals: the goal set's max_relator_length differs from the engine's");
-        if (gs->cyclical != g->cyclical) return fail("greedy_set_goals: the goal set's cyclical flag differs from the engine's");
-        if (gs->device != g->device) return fail("greedy_set_goals: the goal set lives on another device");
-        if (gs->n_entries >= (int64_t)0xFFFFFFFF) {  // the bucket kernel packs a hit's entry into 32 bits beside its candidate
-            acs::set_last_error("greedy_set_goals: goal sets of 2^32 - 1 entries or more are not supported");
-            return ACS_ERR_UNSUPPORTED;
-        }
+        if (gs->mrl != g->mrl)
+            return fail(ACS_ERR_INVALID, "greedy_set_goals: the goal set's max_relator_length differs from the engine's");
+        if (gs->cyclical != g->cyclical)
+            return fail(ACS_ERR_INVALID, "greedy_set_goals: the goal set's cyclical flag differs from the engine's");
+        if (gs->device != g->device) return fail(ACS_ERR_INVALID, "greedy_set_goals: the goal set lives on another device");
+        if (gs->n_entries >= (int64_t)0xFFFFFFFF)  // the bucket kernel packs a hit's entry into 32 bits beside its candidate
+            return fail(ACS_ERR_UNSUPPORTED, "greedy_set_goals: goal sets of 2^32 - 1 entries or more are not supported");
     }
     g->goals = gs;
     return ACS_OK;
@@ -760,20 +700,14 @@ extern "C" int acs_greedy_set_goals(acs_greedy* g, const acs_goalset* gs) {
 
 extern "C" int acs_greedy_goal_hit_elements(acs_greedy* g, int32_t* h_elem) {
     if (!g || !h_elem) return ACS_ERR_INVALID;
-    if (!g->ran) {
-        acs::set_last_error("greedy: no completed run");
-        return ACS_ERR_INVALID;
-    }
+    if (!g->ran) return fail(ACS_ERR_INVALID, "greedy: no completed run");
     for (int s = 0; s < g->n_search; ++s) h_elem[s] = g->ran_with_goals ? g->h_goal_g[s] : -1;
     return ACS_OK;
 }
 
 extern "C" int acs_greedy_goal_hits(acs_greedy* g, int64_t* h_entry) {
     if (!g || !h_entry) return ACS_ERR_INVALID;
-    if (!g->ran) {
-        acs::set_last_error("greedy: no completed run");
-        return ACS_ERR_INVALID;
-    }
+    if (!g->ran) return fail(ACS_ERR_INVALID, "greedy: no completed run");
     for (int s = 0; s < g->n_search; ++s) h_entry[s] = g->ran_with_goals ? g->h_rec[s].goal : -1;
     return ACS_OK;
 }

@@ -118,14 +118,16 @@ struct GbShared {
 };
 enum : uint32_t { GB_CONT = 0, GB_INTERRUPT = 1, GB_BUDGET = 2, GB_SOLVED = 3, GB_ERROR = 4, GB_GOAL = 5 };
 
+// words per sort record: the key, the node index and one spare word (a record of its own, not a node record)
+__host__ __device__ constexpr int gb_rec_words(int W) { return 2 * W + 2; }
 template <int W>
 __device__ __forceinline__ uint64_t* gb_rec(uint64_t* sortbuf, uint32_t i) {
-    return sortbuf + (size_t)i * (2 * W + 2);
+    return sortbuf + (size_t)i * gb_rec_words(W);
 }
 template <int W>
 __device__ __forceinline__ Key<W> gb_rec_key(const uint64_t* sortbuf, uint32_t i) {
     Key<W> k;
-    const uint64_t* p = sortbuf + (size_t)i * (2 * W + 2);
+    const uint64_t* p = sortbuf + (size_t)i * gb_rec_words(W);
 #pragma unroll
     for (int t = 0; t < 2 * W; ++t) k.k[t] = p[t];
     return k;
@@ -201,7 +203,7 @@ __global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS)
     if (sidx >= A.n_search) return;
     if (X.retry_only && A.rec[sidx].status != kGbFallback) return;
     const int tid = threadIdx.x;
-    constexpr int RS = 2 * W + 2;  // words per sort record
+    constexpr int RS = gb_rec_words(W);
     uint64_t* keys = A.keys + (uint64_t)sidx * A.cap * 2 * W;
     uint64_t* parent = A.parent + (uint64_t)sidx * A.cap;
     uint64_t* table = A.table + (uint64_t)sidx * A.tcap;
@@ -219,7 +221,7 @@ __global__ void __launch_bounds__(kGbThreads, GB_MIN_BLOCKS)
     Key<W> root;
 #pragma unroll
     for (int i = 0; i < 2 * W; ++i) root.k[i] = A.roots[(uint64_t)sidx * 2 * W + i];
-    const int L0 = (int)(root.k[W - 1] >> 58) + (int)(root.k[2 * W - 1] >> 58);
+    const int L0 = key_total_len<W>(root);
     if (tid == 0) {
         store_key<W>(keys, 0, root);
         parent[0] = kNone;

@@ -598,9 +598,9 @@ __global__ void __launch_bounds__(128) mb_decide_kernel(const MbEngine E) {
         M.sol_len = 2;
         if (goal_here) {
             const uint64_t e = goal & 0xFFFFFFFFull;
-            const int W = st->mrl <= 29 ? 1 : 2;
-            const uint64_t* q = E.goals.nodes + e * (2 * W + 2);  // the goal state's key: lengths in the top bits
-            M.sol_len = (int32_t)(q[W - 1] >> 58) + (int32_t)(q[2 * W - 1] >> 58);
+            const int W = key_words(st->mrl);
+            const uint64_t* q = E.goals.nodes + e * node_words(W);  // the goal state's key
+            M.sol_len = key_len(q, W, 0) + key_len(q, W, 1);
             E.goal_hit[s] = (int64_t)e;
         }
     } else if (status) {
@@ -690,7 +690,7 @@ __global__ void mb_path_kernel(const MbEngine E, int32_t* paths, int path_cap, i
         if (pos < path_cap) {
             path[2 * pos] = pl < 0 ? -1 : (int32_t)(pl & 15);
             if constexpr (SYM) path[2 * pos] = (path[2 * pos] & 0xFF) | (int32_t)(((uint64_t)tag >> 32) & 15) << 8;
-            path[2 * pos + 1] = (int32_t)(k.k[W - 1] >> 58) + (int32_t)(k.k[2 * W - 1] >> 58);
+            path[2 * pos + 1] = key_total_len<W>(k);
         }
         g = pl < 0 ? -1 : (pl >> 4);
     }
@@ -728,16 +728,6 @@ __global__ void mb_path_kernel(const MbEngine E, int32_t* paths, int path_cap, i
     }
 }
 
-template <int W>
-__global__ void mb_unpack_kernel(const uint64_t* nodes, int8_t* out, uint64_t n, int mrl) {
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    Rel<2 * W> r0, r1;
-    split_key<W>(node_key<W>(nodes, i), r0, r1);
-    unpack_bytes<2 * W>(out + i * 2 * mrl, r0, mrl);
-    unpack_bytes<2 * W>(out + i * 2 * mrl + mrl, r1, mrl);
-}
-
 // committed nodes of every search -> goal-set entries in (search, FIFO id) order; off [n_search + 1] holds
 // each search's first entry, slab [n_search] its first node.  Parent links are rebased onto entry indices.
 template <int W>
@@ -759,19 +749,6 @@ __global__ void mb_adopt_kernel(const uint64_t* nodes, const int64_t* off, const
 using namespace acs;
 
 namespace {
-inline int mb_fail(int code, const std::string& m) {
-    acs::set_last_error(m.c_str());
-    return code;
-}
-#define MB_CUDA(call)                                                                      \
-    do {                                                                                   \
-        cudaError_t e__ = (call);                                                          \
-        if (e__ != cudaSuccess) {                                                          \
-            cudaGetLastError();                                                            \
-            return mb_fail(e__ == cudaErrorMemoryAllocation ? ACS_ERR_NOMEM : ACS_ERR_CUDA, \
-                           std::string(#call) + ": " + cudaGetErrorString(e__));           \
-        }                                                                                  \
-    } while (0)
 constexpr int kMbRing = 4, kMbLag = 2;
 
 // sizes of an engine (shared by acs_bfs_batch_bytes and acs_bfs_batch_create)
@@ -783,19 +760,19 @@ struct MbPlan {
 };
 
 int mb_plan(int n_search, int mrl, const int64_t* max_nodes, int64_t chunk_parents, MbPlan& P) {
-    if (n_search < 1 || !max_nodes) return mb_fail(ACS_ERR_INVALID, "bfs_batch: need at least one search");
-    if (mrl < 1 || mrl > 61) return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch needs 1 <= max_relator_length <= 61");
-    P.W = mrl <= 29 ? 1 : 2;
+    if (n_search < 1 || !max_nodes) return fail(ACS_ERR_INVALID, "bfs_batch: need at least one search");
+    if (const int rc = check_key_mrl(mrl, "bfs_batch")) return rc;
+    P.W = key_words(mrl);
     P.nodes = 0;
     for (int s = 0; s < n_search; ++s) {
-        if (max_nodes[s] < 0) return mb_fail(ACS_ERR_INVALID, "bfs_batch: negative node budget");
+        if (max_nodes[s] < 0) return fail(ACS_ERR_INVALID, "bfs_batch: negative node budget");
         P.nodes += max_nodes[s] + 16;
     }
     // the table stays <= 3/4 full: committed nodes, tombstones and one chunk's tentative claims
     uint64_t t = 1024;
     while (t < 5 * (uint64_t)P.nodes / 2) t <<= 1;
     P.tcap = t;
-    if (P.nodes >= (int64_t)kMbIdx) return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch: too many nodes for one engine");
+    if (P.nodes >= (int64_t)kMbIdx) return fail(ACS_ERR_UNSUPPORTED, "bfs_batch: too many nodes for one engine");
     // parents per chunk after the first: ~4 Mi (candidate ids are 32-bit)
     int64_t chunk = chunk_parents > 0 ? chunk_parents : (int64_t)1 << 22;
     chunk = std::min<int64_t>(chunk, std::max<int64_t>(P.nodes, 1024));
@@ -803,11 +780,11 @@ int mb_plan(int n_search, int mrl, const int64_t* max_nodes, int64_t chunk_paren
     P.chunk = chunk;
     // the log and the bitmap also hold the first chunk, which expands every root
     const int64_t widest = std::max<int64_t>(chunk, n_search);
-    if (widest > ((int64_t)1 << 32) / 12 - 1) return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch: too many searches");
+    if (widest > ((int64_t)1 << 32) / 12 - 1) return fail(ACS_ERR_UNSUPPORTED, "bfs_batch: too many searches");
     P.rec_cap = 12 * widest;
     P.bitmap_words = (12 * widest + 31) / 32 + 8;
     P.nblk = (P.bitmap_words + kScanBlock - 1) / kScanBlock + 1;
-    const int64_t node_bytes = 8 * (2 * P.W + 2);
+    const int64_t node_bytes = 8 * node_words(P.W);
     // per search: control minima, six segment arrays, the state and the root key
     const int64_t per_search = kMbCtrl * 8 + 4 + 8 + 8 + 8 + 8 + 4 + (int64_t)sizeof(MbSearch) + 16 * P.W;
     P.bytes = P.nodes * node_bytes + (int64_t)P.tcap * 8 + P.rec_cap * (16 * P.W + 4 + 4 + 8) + P.bitmap_words * 4 +
@@ -880,13 +857,7 @@ int acs_bfs_batch_create(int device, int n_search, int mrl, const int64_t* max_n
     MbPlan P;
     const int rc = mb_plan(n_search, mrl, max_nodes, chunk_parents, P);
     if (rc != ACS_OK) return rc;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        return mb_fail(ACS_ERR_NO_DEVICE, "no CUDA device visible; there is no CPU fallback");
-    }
-    if (device < 0 || device >= ndev) return mb_fail(ACS_ERR_INVALID, "bfs_batch: device index out of range");
-    MB_CUDA(cudaSetDevice(device));
+    if (const int rc2 = open_device(device, "bfs_batch")) return rc2;
     acs_bfs_batch* b = new acs_bfs_batch();
     b->device = device;
     b->n_search = n_search;
@@ -897,39 +868,30 @@ int acs_bfs_batch_create(int device, int n_search, int mrl, const int64_t* max_n
     b->budgets.assign(max_nodes, max_nodes + n_search);
     auto bail = [&](int code, const std::string& m) {
         acs_bfs_batch_destroy(b);
-        return mb_fail(code, m);
+        return fail(code, m);
     };
     MbEngine& E = b->E;
     E.rec_cap = P.rec_cap;
-#define MB_ALLOC(ptr, bytes)                                                                             \
-    do {                                                                                                 \
-        cudaError_t e__ = cudaMalloc((void**)&(ptr), (size_t)(bytes));                                   \
-        if (e__ != cudaSuccess) {                                                                        \
-            cudaGetLastError();                                                                          \
-            return bail(ACS_ERR_NOMEM, std::string("bfs_batch: cudaMalloc(" #ptr "): ") + cudaGetErrorString(e__)); \
-        }                                                                                                \
-    } while (0)
-    MB_ALLOC(E.st, sizeof(MbState));
-    MB_ALLOC(E.srch, (size_t)n_search * sizeof(MbSearch));
-    MB_ALLOC(E.nodes, (size_t)P.nodes * 8 * (2 * P.W + 2));
-    MB_ALLOC(E.table, (size_t)P.tcap * 8);
-    MB_ALLOC(E.log_keys, (size_t)P.rec_cap * 16 * P.W);
-    MB_ALLOC(E.log_c, (size_t)P.rec_cap * 4);
-    MB_ALLOC(E.log_s, (size_t)P.rec_cap * 4);
-    MB_ALLOC(E.rec_slot, (size_t)P.rec_cap * 8);
-    MB_ALLOC(E.cursor, 8);
-    MB_ALLOC(E.bitmap, (size_t)P.bitmap_words * 4);
-    MB_ALLOC(E.rt, (size_t)(P.bitmap_words + 1) * sizeof(uint2));
-    MB_ALLOC(E.bsums, (size_t)P.nblk * 4);
-    MB_ALLOC(E.ctrl, (size_t)n_search * kMbCtrl * 8);
-    MB_ALLOC(E.seg_search, (size_t)n_search * 4);
-    MB_ALLOC(E.seg_head, (size_t)n_search * 8);
-    MB_ALLOC(E.seg_off, (size_t)(n_search + 1) * 8);
-    MB_ALLOC(E.seg_limit, (size_t)n_search * 8);
-    MB_ALLOC(E.seg_base, (size_t)n_search * 8);
-    MB_ALLOC(E.seg_of, (size_t)n_search * 4);
-    MB_ALLOC(b->d_roots, (size_t)n_search * 16 * P.W);
-#undef MB_ALLOC
+    ACS_ALLOC(E.st, sizeof(MbState), acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.srch, (size_t)n_search * sizeof(MbSearch), acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.nodes, (size_t)P.nodes * 8 * node_words(P.W), acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.table, (size_t)P.tcap * 8, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.log_keys, (size_t)P.rec_cap * 16 * P.W, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.log_c, (size_t)P.rec_cap * 4, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.log_s, (size_t)P.rec_cap * 4, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.rec_slot, (size_t)P.rec_cap * 8, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.cursor, 8, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.bitmap, (size_t)P.bitmap_words * 4, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.rt, (size_t)(P.bitmap_words + 1) * sizeof(uint2), acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.bsums, (size_t)P.nblk * 4, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.ctrl, (size_t)n_search * kMbCtrl * 8, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.seg_search, (size_t)n_search * 4, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.seg_head, (size_t)n_search * 8, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.seg_off, (size_t)(n_search + 1) * 8, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.seg_limit, (size_t)n_search * 8, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.seg_base, (size_t)n_search * 8, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(E.seg_of, (size_t)n_search * 4, acs_bfs_batch_destroy(b));
+    ACS_ALLOC(b->d_roots, (size_t)n_search * 16 * P.W, acs_bfs_batch_destroy(b));
     if (cudaMallocHost((void**)&b->h_ring, kMbRing * sizeof(MbState)) != cudaSuccess)
         return bail(ACS_ERR_NOMEM, "bfs_batch: cudaMallocHost");
     if (cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking) != cudaSuccess)
@@ -971,27 +933,27 @@ template <int W>
 int mb_paths(acs_bfs_batch* b, int32_t* h_paths, int path_cap, std::vector<int32_t>& plen) {
     const int n = b->n_search;
     cudaStream_t s = b->stream;
-    MB_CUDA(cudaSetDevice(b->device));
+    ACS_CUDA(cudaSetDevice(b->device));
     const int cap = std::max(path_cap, 1);  // the kernel writes the first pair of every solved path
     if (!b->d_paths || cap > b->d_path_cap) {
         if (b->d_paths) cudaFree(b->d_paths);
         b->d_paths = nullptr;
         b->d_path_cap = 0;
-        MB_CUDA(cudaMalloc((void**)&b->d_paths, (size_t)n * cap * 2 * sizeof(int32_t)));
+        ACS_CUDA(cudaMalloc((void**)&b->d_paths, (size_t)n * cap * 2 * sizeof(int32_t)));
         b->d_path_cap = cap;
     }
-    if (!b->d_plen) MB_CUDA(cudaMalloc((void**)&b->d_plen, (size_t)n * sizeof(int32_t)));
+    if (!b->d_plen) ACS_CUDA(cudaMalloc((void**)&b->d_plen, (size_t)n * sizeof(int32_t)));
     if (b->symmetric) mb_path_kernel<W, true><<<(n + 127) / 128, 128, 0, s>>>(b->E, b->d_paths, cap, b->d_plen);
     else mb_path_kernel<W, false><<<(n + 127) / 128, 128, 0, s>>>(b->E, b->d_paths, cap, b->d_plen);
-    MB_CUDA(cudaGetLastError());
+    ACS_CUDA(cudaGetLastError());
     plen.resize((size_t)n);
-    MB_CUDA(cudaMemcpyAsync(plen.data(), b->d_plen, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    MB_CUDA(cudaStreamSynchronize(s));
+    ACS_CUDA(cudaMemcpyAsync(plen.data(), b->d_plen, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    ACS_CUDA(cudaStreamSynchronize(s));
     for (int i = 0; i < n; ++i)
         if (plen[i] > path_cap)
-            return mb_fail(ACS_ERR_INVALID, "bfs_batch: a solution path is longer than path_cap (see path_len)");
+            return fail(ACS_ERR_INVALID, "bfs_batch: a solution path is longer than path_cap (see path_len)");
     if (h_paths && path_cap > 0)
-        MB_CUDA(cudaMemcpy(h_paths, b->d_paths, (size_t)n * path_cap * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost));
+        ACS_CUDA(cudaMemcpy(h_paths, b->d_paths, (size_t)n * path_cap * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost));
     return ACS_OK;
 }
 
@@ -999,7 +961,7 @@ template <int W>
 int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int path_cap, acs_search_result* results) {
     const int n = b->n_search, mrl = b->mrl;
     MbEngine& E = b->E;
-    if (b->adopted) return mb_fail(ACS_ERR_INVALID, "bfs_batch: the engine's states were handed to a goal set");
+    if (b->adopted) return fail(ACS_ERR_INVALID, "bfs_batch: the engine's states were handed to a goal set");
     std::vector<MbSearch> init((size_t)n);
     std::vector<uint64_t> roots((size_t)n * 2 * W, 0);
     std::vector<uint8_t> root_g((size_t)n, 0);
@@ -1016,10 +978,10 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
         M.sol_gid = -1;
         Key<W> root;
         int lens[2];
-        bool valid;
-        if (!pack_root<W>(h_pres + (size_t)s * 2 * mrl, mrl, root, lens, valid))
-            return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch: letters outside {+-1,+-2} are not supported by the packed search");
-        if (!valid) {  // breadth_first.py:36-38 asserts is_array_valid_presentation
+        const RootCheck rc = pack_root<W>(h_pres + (size_t)s * 2 * mrl, mrl, root, lens);
+        if (rc == RootCheck::bad_letter)
+            return fail(ACS_ERR_UNSUPPORTED, "bfs_batch: letters outside {+-1,+-2} are not supported by the packed search");
+        if (rc != RootCheck::ok) {  // breadth_first.py:36-38 asserts is_array_valid_presentation
             M.status = ACS_ROW_ASSERT;
             M.done = 1;
             M.n_nodes = 0;
@@ -1043,26 +1005,26 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
     st.used = n_valid;
     st.explore = b->explore;
     cudaStream_t s = b->stream;
-    MB_CUDA(cudaSetDevice(b->device));
-    MB_CUDA(cudaMemsetAsync(E.table, 0, b->plan.tcap * sizeof(uint64_t), s));
-    if (E.goal_hit) MB_CUDA(cudaMemsetAsync(E.goal_hit, 0xFF, (size_t)n * sizeof(int64_t), s));
-    if (E.goal_hit_g) MB_CUDA(cudaMemsetAsync(E.goal_hit_g, 0xFF, (size_t)n * sizeof(int32_t), s));
+    ACS_CUDA(cudaSetDevice(b->device));
+    ACS_CUDA(cudaMemsetAsync(E.table, 0, b->plan.tcap * sizeof(uint64_t), s));
+    if (E.goal_hit) ACS_CUDA(cudaMemsetAsync(E.goal_hit, 0xFF, (size_t)n * sizeof(int64_t), s));
+    if (E.goal_hit_g) ACS_CUDA(cudaMemsetAsync(E.goal_hit_g, 0xFF, (size_t)n * sizeof(int32_t), s));
     b->h_ring[0] = st;  // pinned staging for the async upload
-    MB_CUDA(cudaMemcpyAsync(E.st, &b->h_ring[0], sizeof(MbState), cudaMemcpyHostToDevice, s));
-    MB_CUDA(cudaMemcpyAsync(E.srch, init.data(), init.size() * sizeof(MbSearch), cudaMemcpyHostToDevice, s));
-    MB_CUDA(cudaMemcpyAsync(b->d_roots, roots.data(), roots.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    if (b->symmetric) MB_CUDA(cudaMemcpyAsync(b->d_root_g, root_g.data(), root_g.size(), cudaMemcpyHostToDevice, s));
+    ACS_CUDA(cudaMemcpyAsync(E.st, &b->h_ring[0], sizeof(MbState), cudaMemcpyHostToDevice, s));
+    ACS_CUDA(cudaMemcpyAsync(E.srch, init.data(), init.size() * sizeof(MbSearch), cudaMemcpyHostToDevice, s));
+    ACS_CUDA(cudaMemcpyAsync(b->d_roots, roots.data(), roots.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    if (b->symmetric) ACS_CUDA(cudaMemcpyAsync(b->d_root_g, root_g.data(), root_g.size(), cudaMemcpyHostToDevice, s));
     E.root_g = b->symmetric ? b->d_root_g : nullptr;
-    MB_CUDA(cudaStreamSynchronize(s));  // the staging copies above read host memory that goes out of scope
-    MB_CUDA(cudaEventRecord(b->ev0, s));
+    ACS_CUDA(cudaStreamSynchronize(s));  // the staging copies above read host memory that goes out of scope
+    ACS_CUDA(cudaEventRecord(b->ev0, s));
     mb_init_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(E, b->d_roots);
     if (b->goals) mb_goal_roots_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(E);
     mb_plan_kernel<<<1, 32, 0, s>>>(E, 1);
-    MB_CUDA(cudaGetLastError());
+    ACS_CUDA(cudaGetLastError());
     const int decide_blocks = (n + 127) / 128;
     for (int64_t chunk = 0;; ++chunk) {
         if (chunk >= kMbLag) {
-            MB_CUDA(cudaEventSynchronize(b->ring_ev[(chunk - kMbLag) % kMbRing]));
+            ACS_CUDA(cudaEventSynchronize(b->ring_ev[(chunk - kMbLag) % kMbRing]));
             if (b->h_ring[(chunk - kMbLag) % kMbRing].done) break;
         }
         mb_prep_kernel<<<b->sms * 2, 256, 0, s>>>(E);
@@ -1083,21 +1045,21 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
         if (b->symmetric) mb_commit_kernel<W, true><<<b->commit_blocks, 256, 0, s>>>(E);
         else mb_commit_kernel<W, false><<<b->commit_blocks, 256, 0, s>>>(E);
         mb_plan_kernel<<<1, 32, 0, s>>>(E, 0);
-        MB_CUDA(cudaGetLastError());
-        MB_CUDA(cudaMemcpyAsync(&b->h_ring[chunk % kMbRing], E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
-        MB_CUDA(cudaEventRecord(b->ring_ev[chunk % kMbRing], s));
+        ACS_CUDA(cudaGetLastError());
+        ACS_CUDA(cudaMemcpyAsync(&b->h_ring[chunk % kMbRing], E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
+        ACS_CUDA(cudaEventRecord(b->ring_ev[chunk % kMbRing], s));
     }
-    MB_CUDA(cudaEventRecord(b->ev1, s));
+    ACS_CUDA(cudaEventRecord(b->ev1, s));
     MbState fin{};
     b->h_final.resize((size_t)n);
-    MB_CUDA(cudaMemcpyAsync(&fin, E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
-    MB_CUDA(cudaMemcpyAsync(b->h_final.data(), E.srch, (size_t)n * sizeof(MbSearch), cudaMemcpyDeviceToHost, s));
-    MB_CUDA(cudaStreamSynchronize(s));
+    ACS_CUDA(cudaMemcpyAsync(&fin, E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
+    ACS_CUDA(cudaMemcpyAsync(b->h_final.data(), E.srch, (size_t)n * sizeof(MbSearch), cudaMemcpyDeviceToHost, s));
+    ACS_CUDA(cudaStreamSynchronize(s));
     if (fin.ierr) {
         std::string m = "bfs_batch: internal error:";
         if (fin.ierr & MB_IERR_TABLE_FULL) m += " visited table full (more than 3/4 of its slots used)";
         if (fin.ierr & MB_IERR_SLAB_FULL) m += " node slab of a search full";
-        return mb_fail(ACS_ERR_CUDA, m);
+        return fail(ACS_ERR_CUDA, m);
     }
     b->ran = true;
     float ms = 0.f;
@@ -1141,31 +1103,20 @@ int acs_bfs_batch_run(acs_bfs_batch* b, const int8_t* h_presentations, int32_t* 
 
 int acs_bfs_batch_paths(acs_bfs_batch* b, int32_t* h_paths, int path_cap) {
     if (!b || path_cap < 0 || (!h_paths && path_cap > 0)) return ACS_ERR_INVALID;
-    if (!b->ran) return mb_fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
+    if (!b->ran) return fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
     std::vector<int32_t> plen;
     return b->W == 1 ? mb_paths<1>(b, h_paths, path_cap, plen) : mb_paths<2>(b, h_paths, path_cap, plen);
 }
 
 int acs_bfs_batch_visited(acs_bfs_batch* b, int search, int8_t* h_out, int64_t cap_rows, int64_t* n_out) {
     if (!b || search < 0 || search >= b->n_search || (!h_out && cap_rows > 0)) return ACS_ERR_INVALID;
-    if (!b->ran) return mb_fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
-    MB_CUDA(cudaSetDevice(b->device));
+    if (!b->ran) return fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
+    ACS_CUDA(cudaSetDevice(b->device));
     const MbSearch& f = b->h_final[search];
     const int64_t n = std::min<int64_t>(f.n_nodes, std::max<int64_t>(cap_rows, 0));
     if (n_out) *n_out = n;
-    if (n == 0) return ACS_OK;
-    int8_t* d = nullptr;
-    MB_CUDA(cudaMalloc((void**)&d, (size_t)n * 2 * b->mrl));
-    const uint64_t* slab = b->E.nodes + (size_t)f.slab * (2 * b->W + 2);
-    const unsigned grid = (unsigned)((n + 255) / 256);
-    if (b->W == 1) mb_unpack_kernel<1><<<grid, 256, 0, b->stream>>>(slab, d, (uint64_t)n, b->mrl);
-    else mb_unpack_kernel<2><<<grid, 256, 0, b->stream>>>(slab, d, (uint64_t)n, b->mrl);
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaMemcpyAsync(h_out, d, (size_t)n * 2 * b->mrl, cudaMemcpyDeviceToHost, b->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);
-    cudaFree(d);
-    MB_CUDA(e);
-    return ACS_OK;
+    const uint64_t* slab = b->E.nodes + (size_t)f.slab * node_words(b->W);
+    return records_to_host(b->W, slab, node_words(b->W), n, b->mrl, h_out, nullptr, b->stream);
 }
 
 }  // extern "C"
@@ -1177,21 +1128,21 @@ int acs_bfs_batch_set_goals(acs_bfs_batch* b, const acs_goalset* g, int stop_at_
     if (!b) return ACS_ERR_INVALID;
     if (g) {
         if (g->mrl != b->mrl)
-            return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set's max_relator_length differs from the engine's");
+            return fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set's max_relator_length differs from the engine's");
         if (g->cyclical != b->cyclical)
-            return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set's cyclical flag differs from the engine's");
+            return fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set's cyclical flag differs from the engine's");
         if (g->device != b->device)
-            return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set lives on another device");
+            return fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set lives on another device");
         if (b->symmetric && !g->symmetric)  // an orbit search knows only the orbit of a child
-            return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_goals: an orbit search needs a symmetric goal set");
+            return fail(ACS_ERR_INVALID, "bfs_batch_set_goals: an orbit search needs a symmetric goal set");
         if (g->n_entries >= (int64_t)0xFFFFFFFF)  // a hit packs the entry into 32 bits beside its candidate id
-            return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch_set_goals: goal sets of 2^32 - 1 entries or more are not supported");
+            return fail(ACS_ERR_UNSUPPORTED, "bfs_batch_set_goals: goal sets of 2^32 - 1 entries or more are not supported");
         if (!b->E.goal_hit) {
-            MB_CUDA(cudaSetDevice(b->device));
-            MB_CUDA(cudaMalloc((void**)&b->E.goal_hit, (size_t)b->n_search * sizeof(int64_t)));
-            MB_CUDA(cudaMemset(b->E.goal_hit, 0xFF, (size_t)b->n_search * sizeof(int64_t)));
-            MB_CUDA(cudaMalloc((void**)&b->E.goal_hit_g, (size_t)b->n_search * sizeof(int32_t)));
-            MB_CUDA(cudaMemset(b->E.goal_hit_g, 0xFF, (size_t)b->n_search * sizeof(int32_t)));
+            ACS_CUDA(cudaSetDevice(b->device));
+            ACS_CUDA(cudaMalloc((void**)&b->E.goal_hit, (size_t)b->n_search * sizeof(int64_t)));
+            ACS_CUDA(cudaMemset(b->E.goal_hit, 0xFF, (size_t)b->n_search * sizeof(int64_t)));
+            ACS_CUDA(cudaMalloc((void**)&b->E.goal_hit_g, (size_t)b->n_search * sizeof(int32_t)));
+            ACS_CUDA(cudaMemset(b->E.goal_hit_g, 0xFF, (size_t)b->n_search * sizeof(int32_t)));
         }
         b->E.goals = g->view();
     } else {
@@ -1204,36 +1155,36 @@ int acs_bfs_batch_set_goals(acs_bfs_batch* b, const acs_goalset* g, int stop_at_
 
 int acs_bfs_batch_goal_hits(acs_bfs_batch* b, int64_t* h_entry) {
     if (!b || !h_entry) return ACS_ERR_INVALID;
-    if (!b->ran) return mb_fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
+    if (!b->ran) return fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
     if (!b->E.goal_hit) {
         std::fill(h_entry, h_entry + b->n_search, (int64_t)-1);
         return ACS_OK;
     }
-    MB_CUDA(cudaSetDevice(b->device));
-    MB_CUDA(cudaMemcpyAsync(h_entry, b->E.goal_hit, (size_t)b->n_search * sizeof(int64_t), cudaMemcpyDeviceToHost,
+    ACS_CUDA(cudaSetDevice(b->device));
+    ACS_CUDA(cudaMemcpyAsync(h_entry, b->E.goal_hit, (size_t)b->n_search * sizeof(int64_t), cudaMemcpyDeviceToHost,
                             b->stream));
-    MB_CUDA(cudaStreamSynchronize(b->stream));
+    ACS_CUDA(cudaStreamSynchronize(b->stream));
     return ACS_OK;
 }
 
 int acs_bfs_batch_goal_hit_elements(acs_bfs_batch* b, int32_t* h_elem) {
     if (!b || !h_elem) return ACS_ERR_INVALID;
-    if (!b->ran) return mb_fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
+    if (!b->ran) return fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
     if (!b->E.goal_hit_g) {
         std::fill(h_elem, h_elem + b->n_search, -1);
         return ACS_OK;
     }
-    MB_CUDA(cudaSetDevice(b->device));
-    MB_CUDA(cudaMemcpyAsync(h_elem, b->E.goal_hit_g, (size_t)b->n_search * sizeof(int32_t), cudaMemcpyDeviceToHost,
+    ACS_CUDA(cudaSetDevice(b->device));
+    ACS_CUDA(cudaMemcpyAsync(h_elem, b->E.goal_hit_g, (size_t)b->n_search * sizeof(int32_t), cudaMemcpyDeviceToHost,
                             b->stream));
-    MB_CUDA(cudaStreamSynchronize(b->stream));
+    ACS_CUDA(cudaStreamSynchronize(b->stream));
     return ACS_OK;
 }
 
 int acs_goalset_from_bfs_batch(acs_bfs_batch* b, acs_goalset** out) {
     if (!b || !out) return ACS_ERR_INVALID;
     *out = nullptr;
-    if (!b->ran) return mb_fail(ACS_ERR_INVALID, "goalset_from_bfs_batch: the engine has no completed run");
+    if (!b->ran) return fail(ACS_ERR_INVALID, "goalset_from_bfs_batch: the engine has no completed run");
     const int n = b->n_search;
     std::vector<int64_t> off((size_t)n + 1, 0), slab((size_t)n, 0);
     for (int s = 0; s < n; ++s) {
@@ -1241,8 +1192,8 @@ int acs_goalset_from_bfs_batch(acs_bfs_batch* b, acs_goalset** out) {
         slab[s] = b->h_final[s].slab;
     }
     const int64_t total = off[n];
-    MB_CUDA(cudaSetDevice(b->device));
-    MB_CUDA(cudaStreamSynchronize(b->stream));
+    ACS_CUDA(cudaSetDevice(b->device));
+    ACS_CUDA(cudaStreamSynchronize(b->stream));
     // the engine is spent from here on: free its table and logs before the entries are allocated
     MbEngine& E = b->E;
     for (void** p : {(void**)&E.table, (void**)&E.log_keys, (void**)&E.log_c, (void**)&E.log_s, (void**)&E.rec_slot,
@@ -1260,7 +1211,7 @@ int acs_goalset_from_bfs_batch(acs_bfs_batch* b, acs_goalset** out) {
     g->symmetric = b->symmetric;
     g->n_entries = total;
     int64_t* d_idx = nullptr;
-    cudaError_t e = cudaMalloc((void**)&g->nodes, (size_t)std::max<int64_t>(total, 1) * 8 * (2 * b->W + 2));
+    cudaError_t e = cudaMalloc((void**)&g->nodes, (size_t)std::max<int64_t>(total, 1) * 8 * node_words(b->W));
     if (e == cudaSuccess) e = cudaMalloc((void**)&d_idx, (2 * (size_t)n + 1) * sizeof(int64_t));
     if (e == cudaSuccess) e = cudaMemcpyAsync(d_idx, off.data(), off.size() * 8, cudaMemcpyHostToDevice, b->stream);
     if (e == cudaSuccess)
@@ -1274,10 +1225,8 @@ int acs_goalset_from_bfs_batch(acs_bfs_batch* b, acs_goalset** out) {
     if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);  // the host vectors above go out of scope
     if (d_idx) cudaFree(d_idx);
     if (e != cudaSuccess) {
-        cudaGetLastError();
         goalset_free(g);
-        return mb_fail(e == cudaErrorMemoryAllocation ? ACS_ERR_NOMEM : ACS_ERR_CUDA,
-                       std::string("goalset_from_bfs_batch: ") + cudaGetErrorString(e));
+        return cuda_fail(e, "goalset_from_bfs_batch");
     }
     cudaFree(E.nodes);
     E.nodes = nullptr;
@@ -1299,13 +1248,13 @@ int acs_bfs_batch_set_symmetric(acs_bfs_batch* b, int symmetric) {
     if (!b) return ACS_ERR_INVALID;
     if (symmetric) {
         if (b->goals && !b->goals->symmetric)
-            return mb_fail(ACS_ERR_INVALID, "bfs_batch_set_symmetric: an orbit search needs a symmetric goal set");
+            return fail(ACS_ERR_INVALID, "bfs_batch_set_symmetric: an orbit search needs a symmetric goal set");
         if (b->n_search >= (1 << kMbSymShift))
-            return mb_fail(ACS_ERR_UNSUPPORTED, "bfs_batch_set_symmetric: orbit search supports fewer than 2^28 searches");
+            return fail(ACS_ERR_UNSUPPORTED, "bfs_batch_set_symmetric: orbit search supports fewer than 2^28 searches");
         if (!b->E.log_g) {
-            MB_CUDA(cudaSetDevice(b->device));
-            MB_CUDA(cudaMalloc((void**)&b->E.log_g, (size_t)b->E.rec_cap));
-            MB_CUDA(cudaMalloc((void**)&b->d_root_g, (size_t)b->n_search));
+            ACS_CUDA(cudaSetDevice(b->device));
+            ACS_CUDA(cudaMalloc((void**)&b->E.log_g, (size_t)b->E.rec_cap));
+            ACS_CUDA(cudaMalloc((void**)&b->d_root_g, (size_t)b->n_search));
         }
     }
     b->symmetric = symmetric ? 1 : 0;

@@ -114,7 +114,7 @@ struct PbShard {
 };
 
 __device__ __forceinline__ int64_t node_gid_rt(const uint64_t* nodes, int W, int64_t idx) {
-    return (int64_t)nodes[idx * (2 * W + 2) + 2 * W + 1];
+    return (int64_t)nodes[idx * node_words(W) + 2 * W + 1];
 }
 
 __device__ __forceinline__ void st_release_sys(uint64_t* p, uint64_t v) {
@@ -1130,23 +1130,8 @@ __global__ void pb_lookup_kernel(const PbShard S, int64_t value, long long* out)
         out[0] = 1;
         out[1] = par < 0 ? -1 : (par >> 4);
         out[2] = par < 0 ? -1 : (par & 15);
-        out[3] = (long long)(k.k[W - 1] >> 58) + (long long)(k.k[2 * W - 1] >> 58);
+        out[3] = key_total_len<W>(k);
     }
-}
-
-// visited nodes -> int8 rows and global ids (local order)
-template <int W>
-__global__ void pb_unpack_kernel(const uint64_t* nodes, int8_t* out, int64_t* gid_out, uint64_t n, int mrl) {
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    Key<W> k;
-    int64_t par, g;
-    node_load<W>(nodes, i, k, par, g);
-    Rel<2 * W> r0, r1;
-    split_key<W>(k, r0, r1);
-    unpack_bytes<2 * W>(out + i * 2 * mrl, r0, mrl);
-    unpack_bytes<2 * W>(out + i * 2 * mrl + mrl, r1, mrl);
-    gid_out[i] = g;
 }
 
 // all shards in this process: path of node `node` from the root, then (extra_action, extra_len)
@@ -1167,7 +1152,7 @@ __global__ void pb_path_kernel(const PbShard* shards, int n_shards, int64_t node
                 int64_t pl = 0, gg = -1;
                 if (lo < n) node_load<W>(S.nodes, (uint64_t)lo, k, pl, gg);
                 if (lo < n && gg == g) {
-                    L = (int)(k.k[W - 1] >> 58) + (int)(k.k[2 * W - 1] >> 58);
+                    L = key_total_len<W>(k);
                     par = pl < 0 ? -1 : (pl >> 4);
                     act = pl < 0 ? -1 : (int)(pl & 15);
                     break;
@@ -1198,19 +1183,6 @@ __global__ void pb_path_kernel(const PbShard* shards, int n_shards, int64_t node
 using namespace acs;
 
 namespace {
-inline int pb_fail(int code, const std::string& m) {
-    acs::set_last_error(m.c_str());
-    return code;
-}
-#define PB_CUDA(call)                                                                      \
-    do {                                                                                   \
-        cudaError_t e__ = (call);                                                          \
-        if (e__ != cudaSuccess) {                                                          \
-            cudaGetLastError();                                                            \
-            return pb_fail(e__ == cudaErrorMemoryAllocation ? ACS_ERR_NOMEM : ACS_ERR_CUDA, \
-                           std::string(#call) + ": " + cudaGetErrorString(e__));           \
-        }                                                                                  \
-    } while (0)
 inline int64_t align256(int64_t x) { return (x + 255) / 256 * 256; }
 constexpr int kRing = 4, kLag = 2;
 }  // namespace
@@ -1248,22 +1220,16 @@ int acs_pbfs_create(int device, int rank, int world, int mrl, int64_t max_nodes,
                     acs_pbfs** out) {
     if (!out) return ACS_ERR_INVALID;
     *out = nullptr;
-    if (mrl < 1 || mrl > 61) return pb_fail(ACS_ERR_UNSUPPORTED, "bfs needs 1 <= max_relator_length <= 61");
+    if (const int rc = check_key_mrl(mrl, "bfs")) return rc;
     if (world < 1 || world > kPbMaxWorld || rank < 0 || rank >= world || max_nodes < 0)
-        return pb_fail(ACS_ERR_INVALID, "pbfs: bad rank / world / budget");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        return pb_fail(ACS_ERR_NO_DEVICE, "no CUDA device visible; there is no CPU fallback");
-    }
-    if (device < 0 || device >= ndev) return pb_fail(ACS_ERR_INVALID, "pbfs: device index out of range");
-    PB_CUDA(cudaSetDevice(device));
+        return fail(ACS_ERR_INVALID, "pbfs: bad rank / world / budget");
+    if (const int rc = open_device(device, "pbfs")) return rc;
     acs_pbfs* b = new acs_pbfs();
     b->device = device;
     b->rank = rank;
     b->world = world;
     b->mrl = mrl;
-    b->W = mrl <= 29 ? 1 : 2;
+    b->W = key_words(mrl);
     b->cyclical = cyclical ? 1 : 0;
     b->budget = max_nodes;
     // hash partitioning is balanced to a few sigma of sqrt(n/world); the budget test overshoots by <= 11
@@ -1273,7 +1239,7 @@ int acs_pbfs_create(int device, int rank, int world, int mrl, int64_t max_nodes,
     b->tcap = t;
     auto bail = [&](int code, const std::string& m) {
         acs_pbfs_destroy(b);
-        return pb_fail(code, m);
+        return fail(code, m);
     };
     if (t > (1ull << 31)) return bail(ACS_ERR_UNSUPPORTED, "pbfs: more than 2^30 nodes per rank: use more GPUs");
     // chunk size: per-rank work of ~4 Mi parents; candidate ids are 32-bit
@@ -1319,25 +1285,16 @@ int acs_pbfs_create(int device, int rank, int world, int mrl, int64_t max_nodes,
     S.off_c = off;
     off = align256(off + (int64_t)world * b->log_cap * 4);
     b->arena_bytes = off;
-#define PB_ALLOC(ptr, bytes)                                                              \
-    do {                                                                                  \
-        cudaError_t e__ = cudaMalloc((void**)&(ptr), (size_t)(bytes));                    \
-        if (e__ != cudaSuccess) {                                                         \
-            cudaGetLastError();                                                           \
-            return bail(ACS_ERR_NOMEM, std::string("cudaMalloc(" #ptr "): ") + cudaGetErrorString(e__)); \
-        }                                                                                 \
-    } while (0)
-    PB_ALLOC(S.arena, b->arena_bytes);
-    PB_ALLOC(S.st, sizeof(PbState));
-    PB_ALLOC(S.nodes, (size_t)b->cap_local * 8 * (2 * b->W + 2));
-    PB_ALLOC(S.table, (size_t)b->tcap * 8);
-    PB_ALLOC(S.rt, (size_t)(S.bitmap_words + 1) * sizeof(uint4));
-    PB_ALLOC(S.cursors, kPbMaxWorld * kCurStride * 8);
-    PB_ALLOC(S.cstart, kPbMaxWorld * 8);
-    PB_ALLOC(S.ctrl_local, kCtrlWords * 8);
-    PB_ALLOC(b->d_path, (size_t)b->path_cap * 2 * sizeof(int32_t) + 16);
-    PB_ALLOC(b->d_small, 8 * sizeof(long long));
-#undef PB_ALLOC
+    ACS_ALLOC(S.arena, b->arena_bytes, acs_pbfs_destroy(b));
+    ACS_ALLOC(S.st, sizeof(PbState), acs_pbfs_destroy(b));
+    ACS_ALLOC(S.nodes, (size_t)b->cap_local * 8 * node_words(b->W), acs_pbfs_destroy(b));
+    ACS_ALLOC(S.table, (size_t)b->tcap * 8, acs_pbfs_destroy(b));
+    ACS_ALLOC(S.rt, (size_t)(S.bitmap_words + 1) * sizeof(uint4), acs_pbfs_destroy(b));
+    ACS_ALLOC(S.cursors, kPbMaxWorld * kCurStride * 8, acs_pbfs_destroy(b));
+    ACS_ALLOC(S.cstart, kPbMaxWorld * 8, acs_pbfs_destroy(b));
+    ACS_ALLOC(S.ctrl_local, kCtrlWords * 8, acs_pbfs_destroy(b));
+    ACS_ALLOC(b->d_path, (size_t)b->path_cap * 2 * sizeof(int32_t) + 16, acs_pbfs_destroy(b));
+    ACS_ALLOC(b->d_small, 8 * sizeof(long long), acs_pbfs_destroy(b));
     // flags / control inboxes start at zero (epochs start at 1)
     if (cudaMemset(S.arena, 0, (size_t)zero_bytes) != cudaSuccess) return bail(ACS_ERR_CUDA, "pbfs: memset(arena)");
     if (cudaMallocHost((void**)&b->h_ring, kRing * sizeof(PbState)) != cudaSuccess)
@@ -1442,9 +1399,9 @@ void acs_pbfs_destroy(acs_pbfs* b) {
 int acs_pbfs_export(acs_pbfs* b, void* handle64) {
     if (!b || !handle64) return ACS_ERR_INVALID;
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "handle size");
-    PB_CUDA(cudaSetDevice(b->device));
+    ACS_CUDA(cudaSetDevice(b->device));
     cudaIpcMemHandle_t h;
-    PB_CUDA(cudaIpcGetMemHandle(&h, b->S.arena));
+    ACS_CUDA(cudaIpcGetMemHandle(&h, b->S.arena));
     std::memcpy(handle64, &h, 64);
     return ACS_OK;
 }
@@ -1452,13 +1409,13 @@ int acs_pbfs_export(acs_pbfs* b, void* handle64) {
 /* handles: world x 64 bytes in rank order (as gathered from acs_pbfs_export on every rank) */
 int acs_pbfs_connect(acs_pbfs* b, const void* handles) {
     if (!b || !handles) return ACS_ERR_INVALID;
-    PB_CUDA(cudaSetDevice(b->device));
+    ACS_CUDA(cudaSetDevice(b->device));
     for (int r = 0; r < b->world; ++r) {
         if (r == b->rank) continue;
         cudaIpcMemHandle_t h;
         std::memcpy(&h, static_cast<const char*>(handles) + 64 * r, 64);
         void* p = nullptr;
-        PB_CUDA(cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
+        ACS_CUDA(cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
         b->ipc_opened[r] = p;
         b->S.peer[r] = static_cast<char*>(p);
     }
@@ -1470,17 +1427,17 @@ int acs_pbfs_connect(acs_pbfs* b, const void* handles) {
 int acs_pbfs_connect_local(acs_pbfs** shards, int n) {
     if (!shards || n < 1) return ACS_ERR_INVALID;
     for (int i = 0; i < n; ++i)
-        if (!shards[i] || shards[i]->world != n || shards[i]->rank != i) return pb_fail(ACS_ERR_INVALID, "pbfs: shards must be ranks 0..n-1 of a world of n");
+        if (!shards[i] || shards[i]->world != n || shards[i]->rank != i) return fail(ACS_ERR_INVALID, "pbfs: shards must be ranks 0..n-1 of a world of n");
     for (int i = 0; i < n; ++i) {
         for (int j = 0; j < n; ++j) {
             shards[i]->S.peer[j] = shards[j]->S.arena;
             if (shards[i]->device != shards[j]->device) {
-                PB_CUDA(cudaSetDevice(shards[i]->device));
+                ACS_CUDA(cudaSetDevice(shards[i]->device));
                 int can = 0;
-                PB_CUDA(cudaDeviceCanAccessPeer(&can, shards[i]->device, shards[j]->device));
-                if (!can) return pb_fail(ACS_ERR_UNSUPPORTED, "pbfs: no peer access between the devices");
+                ACS_CUDA(cudaDeviceCanAccessPeer(&can, shards[i]->device, shards[j]->device));
+                if (!can) return fail(ACS_ERR_UNSUPPORTED, "pbfs: no peer access between the devices");
                 cudaError_t e = cudaDeviceEnablePeerAccess(shards[j]->device, 0);
-                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) PB_CUDA(e);
+                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) ACS_CUDA(e);
                 cudaGetLastError();
             }
         }
@@ -1488,12 +1445,12 @@ int acs_pbfs_connect_local(acs_pbfs** shards, int n) {
     }
     // device array of the pointer blocks for the path kernel
     acs_pbfs* b0 = shards[0];
-    PB_CUDA(cudaSetDevice(b0->device));
+    ACS_CUDA(cudaSetDevice(b0->device));
     if (b0->d_shards) cudaFree(b0->d_shards);
     b0->d_shards = nullptr;
-    PB_CUDA(cudaMalloc((void**)&b0->d_shards, n * sizeof(PbShard)));
+    ACS_CUDA(cudaMalloc((void**)&b0->d_shards, n * sizeof(PbShard)));
     for (int i = 0; i < n; ++i)
-        PB_CUDA(cudaMemcpy(b0->d_shards + i, &shards[i]->S, sizeof(PbShard), cudaMemcpyHostToDevice));
+        ACS_CUDA(cudaMemcpy(b0->d_shards + i, &shards[i]->S, sizeof(PbShard), cudaMemcpyHostToDevice));
     b0->n_group = n;
     return ACS_OK;
 }
@@ -1510,10 +1467,10 @@ int pb_run_impl(acs_pbfs** sh, int n_local, const int8_t* h_presentation, int32_
     const int world = b0->world;
     Key<W> root;
     int lens[2];
-    bool valid;
-    if (!pack_root<W>(h_presentation, b0->mrl, root, lens, valid))
-        return pb_fail(ACS_ERR_UNSUPPORTED, "bfs: letters outside {+-1,+-2} are not supported by the packed search");
-    if (!valid) {  // breadth_first.py:36-38 asserts is_array_valid_presentation
+    const RootCheck rc0 = pack_root<W>(h_presentation, b0->mrl, root, lens);
+    if (rc0 == RootCheck::bad_letter)
+        return fail(ACS_ERR_UNSUPPORTED, "bfs: letters outside {+-1,+-2} are not supported by the packed search");
+    if (rc0 != RootCheck::ok) {  // breadth_first.py:36-38 asserts is_array_valid_presentation
         res->status = ACS_ROW_ASSERT;
         return ACS_OK;
     }
@@ -1525,11 +1482,11 @@ int pb_run_impl(acs_pbfs** sh, int n_local, const int8_t* h_presentation, int32_
 
     for (int i = 0; i < n_local; ++i) {
         acs_pbfs* b = sh[i];
-        if (!b->connected) return pb_fail(ACS_ERR_INVALID, "pbfs: shard is not connected to its peers");
-        PB_CUDA(cudaSetDevice(b->device));
+        if (!b->connected) return fail(ACS_ERR_INVALID, "pbfs: shard is not connected to its peers");
+        ACS_CUDA(cudaSetDevice(b->device));
         cudaStream_t s = stream_of(b);
-        PB_CUDA(cudaMemsetAsync(b->S.table, 0, b->tcap * sizeof(uint64_t), s));
-        PB_CUDA(cudaMemsetAsync(b->S.cursors, 0, kPbMaxWorld * kCurStride * 8, s));
+        ACS_CUDA(cudaMemsetAsync(b->S.table, 0, b->tcap * sizeof(uint64_t), s));
+        ACS_CUDA(cudaMemsetAsync(b->S.cursors, 0, kPbMaxWorld * kCurStride * 8, s));
         PbState st{};
         st.budget = b->budget;
         st.cap_local = b->cap_local;
@@ -1550,42 +1507,39 @@ int pb_run_impl(acs_pbfs** sh, int n_local, const int8_t* h_presentation, int32_
         st.min_len = lens[0] + lens[1];
         st.sol_gid = -1;
         b->h_ring[0] = st;  // pinned staging for the async upload
-        PB_CUDA(cudaMemcpyAsync(b->S.st, &b->h_ring[0], sizeof(PbState), cudaMemcpyHostToDevice, s));
+        ACS_CUDA(cudaMemcpyAsync(b->S.st, &b->h_ring[0], sizeof(PbState), cudaMemcpyHostToDevice, s));
         if (b->rank == owner) {
             // the root is record 0 of the owner's own (owner -> owner) log, node 0 of its shard, and
             // sits in the first slot of its 4-slot bucket (where the insert kernel's probe starts)
             const uint64_t log_pos = (uint64_t)owner * (uint64_t)b->log_cap;
             const uint64_t slot_val = ((h >> 41) << 40) | (log_pos + 1);
-            const int64_t none = -1, zero = 0;
             const unsigned long long one = 1;
             const uint32_t c0 = 0;
             char* arena = b->S.arena;
-            uint64_t node0[2 * W + 2];
-            for (int k = 0; k < 2 * W; ++k) node0[k] = root.k[k];
-            node0[2 * W] = (uint64_t)none;
-            node0[2 * W + 1] = (uint64_t)zero;
-            PB_CUDA(cudaMemcpyAsync(b->S.nodes, node0, sizeof(node0), cudaMemcpyHostToDevice, s));
-            PB_CUDA(cudaMemcpyAsync(arena + b->S.off_keys + log_pos * sizeof(root), &root, sizeof(root), cudaMemcpyHostToDevice, s));
-            PB_CUDA(cudaMemcpyAsync(arena + b->S.off_c + log_pos * 4, &c0, 4, cudaMemcpyHostToDevice, s));
-            PB_CUDA(cudaMemcpyAsync(b->S.cursors + owner * kCurStride, &one, 8, cudaMemcpyHostToDevice, s));
-            PB_CUDA(cudaMemcpyAsync(b->S.table + ((h & (b->tcap - 1)) & ~3ull), &slot_val, 8, cudaMemcpyHostToDevice, s));
+            uint64_t node0[node_words(W)];
+            node_pack<W>(root, -1, 0, node0);
+            ACS_CUDA(cudaMemcpyAsync(b->S.nodes, node0, sizeof(node0), cudaMemcpyHostToDevice, s));
+            ACS_CUDA(cudaMemcpyAsync(arena + b->S.off_keys + log_pos * sizeof(root), &root, sizeof(root), cudaMemcpyHostToDevice, s));
+            ACS_CUDA(cudaMemcpyAsync(arena + b->S.off_c + log_pos * 4, &c0, 4, cudaMemcpyHostToDevice, s));
+            ACS_CUDA(cudaMemcpyAsync(b->S.cursors + owner * kCurStride, &one, 8, cudaMemcpyHostToDevice, s));
+            ACS_CUDA(cudaMemcpyAsync(b->S.table + ((h & (b->tcap - 1)) & ~3ull), &slot_val, 8, cudaMemcpyHostToDevice, s));
         }
-        PB_CUDA(cudaStreamSynchronize(s));  // the staging copies above read host stack memory
+        ACS_CUDA(cudaStreamSynchronize(s));  // the staging copies above read host stack memory
     }
-    PB_CUDA(cudaSetDevice(b0->device));
-    PB_CUDA(cudaEventRecord(b0->ev0, stream_of(b0)));
+    ACS_CUDA(cudaSetDevice(b0->device));
+    ACS_CUDA(cudaEventRecord(b0->ev0, stream_of(b0)));
 
     auto each = [&](auto&& fn) -> int {
         for (int i = 0; i < n_local; ++i) {
             acs_pbfs* b = sh[i];
             if (!same_device) {
                 cudaError_t e = cudaSetDevice(b->device);
-                if (e != cudaSuccess) return pb_fail(ACS_ERR_CUDA, cudaGetErrorString(e));
+                if (e != cudaSuccess) return fail(ACS_ERR_CUDA, cudaGetErrorString(e));
             }
             fn(b, stream_of(b));
         }
         cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return pb_fail(ACS_ERR_CUDA, std::string("pbfs launch: ") + cudaGetErrorString(e));
+        if (e != cudaSuccess) return fail(ACS_ERR_CUDA, std::string("pbfs launch: ") + cudaGetErrorString(e));
         return ACS_OK;
     };
     int rc = ACS_OK;
@@ -1606,7 +1560,7 @@ int pb_run_impl(acs_pbfs** sh, int n_local, const int8_t* h_presentation, int32_
     mark();
     for (int64_t chunk = 0;; ++chunk) {
         if (chunk >= kLag) {
-            PB_CUDA(cudaEventSynchronize(b0->ring_ev[(chunk - kLag) % kRing]));
+            ACS_CUDA(cudaEventSynchronize(b0->ring_ev[(chunk - kLag) % kRing]));
             if (b0->h_ring[(chunk - kLag) % kRing].done) break;
         }
 #define PB_PHASE(expr)                                       \
@@ -1648,21 +1602,21 @@ int pb_run_impl(acs_pbfs** sh, int n_local, const int8_t* h_presentation, int32_
         PB_PHASE((pb_decide_kernel<<<1, kCtrlWords, 0, s>>>(b->S)));
         PB_PHASE((pb_commit_kernel<W><<<b->commit_blocks, 256, 0, s>>>(b->S)));
 #undef PB_PHASE
-        if (!same_device) PB_CUDA(cudaSetDevice(b0->device));
-        PB_CUDA(cudaMemcpyAsync(&b0->h_ring[chunk % kRing], b0->S.st, sizeof(PbState), cudaMemcpyDeviceToHost, stream_of(b0)));
-        PB_CUDA(cudaEventRecord(b0->ring_ev[chunk % kRing], stream_of(b0)));
+        if (!same_device) ACS_CUDA(cudaSetDevice(b0->device));
+        ACS_CUDA(cudaMemcpyAsync(&b0->h_ring[chunk % kRing], b0->S.st, sizeof(PbState), cudaMemcpyDeviceToHost, stream_of(b0)));
+        ACS_CUDA(cudaEventRecord(b0->ring_ev[chunk % kRing], stream_of(b0)));
     }
-    PB_CUDA(cudaEventRecord(b0->ev1, stream_of(b0)));
+    ACS_CUDA(cudaEventRecord(b0->ev1, stream_of(b0)));
     int ierr = 0;
     for (int i = 0; i < n_local; ++i) {
         acs_pbfs* b = sh[i];
-        PB_CUDA(cudaSetDevice(b->device));
-        PB_CUDA(cudaStreamSynchronize(stream_of(b)));
-        PB_CUDA(cudaMemcpy(&b->h_final, b->S.st, sizeof(PbState), cudaMemcpyDeviceToHost));
+        ACS_CUDA(cudaSetDevice(b->device));
+        ACS_CUDA(cudaStreamSynchronize(stream_of(b)));
+        ACS_CUDA(cudaMemcpy(&b->h_final, b->S.st, sizeof(PbState), cudaMemcpyDeviceToHost));
         b->epoch = b->h_final.epoch;
         ierr |= b->h_final.ierr;
     }
-    PB_CUDA(cudaSetDevice(b0->device));
+    ACS_CUDA(cudaSetDevice(b0->device));
     const PbState& f = b0->h_final;
     if (ierr) {
         std::string m = "pbfs: internal error:";
@@ -1670,7 +1624,7 @@ int pb_run_impl(acs_pbfs** sh, int n_local, const int8_t* h_presentation, int32_
         if (ierr & IERR_TABLE_FULL) m += " visited table full";
         if (ierr & IERR_SHARD_FULL) m += " shard capacity exceeded (skewed partition)";
         if (ierr & IERR_TIMEOUT) m += " timed out waiting for a peer rank";
-        return pb_fail(ACS_ERR_CUDA, m);
+        return fail(ACS_ERR_CUDA, m);
     }
     res->solved = f.solved;
     res->status = f.status;
@@ -1710,13 +1664,13 @@ int pb_run_impl(acs_pbfs** sh, int n_local, const int8_t* h_presentation, int32_
         int32_t* d_len = b0->d_path + 2 * (size_t)b0->path_cap;
         cudaStream_t s = stream_of(b0);
         pb_path_kernel<W><<<1, 1, 0, s>>>(b0->d_shards, world, f.sol_gid / 12, (int)(f.sol_gid % 12), 2, b0->d_path, cap, d_len);
-        PB_CUDA(cudaGetLastError());
+        ACS_CUDA(cudaGetLastError());
         int32_t plen = 0;
-        PB_CUDA(cudaMemcpyAsync(&plen, d_len, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-        PB_CUDA(cudaStreamSynchronize(s));
+        ACS_CUDA(cudaMemcpyAsync(&plen, d_len, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        ACS_CUDA(cudaStreamSynchronize(s));
         res->path_len = plen;
         if (h_path && cap > 0)
-            PB_CUDA(cudaMemcpy(h_path, b0->d_path, (size_t)std::min(plen, cap) * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost));
+            ACS_CUDA(cudaMemcpy(h_path, b0->d_path, (size_t)std::min(plen, cap) * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost));
     }
     return ACS_OK;
 }
@@ -1734,7 +1688,7 @@ int acs_pbfs_run(acs_pbfs** shards, int n_local, const int8_t* h_presentation, i
     if (!shards || n_local < 1 || !shards[0] || !h_presentation || !res) return ACS_ERR_INVALID;
     for (int i = 0; i < n_local; ++i)
         if (!shards[i] || shards[i]->W != shards[0]->W || shards[i]->world != shards[0]->world) return ACS_ERR_INVALID;
-    if (n_local != 1 && n_local != shards[0]->world) return pb_fail(ACS_ERR_INVALID, "pbfs: pass one shard or all of them");
+    if (n_local != 1 && n_local != shards[0]->world) return fail(ACS_ERR_INVALID, "pbfs: pass one shard or all of them");
     return shards[0]->W == 1 ? pb_run_impl<1>(shards, n_local, h_presentation, h_path, path_cap, res)
                              : pb_run_impl<2>(shards, n_local, h_presentation, h_path, path_cap, res);
 }
@@ -1742,39 +1696,22 @@ int acs_pbfs_run(acs_pbfs** shards, int n_local, const int8_t* h_presentation, i
 /* out4 = {found on this rank, parent global id (-1 root), action (-1 root), total length} */
 int acs_pbfs_lookup(acs_pbfs* b, int64_t gid, int64_t* out4) {
     if (!b || !out4) return ACS_ERR_INVALID;
-    PB_CUDA(cudaSetDevice(b->device));
+    ACS_CUDA(cudaSetDevice(b->device));
     if (b->W == 1) pb_lookup_kernel<1><<<1, 1, 0, b->stream>>>(b->S, gid, b->d_small);
     else pb_lookup_kernel<2><<<1, 1, 0, b->stream>>>(b->S, gid, b->d_small);
-    PB_CUDA(cudaGetLastError());
-    PB_CUDA(cudaMemcpyAsync(out4, b->d_small, 4 * sizeof(long long), cudaMemcpyDeviceToHost, b->stream));
-    PB_CUDA(cudaStreamSynchronize(b->stream));
+    ACS_CUDA(cudaGetLastError());
+    ACS_CUDA(cudaMemcpyAsync(out4, b->d_small, 4 * sizeof(long long), cudaMemcpyDeviceToHost, b->stream));
+    ACS_CUDA(cudaStreamSynchronize(b->stream));
     return ACS_OK;
 }
 
 /* this rank's visited states (int8 rows) and their global ids (= FIFO positions), local order */
 int acs_pbfs_visited(acs_pbfs* b, int64_t* h_gid, int8_t* h_rows, int64_t cap_rows, int64_t* n_out) {
     if (!b || (cap_rows > 0 && (!h_gid || !h_rows))) return ACS_ERR_INVALID;
-    PB_CUDA(cudaSetDevice(b->device));
+    ACS_CUDA(cudaSetDevice(b->device));
     const int64_t n = std::min<int64_t>(b->h_final.n_local, std::max<int64_t>(cap_rows, 0));
     if (n_out) *n_out = n;
-    if (n == 0) return ACS_OK;
-    int8_t* d = nullptr;
-    int64_t* dg = nullptr;
-    PB_CUDA(cudaMalloc((void**)&d, (size_t)n * 2 * b->mrl));
-    if (cudaMalloc((void**)&dg, (size_t)n * 8) != cudaSuccess) {
-        cudaFree(d);
-        cudaGetLastError();
-        return pb_fail(ACS_ERR_NOMEM, "pbfs: cudaMalloc(visited ids)");
-    }
-    if (b->W == 1) pb_unpack_kernel<1><<<(unsigned)((n + 255) / 256), 256, 0, b->stream>>>(b->S.nodes, d, dg, (uint64_t)n, b->mrl);
-    else pb_unpack_kernel<2><<<(unsigned)((n + 255) / 256), 256, 0, b->stream>>>(b->S.nodes, d, dg, (uint64_t)n, b->mrl);
-    cudaError_t e = cudaMemcpyAsync(h_rows, d, (size_t)n * 2 * b->mrl, cudaMemcpyDeviceToHost, b->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(h_gid, dg, (size_t)n * 8, cudaMemcpyDeviceToHost, b->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);
-    cudaFree(dg);
-    cudaFree(d);
-    PB_CUDA(e);
-    return ACS_OK;
+    return records_to_host(b->W, b->S.nodes, node_words(b->W), n, b->mrl, h_rows, h_gid, b->stream);
 }
 
 /* counters of the last run on this rank: {n_local, chunks, records sent, records received, chunk_cap, log_cap (records per source),

@@ -307,7 +307,7 @@ __global__ void sb_lookup_kernel(const acs_sbfs_args A, int64_t value, long long
         out[0] = 1;
         out[1] = A.parent[lo] < 0 ? -1 : (A.parent[lo] >> 4);
         out[2] = A.parent[lo] < 0 ? -1 : (A.parent[lo] & 15);
-        out[3] = (long long)(k.k[W - 1] >> 58) + (long long)(k.k[2 * W - 1] >> 58);
+        out[3] = key_total_len<W>(k);
     }
 }
 
@@ -320,25 +320,22 @@ using namespace acs;
         acs::set_last_error("sbfs: bad argument block");                             \
         return ACS_ERR_INVALID;                                                      \
     }
-#define SB_LAUNCHED()                                                \
-    do {                                                             \
-        cudaError_t e__ = cudaGetLastError();                        \
-        if (e__ != cudaSuccess) {                                    \
-            acs::set_last_error(cudaGetErrorString(e__));            \
-            return ACS_ERR_CUDA;                                     \
-        }                                                            \
-        return ACS_OK;                                               \
-    } while (0)
+// the error of the launches just made, if any
+static int launched() {
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? ACS_OK : cuda_fail(e, "sbfs launch");
+}
 
 extern "C" {
 
 int acs_sbfs_pack_root(const int8_t* h_presentation, int mrl, uint64_t* key_out /*[4]*/, uint64_t* hash_out,
                        int* total_len, int* valid) {
-    if (!h_presentation || !key_out || !hash_out || !total_len || !valid || mrl < 1 || mrl > 61) return ACS_ERR_INVALID;
+    if (!h_presentation || !key_out || !hash_out || !total_len || !valid || mrl < 1 || mrl > kMaxKeyMrl)
+        return ACS_ERR_INVALID;
     int lens[2];
     bool v;
     std::memset(key_out, 0, 4 * sizeof(uint64_t));
-    if (mrl <= 29) {
+    if (key_words(mrl) == 1) {
         Key<1> k;
         if (!pack_root<1>(h_presentation, mrl, k, lens, v)) return ACS_ERR_UNSUPPORTED;
         std::memcpy(key_out, k.k, sizeof(k.k));
@@ -369,7 +366,7 @@ int acs_sbfs_expand(const acs_sbfs_args* A, int phase, void* stream) {
         if (phase == 0) sb_expand_kernel<2, 0><<<blocks, kSbThreads, 0, s>>>(*A);
         else sb_expand_kernel<2, 1><<<blocks, kSbThreads, 0, s>>>(*A);
     }
-    SB_LAUNCHED();
+    return launched();
 }
 
 int acs_sbfs_insert_mark(const acs_sbfs_args* A, void* stream) {
@@ -384,7 +381,7 @@ int acs_sbfs_insert_mark(const acs_sbfs_args* A, void* stream) {
     if (A->W == 1) sb_insert_kernel<1><<<blocks, 256, 0, s>>>(*A);
     else sb_insert_kernel<2><<<blocks, 256, 0, s>>>(*A);
     sb_mark_kernel<<<blocks, 256, 0, s>>>(*A);
-    SB_LAUNCHED();
+    return launched();
 }
 
 int acs_sbfs_scan(const uint32_t* d_bitmap, uint32_t* d_prefix, int64_t nwords, void* stream) {
@@ -397,20 +394,20 @@ int acs_sbfs_scan(const uint32_t* d_bitmap, uint32_t* d_prefix, int64_t nwords, 
     sb_scan_top_kernel<<<1, kScanThreads, 0, s>>>(block_sums, nblocks, d_prefix + nwords);
     if (nblocks > 0)
         sb_scan_final_kernel<<<(unsigned)nblocks, kScanThreads, 0, s>>>(d_bitmap, block_sums, d_prefix, nwords);
-    SB_LAUNCHED();
+    return launched();
 }
 
 int acs_sbfs_cut(const acs_sbfs_args* A, void* stream) {
     SB_CHECK(A);
     if (A->nparents <= 0) return ACS_OK;
     sb_cut_kernel<<<(unsigned)((A->nparents + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(*A);
-    SB_LAUNCHED();
+    return launched();
 }
 
 int acs_sbfs_rank_at(const acs_sbfs_args* A, uint64_t* d_out2, void* stream) {
     SB_CHECK(A);
     sb_rank_at_kernel<<<1, 1, 0, static_cast<cudaStream_t>(stream)>>>(*A, (unsigned long long*)d_out2);
-    SB_LAUNCHED();
+    return launched();
 }
 
 int acs_sbfs_commit(const acs_sbfs_args* A, void* stream) {
@@ -420,13 +417,13 @@ int acs_sbfs_commit(const acs_sbfs_args* A, void* stream) {
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     if (A->W == 1) sb_commit_kernel<1><<<blocks, 256, 0, s>>>(*A);
     else sb_commit_kernel<2><<<blocks, 256, 0, s>>>(*A);
-    SB_LAUNCHED();
+    return launched();
 }
 
 int acs_sbfs_lower_bound(const int64_t* d_gid, int64_t n, int64_t value, int64_t* d_out, void* stream) {
     if (!d_gid || !d_out || n < 0) return ACS_ERR_INVALID;
     sb_lower_bound_kernel<<<1, 1, 0, static_cast<cudaStream_t>(stream)>>>(d_gid, n, value, (long long*)d_out);
-    SB_LAUNCHED();
+    return launched();
 }
 
 int acs_sbfs_lookup(const acs_sbfs_args* A, int64_t gid, int64_t* d_out4, void* stream) {
@@ -434,17 +431,17 @@ int acs_sbfs_lookup(const acs_sbfs_args* A, int64_t gid, int64_t* d_out4, void* 
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     if (A->W == 1) sb_lookup_kernel<1><<<1, 1, 0, s>>>(*A, gid, (long long*)d_out4);
     else sb_lookup_kernel<2><<<1, 1, 0, s>>>(*A, gid, (long long*)d_out4);
-    SB_LAUNCHED();
+    return launched();
 }
 
 int acs_sbfs_unpack(const uint64_t* d_keys, int8_t* d_out, int64_t n, int mrl, void* stream) {
     if (n <= 0) return ACS_OK;
-    if (!d_keys || !d_out || mrl < 1 || mrl > 61) return ACS_ERR_INVALID;
+    if (!d_keys || !d_out || mrl < 1 || mrl > kMaxKeyMrl) return ACS_ERR_INVALID;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const unsigned blocks = (unsigned)((n + 255) / 256);
-    if (mrl <= 29) keys_unpack_kernel<1><<<blocks, 256, 0, s>>>(d_keys, d_out, (uint64_t)n, mrl);
-    else keys_unpack_kernel<2><<<blocks, 256, 0, s>>>(d_keys, d_out, (uint64_t)n, mrl);
-    SB_LAUNCHED();
+    if (key_words(mrl) == 1) records_unpack_kernel<1><<<blocks, 256, 0, s>>>(d_keys, 2, nullptr, d_out, (uint64_t)n, mrl);
+    else records_unpack_kernel<2><<<blocks, 256, 0, s>>>(d_keys, 4, nullptr, d_out, (uint64_t)n, mrl);
+    return launched();
 }
 
 }  // extern "C"

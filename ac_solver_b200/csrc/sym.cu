@@ -32,10 +32,7 @@ using namespace acs;
 
 extern "C" int acs_canonical_form(int device, int mrl, const int8_t* h_rows, int64_t n, int8_t* h_out, uint8_t* h_elem) {
     if (n < 0 || (n > 0 && (!h_rows || !h_out || !h_elem))) return ACS_ERR_INVALID;
-    if (mrl < 1 || mrl > 61) {
-        set_last_error("canonical_form needs 1 <= max_relator_length <= 61");
-        return ACS_ERR_UNSUPPORTED;
-    }
+    if (const int rc = check_key_mrl(mrl, "canonical_form")) return rc;
     for (int64_t r = 0; r < n; ++r) {  // right-padded rows of letters in {+-1, +-2}
         for (int h = 0; h < 2; ++h) {
             bool pad = false;
@@ -50,27 +47,17 @@ extern "C" int acs_canonical_form(int device, int mrl, const int8_t* h_rows, int
         }
     }
     if (n == 0) return ACS_OK;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        set_last_error("no CUDA device visible; there is no CPU fallback");
-        return ACS_ERR_NO_DEVICE;
-    }
-    if (device < 0 || device >= ndev) {
-        set_last_error("canonical_form: device index out of range");
-        return ACS_ERR_INVALID;
-    }
+    if (const int rc = open_device(device, "canonical_form")) return rc;
     const size_t bytes = (size_t)n * 2 * mrl;
     int8_t *d_in = nullptr, *d_out = nullptr;
     uint8_t* d_elem = nullptr;
-    cudaError_t e = cudaSetDevice(device);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&d_in, bytes);
+    cudaError_t e = cudaMalloc((void**)&d_in, bytes);
     if (e == cudaSuccess) e = cudaMalloc((void**)&d_out, bytes);
     if (e == cudaSuccess) e = cudaMalloc((void**)&d_elem, (size_t)n);
     if (e == cudaSuccess) e = cudaMemcpy(d_in, h_rows, bytes, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) {
         const unsigned grid = (unsigned)((n + 255) / 256);
-        if (mrl <= 29) canonical_form_kernel<1><<<grid, 256>>>(d_in, d_out, d_elem, n, mrl);
+        if (key_words(mrl) == 1) canonical_form_kernel<1><<<grid, 256>>>(d_in, d_out, d_elem, n, mrl);
         else canonical_form_kernel<2><<<grid, 256>>>(d_in, d_out, d_elem, n, mrl);
         e = cudaGetLastError();
     }
@@ -79,10 +66,5 @@ extern "C" int acs_canonical_form(int device, int mrl, const int8_t* h_rows, int
     cudaFree(d_in);
     cudaFree(d_out);
     cudaFree(d_elem);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        set_last_error((std::string("canonical_form: ") + cudaGetErrorString(e)).c_str());
-        return e == cudaErrorMemoryAllocation ? ACS_ERR_NOMEM : ACS_ERR_CUDA;
-    }
-    return ACS_OK;
+    return e == cudaSuccess ? ACS_OK : cuda_fail(e, "canonical_form");
 }

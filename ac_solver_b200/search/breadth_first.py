@@ -12,14 +12,7 @@ import numpy as np
 
 from .. import _lib
 from ..envs.utils import is_array_valid_presentation
-
-
-def _raise_for(status):
-    if status == _lib.ROW_ASSERT:
-        raise AssertionError("a move produced an invalid presentation (empty relator): "
-                             "the reference raises AssertionError here (envs/utils.py:261-263)")
-    if status == _lib.ROW_INDEX:
-        raise IndexError("index 0 is out of bounds for axis 0 with size 0")
+from ._common import _raise_for, check_row, check_rows, fetch_goal_hits, fetch_visited, search_info
 
 
 def bfs_device(presentation, max_nodes_to_explore=10000, cyclically_reduce_after_moves=False,
@@ -29,12 +22,7 @@ def bfs_device(presentation, max_nodes_to_explore=10000, cyclically_reduce_after
     on request, the visited states in insertion order as int8 rows."""
     L = _lib.lib()
     dev = _lib.default_device() if device is None else device
-    p = np.asarray(presentation)
-    if p.ndim != 1 or p.size % 2 or p.size == 0:
-        raise AssertionError(f"{presentation} is not a valid presentation")
-    if p.size and (np.abs(p).max() > 2):
-        raise ValueError("the GPU search supports the two-generator alphabet {+-1, +-2} only")
-    p8 = np.ascontiguousarray(p, dtype=np.int8)
+    p8 = check_row(presentation)
     mrl = p8.size // 2
     h = C.c_void_p()
     _lib.check(L.acs_bfs_create(None, dev, mrl, int(max_nodes_to_explore), int(bool(cyclically_reduce_after_moves)),
@@ -44,18 +32,9 @@ def bfs_device(presentation, max_nodes_to_explore=10000, cyclically_reduce_after
         path = np.zeros((cap, 2), np.int32)
         res = _lib.SearchResult()
         _lib.check(L.acs_bfs_run(h, p8.ctypes.data, path.ctypes.data, cap, C.byref(res)))
-        info = {
-            "n_visited": int(res.n_visited), "n_expanded": int(res.n_expanded), "n_moves": int(res.n_moves),
-            "frontier_left": int(res.frontier_left), "budget_hit": bool(res.budget_hit),
-            "n_levels": int(res.n_levels), "status": int(res.status),
-            "minlen_log": [int(res.minlen_log[i]) for i in range(res.n_minlen)],
-            "seconds_device": float(res.seconds_device),
-        }
+        info = search_info(res)
         if want_visited and res.status == 0:
-            vis = np.zeros((max(int(res.n_visited), 1), 2 * mrl), np.int8)
-            n_out = C.c_int64(0)
-            _lib.check(L.acs_bfs_visited(h, vis.ctypes.data, vis.shape[0], C.byref(n_out)))
-            info["visited"] = vis[: n_out.value]
+            info["visited"] = fetch_visited(L.acs_bfs_visited, res.n_visited, 2 * mrl, h)
     finally:
         L.acs_bfs_destroy(h)
     _raise_for(res.status)
@@ -70,17 +49,13 @@ DEFAULT_MAX_TOTAL_BYTES = 128 << 30
 
 def _batch_inputs(presentations, max_nodes_to_explore):
     """Validate a batch on the host, before any GPU work -> (int8 rows, int64 budgets)."""
-    P = np.asarray(presentations)
-    if P.ndim != 2 or P.shape[1] % 2 or P.shape[1] == 0:
-        raise ValueError("presentations must be [S, 2*max_relator_length]")
-    if P.size and np.abs(P.astype(np.int64)).max() > 2:  # wide: abs(int8 -128) is -128
-        raise ValueError("the GPU search supports the two-generator alphabet {+-1, +-2} only")
+    P = check_rows(presentations)
     budgets = np.broadcast_to(np.asarray(max_nodes_to_explore, dtype=np.int64), (P.shape[0],))
     if np.ndim(max_nodes_to_explore) > 1 or (budgets < 0).any():
         raise ValueError("max_nodes_to_explore must be one non-negative int or one per row")
     for k in range(P.shape[0]):  # breadth_first.py:36-38
         assert is_array_valid_presentation(P[k]), f"row {k}: {P[k].tolist()} is not a valid presentation"
-    return np.ascontiguousarray(P, dtype=np.int8), np.ascontiguousarray(budgets)
+    return P, np.ascontiguousarray(budgets)
 
 
 def _engine_bytes(L, mrl, budgets, chunk_parents):
@@ -143,30 +118,17 @@ class _BatchEngine:
             paths = np.zeros((S, cap, 2), np.int32)
             rc = L.acs_bfs_batch_paths(self.h, paths.ctypes.data, cap)
         _lib.check(rc)
-        hits = None
+        goal_info = None
         if self.goals is not None:
-            hits = np.full(S, -1, np.int64)
-            _lib.check(L.acs_bfs_batch_goal_hits(self.h, hits.ctypes.data))
-            elems = np.full(S, -1, np.int32)
-            _lib.check(L.acs_bfs_batch_goal_hit_elements(self.h, elems.ctypes.data))
+            goal_info = fetch_goal_hits(L.acs_bfs_batch_goal_hits, L.acs_bfs_batch_goal_hit_elements, self.h, S)
         out = []
         for s in range(S):
             r = res[s]
-            info = {
-                "n_visited": int(r.n_visited), "n_expanded": int(r.n_expanded), "n_moves": int(r.n_moves),
-                "frontier_left": int(r.frontier_left), "budget_hit": bool(r.budget_hit),
-                "n_levels": int(r.n_levels), "status": int(r.status),
-                "minlen_log": [int(r.minlen_log[i]) for i in range(r.n_minlen)],
-                "seconds_device": float(r.seconds_device),
-            }
-            if hits is not None:
-                info["goal"] = int(hits[s]) if hits[s] >= 0 else None
-                info["goal_element"] = int(elems[s]) if hits[s] >= 0 else None
+            info = search_info(r)
+            if goal_info is not None:
+                info.update(goal_info[s])
             if want_visited and r.status == 0:
-                vis = np.zeros((max(int(r.n_visited), 1), self.P8.shape[1]), np.int8)
-                n_out = C.c_int64(0)
-                _lib.check(L.acs_bfs_batch_visited(self.h, s, vis.ctypes.data, vis.shape[0], C.byref(n_out)))
-                info["visited"] = vis[: n_out.value]
+                info["visited"] = fetch_visited(L.acs_bfs_batch_visited, r.n_visited, self.P8.shape[1], self.h, s)
             plist = [(int(a), int(l)) for a, l in paths[s, : r.path_len]] if r.solved else None
             out.append((bool(r.solved), plist, info))
         return out

@@ -16,6 +16,7 @@ import numpy as np
 
 from .. import _lib
 from ..envs.utils import generate_trivial_states, is_array_valid_presentation
+from ._common import check_rows
 from .breadth_first import DEFAULT_MAX_BYTES, _BatchEngine, _batch_inputs, bfs_batch
 
 # the move that undoes each of the 12 moves when relators are only freely reduced (bfs_common.cuh, skip_moves):
@@ -46,13 +47,8 @@ PI = [[int(T >> (4 * m) & 15) for m in range(12)] for T in (
 
 def _goal_rows(rows, cyclical):
     """Validate goal rows on the host -> int8 rows.  A row must be a state a search can generate."""
-    R = np.asarray(rows)
-    if R.ndim != 2 or R.shape[1] % 2 or R.shape[1] == 0:
-        raise ValueError("goal rows must be [n, 2*max_relator_length]")
-    if R.size and np.abs(R.astype(np.int64)).max() > 2:
-        raise ValueError("the GPU search supports the two-generator alphabet {+-1, +-2} only")
-    mrl = R.shape[1] // 2
-    R8 = np.ascontiguousarray(R, dtype=np.int8)
+    R8 = check_rows(rows, "goal rows must be [n, 2*max_relator_length]")
+    mrl = R8.shape[1] // 2
     for k in range(R8.shape[0]):
         if not is_array_valid_presentation(R8[k]):
             raise ValueError(f"goal row {k}: {R8[k].tolist()} is not a valid presentation "

@@ -11,7 +11,19 @@ import ctypes as C
 import numpy as np
 
 from .. import _lib
-from .breadth_first import _check_goals, _raise_for
+from ._common import _raise_for, check_rows, fetch_goal_hits, fetch_visited, search_info
+from .breadth_first import _check_goals
+
+
+def _rows(res, paths, goal_info=None):
+    """(solved, path, info) of every search of a run; ``goal_info`` from ``fetch_goal_hits`` for a goal run."""
+    out = []
+    for s, r in enumerate(res):
+        info = search_info(r, "rounds")
+        if goal_info is not None:
+            info.update(goal_info[s])
+        out.append((bool(r.solved), [(int(a), int(l)) for a, l in paths[s, : r.path_len]], info))
+    return out
 
 
 def greedy_search_batch(presentations, max_nodes_to_explore=10000, cyclically_reduce_after_moves=False,
@@ -31,12 +43,7 @@ def greedy_search_batch(presentations, max_nodes_to_explore=10000, cyclically_re
     plain search exactly."""
     L = _lib.lib()
     dev = _lib.default_device() if device is None else device
-    P = np.asarray(presentations)
-    if P.ndim != 2 or P.shape[1] % 2 or P.shape[1] == 0:
-        raise ValueError("presentations must be [S, 2*max_relator_length]")
-    if P.size and np.abs(P).max() > 2:
-        raise ValueError("the GPU search supports the two-generator alphabet {+-1, +-2} only")
-    P8 = np.ascontiguousarray(P, dtype=np.int8)
+    P8 = check_rows(presentations)
     S, w = P8.shape
     mrl = w // 2
     _check_goals(goals, mrl, cyclically_reduce_after_moves, dev)
@@ -47,44 +54,26 @@ def greedy_search_batch(presentations, max_nodes_to_explore=10000, cyclically_re
     h = C.c_void_p()
     _lib.check(L.acs_greedy_create(dev, S, mrl, budget, int(bool(cyclically_reduce_after_moves)), path_cap,
                                    C.byref(h)))
-    out = []
     try:
         if goals is not None:
             _lib.check(L.acs_greedy_set_goals(h, goals.handle))
         paths = np.zeros((S, path_cap, 2), np.int32)
         res = (_lib.SearchResult * S)()
         _lib.check(L.acs_greedy_run(h, P8.ctypes.data, paths.ctypes.data, res))
-        hits = None
+        need = max(r.path_len for r in res)
+        if need > path_cap:  # deeper than the buffer: the reference has no limit -- run again with room
+            L.acs_greedy_destroy(h)
+            h = None
+            return greedy_search_batch(presentations, max_nodes_to_explore, cyclically_reduce_after_moves, want_visited,
+                                       device, path_cap=int(need) + 4, goals=goals)
+        goal_info = None
         if goals is not None:
-            hits = np.full(S, -1, np.int64)
-            _lib.check(L.acs_greedy_goal_hits(h, hits.ctypes.data))
-            elems = np.full(S, -1, np.int32)
-            _lib.check(L.acs_greedy_goal_hit_elements(h, elems.ctypes.data))
-        for s in range(S):
-            r = res[s]
-            info = {
-                "n_visited": int(r.n_visited), "n_expanded": int(r.n_expanded), "n_moves": int(r.n_moves),
-                "frontier_left": int(r.frontier_left), "budget_hit": bool(r.budget_hit), "status": int(r.status),
-                "minlen_log": [int(r.minlen_log[i]) for i in range(r.n_minlen)],
-                "seconds_device": float(r.seconds_device),
-                # bucket rounds of the CTA-per-search kernel; -1: served by the one-warp heap kernel
-                "rounds": int(r.n_levels),
-            }
-            if hits is not None:
-                info["goal"] = int(hits[s]) if hits[s] >= 0 else None
-                info["goal_element"] = int(elems[s]) if hits[s] >= 0 else None
-            if r.path_len > path_cap:  # deeper than the buffer: the reference has no limit -- run again with room
-                L.acs_greedy_destroy(h)
-                h = None
-                return greedy_search_batch(presentations, max_nodes_to_explore, cyclically_reduce_after_moves, want_visited,
-                                           device, path_cap=int(max(res[i].path_len for i in range(S))) + 4, goals=goals)
-            if want_visited and r.status == 0:
-                vis = np.zeros((max(int(r.n_visited), 1), w), np.int8)
-                n_out = C.c_int64(0)
-                _lib.check(L.acs_greedy_visited(h, s, vis.ctypes.data, vis.shape[0], C.byref(n_out)))
-                info["visited"] = vis[: n_out.value]
-            plist = [(int(a), int(l)) for a, l in paths[s, : r.path_len]]
-            out.append((bool(r.solved), plist, info))
+            goal_info = fetch_goal_hits(L.acs_greedy_goal_hits, L.acs_greedy_goal_hit_elements, h, S)
+        out = _rows(res, paths, goal_info)
+        if want_visited:
+            for s, (_, _, info) in enumerate(out):
+                if info["status"] == 0:
+                    info["visited"] = fetch_visited(L.acs_greedy_visited, info["n_visited"], w, h, s)
     finally:
         if h is not None:
             L.acs_greedy_destroy(h)
@@ -106,11 +95,7 @@ def greedy_search_groups(groups, max_nodes_to_explore=10000, cyclically_reduce_a
     arrays, handles = [], []
     try:
         for P in groups:
-            P8 = np.ascontiguousarray(np.asarray(P), dtype=np.int8)
-            if P8.ndim != 2 or P8.shape[1] % 2 or P8.shape[1] == 0:
-                raise ValueError("every group must be [S, 2*max_relator_length]")
-            if P8.size and np.abs(P8).max() > 2:
-                raise ValueError("the GPU search supports the two-generator alphabet {+-1, +-2} only")
+            P8 = check_rows(P, "every group must be [S, 2*max_relator_length]")
             h = C.c_void_p()
             _lib.check(L.acs_greedy_create(dev, P8.shape[0], P8.shape[1] // 2, budget, int(bool(cyclically_reduce_after_moves)),
                                            int(path_cap), C.byref(h)))
@@ -137,15 +122,7 @@ def greedy_search_groups(groups, max_nodes_to_explore=10000, cyclically_reduce_a
             out.append(greedy_search_batch(arrays[k], budget, cyclically_reduce_after_moves, device=dev,
                                            path_cap=int(max(res[s].path_len for s in range(S))) + 4))
             continue
-        rows = []
-        for s in range(S):
-            r = res[s]
-            info = {"n_visited": int(r.n_visited), "n_expanded": int(r.n_expanded), "n_moves": int(r.n_moves),
-                    "frontier_left": int(r.frontier_left), "budget_hit": bool(r.budget_hit), "status": int(r.status),
-                    "minlen_log": [int(r.minlen_log[i]) for i in range(r.n_minlen)], "seconds_device": float(r.seconds_device),
-                    "rounds": int(r.n_levels)}
-            rows.append((bool(r.solved), [(int(a), int(l)) for a, l in paths[s, : r.path_len]], info))
-        out.append(rows)
+        out.append(_rows(res, paths))
     return out
 
 

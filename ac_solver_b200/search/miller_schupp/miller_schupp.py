@@ -64,7 +64,8 @@ def trivialize_miller_schupp_through_search(min_n, max_n, min_w_len, max_w_len, 
     """miller_schupp.py:95-177.  ``search_fn`` is this package's ``greedy_search`` or ``bfs``.
     Returns (solved_rels, unsolved_rels, solved_paths) in the reference's order."""
     assert search_fn.__name__ in ["greedy_search", "bfs"], f"expect search_fn to be greedy or bfs; got {search_fn.__name__}"
-    from ..breadth_first import _raise_for, bfs_batch
+    from .._common import _raise_for
+    from ..breadth_first import bfs_batch
     from ..greedy import greedy_search_batch
 
     rels = {n: generate_miller_schupp_presentations(n, max_w_len) for n in range(min_n, max_n + 1)}

@@ -19,33 +19,11 @@ import ctypes as C
 import numpy as np
 
 from .. import _lib
-
-
-def _check_presentation(presentation):
-    p = np.asarray(presentation)
-    if p.ndim != 1 or p.size % 2 or p.size == 0:
-        raise AssertionError(f"{presentation} is not a valid presentation")
-    if p.size and (np.abs(p).max() > 2):
-        raise ValueError("the GPU search supports the two-generator alphabet {+-1, +-2} only")
-    return np.ascontiguousarray(p, dtype=np.int8)
-
-
-def _raise_for(status):
-    if status == _lib.ROW_ASSERT:
-        raise AssertionError("a move produced an invalid presentation (empty relator): "
-                             "the reference raises AssertionError here (envs/utils.py:261-263)")
-    if status == _lib.ROW_INDEX:
-        raise IndexError("index 0 is out of bounds for axis 0 with size 0")
+from ._common import _raise_for, check_row, search_info
 
 
 def _info(res, stats_list):
-    info = {
-        "n_visited": int(res.n_visited), "n_expanded": int(res.n_expanded), "n_moves": int(res.n_moves),
-        "frontier_left": int(res.frontier_left), "budget_hit": bool(res.budget_hit),
-        "n_levels": int(res.n_levels), "status": int(res.status),
-        "minlen_log": [int(res.minlen_log[i]) for i in range(res.n_minlen)],
-        "seconds_device": float(res.seconds_device),
-    }
+    info = search_info(res)
     st = stats_list[0]
     info.update(n_local=[int(s[0]) for s in stats_list], chunks=int(st[1]),
                 records_sent=[int(s[2]) for s in stats_list], records_recv=[int(s[3]) for s in stats_list],
@@ -119,7 +97,7 @@ class PartitionedBfs:
     def run(self, presentation, want_visited=False):
         """-> (solved, path|None, info), identical on every rank."""
         torch = self.torch
-        p8 = _check_presentation(presentation)
+        p8 = check_row(presentation)
         if p8.size != 2 * self.mrl:
             raise ValueError("presentation length does not match this search's max_relator_length")
         n = len(self.handles)
@@ -200,7 +178,7 @@ def bfs_partitioned(presentation, max_nodes_to_explore=10000, cyclically_reduce_
     """Partitioned ``bfs``: call on every rank of the process group with the same arguments.
     Returns ``(solved, path|None, info)`` on every rank; ``info["visited"]`` (rank 0, on request)
     holds the visited states in the reference's insertion order."""
-    p8 = _check_presentation(presentation)
+    p8 = check_row(presentation)
     with PartitionedBfs(p8.size // 2, max_nodes_to_explore, cyclically_reduce_after_moves, group=group,
                         sim_world=sim_world, chunk_parents=chunk_parents, device=device) as eng:
         solved, path, info = eng.run(p8, want_visited=want_visited)

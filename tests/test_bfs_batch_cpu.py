@@ -22,6 +22,23 @@ def test_bfs_batch_rejects_bad_shapes_and_alphabet():
         bfs_batch(np.array([[1, 0, 2, 0]]), -1)
 
 
+def test_every_search_refuses_int8_minus_128_on_the_host():
+    """abs() of int8 -128 is -128, so a plain abs test lets it through to the library: every wrapper checks
+    the alphabet wide and raises the same ValueError as bfs_batch, before any device work."""
+    from ac_solver_b200 import greedy_search, greedy_search_batch
+    from ac_solver_b200.search.breadth_first import bfs_device
+    from ac_solver_b200.search.greedy import greedy_search_groups
+    from ac_solver_b200.search.partitioned import bfs_partitioned
+
+    row = np.array([1, -128, 2, 0], np.int8)
+    calls = [lambda: bfs_device(row, 10), lambda: bfs_partitioned(row, 10, sim_world=1),
+             lambda: greedy_search(row, 10), lambda: greedy_search_batch(row[None, :], 10),
+             lambda: greedy_search_groups([row[None, :]], 10)]
+    for call in calls:
+        with pytest.raises(ValueError, match="alphabet"):
+            call()
+
+
 def test_bfs_batch_names_the_invalid_row():
     from ac_solver_b200 import bfs_batch, bfs_groups
 
