@@ -113,6 +113,15 @@ _SIGS = {
     "acs_canonical_form": (C.c_int, [C.c_int, C.c_int, _P, C.c_int64, _P, _P]),
     "acs_bfs_batch_set_symmetric": (C.c_int, [_P, C.c_int]),
     "acs_bfs_batch_goal_hit_elements": (C.c_int, [_P, _P]),
+    "acs_beam_bytes": (C.c_int, [C.c_int, C.c_int, C.c_int64, _P, C.c_int, C.POINTER(C.c_int64)]),
+    "acs_beam_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int64, _P, C.c_int, C.c_int, C.POINTER(_P)]),
+    "acs_beam_set_goals": (C.c_int, [_P, _P]),
+    "acs_beam_run": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(SearchResult)]),
+    "acs_beam_paths": (C.c_int, [_P, _P, C.c_int]),
+    "acs_beam_visited": (C.c_int, [_P, C.c_int, _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "acs_beam_goal_hits": (C.c_int, [_P, _P]),
+    "acs_beam_goal_hit_elements": (C.c_int, [_P, _P]),
+    "acs_beam_destroy": (None, [_P]),
     "acs_goalset_from_rows_symmetric": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, C.c_int64, C.POINTER(_P)]),
     "acs_goalset_is_symmetric": (C.c_int, [_P, C.POINTER(C.c_int)]),
     "acs_goalset_path_frame": (C.c_int, [_P, C.c_int64, C.POINTER(C.c_int), _P, C.c_int, C.POINTER(C.c_int),

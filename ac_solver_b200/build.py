@@ -15,7 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libacsolver_b200.so")
-SOURCES = ["capi.cu", "moves_kernel.cu", "generic_kernel.cu", "greedy.cu", "sbfs.cu", "pbfs.cu", "mbfs.cu", "goalset.cu", "sym.cu", "ball.cu", "ppo_kernels.cu"]
+SOURCES = ["capi.cu", "moves_kernel.cu", "generic_kernel.cu", "greedy.cu", "sbfs.cu", "pbfs.cu", "mbfs.cu", "beam.cu", "goalset.cu", "sym.cu", "ball.cu", "ppo_kernels.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17",

@@ -64,25 +64,30 @@ def _engine_bytes(L, mrl, budgets, chunk_parents):
     return b.value
 
 
-def _split(L, mrl, budgets, chunk_parents, max_bytes):
+def _split_by(engine_bytes, budgets, max_bytes):
     """Consecutive row ranges whose engines each need at most max_bytes (a single row may need more)
-    -> list of (lo, hi, bytes).  An engine's size grows with its rows, so each range end is found by
-    bisection."""
+    -> list of (lo, hi, bytes), where ``engine_bytes(budgets[lo:hi])`` is the size of the engine of rows
+    [lo, hi).  An engine's size grows with its rows, so each range end is found by bisection."""
     parts, lo = [], 0
     S = len(budgets)
     while lo < S:
         good, bad = lo + 1, S + 1  # rows [lo, good) fit (or are a single row); [lo, bad) do not
-        if _engine_bytes(L, mrl, budgets[lo:S], chunk_parents) <= max_bytes:
+        if engine_bytes(budgets[lo:S]) <= max_bytes:
             good = S
         while bad - good > 1 and good < S:
             mid = (good + bad) // 2
-            if _engine_bytes(L, mrl, budgets[lo:mid], chunk_parents) <= max_bytes:
+            if engine_bytes(budgets[lo:mid]) <= max_bytes:
                 good = mid
             else:
                 bad = mid
-        parts.append((lo, good, _engine_bytes(L, mrl, budgets[lo:good], chunk_parents)))
+        parts.append((lo, good, engine_bytes(budgets[lo:good])))
         lo = good
     return parts
+
+
+def _split(L, mrl, budgets, chunk_parents, max_bytes):
+    """``_split_by`` for ``bfs_batch`` engines."""
+    return _split_by(lambda b: _engine_bytes(L, mrl, b, chunk_parents), budgets, max_bytes)
 
 
 class _BatchEngine:

@@ -296,6 +296,44 @@ int acs_goalset_path_frame(const acs_goalset *g, int64_t entry, int *root, int32
 int acs_bfs_batch_goal_hit_elements(acs_bfs_batch *b, int32_t *h_elem /* [n_search] */);
 int acs_greedy_goal_hit_elements(acs_greedy *g, int32_t *h_elem /* [n_search] */);
 
+/* Batched beam search (csrc/beam.cu): n_search independent searches of the same mrl and cyclical flag, one
+ * node budget each, advanced together level by level through the same kernel launches on one GPU.  A search
+ * keeps a visited list V = [root] and a beam = [root].  At each level the candidates c = 12*i + m (move m of
+ * beam node i) are walked in increasing c: the first that raises (results[s].status), has total length 2 or
+ * is in the goal set ends the search and nothing of that level is kept.  Otherwise the children whose state
+ * is not in V, each at its smallest c, are ordered by (total length, c) and the first
+ * min(beam_width, max_nodes[s] - |V|) become the next beam, appended to V in that order.  A search stops
+ * after a level whose next beam is empty, that brought |V| to max_nodes[s] (budget_hit), or the
+ * max_depth-th level.  Counters and paths are those of acs_bfs_batch_run: n_moves counts candidates up to
+ * and including the one that ended the search, n_expanded the beam nodes expanded, frontier_left the beam
+ * nodes left, n_levels the levels kept, minlen_log every new minimal total length in (level, c) order.
+ * Orbit (symmetric) search is not offered by this engine; symmetric goal sets are.
+ * acs_beam_bytes: device bytes an engine for these arguments allocates (for planning batches).
+ * acs_beam_create: 1 <= beam_width <= 2^24, every max_nodes[s] >= 1, max_depth >= 1 or 0 for no limit,
+ * 1 <= mrl <= 61; anything else is ACS_ERR_INVALID / ACS_ERR_UNSUPPORTED before any device work.
+ * acs_beam_run: h_presentations [n_search, 2*mrl] (a row that is not right-padded or has an empty relator
+ * gets status ACS_ROW_ASSERT and is not searched); h_paths [n_search, path_cap, 2] int32 (action,
+ * total_length) pairs; results [n_search].  A path longer than path_cap makes the run return
+ * ACS_ERR_INVALID with every other result filled (results[s].path_len holds the needed length);
+ * acs_beam_paths then fetches the paths of that run into a larger buffer without searching again.
+ * acs_beam_visited: V of search `search` of the last run, in order, as int8 rows.
+ * acs_beam_set_goals: goal set of the next runs (may be NULL; must outlive those runs), exact or symmetric;
+ * its mrl, cyclical flag and device must be b's, else ACS_ERR_INVALID.  A root in the set is a hit at depth
+ * 0 with the path [(-1, L0)].  acs_beam_goal_hits / acs_beam_goal_hit_elements: as for acs_bfs_batch. */
+typedef struct acs_beam acs_beam;
+int acs_beam_bytes(int n_search, int mrl, int64_t beam_width, const int64_t *max_nodes, int max_depth,
+                   int64_t *bytes_out);
+int acs_beam_create(int device, int n_search, int mrl, int64_t beam_width, const int64_t *max_nodes /* [n_search] */,
+                    int max_depth, int cyclical, acs_beam **out);
+int acs_beam_set_goals(acs_beam *b, const acs_goalset *g);
+int acs_beam_run(acs_beam *b, const int8_t *h_presentations, int32_t *h_paths, int path_cap,
+                 acs_search_result *results /* [n_search] */);
+int acs_beam_paths(acs_beam *b, int32_t *h_paths, int path_cap);
+int acs_beam_visited(acs_beam *b, int search, int8_t *h_out, int64_t cap_rows, int64_t *n_out);
+int acs_beam_goal_hits(acs_beam *b, int64_t *h_entry /* [n_search] */);
+int acs_beam_goal_hit_elements(acs_beam *b, int32_t *h_elem /* [n_search] */);
+void acs_beam_destroy(acs_beam *b);
+
 /* ---- hash-partitioned multi-GPU BFS: per-rank device kernels --------------------------------- */
 /* The host loop (ac_solver_b200/search/sharded.py, one process per GPU, torch.distributed/NCCL
  * for the all-to-all and the small all-reduces) drives these on caller-allocated device buffers.
