@@ -47,6 +47,7 @@
 #include "bfs_common.cuh"
 #include "goalset.cuh"
 #include "mb_engine.cuh"
+#include "mb_host.cuh"
 
 namespace acs {
 
@@ -245,62 +246,12 @@ __global__ void __launch_bounds__(128) bm_decide_kernel(const BmEngine B) {
     const uint64_t off = (uint64_t)E.seg_off[k], F = (uint64_t)E.seg_off[k + 1] - off;
     const uint64_t c0 = 12 * off, head = (uint64_t)M.head;
     uint64_t limit = 12 * F;  // candidates evaluated: up to the event, or all
-    const unsigned long long sol = red[kMbSol], err = red[kMbErr], goal = red[kMbGoal];
-    bool sol_here = false, goal_here = false;
-    int status = 0;
-    uint64_t ev = 0;
-    if (sol != ~0ull) {
-        ev = sol - c0;
-        limit = ev;
-        sol_here = true;
-    }
-    if (goal != ~0ull && (goal >> 32) - c0 < limit) {  // on the solving child itself the solve wins
-        ev = (goal >> 32) - c0;
-        limit = ev;
-        sol_here = goal_here = true;
-    }
-    if (err != ~0ull && (err >> 2) - c0 < limit) {
-        ev = (err >> 2) - c0;
-        limit = ev;
-        status = (int)(err & 3);
-        sol_here = goal_here = false;
-    }
-    const uint64_t c_limit = limit + (sol_here ? 1 : 0);
-    int min_len = M.min_len;
-    for (;;) {  // new minimal lengths in candidate order
-        unsigned long long best = ~0ull;
-        int bestL = -1;
-        for (int L = 0; L < min_len && L < 128; ++L) {
-            const unsigned long long g = red[kMbLen0 + L];
-            if (g != ~0ull && g - c0 < c_limit && g < best) {
-                best = g;
-                bestL = L;
-            }
-        }
-        if (bestL < 0) break;
-        min_len = bestL;
-        if (M.n_minlen < 128) M.minlen_log[M.n_minlen++] = bestL;
-    }
-    M.min_len = min_len;
+    const MbEvent ev = mb_event(red, red[kMbSol], c0, limit);
+    mb_minlen_log(M, red, c0, limit, ev.solved);
     E.seg_limit[k] = 0;
-    if (sol_here || status) {
+    if (ev.solved || ev.status) {
         M.done = 1;
-        M.n_expanded = (int64_t)((12 * head + ev) / 12 + 1);
-        if (status) {
-            M.status = status;
-            M.err_code = (int64_t)(((12 * head + ev) << 2) | (uint64_t)status);
-            return;
-        }
-        M.solved = 1;
-        M.sol_gid = (int64_t)(12 * head + ev);
-        M.sol_len = 2;
-        if (goal_here) {
-            const uint64_t e = goal & 0xFFFFFFFFull;
-            const int W = key_words(st->mrl);
-            const uint64_t* q = E.goals.nodes + e * node_words(W);
-            M.sol_len = key_len(q, W, 0) + key_len(q, W, 1);
-            E.goal_hit[s] = (int64_t)e;
-        }
+        mb_end_at(E, M, s, red, ev, head);
         return;
     }
     uint32_t* h = B.hist + (int64_t)k * kBmLens;
@@ -388,8 +339,6 @@ __global__ void __launch_bounds__(kBmSelT) bm_select_kernel(const BmEngine B) {
 using namespace acs;
 
 namespace {
-constexpr int kBmRing = 4, kBmLag = 2;
-
 // sizes of an engine (shared by acs_beam_bytes and acs_beam_create)
 struct BmPlan {
     int W;
@@ -436,25 +385,19 @@ int bm_plan(int n_search, int mrl, int64_t width, const int64_t* max_nodes, int 
 }
 }  // namespace
 
-struct acs_beam {
-    int device = 0, n_search = 0, mrl = 0, W = 1, cyclical = 0;
+struct acs_beam : MbHost {
     BmPlan plan{};
     BmEngine B{};
-    uint64_t* d_roots = nullptr;
-    int32_t* d_paths = nullptr;
-    int32_t* d_plen = nullptr;
-    int d_path_cap = 0;
-    std::vector<int64_t> budgets;
-    std::vector<MbSearch> h_final;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr, ring_ev[kBmRing] = {};
-    MbState* h_ring = nullptr;  // pinned [kBmRing]
-    int sms = 148;
-    int expand_blocks = 148, expand_wpb = 8, insert_blocks = 148;
-    size_t expand_smem = 0;
-    bool ran = false;
-    const acs_goalset* goals = nullptr;  // acs_beam_set_goals
 };
+
+// launch sizes from the kernels' occupancy
+template <int W>
+static void bm_size_launches(acs_beam* b) {
+    b->expand_smem = (size_t)b->expand_wpb * mb_stage_bytes_per_warp<W>();
+    b->expand_blocks = mb_blocks(*b, mb_expand_kernel<W, true, false, false>, 32 * b->expand_wpb, b->expand_smem);
+    b->insert_blocks = mb_blocks(*b, bm_insert_kernel<W>, 256, 0);
+    cudaGetLastError();
+}
 
 extern "C" {
 
@@ -470,23 +413,9 @@ int acs_beam_bytes(int n_search, int mrl, int64_t beam_width, const int64_t* max
 
 void acs_beam_destroy(acs_beam* b) {
     if (!b) return;
-    cudaSetDevice(b->device);
-    if (b->stream) {
-        cudaStreamSynchronize(b->stream);
-        cudaStreamDestroy(b->stream);
-    }
-    if (b->ev0) cudaEventDestroy(b->ev0);
-    if (b->ev1) cudaEventDestroy(b->ev1);
-    for (auto e : b->ring_ev)
-        if (e) cudaEventDestroy(e);
-    MbEngine& E = b->B.E;
-    void* ptrs[] = {E.st, E.srch, E.nodes, E.table, E.log_keys, E.log_c, E.log_s, E.cursor, E.bitmap, E.ctrl,
-                    E.seg_search, E.seg_head, E.seg_off, E.seg_limit, E.seg_base, E.seg_of, E.goal_hit, E.goal_hit_g,
-                    b->B.ltab, b->B.lmask, b->B.rec_of, b->B.wlen, b->B.hist, b->d_roots, b->d_paths, b->d_plen};
-    for (void* p : ptrs)
+    mb_close(*b, b->B.E);
+    for (void* p : {(void*)b->B.ltab, (void*)b->B.lmask, (void*)b->B.rec_of, (void*)b->B.wlen, (void*)b->B.hist})
         if (p) cudaFree(p);
-    if (b->h_ring) cudaFreeHost(b->h_ring);
-    cudaGetLastError();
     delete b;
 }
 
@@ -499,67 +428,26 @@ int acs_beam_create(int device, int n_search, int mrl, int64_t beam_width, const
     if (rc != ACS_OK) return rc;
     if (const int rc2 = open_device(device, "beam")) return rc2;
     acs_beam* b = new acs_beam();
-    b->device = device;
-    b->n_search = n_search;
-    b->mrl = mrl;
-    b->W = P.W;
-    b->cyclical = cyclical ? 1 : 0;
+    mb_init(*b, device, n_search, mrl, P.W, cyclical, max_nodes);
     b->plan = P;
-    b->budgets.assign(max_nodes, max_nodes + n_search);
     BmEngine& B = b->B;
     B.width = beam_width;
     B.max_depth = max_depth;
-    MbEngine& E = B.E;
-    E.rec_cap = P.rec_cap;
-    ACS_ALLOC(E.st, sizeof(MbState), acs_beam_destroy(b));
-    ACS_ALLOC(E.srch, (size_t)n_search * sizeof(MbSearch), acs_beam_destroy(b));
-    ACS_ALLOC(E.nodes, (size_t)P.nodes * 8 * node_words(P.W), acs_beam_destroy(b));
-    ACS_ALLOC(E.table, (size_t)P.tcap * 8, acs_beam_destroy(b));
-    ACS_ALLOC(E.log_keys, (size_t)P.rec_cap * 16 * P.W, acs_beam_destroy(b));
-    ACS_ALLOC(E.log_c, (size_t)P.rec_cap * 4, acs_beam_destroy(b));
-    ACS_ALLOC(E.log_s, (size_t)P.rec_cap * 4, acs_beam_destroy(b));
-    ACS_ALLOC(E.cursor, 8, acs_beam_destroy(b));
-    ACS_ALLOC(E.bitmap, (size_t)P.bitmap_words * 4, acs_beam_destroy(b));
-    ACS_ALLOC(E.ctrl, (size_t)n_search * kMbCtrl * 8, acs_beam_destroy(b));
-    ACS_ALLOC(E.seg_search, (size_t)n_search * 4, acs_beam_destroy(b));
-    ACS_ALLOC(E.seg_head, (size_t)n_search * 8, acs_beam_destroy(b));
-    ACS_ALLOC(E.seg_off, (size_t)(n_search + 1) * 8, acs_beam_destroy(b));
-    ACS_ALLOC(E.seg_limit, (size_t)n_search * 8, acs_beam_destroy(b));
-    ACS_ALLOC(E.seg_base, (size_t)n_search * 8, acs_beam_destroy(b));
-    ACS_ALLOC(E.seg_of, (size_t)n_search * 4, acs_beam_destroy(b));
-    ACS_ALLOC(B.ltab, (size_t)P.ltab_slots * 8, acs_beam_destroy(b));
-    ACS_ALLOC(B.lmask, 8, acs_beam_destroy(b));
-    ACS_ALLOC(B.rec_of, (size_t)P.rec_cap * 4, acs_beam_destroy(b));
-    ACS_ALLOC(B.wlen, (size_t)P.rec_cap, acs_beam_destroy(b));
-    ACS_ALLOC(B.hist, (size_t)n_search * kBmLens * 4, acs_beam_destroy(b));
-    ACS_ALLOC(b->d_roots, (size_t)n_search * 16 * P.W, acs_beam_destroy(b));
-    auto bail = [&](int code, const std::string& m) {
-        acs_beam_destroy(b);
-        return fail(code, m);
+    auto alloc = [&]() -> int {
+        if (const int r = mb_alloc(b, B.E, P.nodes, P.tcap, P.rec_cap, P.bitmap_words)) return r;
+        ACS_ALLOC(B.ltab, (size_t)P.ltab_slots * 8, (void)0);
+        ACS_ALLOC(B.lmask, 8, (void)0);
+        ACS_ALLOC(B.rec_of, (size_t)P.rec_cap * 4, (void)0);
+        ACS_ALLOC(B.wlen, (size_t)P.rec_cap, (void)0);
+        ACS_ALLOC(B.hist, (size_t)n_search * kBmLens * 4, (void)0);
+        return mb_open(*b, "beam");
     };
-    if (cudaMallocHost((void**)&b->h_ring, kBmRing * sizeof(MbState)) != cudaSuccess)
-        return bail(ACS_ERR_NOMEM, "beam: cudaMallocHost");
-    if (cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking) != cudaSuccess)
-        return bail(ACS_ERR_CUDA, "beam: cudaStreamCreate");
-    cudaEventCreate(&b->ev0);
-    cudaEventCreate(&b->ev1);
-    for (auto& e : b->ring_ev) cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
-    cudaDeviceProp prop{};
-    if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) b->sms = prop.multiProcessorCount;
-    b->expand_smem = (size_t)b->expand_wpb * (P.W == 1 ? mb_stage_bytes_per_warp<1>() : mb_stage_bytes_per_warp<2>());
-    int per_sm = 1, ib = 1;
-    if (P.W == 1) {
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mb_expand_kernel<1, true, false, false>, 32 * b->expand_wpb,
-                                                      b->expand_smem);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ib, bm_insert_kernel<1>, 256, 0);
-    } else {
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mb_expand_kernel<2, true, false, false>, 32 * b->expand_wpb,
-                                                      b->expand_smem);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ib, bm_insert_kernel<2>, 256, 0);
+    if (const int r = alloc()) {
+        acs_beam_destroy(b);
+        return r;
     }
-    cudaGetLastError();
-    b->expand_blocks = b->sms * std::max(per_sm, 1);
-    b->insert_blocks = b->sms * std::max(ib, 1);
+    if (P.W == 1) bm_size_launches<1>(b);
+    else bm_size_launches<2>(b);
     *out = b;
     return ACS_OK;
 }
@@ -568,98 +456,27 @@ int acs_beam_create(int device, int n_search, int mrl, int64_t beam_width, const
 
 namespace {
 
-// Paths of the solved searches of the last run (see mb_paths in mbfs.cu)
-template <int W>
-int bm_paths(acs_beam* b, int32_t* h_paths, int path_cap, std::vector<int32_t>& plen) {
-    const int n = b->n_search;
-    cudaStream_t s = b->stream;
-    ACS_CUDA(cudaSetDevice(b->device));
-    const int cap = std::max(path_cap, 1);
-    if (!b->d_paths || cap > b->d_path_cap) {
-        if (b->d_paths) cudaFree(b->d_paths);
-        b->d_paths = nullptr;
-        b->d_path_cap = 0;
-        ACS_CUDA(cudaMalloc((void**)&b->d_paths, (size_t)n * cap * 2 * sizeof(int32_t)));
-        b->d_path_cap = cap;
-    }
-    if (!b->d_plen) ACS_CUDA(cudaMalloc((void**)&b->d_plen, (size_t)n * sizeof(int32_t)));
-    mb_path_kernel<W, false><<<(n + 127) / 128, 128, 0, s>>>(b->B.E, b->d_paths, cap, b->d_plen);
-    ACS_CUDA(cudaGetLastError());
-    plen.resize((size_t)n);
-    ACS_CUDA(cudaMemcpyAsync(plen.data(), b->d_plen, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    ACS_CUDA(cudaStreamSynchronize(s));
-    for (int i = 0; i < n; ++i)
-        if (plen[i] > path_cap) return fail(ACS_ERR_INVALID, "beam: a solution path is longer than path_cap (see path_len)");
-    if (h_paths && path_cap > 0) {
-        ACS_CUDA(cudaMemcpyAsync(h_paths, b->d_paths, (size_t)n * path_cap * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-        ACS_CUDA(cudaStreamSynchronize(s));
-    }
-    return ACS_OK;
-}
-
 template <int W>
 int bm_run_impl(acs_beam* b, const int8_t* h_pres, int32_t* h_paths, int path_cap, acs_search_result* results) {
-    const int n = b->n_search, mrl = b->mrl;
+    const int n = b->n_search;
     BmEngine& B = b->B;
     MbEngine& E = B.E;
-    std::vector<MbSearch> init((size_t)n);
-    std::vector<uint64_t> roots((size_t)n * 2 * W, 0);
-    int64_t slab = 0;
-    // every row is checked before any device work
-    for (int s = 0; s < n; ++s) {
-        Key<W> root;
-        int lens[2];
-        if (pack_root<W>(h_pres + (size_t)s * 2 * mrl, mrl, root, lens) == RootCheck::bad_letter)
-            return fail(ACS_ERR_UNSUPPORTED, "beam: letters outside {+-1,+-2} are not supported by the packed search");
-    }
-    for (int s = 0; s < n; ++s) {
-        MbSearch& M = init[s];
-        std::memset(&M, 0, sizeof(M));
-        M.budget = b->budgets[s];
-        M.cap = b->budgets[s];
-        M.slab = slab;
-        slab += M.cap;
-        M.n_nodes = 1;
-        M.level_end = 1;
-        M.sol_gid = -1;
-        Key<W> root;
-        int lens[2];
-        if (pack_root<W>(h_pres + (size_t)s * 2 * mrl, mrl, root, lens) != RootCheck::ok) {
-            M.status = ACS_ROW_ASSERT;  // is_array_valid_presentation fails: nothing is searched
-            M.done = 1;
-            M.n_nodes = 0;
-            continue;
-        }
-        M.min_len = lens[0] + lens[1];
-        for (int i = 0; i < 2 * W; ++i) roots[(size_t)s * 2 * W + i] = root.k[i];
-    }
+    MbRoots R;  // slabs of exactly the budget: a level commits at most budget - |V| nodes
+    if (const int rc = mb_pack_roots<W>(*b, h_pres, 0, false, "beam", R)) return rc;
     MbState st{};
     st.chunk_cap = b->plan.chunk;
     st.tmask = b->plan.tcap - 1;
-    st.mrl = mrl;
+    st.mrl = b->mrl;
     st.cyclical = b->cyclical;
     st.n_search = n;
+    if (const int rc = mb_run_begin<W>(*b, E, st, R, nullptr)) return rc;
     cudaStream_t s = b->stream;
-    ACS_CUDA(cudaSetDevice(b->device));
-    ACS_CUDA(cudaMemsetAsync(E.table, 0, b->plan.tcap * sizeof(uint64_t), s));
-    if (E.goal_hit) ACS_CUDA(cudaMemsetAsync(E.goal_hit, 0xFF, (size_t)n * sizeof(int64_t), s));
-    if (E.goal_hit_g) ACS_CUDA(cudaMemsetAsync(E.goal_hit_g, 0xFF, (size_t)n * sizeof(int32_t), s));
-    b->h_ring[0] = st;  // pinned staging for the async upload
-    ACS_CUDA(cudaMemcpyAsync(E.st, &b->h_ring[0], sizeof(MbState), cudaMemcpyHostToDevice, s));
-    ACS_CUDA(cudaMemcpyAsync(E.srch, init.data(), init.size() * sizeof(MbSearch), cudaMemcpyHostToDevice, s));
-    ACS_CUDA(cudaMemcpyAsync(b->d_roots, roots.data(), roots.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    E.root_g = nullptr;
-    ACS_CUDA(cudaStreamSynchronize(s));  // the staging copies above read host memory that goes out of scope
-    ACS_CUDA(cudaEventRecord(b->ev0, s));
-    mb_init_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(E, b->d_roots);
-    if (b->goals) mb_goal_roots_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(E);
-    ACS_CUDA(cudaGetLastError());
     const int decide_blocks = (n + 127) / 128;
     const int select_blocks = std::min(n, b->sms * 8);
     for (int64_t chunk = 0;; ++chunk) {
-        if (chunk >= kBmLag) {
-            ACS_CUDA(cudaEventSynchronize(b->ring_ev[(chunk - kBmLag) % kBmRing]));
-            if (b->h_ring[(chunk - kBmLag) % kBmRing].done) break;
+        if (const int done = mb_ring_done(*b, chunk)) {
+            if (done < 0) return done;
+            break;
         }
         bm_plan_kernel<<<1, 32, 0, s>>>(B, chunk == 0);
         bm_prep_kernel<<<b->sms * 2, 256, 0, s>>>(B);
@@ -673,39 +490,11 @@ int bm_run_impl(acs_beam* b, const int8_t* h_pres, int32_t* h_paths, int path_ca
         bm_decide_kernel<<<decide_blocks, 128, 0, s>>>(B);
         bm_select_kernel<W><<<select_blocks, kBmSelT, 0, s>>>(B);
         ACS_CUDA(cudaGetLastError());
-        ACS_CUDA(cudaMemcpyAsync(&b->h_ring[chunk % kBmRing], E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
-        ACS_CUDA(cudaEventRecord(b->ring_ev[chunk % kBmRing], s));
+        if (const int rc = mb_ring_publish(*b, E, chunk)) return rc;
     }
-    ACS_CUDA(cudaEventRecord(b->ev1, s));
-    MbState fin{};
-    b->h_final.resize((size_t)n);
-    ACS_CUDA(cudaMemcpyAsync(&fin, E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
-    ACS_CUDA(cudaMemcpyAsync(b->h_final.data(), E.srch, (size_t)n * sizeof(MbSearch), cudaMemcpyDeviceToHost, s));
-    ACS_CUDA(cudaStreamSynchronize(s));
-    if (fin.ierr) return fail(ACS_ERR_CUDA, "beam: internal error: a hash table is full");
-    b->ran = true;
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, b->ev0, b->ev1);
-    std::vector<int32_t> plen((size_t)n);
-    const int rc = bm_paths<W>(b, h_paths, path_cap, plen);
-    for (int i = 0; i < n; ++i) {
-        const MbSearch& f = b->h_final[i];
-        acs_search_result* r = results + i;
-        std::memset(r, 0, sizeof(*r));
-        r->solved = f.solved;
-        r->status = f.status;
-        r->budget_hit = f.budget_hit;
-        r->path_len = plen[i];
-        r->seconds_device = ms * 1e-3;
-        if (f.status == ACS_ROW_ASSERT && f.n_nodes == 0) continue;  // invalid root: nothing searched
-        r->n_visited = f.n_nodes;
-        r->n_expanded = f.n_expanded;
-        r->n_moves = f.solved ? f.sol_gid + 1 : (f.status ? (int64_t)(((uint64_t)f.err_code >> 2) + 1) : f.n_expanded * 12);
-        r->frontier_left = f.n_nodes - f.n_expanded;
-        r->n_levels = f.levels;
-        r->n_minlen = f.n_minlen;
-        for (int j = 0; j < f.n_minlen && j < 128; ++j) r->minlen_log[j] = f.minlen_log[j];
-    }
+    int ierr = 0;
+    const int rc = mb_run_end<W>(*b, E, false, "beam", h_paths, path_cap, results, ierr);
+    if (ierr) return fail(ACS_ERR_CUDA, "beam: internal error: a hash table is full");
     return rc;
 }
 
@@ -722,74 +511,29 @@ int acs_beam_run(acs_beam* b, const int8_t* h_presentations, int32_t* h_paths, i
 
 int acs_beam_paths(acs_beam* b, int32_t* h_paths, int path_cap) {
     if (!b || path_cap < 0 || (!h_paths && path_cap > 0)) return ACS_ERR_INVALID;
-    if (!b->ran) return fail(ACS_ERR_INVALID, "beam: no completed run");
-    std::vector<int32_t> plen;
-    return b->W == 1 ? bm_paths<1>(b, h_paths, path_cap, plen) : bm_paths<2>(b, h_paths, path_cap, plen);
+    return mb_paths_again(*b, b->B.E, false, "beam", h_paths, path_cap);
 }
 
 int acs_beam_visited(acs_beam* b, int search, int8_t* h_out, int64_t cap_rows, int64_t* n_out) {
     if (!b || search < 0 || search >= b->n_search || (!h_out && cap_rows > 0)) return ACS_ERR_INVALID;
-    if (!b->ran) return fail(ACS_ERR_INVALID, "beam: no completed run");
-    ACS_CUDA(cudaSetDevice(b->device));
-    const MbSearch& f = b->h_final[search];
-    const int64_t n = std::min<int64_t>(f.n_nodes, std::max<int64_t>(cap_rows, 0));
-    if (n_out) *n_out = n;
-    const uint64_t* slab = b->B.E.nodes + (size_t)f.slab * node_words(b->W);
-    return records_to_host(b->W, slab, node_words(b->W), n, b->mrl, h_out, nullptr, b->stream);
+    return mb_visited(*b, b->B.E, "beam", search, h_out, cap_rows, n_out);
 }
 
 int acs_beam_set_goals(acs_beam* b, const acs_goalset* g) {
     if (!b) return ACS_ERR_INVALID;
-    if (g) {
-        if (g->mrl != b->mrl)
-            return fail(ACS_ERR_INVALID, "beam_set_goals: the goal set's max_relator_length differs from the engine's");
-        if (g->cyclical != b->cyclical)
-            return fail(ACS_ERR_INVALID, "beam_set_goals: the goal set's cyclical flag differs from the engine's");
-        if (g->device != b->device) return fail(ACS_ERR_INVALID, "beam_set_goals: the goal set lives on another device");
-        if (g->n_entries >= (int64_t)0xFFFFFFFF)  // a hit packs the entry into 32 bits beside its candidate id
-            return fail(ACS_ERR_UNSUPPORTED, "beam_set_goals: goal sets of 2^32 - 1 entries or more are not supported");
-        MbEngine& E = b->B.E;
-        if (!E.goal_hit) {
-            ACS_CUDA(cudaSetDevice(b->device));
-            ACS_CUDA(cudaMalloc((void**)&E.goal_hit, (size_t)b->n_search * sizeof(int64_t)));
-            ACS_CUDA(cudaMemset(E.goal_hit, 0xFF, (size_t)b->n_search * sizeof(int64_t)));
-            ACS_CUDA(cudaMalloc((void**)&E.goal_hit_g, (size_t)b->n_search * sizeof(int32_t)));
-            ACS_CUDA(cudaMemset(E.goal_hit_g, 0xFF, (size_t)b->n_search * sizeof(int32_t)));
-        }
-        E.goals = g->view();
-    } else {
-        b->B.E.goals = GoalView{nullptr, nullptr, 0, 0};
-    }
-    b->goals = g;
-    return ACS_OK;
+    if (g)
+        if (const int rc = goalset_check(g, b->mrl, b->cyclical, b->device, false, "beam")) return rc;
+    return mb_set_goals(*b, b->B.E, g);
 }
 
 int acs_beam_goal_hits(acs_beam* b, int64_t* h_entry) {
     if (!b || !h_entry) return ACS_ERR_INVALID;
-    if (!b->ran) return fail(ACS_ERR_INVALID, "beam: no completed run");
-    if (!b->B.E.goal_hit) {
-        std::fill(h_entry, h_entry + b->n_search, (int64_t)-1);
-        return ACS_OK;
-    }
-    ACS_CUDA(cudaSetDevice(b->device));
-    ACS_CUDA(cudaMemcpyAsync(h_entry, b->B.E.goal_hit, (size_t)b->n_search * sizeof(int64_t), cudaMemcpyDeviceToHost,
-                             b->stream));
-    ACS_CUDA(cudaStreamSynchronize(b->stream));
-    return ACS_OK;
+    return mb_goal_hits<int64_t>(*b, b->B.E.goal_hit, h_entry, "beam");
 }
 
 int acs_beam_goal_hit_elements(acs_beam* b, int32_t* h_elem) {
     if (!b || !h_elem) return ACS_ERR_INVALID;
-    if (!b->ran) return fail(ACS_ERR_INVALID, "beam: no completed run");
-    if (!b->B.E.goal_hit_g) {
-        std::fill(h_elem, h_elem + b->n_search, -1);
-        return ACS_OK;
-    }
-    ACS_CUDA(cudaSetDevice(b->device));
-    ACS_CUDA(cudaMemcpyAsync(h_elem, b->B.E.goal_hit_g, (size_t)b->n_search * sizeof(int32_t), cudaMemcpyDeviceToHost,
-                             b->stream));
-    ACS_CUDA(cudaStreamSynchronize(b->stream));
-    return ACS_OK;
+    return mb_goal_hits<int32_t>(*b, b->B.E.goal_hit_g, h_elem, "beam");
 }
 
 }  // extern "C"

@@ -103,6 +103,18 @@ __global__ void gs_path_kernel(const uint64_t* nodes, int64_t entry, int32_t* pa
     }
 }
 
+int goalset_check(const acs_goalset* g, int mrl, int cyclical, int device, bool orbit, const char* who) {
+    const std::string w = std::string(who) + "_set_goals: ";
+    if (g->mrl != mrl) return fail(ACS_ERR_INVALID, w + "the goal set's max_relator_length differs from the engine's");
+    if (g->cyclical != cyclical) return fail(ACS_ERR_INVALID, w + "the goal set's cyclical flag differs from the engine's");
+    if (g->device != device) return fail(ACS_ERR_INVALID, w + "the goal set lives on another device");
+    if (orbit && !g->symmetric)  // an orbit search knows only the orbit of a child
+        return fail(ACS_ERR_INVALID, w + "an orbit search needs a symmetric goal set");
+    if (g->n_entries >= (int64_t)0xFFFFFFFF)  // a hit packs the entry into 32 bits beside its candidate id
+        return fail(ACS_ERR_UNSUPPORTED, w + "goal sets of 2^32 - 1 entries or more are not supported");
+    return ACS_OK;
+}
+
 int goalset_index(acs_goalset* g, cudaStream_t s) {
     uint64_t t = 1024;
     while (t < 2 * (uint64_t)g->n_entries) t <<= 1;

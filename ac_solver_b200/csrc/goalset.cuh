@@ -72,6 +72,9 @@ namespace acs {
 // Allocates and fills the index of g's nodes (g->nodes holds n_entries entries) and counts its distinct
 // states.  Returns ACS_OK or an error code with the message set.
 int goalset_index(acs_goalset* g, cudaStream_t s);
+// ACS_OK when an engine of max_relator_length mrl, `cyclical` flag and device `device` can search with goal set g
+// (an orbit search needs a symmetric set); otherwise an error code with the text "<who>_set_goals: ..."
+int goalset_check(const acs_goalset* g, int mrl, int cyclical, int device, bool orbit, const char* who);
 // Frees what g owns and g itself.
 void goalset_free(acs_goalset* g);
 }  // namespace acs

@@ -685,15 +685,8 @@ extern "C" int acs_greedy_visited(acs_greedy* g, int search, int8_t* h_out, int6
 
 extern "C" int acs_greedy_set_goals(acs_greedy* g, const acs_goalset* gs) {
     if (!g) return ACS_ERR_INVALID;
-    if (gs) {
-        if (gs->mrl != g->mrl)
-            return fail(ACS_ERR_INVALID, "greedy_set_goals: the goal set's max_relator_length differs from the engine's");
-        if (gs->cyclical != g->cyclical)
-            return fail(ACS_ERR_INVALID, "greedy_set_goals: the goal set's cyclical flag differs from the engine's");
-        if (gs->device != g->device) return fail(ACS_ERR_INVALID, "greedy_set_goals: the goal set lives on another device");
-        if (gs->n_entries >= (int64_t)0xFFFFFFFF)  // the bucket kernel packs a hit's entry into 32 bits beside its candidate
-            return fail(ACS_ERR_UNSUPPORTED, "greedy_set_goals: goal sets of 2^32 - 1 entries or more are not supported");
-    }
+    if (gs)
+        if (const int rc = goalset_check(gs, g->mrl, g->cyclical, g->device, false, "greedy")) return rc;
     g->goals = gs;
     return ACS_OK;
 }

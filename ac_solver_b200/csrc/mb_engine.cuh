@@ -89,6 +89,82 @@ __device__ __forceinline__ uint64_t mb_rank(const uint2* rt, uint64_t c) {
     return e.x + __popc(e.y & ((1u << (c & 31)) - 1u));
 }
 
+// ---- the segment event rule (decide kernels) ---------------------------------------------------------
+struct MbEvent {
+    bool solved, goal;  // a solving or goal child ends the search (goal: the goal test fired)
+    int status;         // or a raising child: the reference's status
+    uint64_t offset;    // the event's candidate offset from the segment's first candidate id
+};
+
+// The event that ends a segment's search among its candidates c0 + [0, limit), which lowers limit to the event:
+// the first solving child `sol` (~0: none), a goal child before it (on the solving child itself the solve wins),
+// then a raising child before either.
+__device__ __forceinline__ MbEvent mb_event(const unsigned long long* red, unsigned long long sol, uint64_t c0,
+                                            uint64_t& limit) {
+    MbEvent ev{false, false, 0, 0};
+    const unsigned long long err = red[kMbErr], goal = red[kMbGoal];
+    if (sol != ~0ull && sol - c0 < limit) {
+        ev.offset = limit = sol - c0;
+        ev.solved = true;
+    }
+    if (goal != ~0ull && (goal >> 32) - c0 < limit) {
+        ev.offset = limit = (goal >> 32) - c0;
+        ev.solved = ev.goal = true;
+    }
+    if (err != ~0ull && (err >> 2) - c0 < limit) {  // the reference raises here, before anything later
+        ev.offset = limit = (err >> 2) - c0;
+        ev.status = (int)(err & 3);
+        ev.solved = ev.goal = false;
+    }
+    return ev;
+}
+
+// The counters of a search that event ev of its segment (first candidate id 12 * head) ended, and the goal
+// entry it stopped at
+__device__ __forceinline__ void mb_end_at(const MbEngine& E, MbSearch& M, int s, const unsigned long long* red,
+                                          const MbEvent& ev, uint64_t head) {
+    const uint64_t c = 12 * head + ev.offset;
+    M.n_expanded = (int64_t)(c / 12 + 1);
+    if (ev.status) {
+        M.status = ev.status;
+        M.err_code = (int64_t)((c << 2) | (uint64_t)ev.status);
+        return;
+    }
+    M.solved = 1;
+    M.sol_gid = (int64_t)c;
+    M.sol_len = 2;
+    if (ev.goal) {
+        const uint64_t e = red[kMbGoal] & 0xFFFFFFFFull;
+        const int W = key_words(E.st->mrl);
+        const uint64_t* q = E.goals.nodes + e * node_words(W);  // the goal state's key
+        M.sol_len = key_len(q, W, 0) + key_len(q, W, 1);
+        E.goal_hit[s] = (int64_t)e;
+    }
+}
+
+// "New minimal length found" events in the reference's order, up to the segment's event: the first child of each
+// new minimal total length among candidates c0 + [0, limit), and the solving child itself
+__device__ __forceinline__ void mb_minlen_log(MbSearch& M, const unsigned long long* red, uint64_t c0, uint64_t limit,
+                                              bool solved) {
+    const uint64_t c_limit = limit + (solved ? 1 : 0);
+    int min_len = M.min_len;
+    for (;;) {
+        unsigned long long best = ~0ull;
+        int bestL = -1;
+        for (int L = 0; L < min_len && L < 128; ++L) {
+            const unsigned long long g = red[kMbLen0 + L];
+            if (g != ~0ull && g - c0 < c_limit && g < best) {
+                best = g;
+                bestL = L;
+            }
+        }
+        if (bestL < 0) break;
+        min_len = bestL;
+        if (M.n_minlen < 128) M.minlen_log[M.n_minlen++] = bestL;
+    }
+    M.min_len = min_len;
+}
+
 // ---- init: roots into their slabs and the table ----------------------------------------------
 template <int W>
 __global__ void mb_init_kernel(const MbEngine E, const uint64_t* roots) {

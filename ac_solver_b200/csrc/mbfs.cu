@@ -52,6 +52,7 @@
 #include "bfs_common.cuh"
 #include "goalset.cuh"
 #include "mb_engine.cuh"
+#include "mb_host.cuh"
 
 namespace acs {
 
@@ -305,70 +306,15 @@ __global__ void __launch_bounds__(128) mb_decide_kernel(const MbEngine E) {
         cut_p = lo;
         if (12 * (cut_p + 1) < limit) limit = 12 * (cut_p + 1);
     }
-    const unsigned long long sol = st->explore ? ~0ull : red[kMbSol], err = red[kMbErr], goal = red[kMbGoal];
-    bool sol_here = false, goal_here = false;
-    int status = 0;
-    uint64_t sol_l = 0, err_l = 0;
-    if (sol != ~0ull && sol - c0 < limit) {  // solved at or before the cut parent
-        sol_l = sol - c0;
-        limit = sol_l;
-        sol_here = true;
-        cut = false;
-    }
-    if (goal != ~0ull && (goal >> 32) - c0 < limit) {  // a goal child; on the solving child itself the solve wins
-        sol_l = (goal >> 32) - c0;
-        limit = sol_l;
-        sol_here = true;
-        goal_here = true;
-        cut = false;
-    }
-    if (err != ~0ull && (err >> 2) - c0 < limit) {  // the reference raises here, before anything later
-        err_l = (err >> 2) - c0;
-        limit = err_l;
-        status = (int)(err & 3);
-        sol_here = false;
-        goal_here = false;
-        cut = false;
-    }
-    // "New minimal length found" events in reference order
-    const uint64_t c_limit = limit + (sol_here ? 1 : 0);
-    int min_len = M.min_len;
-    for (;;) {
-        unsigned long long best = ~0ull;
-        int bestL = -1;
-        for (int L = 0; L < min_len && L < 128; ++L) {
-            const unsigned long long g = red[kMbLen0 + L];
-            if (g != ~0ull && g - c0 < c_limit && g < best) {
-                best = g;
-                bestL = L;
-            }
-        }
-        if (bestL < 0) break;
-        min_len = bestL;
-        if (M.n_minlen < 128) M.minlen_log[M.n_minlen++] = bestL;
-    }
-    M.min_len = min_len;
+    const MbEvent ev = mb_event(red, st->explore ? ~0ull : red[kMbSol], c0, limit);
+    mb_minlen_log(M, red, c0, limit, ev.solved);
     const uint64_t cg = mb_rank(E.rt, c0 + limit) - r0;
     E.seg_limit[k] = (int64_t)(c0 + limit);
     E.seg_base[k] = M.slab + (int64_t)n_nodes - (int64_t)r0;
     if ((int64_t)(n_nodes + cg) > M.cap) atomicOr(&st->ierr, MB_IERR_SLAB_FULL);  // the commit drops the excess
     M.n_nodes = (int64_t)(n_nodes + cg);
-    if (sol_here) {
-        M.solved = 1;
-        M.sol_gid = (int64_t)(12 * head + sol_l);
-        M.n_expanded = M.sol_gid / 12 + 1;
-        M.sol_len = 2;
-        if (goal_here) {
-            const uint64_t e = goal & 0xFFFFFFFFull;
-            const int W = key_words(st->mrl);
-            const uint64_t* q = E.goals.nodes + e * node_words(W);  // the goal state's key
-            M.sol_len = key_len(q, W, 0) + key_len(q, W, 1);
-            E.goal_hit[s] = (int64_t)e;
-        }
-    } else if (status) {
-        M.status = status;
-        M.err_code = (int64_t)(((12 * head + err_l) << 2) | (uint64_t)status);
-        M.n_expanded = (int64_t)((12 * head + err_l) / 12 + 1);
+    if (ev.solved || ev.status) {
+        mb_end_at(E, M, s, red, ev, head);
     } else if (cut) {
         M.budget_hit = 1;
         M.n_expanded = (int64_t)(head + cut_p + 1);
@@ -438,8 +384,6 @@ __global__ void mb_adopt_kernel(const uint64_t* nodes, const int64_t* off, const
 using namespace acs;
 
 namespace {
-constexpr int kMbRing = 4, kMbLag = 2;
-
 // sizes of an engine (shared by acs_bfs_batch_bytes and acs_bfs_batch_create)
 struct MbPlan {
     int W;
@@ -482,29 +426,26 @@ int mb_plan(int n_search, int mrl, const int64_t* max_nodes, int64_t chunk_paren
 }
 }  // namespace
 
-struct acs_bfs_batch {
-    int device = 0, n_search = 0, mrl = 0, W = 1, cyclical = 0;
+struct acs_bfs_batch : MbHost {
     MbPlan plan{};
     MbEngine E{};
-    uint64_t* d_roots = nullptr;
-    int32_t* d_paths = nullptr;
-    int32_t* d_plen = nullptr;
-    int d_path_cap = 0;
-    std::vector<int64_t> budgets;
-    std::vector<MbSearch> h_final;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr, ring_ev[kMbRing] = {};
-    MbState* h_ring = nullptr;  // pinned [kMbRing]
-    int sms = 148;
-    int expand_blocks = 148, expand_blocks_sym = 148, expand_wpb = 8, insert_blocks = 148, commit_blocks = 148;
-    size_t expand_smem = 0;
-    bool ran = false;
-    const acs_goalset* goals = nullptr;  // acs_bfs_batch_set_goals
+    int expand_blocks_sym = 148, commit_blocks = 148;
     int explore = 0;                     // stop_at_trivial == 0
     bool adopted = false;                // the nodes went to a goal set (acs_goalset_from_bfs_batch)
     int symmetric = 0;                   // orbit search (acs_bfs_batch_set_symmetric)
     uint8_t* d_root_g = nullptr;         // [n_search] each root's element, with E.log_g allocated by set_symmetric
 };
+
+// launch sizes from the kernels' occupancy
+template <int W>
+static void mb_size_launches(acs_bfs_batch* b) {
+    b->expand_smem = (size_t)b->expand_wpb * mb_stage_bytes_per_warp<W>();
+    b->expand_blocks = mb_blocks(*b, mb_expand_kernel<W, true, false>, 32 * b->expand_wpb, b->expand_smem);
+    b->expand_blocks_sym = mb_blocks(*b, mb_expand_kernel<W, true, true>, 32 * b->expand_wpb, b->expand_smem);
+    b->insert_blocks = mb_blocks(*b, mb_insert_kernel<W>, 256, 0);
+    b->commit_blocks = mb_blocks(*b, mb_commit_kernel<W, false>, 256, 0);
+    cudaGetLastError();
+}
 
 extern "C" {
 
@@ -519,23 +460,8 @@ int acs_bfs_batch_bytes(int n_search, int mrl, const int64_t* max_nodes, int64_t
 
 void acs_bfs_batch_destroy(acs_bfs_batch* b) {
     if (!b) return;
-    cudaSetDevice(b->device);
-    if (b->stream) {
-        cudaStreamSynchronize(b->stream);
-        cudaStreamDestroy(b->stream);
-    }
-    if (b->ev0) cudaEventDestroy(b->ev0);
-    if (b->ev1) cudaEventDestroy(b->ev1);
-    for (auto e : b->ring_ev)
-        if (e) cudaEventDestroy(e);
-    MbEngine& E = b->E;
-    void* ptrs[] = {E.st, E.srch, E.nodes, E.table, E.log_keys, E.log_c, E.log_s, E.rec_slot, E.cursor, E.bitmap, E.rt,
-                    E.bsums, E.ctrl, E.seg_search, E.seg_head, E.seg_off, E.seg_limit, E.seg_base, E.seg_of,
-                    E.goal_hit, E.goal_hit_g, E.log_g, b->d_root_g, b->d_roots, b->d_paths, b->d_plen};
-    for (void* p : ptrs)
-        if (p) cudaFree(p);
-    if (b->h_ring) cudaFreeHost(b->h_ring);
-    cudaGetLastError();
+    mb_close(*b, b->E);
+    if (b->d_root_g) cudaFree(b->d_root_g);
     delete b;
 }
 
@@ -548,66 +474,22 @@ int acs_bfs_batch_create(int device, int n_search, int mrl, const int64_t* max_n
     if (rc != ACS_OK) return rc;
     if (const int rc2 = open_device(device, "bfs_batch")) return rc2;
     acs_bfs_batch* b = new acs_bfs_batch();
-    b->device = device;
-    b->n_search = n_search;
-    b->mrl = mrl;
-    b->W = P.W;
-    b->cyclical = cyclical ? 1 : 0;
+    mb_init(*b, device, n_search, mrl, P.W, cyclical, max_nodes);
     b->plan = P;
-    b->budgets.assign(max_nodes, max_nodes + n_search);
-    auto bail = [&](int code, const std::string& m) {
-        acs_bfs_batch_destroy(b);
-        return fail(code, m);
-    };
     MbEngine& E = b->E;
-    E.rec_cap = P.rec_cap;
-    ACS_ALLOC(E.st, sizeof(MbState), acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.srch, (size_t)n_search * sizeof(MbSearch), acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.nodes, (size_t)P.nodes * 8 * node_words(P.W), acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.table, (size_t)P.tcap * 8, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.log_keys, (size_t)P.rec_cap * 16 * P.W, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.log_c, (size_t)P.rec_cap * 4, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.log_s, (size_t)P.rec_cap * 4, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.rec_slot, (size_t)P.rec_cap * 8, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.cursor, 8, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.bitmap, (size_t)P.bitmap_words * 4, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.rt, (size_t)(P.bitmap_words + 1) * sizeof(uint2), acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.bsums, (size_t)P.nblk * 4, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.ctrl, (size_t)n_search * kMbCtrl * 8, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.seg_search, (size_t)n_search * 4, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.seg_head, (size_t)n_search * 8, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.seg_off, (size_t)(n_search + 1) * 8, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.seg_limit, (size_t)n_search * 8, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.seg_base, (size_t)n_search * 8, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(E.seg_of, (size_t)n_search * 4, acs_bfs_batch_destroy(b));
-    ACS_ALLOC(b->d_roots, (size_t)n_search * 16 * P.W, acs_bfs_batch_destroy(b));
-    if (cudaMallocHost((void**)&b->h_ring, kMbRing * sizeof(MbState)) != cudaSuccess)
-        return bail(ACS_ERR_NOMEM, "bfs_batch: cudaMallocHost");
-    if (cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking) != cudaSuccess)
-        return bail(ACS_ERR_CUDA, "bfs_batch: cudaStreamCreate");
-    cudaEventCreate(&b->ev0);
-    cudaEventCreate(&b->ev1);
-    for (auto& e : b->ring_ev) cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
-    cudaDeviceProp prop{};
-    if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) b->sms = prop.multiProcessorCount;
-    b->expand_smem = (size_t)b->expand_wpb * (P.W == 1 ? mb_stage_bytes_per_warp<1>() : mb_stage_bytes_per_warp<2>());
-    int per_sm = 1, per_sm_sym = 1, ib = 1, cb = 1;
-    if (P.W == 1) {
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mb_expand_kernel<1, true, false>, 32 * b->expand_wpb, b->expand_smem);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_sym, mb_expand_kernel<1, true, true>, 32 * b->expand_wpb, b->expand_smem);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ib, mb_insert_kernel<1>, 256, 0);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cb, mb_commit_kernel<1, false>, 256, 0);
-    } else {
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mb_expand_kernel<2, true, false>, 32 * b->expand_wpb, b->expand_smem);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_sym, mb_expand_kernel<2, true, true>, 32 * b->expand_wpb, b->expand_smem);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ib, mb_insert_kernel<2>, 256, 0);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cb, mb_commit_kernel<2, false>, 256, 0);
+    auto alloc = [&]() -> int {
+        if (const int r = mb_alloc(b, E, P.nodes, P.tcap, P.rec_cap, P.bitmap_words)) return r;
+        ACS_ALLOC(E.rec_slot, (size_t)P.rec_cap * 8, (void)0);
+        ACS_ALLOC(E.rt, (size_t)(P.bitmap_words + 1) * sizeof(uint2), (void)0);
+        ACS_ALLOC(E.bsums, (size_t)P.nblk * 4, (void)0);
+        return mb_open(*b, "bfs_batch");
+    };
+    if (const int r = alloc()) {
+        acs_bfs_batch_destroy(b);
+        return r;
     }
-    cudaGetLastError();
-    b->expand_blocks = b->sms * std::max(per_sm, 1);
-    b->expand_blocks_sym = b->sms * std::max(per_sm_sym, 1);
-    b->insert_blocks = b->sms * std::max(ib, 1);
-    b->commit_blocks = b->sms * std::max(cb, 1);
+    if (P.W == 1) mb_size_launches<1>(b);
+    else mb_size_launches<2>(b);
     *out = b;
     return ACS_OK;
 }
@@ -616,105 +498,30 @@ int acs_bfs_batch_create(int device, int n_search, int mrl, const int64_t* max_n
 
 namespace {
 
-// Paths of the solved searches of the last run into h_paths [n_search, path_cap, 2]; plen gets every search's
-// path length (0 if not solved).  A path longer than path_cap is an error, never truncated.
-template <int W>
-int mb_paths(acs_bfs_batch* b, int32_t* h_paths, int path_cap, std::vector<int32_t>& plen) {
-    const int n = b->n_search;
-    cudaStream_t s = b->stream;
-    ACS_CUDA(cudaSetDevice(b->device));
-    const int cap = std::max(path_cap, 1);  // the kernel writes the first pair of every solved path
-    if (!b->d_paths || cap > b->d_path_cap) {
-        if (b->d_paths) cudaFree(b->d_paths);
-        b->d_paths = nullptr;
-        b->d_path_cap = 0;
-        ACS_CUDA(cudaMalloc((void**)&b->d_paths, (size_t)n * cap * 2 * sizeof(int32_t)));
-        b->d_path_cap = cap;
-    }
-    if (!b->d_plen) ACS_CUDA(cudaMalloc((void**)&b->d_plen, (size_t)n * sizeof(int32_t)));
-    if (b->symmetric) mb_path_kernel<W, true><<<(n + 127) / 128, 128, 0, s>>>(b->E, b->d_paths, cap, b->d_plen);
-    else mb_path_kernel<W, false><<<(n + 127) / 128, 128, 0, s>>>(b->E, b->d_paths, cap, b->d_plen);
-    ACS_CUDA(cudaGetLastError());
-    plen.resize((size_t)n);
-    ACS_CUDA(cudaMemcpyAsync(plen.data(), b->d_plen, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    ACS_CUDA(cudaStreamSynchronize(s));
-    for (int i = 0; i < n; ++i)
-        if (plen[i] > path_cap)
-            return fail(ACS_ERR_INVALID, "bfs_batch: a solution path is longer than path_cap (see path_len)");
-    if (h_paths && path_cap > 0)
-        ACS_CUDA(cudaMemcpy(h_paths, b->d_paths, (size_t)n * path_cap * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost));
-    return ACS_OK;
-}
-
 template <int W>
 int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int path_cap, acs_search_result* results) {
-    const int n = b->n_search, mrl = b->mrl;
+    const int n = b->n_search;
     MbEngine& E = b->E;
     if (b->adopted) return fail(ACS_ERR_INVALID, "bfs_batch: the engine's states were handed to a goal set");
-    std::vector<MbSearch> init((size_t)n);
-    std::vector<uint64_t> roots((size_t)n * 2 * W, 0);
-    std::vector<uint8_t> root_g((size_t)n, 0);
-    int64_t slab = 0, n_valid = 0;
-    for (int s = 0; s < n; ++s) {
-        MbSearch& M = init[s];
-        std::memset(&M, 0, sizeof(M));
-        M.budget = b->budgets[s];
-        M.cap = b->budgets[s] + 16;
-        M.slab = slab;
-        slab += M.cap;
-        M.n_nodes = 1;
-        M.level_end = 1;
-        M.sol_gid = -1;
-        Key<W> root;
-        int lens[2];
-        const RootCheck rc = pack_root<W>(h_pres + (size_t)s * 2 * mrl, mrl, root, lens);
-        if (rc == RootCheck::bad_letter)
-            return fail(ACS_ERR_UNSUPPORTED, "bfs_batch: letters outside {+-1,+-2} are not supported by the packed search");
-        if (rc != RootCheck::ok) {  // breadth_first.py:36-38 asserts is_array_valid_presentation
-            M.status = ACS_ROW_ASSERT;
-            M.done = 1;
-            M.n_nodes = 0;
-            continue;
-        }
-        M.min_len = lens[0] + lens[1];
-        if (b->symmetric) {
-            int g0 = 0;
-            root = canonical<W>(root, g0);
-            root_g[s] = (uint8_t)g0;
-        }
-        for (int i = 0; i < 2 * W; ++i) roots[(size_t)s * 2 * W + i] = root.k[i];
-        ++n_valid;
-    }
+    MbRoots R;  // slabs of budget + 16 nodes (see the design note)
+    if (const int rc = mb_pack_roots<W>(*b, h_pres, 16, b->symmetric, "bfs_batch", R)) return rc;
     MbState st{};
     st.chunk_cap = b->plan.chunk;
     st.tmask = b->plan.tcap - 1;
-    st.mrl = mrl;
+    st.mrl = b->mrl;
     st.cyclical = b->cyclical;
     st.n_search = n;
-    st.used = n_valid;
+    st.used = R.n_valid;
     st.explore = b->explore;
+    if (const int rc = mb_run_begin<W>(*b, E, st, R, b->symmetric ? b->d_root_g : nullptr)) return rc;
     cudaStream_t s = b->stream;
-    ACS_CUDA(cudaSetDevice(b->device));
-    ACS_CUDA(cudaMemsetAsync(E.table, 0, b->plan.tcap * sizeof(uint64_t), s));
-    if (E.goal_hit) ACS_CUDA(cudaMemsetAsync(E.goal_hit, 0xFF, (size_t)n * sizeof(int64_t), s));
-    if (E.goal_hit_g) ACS_CUDA(cudaMemsetAsync(E.goal_hit_g, 0xFF, (size_t)n * sizeof(int32_t), s));
-    b->h_ring[0] = st;  // pinned staging for the async upload
-    ACS_CUDA(cudaMemcpyAsync(E.st, &b->h_ring[0], sizeof(MbState), cudaMemcpyHostToDevice, s));
-    ACS_CUDA(cudaMemcpyAsync(E.srch, init.data(), init.size() * sizeof(MbSearch), cudaMemcpyHostToDevice, s));
-    ACS_CUDA(cudaMemcpyAsync(b->d_roots, roots.data(), roots.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    if (b->symmetric) ACS_CUDA(cudaMemcpyAsync(b->d_root_g, root_g.data(), root_g.size(), cudaMemcpyHostToDevice, s));
-    E.root_g = b->symmetric ? b->d_root_g : nullptr;
-    ACS_CUDA(cudaStreamSynchronize(s));  // the staging copies above read host memory that goes out of scope
-    ACS_CUDA(cudaEventRecord(b->ev0, s));
-    mb_init_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(E, b->d_roots);
-    if (b->goals) mb_goal_roots_kernel<W><<<(n + 127) / 128, 128, 0, s>>>(E);
     mb_plan_kernel<<<1, 32, 0, s>>>(E, 1);
     ACS_CUDA(cudaGetLastError());
     const int decide_blocks = (n + 127) / 128;
     for (int64_t chunk = 0;; ++chunk) {
-        if (chunk >= kMbLag) {
-            ACS_CUDA(cudaEventSynchronize(b->ring_ev[(chunk - kMbLag) % kMbRing]));
-            if (b->h_ring[(chunk - kMbLag) % kMbRing].done) break;
+        if (const int done = mb_ring_done(*b, chunk)) {
+            if (done < 0) return done;
+            break;
         }
         mb_prep_kernel<<<b->sms * 2, 256, 0, s>>>(E);
         const dim3 eg(b->symmetric ? b->expand_blocks_sym : b->expand_blocks), et(32 * b->expand_wpb);
@@ -735,46 +542,15 @@ int mb_run_impl(acs_bfs_batch* b, const int8_t* h_pres, int32_t* h_paths, int pa
         else mb_commit_kernel<W, false><<<b->commit_blocks, 256, 0, s>>>(E);
         mb_plan_kernel<<<1, 32, 0, s>>>(E, 0);
         ACS_CUDA(cudaGetLastError());
-        ACS_CUDA(cudaMemcpyAsync(&b->h_ring[chunk % kMbRing], E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
-        ACS_CUDA(cudaEventRecord(b->ring_ev[chunk % kMbRing], s));
+        if (const int rc = mb_ring_publish(*b, E, chunk)) return rc;
     }
-    ACS_CUDA(cudaEventRecord(b->ev1, s));
-    MbState fin{};
-    b->h_final.resize((size_t)n);
-    ACS_CUDA(cudaMemcpyAsync(&fin, E.st, sizeof(MbState), cudaMemcpyDeviceToHost, s));
-    ACS_CUDA(cudaMemcpyAsync(b->h_final.data(), E.srch, (size_t)n * sizeof(MbSearch), cudaMemcpyDeviceToHost, s));
-    ACS_CUDA(cudaStreamSynchronize(s));
-    if (fin.ierr) {
+    int ierr = 0;
+    const int rc = mb_run_end<W>(*b, E, b->symmetric, "bfs_batch", h_paths, path_cap, results, ierr);
+    if (ierr) {
         std::string m = "bfs_batch: internal error:";
-        if (fin.ierr & MB_IERR_TABLE_FULL) m += " visited table full (more than 3/4 of its slots used)";
-        if (fin.ierr & MB_IERR_SLAB_FULL) m += " node slab of a search full";
+        if (ierr & MB_IERR_TABLE_FULL) m += " visited table full (more than 3/4 of its slots used)";
+        if (ierr & MB_IERR_SLAB_FULL) m += " node slab of a search full";
         return fail(ACS_ERR_CUDA, m);
-    }
-    b->ran = true;
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, b->ev0, b->ev1);
-    std::vector<int32_t> plen((size_t)n);
-    const int rc = mb_paths<W>(b, h_paths, path_cap, plen);
-    for (int i = 0; i < n; ++i) {
-        const MbSearch& f = b->h_final[i];
-        acs_search_result* r = results + i;
-        std::memset(r, 0, sizeof(*r));
-        r->solved = f.solved;
-        r->status = f.status;
-        r->budget_hit = f.budget_hit;
-        r->path_len = plen[i];
-        if (f.status == ACS_ROW_ASSERT && f.n_nodes == 0) {  // invalid root: the reference asserts before searching
-            r->seconds_device = ms * 1e-3;
-            continue;
-        }
-        r->n_visited = f.n_nodes;
-        r->n_expanded = f.n_expanded;
-        r->n_moves = f.solved ? f.sol_gid + 1 : (f.status ? (int64_t)(((uint64_t)f.err_code >> 2) + 1) : f.n_expanded * 12);
-        r->frontier_left = f.n_nodes - f.n_expanded;
-        r->n_levels = f.levels;
-        r->n_minlen = f.n_minlen;
-        for (int j = 0; j < f.n_minlen && j < 128; ++j) r->minlen_log[j] = f.minlen_log[j];
-        r->seconds_device = ms * 1e-3;
     }
     return rc;
 }
@@ -792,20 +568,12 @@ int acs_bfs_batch_run(acs_bfs_batch* b, const int8_t* h_presentations, int32_t* 
 
 int acs_bfs_batch_paths(acs_bfs_batch* b, int32_t* h_paths, int path_cap) {
     if (!b || path_cap < 0 || (!h_paths && path_cap > 0)) return ACS_ERR_INVALID;
-    if (!b->ran) return fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
-    std::vector<int32_t> plen;
-    return b->W == 1 ? mb_paths<1>(b, h_paths, path_cap, plen) : mb_paths<2>(b, h_paths, path_cap, plen);
+    return mb_paths_again(*b, b->E, b->symmetric, "bfs_batch", h_paths, path_cap);
 }
 
 int acs_bfs_batch_visited(acs_bfs_batch* b, int search, int8_t* h_out, int64_t cap_rows, int64_t* n_out) {
     if (!b || search < 0 || search >= b->n_search || (!h_out && cap_rows > 0)) return ACS_ERR_INVALID;
-    if (!b->ran) return fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
-    ACS_CUDA(cudaSetDevice(b->device));
-    const MbSearch& f = b->h_final[search];
-    const int64_t n = std::min<int64_t>(f.n_nodes, std::max<int64_t>(cap_rows, 0));
-    if (n_out) *n_out = n;
-    const uint64_t* slab = b->E.nodes + (size_t)f.slab * node_words(b->W);
-    return records_to_host(b->W, slab, node_words(b->W), n, b->mrl, h_out, nullptr, b->stream);
+    return mb_visited(*b, b->E, "bfs_batch", search, h_out, cap_rows, n_out);
 }
 
 }  // extern "C"
@@ -815,59 +583,21 @@ extern "C" {
 
 int acs_bfs_batch_set_goals(acs_bfs_batch* b, const acs_goalset* g, int stop_at_trivial) {
     if (!b) return ACS_ERR_INVALID;
-    if (g) {
-        if (g->mrl != b->mrl)
-            return fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set's max_relator_length differs from the engine's");
-        if (g->cyclical != b->cyclical)
-            return fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set's cyclical flag differs from the engine's");
-        if (g->device != b->device)
-            return fail(ACS_ERR_INVALID, "bfs_batch_set_goals: the goal set lives on another device");
-        if (b->symmetric && !g->symmetric)  // an orbit search knows only the orbit of a child
-            return fail(ACS_ERR_INVALID, "bfs_batch_set_goals: an orbit search needs a symmetric goal set");
-        if (g->n_entries >= (int64_t)0xFFFFFFFF)  // a hit packs the entry into 32 bits beside its candidate id
-            return fail(ACS_ERR_UNSUPPORTED, "bfs_batch_set_goals: goal sets of 2^32 - 1 entries or more are not supported");
-        if (!b->E.goal_hit) {
-            ACS_CUDA(cudaSetDevice(b->device));
-            ACS_CUDA(cudaMalloc((void**)&b->E.goal_hit, (size_t)b->n_search * sizeof(int64_t)));
-            ACS_CUDA(cudaMemset(b->E.goal_hit, 0xFF, (size_t)b->n_search * sizeof(int64_t)));
-            ACS_CUDA(cudaMalloc((void**)&b->E.goal_hit_g, (size_t)b->n_search * sizeof(int32_t)));
-            ACS_CUDA(cudaMemset(b->E.goal_hit_g, 0xFF, (size_t)b->n_search * sizeof(int32_t)));
-        }
-        b->E.goals = g->view();
-    } else {
-        b->E.goals = GoalView{nullptr, nullptr, 0, 0};
-    }
-    b->goals = g;
+    if (g)
+        if (const int rc = goalset_check(g, b->mrl, b->cyclical, b->device, b->symmetric, "bfs_batch")) return rc;
+    if (const int rc = mb_set_goals(*b, b->E, g)) return rc;
     b->explore = stop_at_trivial ? 0 : 1;
     return ACS_OK;
 }
 
 int acs_bfs_batch_goal_hits(acs_bfs_batch* b, int64_t* h_entry) {
     if (!b || !h_entry) return ACS_ERR_INVALID;
-    if (!b->ran) return fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
-    if (!b->E.goal_hit) {
-        std::fill(h_entry, h_entry + b->n_search, (int64_t)-1);
-        return ACS_OK;
-    }
-    ACS_CUDA(cudaSetDevice(b->device));
-    ACS_CUDA(cudaMemcpyAsync(h_entry, b->E.goal_hit, (size_t)b->n_search * sizeof(int64_t), cudaMemcpyDeviceToHost,
-                            b->stream));
-    ACS_CUDA(cudaStreamSynchronize(b->stream));
-    return ACS_OK;
+    return mb_goal_hits<int64_t>(*b, b->E.goal_hit, h_entry, "bfs_batch");
 }
 
 int acs_bfs_batch_goal_hit_elements(acs_bfs_batch* b, int32_t* h_elem) {
     if (!b || !h_elem) return ACS_ERR_INVALID;
-    if (!b->ran) return fail(ACS_ERR_INVALID, "bfs_batch: no completed run");
-    if (!b->E.goal_hit_g) {
-        std::fill(h_elem, h_elem + b->n_search, -1);
-        return ACS_OK;
-    }
-    ACS_CUDA(cudaSetDevice(b->device));
-    ACS_CUDA(cudaMemcpyAsync(h_elem, b->E.goal_hit_g, (size_t)b->n_search * sizeof(int32_t), cudaMemcpyDeviceToHost,
-                            b->stream));
-    ACS_CUDA(cudaStreamSynchronize(b->stream));
-    return ACS_OK;
+    return mb_goal_hits<int32_t>(*b, b->E.goal_hit_g, h_elem, "bfs_batch");
 }
 
 int acs_goalset_from_bfs_batch(acs_bfs_batch* b, acs_goalset** out) {

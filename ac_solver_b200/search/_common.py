@@ -1,5 +1,5 @@
 """Plumbing shared by the device search wrappers: host-side input checks, the ``info`` dict of a
-``SearchResult`` and the read-backs of visited states and goal hits."""
+``SearchResult``, the read-backs of visited states and goal hits, and the run of a batched engine."""
 
 from __future__ import annotations
 
@@ -70,3 +70,46 @@ def fetch_goal_hits(hits_fn, elements_fn, h, S):
     _lib.check(elements_fn(h, elems.ctypes.data))
     return [{"goal": int(hits[s]) if hits[s] >= 0 else None, "goal_element": int(elems[s]) if hits[s] >= 0 else None}
             for s in range(S)]
+
+
+class BatchedEngine:
+    """Handle of one batched device engine over the validated rows ``self.P8``: ``api`` names its C functions
+    (``<api>_run``, ``_paths``, ``_visited``, ``_goal_hits``, ``_goal_hit_elements``, ``_destroy``) and ``levels`` is
+    the ``info`` key of its level count.  A subclass creates the engine in ``self.h`` and sets ``self.L``,
+    ``self.P8`` and ``self.goals``."""
+
+    api = levels = None
+
+    def run(self, want_visited, path_cap=256):
+        """One run over the rows -> a list of ``(solved, path|None, info)``."""
+        L, h, P8, api = self.L, self.h, self.P8, self.api
+        S = P8.shape[0]
+        cap = path_cap
+        paths = np.zeros((S, cap, 2), np.int32)
+        res = (_lib.SearchResult * S)()
+        rc = getattr(L, api + "_run")(h, P8.ctypes.data, paths.ctypes.data, cap, res)
+        need = max(int(res[s].path_len) for s in range(S))
+        if rc == _lib.ACS_ERR_INVALID and need > cap:  # a deeper solution than the buffer: fetch the paths again
+            cap = need
+            paths = np.zeros((S, cap, 2), np.int32)
+            rc = getattr(L, api + "_paths")(h, paths.ctypes.data, cap)
+        _lib.check(rc)
+        goal_info = None
+        if self.goals is not None:
+            goal_info = fetch_goal_hits(getattr(L, api + "_goal_hits"), getattr(L, api + "_goal_hit_elements"), h, S)
+        out = []
+        for s in range(S):
+            r = res[s]
+            info = search_info(r, self.levels)
+            if goal_info is not None:
+                info.update(goal_info[s])
+            if want_visited and r.status == 0:
+                info["visited"] = fetch_visited(getattr(L, api + "_visited"), r.n_visited, P8.shape[1], h, s)
+            plist = [(int(a), int(l)) for a, l in paths[s, : r.path_len]] if r.solved else None
+            out.append((bool(r.solved), plist, info))
+        return out
+
+    def destroy(self):
+        if self.h:
+            getattr(self.L, self.api + "_destroy")(self.h)
+            self.h = None

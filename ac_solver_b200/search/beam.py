@@ -11,7 +11,7 @@ import ctypes as C
 import numpy as np
 
 from .. import _lib
-from ._common import fetch_goal_hits, fetch_visited, search_info
+from ._common import BatchedEngine
 from .breadth_first import DEFAULT_MAX_BYTES, _batch_inputs, _check_goals, _split_by
 
 MAX_BEAM_WIDTH = 1 << 24
@@ -23,8 +23,10 @@ def _beam_bytes(L, mrl, beam_width, budgets, max_depth):
     return b.value
 
 
-class _BeamEngine:
+class _BeamEngine(BatchedEngine):
     """One acs_beam engine over rows of a validated batch."""
+
+    api, levels = "acs_beam", "levels"
 
     def __init__(self, L, dev, P8, budgets, beam_width, max_depth, cyclical, goals=None):
         self.L, self.P8 = L, np.ascontiguousarray(P8)
@@ -40,38 +42,6 @@ class _BeamEngine:
         except BaseException:
             self.destroy()
             raise
-
-    def run(self, want_visited, path_cap=256):
-        L, S = self.L, self.S
-        cap = path_cap
-        paths = np.zeros((S, cap, 2), np.int32)
-        res = (_lib.SearchResult * S)()
-        rc = L.acs_beam_run(self.h, self.P8.ctypes.data, paths.ctypes.data, cap, res)
-        need = max(int(res[s].path_len) for s in range(S))
-        if rc == _lib.ACS_ERR_INVALID and need > cap:  # a deeper solution than the buffer: fetch the paths again
-            cap = need
-            paths = np.zeros((S, cap, 2), np.int32)
-            rc = L.acs_beam_paths(self.h, paths.ctypes.data, cap)
-        _lib.check(rc)
-        goal_info = None
-        if self.goals is not None:
-            goal_info = fetch_goal_hits(L.acs_beam_goal_hits, L.acs_beam_goal_hit_elements, self.h, S)
-        out = []
-        for s in range(S):
-            r = res[s]
-            info = search_info(r, levels="levels")
-            if goal_info is not None:
-                info.update(goal_info[s])
-            if want_visited and r.status == 0:
-                info["visited"] = fetch_visited(L.acs_beam_visited, r.n_visited, self.P8.shape[1], self.h, s)
-            plist = [(int(a), int(l)) for a, l in paths[s, : r.path_len]] if r.solved else None
-            out.append((bool(r.solved), plist, info))
-        return out
-
-    def destroy(self):
-        if self.h:
-            self.L.acs_beam_destroy(self.h)
-            self.h = None
 
 
 def _check_args(beam_width, max_depth):

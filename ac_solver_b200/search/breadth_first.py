@@ -12,7 +12,7 @@ import numpy as np
 
 from .. import _lib
 from ..envs.utils import is_array_valid_presentation
-from ._common import _raise_for, check_row, check_rows, fetch_goal_hits, fetch_visited, search_info
+from ._common import BatchedEngine, _raise_for, check_row, check_rows, fetch_visited, search_info
 
 
 def bfs_device(presentation, max_nodes_to_explore=10000, cyclically_reduce_after_moves=False,
@@ -90,8 +90,10 @@ def _split(L, mrl, budgets, chunk_parents, max_bytes):
     return _split_by(lambda b: _engine_bytes(L, mrl, b, chunk_parents), budgets, max_bytes)
 
 
-class _BatchEngine:
+class _BatchEngine(BatchedEngine):
     """One acs_bfs_batch engine over rows [lo, hi) of a validated batch."""
+
+    api, levels = "acs_bfs_batch", "n_levels"
 
     def __init__(self, L, dev, P8, budgets, cyclical, chunk_parents, goals=None, stop_at_trivial=True, symmetric=False):
         self.L, self.P8 = L, np.ascontiguousarray(P8)
@@ -110,38 +112,6 @@ class _BatchEngine:
         except BaseException:
             self.destroy()
             raise
-
-    def run(self, want_visited):
-        L, S = self.L, self.S
-        cap = 256
-        paths = np.zeros((S, cap, 2), np.int32)
-        res = (_lib.SearchResult * S)()
-        rc = L.acs_bfs_batch_run(self.h, self.P8.ctypes.data, paths.ctypes.data, cap, res)
-        need = max(int(res[s].path_len) for s in range(S))
-        if rc == _lib.ACS_ERR_INVALID and need > cap:  # a deeper solution than the buffer: fetch the paths again
-            cap = need
-            paths = np.zeros((S, cap, 2), np.int32)
-            rc = L.acs_bfs_batch_paths(self.h, paths.ctypes.data, cap)
-        _lib.check(rc)
-        goal_info = None
-        if self.goals is not None:
-            goal_info = fetch_goal_hits(L.acs_bfs_batch_goal_hits, L.acs_bfs_batch_goal_hit_elements, self.h, S)
-        out = []
-        for s in range(S):
-            r = res[s]
-            info = search_info(r)
-            if goal_info is not None:
-                info.update(goal_info[s])
-            if want_visited and r.status == 0:
-                info["visited"] = fetch_visited(L.acs_bfs_batch_visited, r.n_visited, self.P8.shape[1], self.h, s)
-            plist = [(int(a), int(l)) for a, l in paths[s, : r.path_len]] if r.solved else None
-            out.append((bool(r.solved), plist, info))
-        return out
-
-    def destroy(self):
-        if self.h:
-            self.L.acs_bfs_batch_destroy(self.h)
-            self.h = None
 
 
 def _check_goals(goals, mrl, cyclical, dev):

@@ -30,11 +30,14 @@ MUST_MATCH = [
     "mb_expand_kernel", "mb_insert_kernel", "mb_commit_kernel", "mb_goal_kernel",
     "greedy_kernel", "greedy_bucket_kernel", "gs_insert_kernel",
     "sb_expand_kernel", "sb_insert_kernel", "canonical_form_kernel",
+    "bm_plan_kernel", "bm_prep_kernel", "bm_insert_kernel", "bm_hist_kernel", "bm_select_kernel",
+    "mb_init_kernel", "mb_goal_roots_kernel", "mb_path_kernel", "mb_plan_kernel", "mb_prep_kernel",
+    "mb_scan_sums_kernel", "mb_scan_top_kernel", "mb_scan_final_kernel", "mb_adopt_kernel",
 ]
 # kernels reported for information (unpack, lookup, path and decide kernels)
 WATCH = MUST_MATCH + [
     "records_unpack_kernel", "keys_unpack_kernel", "pb_unpack_kernel", "mb_unpack_kernel",
-    "mb_decide_kernel", "pb_path_kernel", "pb_lookup_kernel", "mb_path_kernel", "greedy_path_kernel",
+    "mb_decide_kernel", "bm_decide_kernel", "pb_path_kernel", "pb_lookup_kernel", "mb_path_kernel", "greedy_path_kernel",
     "gs_path_kernel", "sb_lookup_kernel", "sb_path_kernel",
 ]
 
